@@ -106,6 +106,10 @@ SIGNATURES = {
     "fcd_solver_wait": (c_int, [_P, c_uint64, _P, c_int32]),
     "fcd_energy_terms": (c_int, [_P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
                                  POINTER(FcdTheta), c_double, _P, _P, _P, _P]),
+    "fcd_patient_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
+    "fcd_patient_terms": (c_int, [_P, c_int64, _P, c_int64, c_int32, c_int64, _P, _P, _P, _P, c_int32, POINTER(FcdTheta),
+                                  _P, _P, _P]),
+    "fcd_qR_change": (c_int, [_P, _P, c_int32, c_int32, _P, _P, _P]),
     "fcd_state_moments": (c_int, [_P, _P, c_int32, _P, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int32, _P,
                                   POINTER(FcdTheta), _P, _P, _P]),
     "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),

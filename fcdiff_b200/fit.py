@@ -33,6 +33,7 @@ the reference cannot execute:
 ``_update_lq_R``: ``"reference"`` reproduces ``nm_to_c(n, m)`` of fit.py:185-186
 (SURVEY 0.3), ``"symmetric"`` uses the unordered pair.
 """
+import collections
 import ctypes
 
 import numpy as np
@@ -41,6 +42,9 @@ import torch
 from . import _dev, _lib, _opt, util
 
 _LOOKUP = {"reference": 0, "symmetric": 1}
+
+# what UnsharedRegionFit.score_patients returns
+PatientScores = collections.namedtuple("PatientScores", "lq_R free_energy free_energy_typical sweeps max_change")
 
 
 def _pi2(pi):
@@ -1165,26 +1169,170 @@ class UnsharedRegionFit(object):
         else:
             if inp['WT'] is None:
                 inp['WT'] = _dev.empty((Ul, C, 2))
-            with _dev.timed(self.profile, "K2b_region_weights"):
-                if use_pt:
-                    _lib.check(lib.fcd_region_weights(_dev.ptr(PT), max(Ul, 1) * pitchC, Ul, C, pitchC,
-                                                      _dev.ptr(qF), _dev.ptr(fstate), _dev.ptr(inp['PsT']),
-                                                      _dev.ptr(inp['kcache']), ctypes.byref(th),
-                                                      _dev.ptr(inp['WT']), _dev.stream()), "fcd_region_weights")
-                else:
-                    _lib.check(lib.fcd_region_weights_em(_dev.ptr(Pe), peStride, pePitch, pe_u0, Ul, C, pitchC,
-                                                         _dev.ptr(qF), _dev.ptr(fstate), _dev.ptr(inp['PsT']),
-                                                         _dev.ptr(inp['kcache']), ctypes.byref(th),
-                                                         _dev.ptr(inp['WT']), _dev.stream()), "fcd_region_weights_em")
-            # (the sweep's in-place arrays are copied in the shadow of the weights kernel: until that launch the
-            # host is on the critical path -- the GPU has only the E-step launched ahead to work on)
-            lqR_new, qR_new = lqR.clone(), qR.clone()
-            with _dev.timed(self.profile, "K2b_sweep"):
-                _lib.check(lib.fcd_estep_qR(_dev.ptr(inp['WT']), C, N, U, u0, Ul, log_pi2, lookup,
-                                            _dev.ptr(qR_new), _dev.ptr(lqR_new), _dev.stream()), "fcd_estep_qR")
+            planes = ("pt", PT, max(Ul, 1) * pitchC) if use_pt else ("em", Pe, peStride, pePitch, pe_u0)
+            (lqR_new, qR_new) = self._weights_and_sweep(planes, inp['WT'], inp['PsT'], inp['kcache'], qF, fstate, th,
+                                                        C, N, U, u0, Ul, pitchC, log_pi2, lookup, lqR, qR)
         if self.shards is not None:
             self.shards.allgather_patients(lqR_new, qR_new, N, U)
         self._mR.set_dev(lqR_new, qR_new, (N, U, 2))
+
+    def _weights_and_sweep(self, planes, WT, PsT, kcache, qF, fstate, th, C, N, U, u0, Ul, pitchC, log_pi2, lookup,
+                           lqR, qR, weights=True):
+        """Region weights WT of the patients [u0, u0 + Ul) (K2b part 1, q_R-independent half of fcdiff/fit.py:187-194)
+        unless ``weights`` is False (WT already holds them), then one Gauss-Seidel sweep (fit.py:176-198) on copies
+        of (lqR, qR); returns the copies.  ``planes``: ("pt", PT, planeStride) patient-major or
+        ("em", Pe, planeStride, pitchU, u0) edge-major responsibility planes."""
+        lib = _lib.load()
+        if weights:
+            with _dev.timed(self.profile, "K2b_region_weights"):
+                if planes[0] == "pt":
+                    (_, PT, ptStride) = planes
+                    _lib.check(lib.fcd_region_weights(_dev.ptr(PT), ptStride, Ul, C, pitchC, _dev.ptr(qF),
+                                                      _dev.ptr(fstate), _dev.ptr(PsT), _dev.ptr(kcache),
+                                                      ctypes.byref(th), _dev.ptr(WT), _dev.stream()),
+                               "fcd_region_weights")
+                else:
+                    (_, Pe, peStride, pePitch, pe_u0) = planes
+                    _lib.check(lib.fcd_region_weights_em(_dev.ptr(Pe), peStride, pePitch, pe_u0, Ul, C, pitchC,
+                                                         _dev.ptr(qF), _dev.ptr(fstate), _dev.ptr(PsT),
+                                                         _dev.ptr(kcache), ctypes.byref(th), _dev.ptr(WT),
+                                                         _dev.stream()), "fcd_region_weights_em")
+        # (the sweep's in-place arrays are copied in the shadow of the weights kernel: until that launch the
+        # host is on the critical path -- the GPU has only the E-step launched ahead to work on)
+        lqR_new, qR_new = lqR.clone(), qR.clone()
+        with _dev.timed(self.profile, "K2b_sweep"):
+            _lib.check(lib.fcd_estep_qR(_dev.ptr(WT), C, N, U, u0, Ul, log_pi2, lookup,
+                                        _dev.ptr(qR_new), _dev.ptr(lqR_new), _dev.stream()), "fcd_estep_qR")
+        return lqR_new, qR_new
+
+    # ------------------------------------------------------------------ held-out patients (new)
+    @staticmethod
+    def _mirror_shape(mirror):
+        """Shape of a posterior array without moving it (None if it was never set)."""
+        if mirror.dev is not None or mirror.fill is not None:
+            return tuple(mirror.shape)
+        if mirror.host is not None:
+            return tuple(np.shape(mirror.host))
+        return None
+
+    def score_patients(self, bt_new, lq_R0=None, max_sweeps=50, tol=1e-9):
+        """Region posteriors and per-patient free energies of subjects the fit was not trained on.
+
+        The fit's current ``model`` (pi, eta, epsilon, gamma, mu, sigma), its q_F and its ``edge_lookup`` are
+        held fixed.  Then the region posteriors of different patients are independent, and the free energy of
+        fcdiff/fit.py:142-155 splits into one share per patient.  The region weights are formed once; each sweep
+        is then exact coordinate ascent on the patients' shares with the symmetric lookup.  With the reference
+        lookup it is the step ``_update_lq_R`` takes (fit.py:176-198).  The fit itself is not changed.
+
+        Parameters
+        ----------
+        bt_new : (C, U') array or CUDA tensor of correlations, same edge order and C as the fit.
+        lq_R0 : (N, U', 2) starting log-posterior; None: uniform, -log 2 (the start of fit.py:84-102).
+        max_sweeps : sweeps run until the largest |change of q_R| over all scored patients and regions is
+            <= ``tol``, or at most this many; 0 evaluates the scores at ``lq_R0``.
+
+        Returns
+        -------
+        PatientScores(lq_R, free_energy, free_energy_typical, sweeps, max_change):
+            lq_R (N, U', 2) float64; free_energy[u] = -E_lp_R,u - E_lM,u + E_lq_R,u (the patient's share of
+            fit.py:148-155); free_energy_typical[u] the same share with every region typical,
+            -N log(1 - pi) - sum_c sum_k q_F log M_k0.  ``free_energy_typical - free_energy`` is a per-subject
+            anomaly score.  sweeps: sweeps run; max_change: the last sweep's largest |change of q_R| (NaN if
+            none ran).
+        """
+        (lq_R, t, sweeps, change) = self._score_terms(bt_new, lq_R0, max_sweeps, tol)
+        N = lq_R.shape[0]
+        free_energy = -t[:, 1]                    # the order of fit.py:148-155: - E_lp_R - E_lM + E_lq_R
+        free_energy = free_energy - t[:, 0]
+        free_energy = free_energy + t[:, 2]
+        typical = -N * float(np.log(_pi2(self.model.pi))[0]) - t[:, 3]
+        return PatientScores(lq_R, free_energy, typical, sweeps, change)
+
+    def _score_terms(self, bt_new, lq_R0, max_sweeps, tol):
+        """`score_patients` up to the per-patient sums: (lq_R, (U', 4) {E_lM, E_lp_R, E_lq_R,
+        sum_c sum_k q_F log M_k0}, sweeps, max_change)."""
+        if self.model is None:
+            raise ValueError("Model has not been initialized.")
+        shF = self._mirror_shape(self._mF)
+        if shF is None:
+            raise ValueError("The fit has no q_F (run() the fit or assign _lq_F first).")
+        if self.shards is not None:
+            raise ValueError("score_patients runs on one GPU: the fit has edge shards.")
+        if '_lM' in self._explicit or '_lp_B_g_F' in self._explicit:
+            raise ValueError("score_patients needs the fused form: the fit holds user-assigned _lM / _lp_B_g_F.")
+        if self.edge_lookup not in _LOOKUP:
+            raise ValueError("edge_lookup must be 'reference' or 'symmetric'")
+        C = int(shF[0])
+        N = util.C_to_N(C)
+        if (N % 1) != 0 or N < 2:
+            raise ValueError("q_F has %d edges: not a triangular number of at least one edge." % C)
+        N = int(N)
+        if len(tuple(bt_new.shape)) != 2 or int(bt_new.shape[0]) != C:
+            raise ValueError("bt_new must be (C, U') with C = %d (got shape %s)" % (C, tuple(bt_new.shape)))
+        U = int(bt_new.shape[1])
+        if U < 1:
+            raise ValueError("bt_new holds no patient")
+        if lq_R0 is not None:
+            lq_R0 = np.ascontiguousarray(lq_R0.cpu().numpy() if torch.is_tensor(lq_R0) else lq_R0, dtype=np.float64)
+            if lq_R0.shape != (N, U, 2):
+                raise ValueError("lq_R0 must be (N, U', 2) = %s (got %s)" % ((N, U, 2), lq_R0.shape))
+        if int(max_sweeps) != max_sweeps or max_sweeps < 0:
+            raise ValueError("max_sweeps must be a non-negative integer")
+        if self.edge_lookup == "reference" and N < 3:
+            raise ValueError("edge_lookup='reference' needs at least 3 regions")
+        max_sweeps = int(max_sweeps)
+
+        lib = _lib.load()
+        prof = self.profile
+        pitchU = _dev.even(U)
+        if torch.is_tensor(bt_new):
+            src = bt_new.to(_dev.device(), torch.float64)
+            bt = src.contiguous() if pitchU == U else _dev.zeros((C, pitchU))
+            if pitchU != U:
+                bt[:, :U].copy_(src)
+        else:
+            bt = _dev.upload_rows(np.asarray(bt_new), pitchU)
+        th = self._theta(use_snapshot=False)
+        PL = _dev.empty((4, C, pitchU))                           # p_0, p_1, p_2, L of the scored patients
+        with _dev.timed(prof, "P0_resp_cache"):
+            _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
+                                          _dev.ptr(PL[3]), _dev.stream()), "fcd_resp_cache")
+        (_, qF) = self._mF.get_dev()
+        fstate = self._mF.get_state()
+        if lq_R0 is None:
+            lqR = torch.full((N * U * 2,), -np.log(2), dtype=torch.float64, device=_dev.device())
+            qR = torch.full((N * U * 2,), float(np.exp(np.float64(-np.log(2)))), dtype=torch.float64,
+                            device=_dev.device())
+        else:
+            (lqR, qR) = (_dev.upload(lq_R0.reshape(-1)), _dev.upload(np.exp(lq_R0).reshape(-1)))
+        (sweeps, change) = (0, float("nan"))
+        if max_sweeps > 0:
+            pitchC = _dev.even(C)
+            (PsT, WT) = (_dev.empty((U, pitchC)), _dev.empty((U, C, 2)))
+            kcache = torch.full((C,), 255, dtype=torch.uint8, device=_dev.device())
+            planes = ("em", PL, C * pitchU, pitchU, 0)
+            log_pi2 = _lib.d3(np.log(_pi2(self.model.pi)))
+            lookup = _LOOKUP[self.edge_lookup]
+            res = _dev.SmallResult(1)
+            while sweeps < max_sweeps:
+                (lqR_new, qR_new) = self._weights_and_sweep(planes, WT, PsT, kcache, qF, fstate, th, C, N, U, 0, U,
+                                                            pitchC, log_pi2, lookup, lqR, qR, weights=sweeps == 0)
+                res.dev.zero_()
+                with _dev.timed(prof, "P1_qR_change"):
+                    _lib.check(lib.fcd_qR_change(_dev.ptr(qR), _dev.ptr(qR_new), N, U, None, _dev.ptr(res.dev),
+                                                 _dev.stream()), "fcd_qR_change")
+                change = float(res.read()[0])
+                (lqR, qR) = (lqR_new, qR_new)
+                sweeps += 1
+                if change <= tol:
+                    break
+        out4 = _dev.empty((U, 4))
+        ws = _dev.empty((max(int(lib.fcd_patient_terms_ws_bytes(C, U)) // 8, 2),))
+        with _dev.timed(prof, "P2_patient_terms"):
+            _lib.check(lib.fcd_patient_terms(_dev.ptr(PL), C * pitchU, _dev.ptr(PL[3]), C, U, pitchU, _dev.ptr(qF),
+                                             _dev.ptr(fstate), _dev.ptr(qR), _dev.ptr(lqR), N, ctypes.byref(th),
+                                             _dev.ptr(out4), _dev.ptr(ws), _dev.stream()), "fcd_patient_terms")
+        return _dev.download(lqR).reshape(N, U, 2), _dev.download(out4), sweeps, change
 
     # ------------------------------------------------------------------ posterior summaries (new)
     def _map_labels(self, mirror, width):

@@ -436,6 +436,26 @@ FCD_API int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
                      const fcd_theta* theta_host, double elm, const void* solver_state,
                      double* out6, double* ws, void* stream);
 
+/* Held-out scoring (csrc/fcd_patients.cu): with theta and q_F of a fitted model fixed, the free energy
+ * (fcdiff/fit.py:142-155) is a sum over patient columns u; these entries keep the sums of `_eval_E_lp_R`,
+ * `_eval_E_lM` and `_eval_E_lq_R` (fit.py:475-539) per patient instead of reducing them to one scalar.
+ *   fcd_patient_terms: out4 [U][4] = {E_lM,u, E_lp_R,u, E_lq_R,u, sum_c sum_k qF[c,k] log M_k0(c,u)} -- the
+ *     last is E_lM,u with every region typical.  The pair weights are those of the edge's own regions
+ *     (n, m) = c_to_nm(c) (fit.py:489-511).  P / L: planes of the scored patients (fcd_resp_cache, all C edges);
+ *     qF / fstate: q_F and its peak states; qR / lqR [N][U][2]; theta_host supplies pi, eta, epsilon.
+ *     ws: fcd_patient_terms_ws_bytes(C, U) bytes of device scratch (no zero fill needed).  A patient's sums
+ *     are bit-identical whichever other patients are scored in the same call: the row partition depends
+ *     on C only and the partials are added in a fixed order.
+ *   fcd_qR_change: out1[0] = max(out1[0], max_{n,u,s} |qR_new - qR_old|) over [N][U][2] (the caller zeroes out1
+ *     first; the maximum of the region sweeps of fit.py:176-198 between two iterates); maxU [U] (may be NULL)
+ *     receives each patient's maximum.  A NaN difference propagates. */
+FCD_API int64_t fcd_patient_terms_ws_bytes(int64_t C, int32_t U);
+FCD_API int fcd_patient_terms(const double* P, int64_t planeStride, const double* L, int64_t C, int32_t U, int64_t pitchU,
+                      const double* qF, const uint8_t* fstate, const double* qR, const double* lqR, int32_t N,
+                      const fcd_theta* theta_host, double* out4, double* ws, void* stream);
+FCD_API int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,
+                  void* stream);
+
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
  * disabled pieces of a mu / sigma update, fcdiff/fit.py:232-237, 542-597,
