@@ -16,6 +16,26 @@
 // per edge-patient); where both regions of the edge are peaked as well the weight is exactly 1 and the factor
 // a_l + b_l p enters a running product (one logarithm per kProdMax factors, fcd_math.cuh), otherwise each
 // weighted term takes its own logarithm.  Unpeaked edges read all three planes.
+//
+// Posteriors of the anomalous connections T and the patients' connection states F~
+// (UnsharedRegionFit.connection_posteriors), for fitted and held-out patients alike.  Given the template state
+// F = k of edge c and the pair state l of its regions (0 both typical, 1 both anomalous, 2 mixed), the
+// generative model (fcdiff/model.py:141-188) gives, with the plane values p of b~[c,u] and a_l, b_l, eps_l of
+// fcd_common.cuh, the exact conditionals
+//   P(F~ = j | k, l, b~) = eps_l p_k / (a_l + b_l p_k)   (j = k),   a_l p_j / (a_l + b_l p_k)   (j != k)
+//   P(T = 1  | k, l, b~) = 0 (l = 0),  1 (l = 1),  eta (eps p_k + a_1 (1 - p_k)) / (a_2 + b_2 p_k)   (l = 2)
+// and the read-outs are their expectations under q_F[c,k] w_l[c,u], the pair weights of the edge's own regions
+// (as fit.py:489-511; the sweep's edge lookup plays no part).
+//   connection_rows_kernel      per (row block, patient) cell, the row partition and lane mapping of
+//                               patient_terms_rows_kernel: q_T[c][u] (and q_F~[c][u][0..2] when MAPS), and the
+//                               cell's sum of q_T over its rows, in row order, into part[b][u];
+//   connection_finish_kernel    expected[u]: the row-block partials in block order; rate[c]: row c of q_T summed
+//                               in a fixed lane order, over U.
+// Tiers: a peaked edge with both regions peaked is one (k*, l*) term (one division); a peaked edge with an
+// undecided region takes the three l terms; an unpeaked edge all nine with q_F weights.  Weights <= 2^-60 are
+// dropped.  Without maps a peaked edge reads its k* plane only, and only for a mixed pair term.  No logarithm is
+// taken, so there is no log table and no SAFE variant; q_T is formed by the same instructions in both variants,
+// so the reductions do not depend on whether the maps are written.
 #include "fcd_common.cuh"
 
 namespace fcd {
@@ -203,6 +223,129 @@ qR_change_kernel(const double* __restrict__ qa, const double* __restrict__ qb, i
     }
 }
 
+// one (k, l) term of weight wt: P(T = 1 | k, l) into t and, when MAPS, P(F~ = . | k, l) into g.  pk = p_k;
+// p: all three planes (read only when MAPS).  The q_T arithmetic is spelled with rounding intrinsics: the
+// compiler may not contract it differently in the two variants (whose other uses of wt and inv differ)
+template <bool MAPS>
+__device__ __forceinline__ void connection_term(const ThetaDev& th, int k, int l, double wt, double pk,
+                                                const double (&p)[3], double& t, double (&g)[3]) {
+    if (l == 1) t = __dadd_rn(t, wt);
+    if (MAPS || l == 2) {
+        const double inv = __ddiv_rn(1.0, mix_rel(th, l, pk));
+        if (l == 2) {
+            const double num = __fma_rn(th.epsilon, pk, __dmul_rn(th.al[1], __dsub_rn(1.0, pk)));
+            t = __fma_rn(wt, __dmul_rn(__dmul_rn(th.eta, num), inv), t);
+        }
+        if (MAPS) {
+            const double s = wt * inv, sa = s * th.al[l], se = s * th.epsl[l];
+#pragma unroll
+            for (int j = 0; j < 3; ++j) g[j] = fma(j == k ? se : sa, p[j], g[j]);
+        }
+    }
+}
+
+template <bool MAPS>
+__global__ void __launch_bounds__(kPtThreads)
+connection_rows_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C, int U, int64_t pitchU,
+                       const double* __restrict__ qF, const uint8_t* __restrict__ fstate,
+                       const double* __restrict__ qR, const __grid_constant__ ThetaDev th, int64_t nb, int64_t rows,
+                       int lanesP, double* __restrict__ qT, double* __restrict__ qFt, double* __restrict__ part) {
+    const int lane = threadIdx.x & 31;
+    const unsigned gw = (blockIdx.x * kPtThreads + threadIdx.x) >> 5;
+    const unsigned tiles = (unsigned)(U + lanesP - 1) / (unsigned)lanesP;
+    const int64_t rb = (int64_t)(gw / tiles) * (32 / lanesP) + lane / lanesP;
+    const int u = (int)(gw % tiles) * lanesP + (lane & (lanesP - 1));
+    if (rb >= nb || u >= U) return;
+    const int64_t c0 = rb * rows;
+    const int64_t c1 = c0 + rows < C ? c0 + rows : C;
+    int n, m;
+    c_to_nm(c0, n, m);
+    const double2* q2 = reinterpret_cast<const double2*>(qR);
+    double acc = 0.0;
+    for (int64_t c = c0; c < c1; ++c) {
+        const int k = __ldg(fstate + c);
+        const double2 qn = __ldg(q2 + (int64_t)n * U + u), qm = __ldg(q2 + (int64_t)m * U + u);
+        const int sn = peak_state2(qn), sm = peak_state2(qm);
+        double w[3];
+        if (sn < 2 && sm < 2) {
+            const int ls = (sn ^ sm) ? 2 : sn;                     // l* of a peaked pair (fit.py:382-406)
+            w[0] = ls == 0 ? 1.0 : 0.0;
+            w[1] = ls == 1 ? 1.0 : 0.0;
+            w[2] = ls == 2 ? 1.0 : 0.0;
+        } else {
+            w[0] = __dmul_rn(qn.x, qm.x);                          // pair_weights, not contracted
+            w[1] = __dmul_rn(qn.y, qm.y);
+            w[2] = __fma_rn(qn.y, qm.x, __dmul_rn(qn.x, qm.y));
+        }
+        const double* pc = P + c * pitchU + u;
+        double p[3] = {0.0, 0.0, 0.0};
+        if (MAPS || (k == 3 && w[2] > kPeakTau)) {
+#pragma unroll
+            for (int j = 0; j < 3; ++j) p[j] = __ldg(pc + j * planeStride);
+        }
+        double t = 0.0, g[3] = {0.0, 0.0, 0.0};
+        if (k < 3) {
+            const double pk = MAPS ? sel3(k, p) : (w[2] > kPeakTau ? __ldg(pc + k * planeStride) : 0.0);
+#pragma unroll
+            for (int l = 0; l < 3; ++l)
+                if (w[l] > kPeakTau) connection_term<MAPS>(th, k, l, w[l], pk, p, t, g);
+        } else {
+            const double f[3] = {__ldg(qF + c * 3), __ldg(qF + c * 3 + 1), __ldg(qF + c * 3 + 2)};
+#pragma unroll
+            for (int kk = 0; kk < 3; ++kk) {
+                if (f[kk] <= kPeakTau) continue;
+#pragma unroll
+                for (int l = 0; l < 3; ++l)
+                    if (w[l] > kPeakTau) connection_term<MAPS>(th, kk, l, __dmul_rn(f[kk], w[l]), p[kk], p, t, g);
+            }
+        }
+        qT[c * U + u] = t;
+        if (MAPS) {
+            double* o = qFt + (c * U + u) * 3;
+            o[0] = g[0];
+            o[1] = g[1];
+            o[2] = g[2];
+        }
+        acc = __dadd_rn(acc, t);
+        if (++m == n) {
+            ++n;
+            m = 0;
+        }
+    }
+    part[rb * U + u] = acc;
+}
+
+// blocks [0, bU): expected[u] for 32 patients each, warps take the row blocks round robin and the eight warp sums
+// are added in warp order; blocks [bU, ...): rate[c] for 8 rows each, one warp per row, lanes stride the patients
+// and the lane sums are added by a fixed butterfly
+__global__ void __launch_bounds__(kPtThreads)
+connection_finish_kernel(const double* __restrict__ part, int64_t nb, const double* __restrict__ qT, int64_t C,
+                         int U, int bU, double* __restrict__ expected, double* __restrict__ rate) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if ((int)blockIdx.x < bU) {
+        __shared__ double s[kPtThreads / 32][32];
+        const int u = blockIdx.x * 32 + lane;
+        double v = 0.0;
+        if (u < U)
+            for (int64_t b = warp; b < nb; b += kPtThreads / 32) v += part[b * U + u];
+        s[warp][lane] = v;
+        __syncthreads();
+        if (warp == 0 && u < U) {
+            double t = s[0][lane];
+            for (int w = 1; w < kPtThreads / 32; ++w) t += s[w][lane];
+            expected[u] = t;
+        }
+        return;
+    }
+    const int64_t c = (int64_t)(blockIdx.x - bU) * (kPtThreads / 32) + warp;
+    if (c >= C) return;
+    const double* row = qT + c * U;
+    double v = 0.0;
+    for (int u = lane; u < U; u += 32) v += row[u];
+    v = warp_sum(v);
+    if (lane == 0) rate[c] = v / U;
+}
+
 }  // namespace fcd
 
 using namespace fcd;
@@ -250,6 +393,46 @@ int fcd_patient_terms(const double* P, int64_t planeStride, const double* L, int
     patient_terms_finish_kernel<<<(unsigned)((U + 31) / 32), kPtThreads, 0, st>>>(ws, nb, qR, lqR, N, U, th.log_pi2[0],
                                                                                 th.log_pi2[1], out4);
     return check_launch("fcd_patient_terms(finish)");
+}
+
+int64_t fcd_connection_ws_bytes(int64_t C, int32_t U) {
+    if (C < 0 || U < 0) return 0;
+    return pt_row_blocks(C) * (int64_t)U * (int64_t)sizeof(double);
+}
+
+int fcd_connection_posteriors(const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                              const double* qF, const uint8_t* fstate, const double* qR, int32_t N,
+                              const fcd_theta* theta_host, double* qT, double* qFt, double* expected, double* rate,
+                              double* ws, void* stream) {
+    FCD_REQUIRE(P != nullptr && qF != nullptr && fstate != nullptr && qR != nullptr && theta_host != nullptr &&
+                qT != nullptr && expected != nullptr && rate != nullptr && ws != nullptr,
+                "fcd_connection_posteriors: NULL argument");
+    FCD_REQUIRE(N >= 2 && N < 65536 && C == (int64_t)N * (N - 1) / 2,
+                "fcd_connection_posteriors: C=%lld is not N(N-1)/2 for N=%d", (long long)C, N);
+    FCD_REQUIRE(U >= 1 && pitchU >= U && planeStride >= C * pitchU, "fcd_connection_posteriors: bad shape");
+    FCD_REQUIRE((reinterpret_cast<uintptr_t>(qR) & 15) == 0, "fcd_connection_posteriors: qR must be 16-byte aligned");
+    const ThetaDev th = make_theta_dev(*theta_host, 0);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t nb = pt_row_blocks(C);
+    const int64_t rows = (C + nb - 1) / nb;
+    int lanesP = 1;
+    while (lanesP < 32 && lanesP < U) lanesP *= 2;
+    const int64_t warps = ((nb + 32 / lanesP - 1) / (32 / lanesP)) * ((U + lanesP - 1) / lanesP);
+    const int64_t grid = (warps * 32 + kPtThreads - 1) / kPtThreads;
+    FCD_REQUIRE(warps < ((int64_t)1 << 26), "fcd_connection_posteriors: %lld patients are too many for one launch",
+                (long long)U);
+    if (qFt != nullptr)
+        connection_rows_kernel<true><<<(unsigned)grid, kPtThreads, 0, st>>>(P, planeStride, C, U, pitchU, qF, fstate,
+                                                                            qR, th, nb, rows, lanesP, qT, qFt, ws);
+    else
+        connection_rows_kernel<false><<<(unsigned)grid, kPtThreads, 0, st>>>(P, planeStride, C, U, pitchU, qF, fstate,
+                                                                             qR, th, nb, rows, lanesP, qT, qFt, ws);
+    int rc = check_launch("fcd_connection_posteriors(rows)");
+    if (rc != 0) return rc;
+    const int64_t bU = (U + 31) / 32, bC = (C + kPtThreads / 32 - 1) / (kPtThreads / 32);
+    FCD_REQUIRE(bU + bC < ((int64_t)1 << 31), "fcd_connection_posteriors: too many edges for one launch");
+    connection_finish_kernel<<<(unsigned)(bU + bC), kPtThreads, 0, st>>>(ws, nb, qT, C, U, (int)bU, expected, rate);
+    return check_launch("fcd_connection_posteriors(finish)");
 }
 
 int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,

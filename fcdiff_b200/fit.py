@@ -45,6 +45,9 @@ _LOOKUP = {"reference": 0, "symmetric": 1}
 
 # what UnsharedRegionFit.score_patients returns
 PatientScores = collections.namedtuple("PatientScores", "lq_R free_energy free_energy_typical sweeps max_change")
+# what UnsharedRegionFit.connection_posteriors returns
+ConnectionPosteriors = collections.namedtuple("ConnectionPosteriors",
+                                              "q_T q_F_tilde expected_anomalous anomalous_rate")
 
 
 def _pi2(pi):
@@ -1251,27 +1254,10 @@ class UnsharedRegionFit(object):
     def _score_terms(self, bt_new, lq_R0, max_sweeps, tol):
         """`score_patients` up to the per-patient sums: (lq_R, (U', 4) {E_lM, E_lp_R, E_lq_R,
         sum_c sum_k q_F log M_k0}, sweeps, max_change)."""
-        if self.model is None:
-            raise ValueError("Model has not been initialized.")
-        shF = self._mirror_shape(self._mF)
-        if shF is None:
-            raise ValueError("The fit has no q_F (run() the fit or assign _lq_F first).")
-        if self.shards is not None:
-            raise ValueError("score_patients runs on one GPU: the fit has edge shards.")
-        if '_lM' in self._explicit or '_lp_B_g_F' in self._explicit:
-            raise ValueError("score_patients needs the fused form: the fit holds user-assigned _lM / _lp_B_g_F.")
+        (C, N) = self._check_readout("score_patients", ('_lM', '_lp_B_g_F'))
         if self.edge_lookup not in _LOOKUP:
             raise ValueError("edge_lookup must be 'reference' or 'symmetric'")
-        C = int(shF[0])
-        N = util.C_to_N(C)
-        if (N % 1) != 0 or N < 2:
-            raise ValueError("q_F has %d edges: not a triangular number of at least one edge." % C)
-        N = int(N)
-        if len(tuple(bt_new.shape)) != 2 or int(bt_new.shape[0]) != C:
-            raise ValueError("bt_new must be (C, U') with C = %d (got shape %s)" % (C, tuple(bt_new.shape)))
-        U = int(bt_new.shape[1])
-        if U < 1:
-            raise ValueError("bt_new holds no patient")
+        U = self._check_bt_new(bt_new, C)
         if lq_R0 is not None:
             lq_R0 = np.ascontiguousarray(lq_R0.cpu().numpy() if torch.is_tensor(lq_R0) else lq_R0, dtype=np.float64)
             if lq_R0.shape != (N, U, 2):
@@ -1285,18 +1271,8 @@ class UnsharedRegionFit(object):
         lib = _lib.load()
         prof = self.profile
         pitchU = _dev.even(U)
-        if torch.is_tensor(bt_new):
-            src = bt_new.to(_dev.device(), torch.float64)
-            bt = src.contiguous() if pitchU == U else _dev.zeros((C, pitchU))
-            if pitchU != U:
-                bt[:, :U].copy_(src)
-        else:
-            bt = _dev.upload_rows(np.asarray(bt_new), pitchU)
         th = self._theta(use_snapshot=False)
-        PL = _dev.empty((4, C, pitchU))                           # p_0, p_1, p_2, L of the scored patients
-        with _dev.timed(prof, "P0_resp_cache"):
-            _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
-                                          _dev.ptr(PL[3]), _dev.stream()), "fcd_resp_cache")
+        PL = self._planes_of(bt_new, C, U, pitchU, th)
         (_, qF) = self._mF.get_dev()
         fstate = self._mF.get_state()
         if lq_R0 is None:
@@ -1333,6 +1309,132 @@ class UnsharedRegionFit(object):
                                              _dev.ptr(fstate), _dev.ptr(qR), _dev.ptr(lqR), N, ctypes.byref(th),
                                              _dev.ptr(out4), _dev.ptr(ws), _dev.stream()), "fcd_patient_terms")
         return _dev.download(lqR).reshape(N, U, 2), _dev.download(out4), sweeps, change
+
+    def _check_readout(self, what, explicit):
+        """Checks a read-out of the fitted model makes before any device work; returns (C, N) of q_F."""
+        if self.model is None:
+            raise ValueError("Model has not been initialized.")
+        shF = self._mirror_shape(self._mF)
+        if shF is None:
+            raise ValueError("The fit has no q_F (run() the fit or assign _lq_F first).")
+        if self.shards is not None:
+            raise ValueError("%s runs on one GPU: the fit has edge shards." % what)
+        if any(name in self._explicit for name in explicit):
+            raise ValueError("%s needs the fused form: the fit holds user-assigned %s." % (what, " / ".join(explicit)))
+        C = int(shF[0])
+        N = util.C_to_N(C)
+        if (N % 1) != 0 or N < 2:
+            raise ValueError("q_F has %d edges: not a triangular number of at least one edge." % C)
+        return C, int(N)
+
+    @staticmethod
+    def _check_bt_new(bt_new, C):
+        """U' of a (C, U') array or tensor of patient correlations."""
+        if len(tuple(bt_new.shape)) != 2 or int(bt_new.shape[0]) != C:
+            raise ValueError("bt_new must be (C, U') with C = %d (got shape %s)" % (C, tuple(bt_new.shape)))
+        U = int(bt_new.shape[1])
+        if U < 1:
+            raise ValueError("bt_new holds no patient")
+        return U
+
+    def _planes_of(self, bt_src, C, U, pitchU, th, with_L=True):
+        """Responsibility planes p_0, p_1, p_2 (and L) [C][pitchU] of the columns of ``bt_src``: a (C, U) host
+        array or CUDA tensor, or a device tensor already padded to (C, pitchU)."""
+        lib = _lib.load()
+        if torch.is_tensor(bt_src):
+            src = bt_src.to(_dev.device(), torch.float64)
+            bt = src.contiguous() if int(src.shape[1]) == pitchU else _dev.zeros((C, pitchU))
+            if int(src.shape[1]) != pitchU:
+                bt[:, :U].copy_(src)
+        else:
+            bt = _dev.upload_rows(np.asarray(bt_src), pitchU)
+        PL = _dev.empty((4 if with_L else 3, C, pitchU))
+        with _dev.timed(self.profile, "P0_resp_cache"):
+            _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
+                                          _dev.ptr(PL[3] if with_L else None), _dev.stream()), "fcd_resp_cache")
+        return PL
+
+    def connection_posteriors(self, bt_new=None, lq_R=None, maps=True):
+        """Posteriors of the anomalous connections T and of the patients' connection states F~.
+
+        For edge c of patient u, with F = k the template state and l the state of the edge's pair of regions
+        (both typical, both anomalous, mixed), T and F~ have closed-form conditionals given b~[c,u] (the
+        generative model of fcdiff/model.py:141-188); the read-outs are their expectations under the fit's
+        q_F[c,k] and the pair weights of q_R (fit.py:382-406).  The model's current theta and q_F are used as
+        they are; the fit itself is not changed.
+
+        Parameters
+        ----------
+        bt_new : None -- the fit's own patients with the fit's q_R; or a (C, U') array or CUDA tensor of
+            held-out patients, same edge order and C as the fit.
+        lq_R : (N, U', 2) region log-posteriors of the held-out patients, typically
+            ``fit.score_patients(bt_new).lq_R``; given if and only if ``bt_new`` is.
+        maps : False returns None for both maps and forms only the reductions (the F~ map is never formed).
+
+        Returns
+        -------
+        ConnectionPosteriors(q_T, q_F_tilde, expected_anomalous, anomalous_rate):
+            q_T (C, U) float64, the probability that connection c of patient u is anomalous (the sampler's t);
+            q_F_tilde (C, U, 3) float64, the posterior of the patient's connection state (the sampler's
+            f_tilde); expected_anomalous (U,) = sum_c q_T, the expected number of anomalous connections per
+            patient; anomalous_rate (C,) = mean_u q_T, the share of the scored patients in whom each connection
+            is anomalous.
+        """
+        (C, N) = self._check_readout("connection_posteriors", ('_lM', '_lp_B_g_F', '_p_Bt_g_Ft'))
+        if (bt_new is None) != (lq_R is None):
+            raise ValueError("connection_posteriors takes bt_new and lq_R together (held-out patients) or "
+                             "neither (the fit's own patients)")
+        (P, planeStride, pitchU, bt_src) = (None, 0, 0, None)
+        if bt_new is None:
+            shR = self._mirror_shape(self._mR)
+            if shR is None:
+                raise ValueError("The fit has no q_R (run() the fit or assign _lq_R first).")
+            inp = self._in
+            if self._shared is not None:
+                U = int(self._shared[2].numel())
+            elif inp is not None:
+                U = int(inp['U'])
+            elif self.bt is not None:
+                U = self._check_bt_new(self.bt, C)
+            else:
+                raise ValueError("The fit has no patients (assign bt or run() the fit first).")
+            if tuple(shR) != (N, U, 2):
+                raise ValueError("the fit's q_R is %s, not (N, U, 2) = %s" % (tuple(shR), (N, U, 2)))
+            key = (tuple(float(v) for v in self.model.mu), tuple(float(v) for v in self.model.sigma))
+            if inp is not None and inp['P'] is not None and inp['cache_key'] == key:
+                (P, planeStride, pitchU) = (inp['P'], max(inp['Cl'], 1) * inp['pitchU'], inp['pitchU'])
+            elif self._shared is not None:
+                raise ValueError("connection_posteriors: the replica-mode fit has no planes for the model's "
+                                 "(mu, sigma) (run() the fit first).")
+            else:
+                bt_src = inp['bt'] if inp is not None else self.bt
+        else:
+            U = self._check_bt_new(bt_new, C)
+            lq = np.ascontiguousarray(lq_R.cpu().numpy() if torch.is_tensor(lq_R) else lq_R, dtype=np.float64)
+            if lq.shape != (N, U, 2):
+                raise ValueError("lq_R must be (N, U', 2) = %s (got %s)" % ((N, U, 2), lq.shape))
+            bt_src = bt_new
+
+        lib = _lib.load()
+        th = self._theta(use_snapshot=False)
+        if P is None:
+            pitchU = _dev.even(U)
+            P = self._planes_of(bt_src, C, U, pitchU, th, with_L=False)
+            planeStride = C * pitchU
+        (_, qF) = self._mF.get_dev()
+        fstate = self._mF.get_state()
+        qR = self._mR.get_dev()[1] if bt_new is None else _dev.upload(np.exp(lq).reshape(-1))
+        qT = _dev.empty((C, U))                     # scratch of the rates without maps
+        qFt = _dev.empty((C, U, 3)) if maps else None
+        (expected, rate) = (_dev.empty((U,)), _dev.empty((C,)))
+        ws = _dev.empty((max(int(lib.fcd_connection_ws_bytes(C, U)) // 8, 1),))
+        with _dev.timed(self.profile, "P3_connection_posteriors"):
+            _lib.check(lib.fcd_connection_posteriors(_dev.ptr(P), planeStride, C, U, pitchU, _dev.ptr(qF),
+                                                     _dev.ptr(fstate), _dev.ptr(qR), N, ctypes.byref(th),
+                                                     _dev.ptr(qT), _dev.ptr(qFt), _dev.ptr(expected), _dev.ptr(rate),
+                                                     _dev.ptr(ws), _dev.stream()), "fcd_connection_posteriors")
+        return ConnectionPosteriors(_dev.download(qT) if maps else None, _dev.download(qFt) if maps else None,
+                                    _dev.download(expected), _dev.download(rate))
 
     # ------------------------------------------------------------------ posterior summaries (new)
     def _map_labels(self, mirror, width):

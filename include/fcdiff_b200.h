@@ -456,6 +456,25 @@ FCD_API int fcd_patient_terms(const double* P, int64_t planeStride, const double
 FCD_API int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,
                   void* stream);
 
+/* Posteriors of the anomalous connections T and of the patients' connection states F~ (csrc/fcd_patients.cu;
+ * no reference counterpart: the reference sums T and F~ out into M_kl, fcdiff/fit.py:409-444, and the sampler
+ * draws them, fcdiff/model.py:141-188).  For edge c = (n, m) = c_to_nm(c) and patient u, with q_F[c,k] and the
+ * pair weights w_l of the edge's own regions (fit.py:382-406):
+ *   qT [C][U]       = sum_k q_F[c,k] sum_l w_l P(T = 1 | F = k, pair state l, b~[c,u])
+ *   qFt [C][U][3]   = sum_k q_F[c,k] sum_l w_l P(F~ = j | F = k, pair state l, b~[c,u])   (may be NULL: not formed)
+ *   expected [U]    = sum_c qT[c][u];   rate [C] = sum_u qT[c][u] / U
+ * P: planes p_0, p_1, p_2 of the scored patients (fcd_resp_cache, all C edges, [3][C][pitchU] with planeStride);
+ * qF / fstate: q_F and its peak states; qR [N][U][2] (16-byte aligned); theta_host supplies eta, epsilon.  qT is
+ * always written (pass scratch when the map is not wanted).  ws: fcd_connection_ws_bytes(C, U) bytes of device
+ * scratch (no zero fill needed).  A patient's maps and expected count are bit-identical whichever other patients
+ * are in the call (the row partition depends on C only, the partials are added in a fixed order), and the three
+ * reductions do not depend on whether qFt is written. */
+FCD_API int64_t fcd_connection_ws_bytes(int64_t C, int32_t U);
+FCD_API int fcd_connection_posteriors(const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                              const double* qF, const uint8_t* fstate, const double* qR, int32_t N,
+                              const fcd_theta* theta_host, double* qT, double* qFt, double* expected, double* rate,
+                              double* ws, void* stream);
+
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
  * disabled pieces of a mu / sigma update, fcdiff/fit.py:232-237, 542-597,
