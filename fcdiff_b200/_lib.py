@@ -113,6 +113,8 @@ SIGNATURES = {
     "fcd_connection_ws_bytes": (c_int64, [c_int64, c_int32]),
     "fcd_connection_posteriors": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, _P, _P, _P, c_int32,
                                           POINTER(FcdTheta), _P, _P, _P, _P, _P, _P]),
+    "fcd_control_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
+    "fcd_control_terms": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_state_moments": (c_int, [_P, _P, c_int32, _P, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int32, _P,
                                   POINTER(FcdTheta), _P, _P, _P]),
     "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),

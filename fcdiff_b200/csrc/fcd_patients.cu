@@ -36,6 +36,15 @@
 // dropped.  Without maps a peaked edge reads its k* plane only, and only for a mixed pair term.  No logarithm is
 // taken, so there is no log table and no SAFE variant; q_T is formed by the same instructions in both variants,
 // so the reductions do not depend on whether the maps are written.
+//
+// Per-subject control log-likelihoods (UnsharedRegionFit.score_controls / classify_subjects): one control's
+// share of E_lp_B_g_F (fcdiff/fit.py:461-472) for a new column x, sum_c sum_k q_F[c,k] log N(x_c; mu_k, sigma_k)
+// with the log density of fit.py:111-114.
+//   control_terms_rows_kernel   per (row block, subject) cell, the row partition and lane mapping of
+//                               patient_terms_rows_kernel: the cell's sum over its rows, in row order, into
+//                               part[b][s];
+//   connection_finish_kernel    (its `expected` blocks only) the row-block partials of each subject in block order.
+// All three weighted terms are evaluated on every element: no tiers, no peak states, no logarithm.
 #include "fcd_common.cuh"
 
 namespace fcd {
@@ -346,6 +355,50 @@ connection_finish_kernel(const double* __restrict__ part, int64_t nb, const doub
     if (lane == 0) rate[c] = v / U;
 }
 
+// per-state constants of log N(x; mu_k, sigma_k) = -((x - mu_k) / sigma_k)^2 / 2 - nc_k, formed once per launch
+struct ControlConsts {
+    double mu[3];
+    double isig[3];     // 1 / sigma_k
+    double nc[3];       // log sigma_k + log sqrt(2 pi)
+};
+
+constexpr int kCtRows = 8;                  // rows whose loads a thread has in flight at once
+
+__global__ void __launch_bounds__(kPtThreads)
+control_terms_rows_kernel(const double* __restrict__ X, int64_t C, int S, int64_t pitchS, const double* __restrict__ qF,
+                          const __grid_constant__ ControlConsts cc, int64_t nb, int64_t rows, int lanesP,
+                          double* __restrict__ part) {
+    const int lane = threadIdx.x & 31;
+    const unsigned gw = (blockIdx.x * kPtThreads + threadIdx.x) >> 5;
+    const unsigned tiles = (unsigned)(S + lanesP - 1) / (unsigned)lanesP;
+    const int64_t rb = (int64_t)(gw / tiles) * (32 / lanesP) + lane / lanesP;
+    const int s = (int)(gw % tiles) * lanesP + (lane & (lanesP - 1));
+    if (rb >= nb || s >= S) return;
+    const int64_t c0 = rb * rows;
+    const int64_t c1 = c0 + rows < C ? c0 + rows : C;
+    double acc = 0.0;
+    for (int64_t cb = c0; cb < c1; cb += kCtRows) {
+        // the column loads of kCtRows rows are issued before any of them is used (bytes in flight, not one row at
+        // a time); a row past the block's end repeats its last row with weight 0 and adds exactly +0.0
+        double x[kCtRows];
+#pragma unroll
+        for (int j = 0; j < kCtRows; ++j) x[j] = ldg_stream1(X + (cb + j < c1 ? cb + j : c1 - 1) * pitchS + s);
+#pragma unroll
+        for (int j = 0; j < kCtRows; ++j) {
+            const bool in = cb + j < c1;
+            const double* q = qF + (in ? cb + j : c1 - 1) * 3;
+            const double g0 = __ldg(q), g1 = __ldg(q + 1), g2 = __ldg(q + 2);   // straight-line code: no branch
+            const double f0 = in ? g0 : 0.0, f1 = in ? g1 : 0.0, f2 = in ? g2 : 0.0;
+            const double z0 = (x[j] - cc.mu[0]) * cc.isig[0], z1 = (x[j] - cc.mu[1]) * cc.isig[1],
+                         z2 = (x[j] - cc.mu[2]) * cc.isig[2];
+            const double l0 = fma(-0.5 * z0, z0, -cc.nc[0]), l1 = fma(-0.5 * z1, z1, -cc.nc[1]),
+                         l2 = fma(-0.5 * z2, z2, -cc.nc[2]);
+            acc += fma(f0, l0, fma(f1, l1, f2 * l2));
+        }
+    }
+    part[rb * S + s] = acc;
+}
+
 }  // namespace fcd
 
 using namespace fcd;
@@ -433,6 +486,44 @@ int fcd_connection_posteriors(const double* P, int64_t planeStride, int64_t C, i
     FCD_REQUIRE(bU + bC < ((int64_t)1 << 31), "fcd_connection_posteriors: too many edges for one launch");
     connection_finish_kernel<<<(unsigned)(bU + bC), kPtThreads, 0, st>>>(ws, nb, qT, C, U, (int)bU, expected, rate);
     return check_launch("fcd_connection_posteriors(finish)");
+}
+
+int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S) {
+    if (C < 0 || S < 0) return 0;
+    return pt_row_blocks(C) * (int64_t)S * (int64_t)sizeof(double);
+}
+
+int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                      const fcd_theta* theta_host, double* out, double* ws, void* stream) {
+    FCD_REQUIRE(X != nullptr && qF != nullptr && theta_host != nullptr && out != nullptr && ws != nullptr,
+                "fcd_control_terms: NULL argument");
+    const int64_t N = (int64_t)((sqrt(8.0 * (double)C + 1.0) + 1.0) * 0.5);
+    FCD_REQUIRE(C >= 1 && N * (N - 1) / 2 == C, "fcd_control_terms: C=%lld is not N(N-1)/2", (long long)C);
+    FCD_REQUIRE(S >= 1 && pitchS >= S, "fcd_control_terms: bad shape");
+    FCD_REQUIRE(((reinterpret_cast<uintptr_t>(X) | reinterpret_cast<uintptr_t>(qF) | reinterpret_cast<uintptr_t>(out) |
+                  reinterpret_cast<uintptr_t>(ws)) & 7) == 0,
+                "fcd_control_terms: X, qF, out and ws must be 8-byte aligned");
+    ControlConsts cc;
+    for (int k = 0; k < 3; ++k) {
+        cc.mu[k] = theta_host->mu[k];
+        cc.isig[k] = 1.0 / theta_host->sigma[k];
+        cc.nc[k] = log(theta_host->sigma[k]) + kHalfLog2Pi;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t nb = pt_row_blocks(C);
+    const int64_t rows = (C + nb - 1) / nb;
+    int lanesP = 1;
+    while (lanesP < 32 && lanesP < S) lanesP *= 2;
+    const int64_t warps = ((nb + 32 / lanesP - 1) / (32 / lanesP)) * ((S + lanesP - 1) / lanesP);
+    const int64_t grid = (warps * 32 + kPtThreads - 1) / kPtThreads;
+    FCD_REQUIRE(warps < ((int64_t)1 << 26), "fcd_control_terms: %lld subjects are too many for one launch",
+                (long long)S);
+    control_terms_rows_kernel<<<(unsigned)grid, kPtThreads, 0, st>>>(X, C, S, pitchS, qF, cc, nb, rows, lanesP, ws);
+    int rc = check_launch("fcd_control_terms(rows)");
+    if (rc != 0) return rc;
+    connection_finish_kernel<<<(unsigned)((S + 31) / 32), kPtThreads, 0, st>>>(ws, nb, nullptr, C, S,
+                                                                              (int)((S + 31) / 32), out, nullptr);
+    return check_launch("fcd_control_terms(finish)");
 }
 
 int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,

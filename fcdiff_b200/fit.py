@@ -37,6 +37,7 @@ import collections
 import ctypes
 
 import numpy as np
+import scipy.special
 import torch
 
 from . import _dev, _lib, _opt, util
@@ -48,6 +49,9 @@ PatientScores = collections.namedtuple("PatientScores", "lq_R free_energy free_e
 # what UnsharedRegionFit.connection_posteriors returns
 ConnectionPosteriors = collections.namedtuple("ConnectionPosteriors",
                                               "q_T q_F_tilde expected_anomalous anomalous_rate")
+# what UnsharedRegionFit.classify_subjects returns
+SubjectScores = collections.namedtuple("SubjectScores",
+                                       "log_odds p_patient control_loglik patient_elbo lq_R sweeps max_change")
 
 
 def _pi2(pi):
@@ -1243,7 +1247,9 @@ class UnsharedRegionFit(object):
             anomaly score.  sweeps: sweeps run; max_change: the last sweep's largest |change of q_R| (NaN if
             none ran).
         """
-        (lq_R, t, sweeps, change) = self._score_terms(bt_new, lq_R0, max_sweeps, tol)
+        return self._patient_scores(*self._score_terms(bt_new, lq_R0, max_sweeps, tol))
+
+    def _patient_scores(self, lq_R, t, sweeps, change):
         N = lq_R.shape[0]
         free_energy = -t[:, 1]                    # the order of fit.py:148-155: - E_lp_R - E_lM + E_lq_R
         free_energy = free_energy - t[:, 0]
@@ -1254,7 +1260,13 @@ class UnsharedRegionFit(object):
     def _score_terms(self, bt_new, lq_R0, max_sweeps, tol):
         """`score_patients` up to the per-patient sums: (lq_R, (U', 4) {E_lM, E_lp_R, E_lq_R,
         sum_c sum_k q_F log M_k0}, sweeps, max_change)."""
-        (C, N) = self._check_readout("score_patients", ('_lM', '_lp_B_g_F'))
+        (C, N, U, lq_R0, max_sweeps) = self._check_score_args("score_patients", bt_new, lq_R0, max_sweeps)
+        return self._score_columns(bt_new, C, N, U, lq_R0, max_sweeps, tol)
+
+    def _check_score_args(self, what, bt_new, lq_R0, max_sweeps):
+        """The checks of `score_patients`, before any device work: (C, N, U', lq_R0 as a host array or None,
+        max_sweeps)."""
+        (C, N) = self._check_readout(what, ('_lM', '_lp_B_g_F'))
         if self.edge_lookup not in _LOOKUP:
             raise ValueError("edge_lookup must be 'reference' or 'symmetric'")
         U = self._check_bt_new(bt_new, C)
@@ -1266,8 +1278,10 @@ class UnsharedRegionFit(object):
             raise ValueError("max_sweeps must be a non-negative integer")
         if self.edge_lookup == "reference" and N < 3:
             raise ValueError("edge_lookup='reference' needs at least 3 regions")
-        max_sweeps = int(max_sweeps)
+        return C, N, U, lq_R0, int(max_sweeps)
 
+    def _score_columns(self, bt_new, C, N, U, lq_R0, max_sweeps, tol):
+        """The device part of `_score_terms` on checked arguments; ``bt_new``: anything `_planes_of` takes."""
         lib = _lib.load()
         prof = self.profile
         pitchU = _dev.even(U)
@@ -1328,26 +1342,41 @@ class UnsharedRegionFit(object):
         return C, int(N)
 
     @staticmethod
-    def _check_bt_new(bt_new, C):
-        """U' of a (C, U') array or tensor of patient correlations."""
+    def _check_bt_new(bt_new, C, name="bt_new"):
+        """U' of a (C, U') array or tensor of subject correlations."""
         if len(tuple(bt_new.shape)) != 2 or int(bt_new.shape[0]) != C:
-            raise ValueError("bt_new must be (C, U') with C = %d (got shape %s)" % (C, tuple(bt_new.shape)))
+            raise ValueError("%s must be (C, U') with C = %d (got shape %s)" % (name, C, tuple(bt_new.shape)))
         U = int(bt_new.shape[1])
         if U < 1:
-            raise ValueError("bt_new holds no patient")
+            raise ValueError("%s holds no subject" % name)
         return U
+
+    @staticmethod
+    def _check_finite(x, name):
+        """Correlations enter the read-outs unvalidated otherwise: a NaN or inf would make every sum it enters
+        non-finite.  One device reduction for a CUDA tensor."""
+        ok = bool(torch.isfinite(x).all()) if torch.is_tensor(x) else bool(np.isfinite(np.asarray(x)).all())
+        if not ok:
+            raise ValueError("%s must hold finite correlations" % name)
+
+    @staticmethod
+    def _columns_on_device(src, C, U, pitchU):
+        """(C, pitchU) float64 device tensor of the columns of ``src``, zero padded: a (C, U) host array or CUDA
+        tensor, or a device tensor already padded to (C, pitchU) (returned as it is)."""
+        if torch.is_tensor(src):
+            src = src.to(_dev.device(), torch.float64)
+            if int(src.shape[1]) == pitchU:
+                return src.contiguous()
+            out = _dev.zeros((C, pitchU))
+            out[:, :U].copy_(src)
+            return out
+        return _dev.upload_rows(np.asarray(src), pitchU)
 
     def _planes_of(self, bt_src, C, U, pitchU, th, with_L=True):
         """Responsibility planes p_0, p_1, p_2 (and L) [C][pitchU] of the columns of ``bt_src``: a (C, U) host
         array or CUDA tensor, or a device tensor already padded to (C, pitchU)."""
         lib = _lib.load()
-        if torch.is_tensor(bt_src):
-            src = bt_src.to(_dev.device(), torch.float64)
-            bt = src.contiguous() if int(src.shape[1]) == pitchU else _dev.zeros((C, pitchU))
-            if int(src.shape[1]) != pitchU:
-                bt[:, :U].copy_(src)
-        else:
-            bt = _dev.upload_rows(np.asarray(bt_src), pitchU)
+        bt = self._columns_on_device(bt_src, C, U, pitchU)
         PL = _dev.empty((4 if with_L else 3, C, pitchU))
         with _dev.timed(self.profile, "P0_resp_cache"):
             _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
@@ -1435,6 +1464,96 @@ class UnsharedRegionFit(object):
                                                      _dev.ptr(ws), _dev.stream()), "fcd_connection_posteriors")
         return ConnectionPosteriors(_dev.download(qT) if maps else None, _dev.download(qFt) if maps else None,
                                     _dev.download(expected), _dev.download(rate))
+
+    # ------------------------------------------------------------------ held-out controls, subjects of unknown group (new)
+    def score_controls(self, b_new=None):
+        """Log-likelihood of each column under the control model, the fit's theta and q_F held fixed.
+
+        For a column x, l_C(x) = sum_c sum_k q_F[c,k] log N(x_c; mu_k, sigma_k): one control's share of
+        E_lp_B_g_F (fcdiff/fit.py:461-472, densities of fit.py:111-114).  The fit itself is not changed.
+
+        Parameters
+        ----------
+        b_new : (C, S) array or CUDA tensor of correlations, same edge order and C as the fit; None: the fit's
+            own controls (``b``, or the control columns of a replica-mode fit's shared inputs).
+
+        Returns
+        -------
+        (S,) float64.
+        """
+        (C, _) = self._check_readout("score_controls", ('_lp_B_g_F',))
+        src = b_new
+        if src is None:
+            if self._shared is not None:
+                (sp, con, _) = self._shared
+                src = sp.X.index_select(1, con)
+            elif self.b is not None:
+                src = self.b
+            else:
+                raise ValueError("The fit has no controls (assign b or pass b_new).")
+        S = self._check_bt_new(src, C, "b_new")
+        self._check_finite(src, "b_new")
+        pitchS = _dev.even(S)
+        return self._control_terms(self._columns_on_device(src, C, S, pitchS), C, S, pitchS)
+
+    def _control_terms(self, X, C, S, pitchS):
+        """(S,) host array: fcd_control_terms of the padded device columns X [C][pitchS]."""
+        lib = _lib.load()
+        th = self._theta(use_snapshot=False)
+        (_, qF) = self._mF.get_dev()
+        out = _dev.empty((S,))
+        ws = _dev.empty((max(int(lib.fcd_control_terms_ws_bytes(C, S)) // 8, 1),))
+        with _dev.timed(self.profile, "P4_control_terms"):
+            _lib.check(lib.fcd_control_terms(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th),
+                                             _dev.ptr(out), _dev.ptr(ws), _dev.stream()), "fcd_control_terms")
+        return _dev.download(out)
+
+    def classify_subjects(self, x_new, prior_patient=None, lq_R0=None, max_sweeps=50, tol=1e-9):
+        """Posterior probability that each column is a patient rather than a control.
+
+        With the fit's theta and q_F held fixed, both groups have a per-subject bound on the log-likelihood:
+        l_C = ``score_controls`` (exact for a one-hot q_F) and l_P = -``score_patients().free_energy``, the
+        patient's share of the evidence bound.  The terms that do not involve the subject (E_lp_F, E_lq_F) are
+        the same in both and cancel, so
+
+            log_odds = l_P - l_C + log(rho / (1 - rho)),    p_patient = expit(log_odds),
+
+        rho the prior probability of the patient group.  For a one-hot q_F, l_P lies below the exact log-evidence
+        of the patient model by KL(q_R || p(R | x)), so ``log_odds`` leans towards the control group by that
+        much.  The columns are uploaded once and feed both models.  The fit itself is not changed.
+
+        Parameters
+        ----------
+        x_new : (C, S) array or CUDA tensor of correlations, same edge order and C as the fit.
+        prior_patient : rho in (0, 1); None: U / (H + U) of the fit's own cohort.
+        lq_R0, max_sweeps, tol : as for ``score_patients``.
+
+        Returns
+        -------
+        SubjectScores(log_odds, p_patient, control_loglik, patient_elbo, lq_R, sweeps, max_change): (S,)
+        float64 arrays l_P - l_C + logit(rho), its expit, l_C and l_P; lq_R, sweeps and max_change are what
+        ``score_patients(x_new, lq_R0, max_sweeps, tol)`` returns.
+        """
+        (C, N, S, lq_R0, max_sweeps) = self._check_score_args("classify_subjects", x_new, lq_R0, max_sweeps)
+        if prior_patient is None:
+            if self._dims is None:
+                raise ValueError("classify_subjects: the fit has no cohort to take the prior from; "
+                                 "pass prior_patient")
+            (_, H, U) = self._dims
+            rho = U / float(H + U)
+        else:
+            rho = float(prior_patient)
+        if not 0.0 < rho < 1.0:
+            raise ValueError("prior_patient must lie in (0, 1) (got %r)" % rho)
+        self._check_finite(x_new, "x_new")
+        pitchS = _dev.even(S)
+        X = self._columns_on_device(x_new, C, S, pitchS)
+        ps = self._patient_scores(*self._score_columns(X, C, N, S, lq_R0, max_sweeps, tol))
+        control = self._control_terms(X, C, S, pitchS)
+        elbo = -ps.free_energy
+        log_odds = (elbo - control) + scipy.special.logit(rho)
+        return SubjectScores(log_odds, scipy.special.expit(log_odds), control, elbo, ps.lq_R, ps.sweeps,
+                             ps.max_change)
 
     # ------------------------------------------------------------------ posterior summaries (new)
     def _map_labels(self, mirror, width):

@@ -1,6 +1,7 @@
 """
 Replica sweeps over the fit: group-label permutations and random restarts
-(BASELINE.json configs[4]; SURVEY 8e "Config 5").  The reference has neither --
+(BASELINE.json configs[4]; SURVEY 8e "Config 5"), and stratified k-fold
+cross-validation of the two-group classifier.  The reference has neither --
 it has no driver beyond ``UnsharedRegionFit.run()`` (fcdiff/fit.py:56-82) -- so
 this module only orchestrates: every replica is one ordinary fit of this
 package on a re-labelled (or re-initialised) copy of the problem.
@@ -220,6 +221,94 @@ def permutation_sweep(corr, labels, n_permutations, model=None, seed=0, fit_opti
     results = _run_replicas(replica_indices(n_permutations + 1, rank, world), run_one,
                             default_streams(world) if streams is None else int(streams))
     return _gather(results, group) if gather else results
+
+
+def stratified_folds(labels, n_folds=5, seed=0):
+    """(S,) int array: the cross-validation fold of every subject.  Each class is shuffled with
+    ``RandomState(seed)`` and dealt round robin over the folds, the patients continuing where the controls
+    stopped: every fold gets each class's count over ``n_folds`` rounded down or up, and the fold sizes differ
+    by at most one."""
+    labels = np.asarray(labels, dtype=bool).reshape(-1)
+    n_folds = int(n_folds)
+    if n_folds < 2:
+        raise ValueError("n_folds must be at least 2")
+    for (cls, name) in ((False, "controls"), (True, "patients")):
+        if int((labels == cls).sum()) < n_folds:
+            raise ValueError("%d %s cannot be spread over %d folds" % (int((labels == cls).sum()), name, n_folds))
+    rng = np.random.RandomState(seed)
+    fold = np.empty(labels.size, dtype=np.int64)
+    start = 0
+    for cls in (False, True):
+        idx = np.flatnonzero(labels == cls)
+        idx = idx[rng.permutation(idx.size)]
+        fold[idx] = (start + np.arange(idx.size)) % n_folds
+        start += idx.size
+    return fold
+
+
+def cross_validate(corr, labels, n_folds=5, model=None, seed=0, fit_options=None, prior_patient=None, streams=None):
+    """
+    Stratified k-fold cross-validation of the two-group classifier
+    (``UnsharedRegionFit.classify_subjects``): every fold is fitted on the
+    other folds' subjects and classifies its own.
+
+    Parameters
+    ----------
+    corr : (C, S) array or CUDA tensor
+        Correlations of ALL subjects, one column per subject.
+    labels : (S,) bool
+        True for patients, False for controls.
+    n_folds, seed
+        Folds of :func:`stratified_folds`.
+    model, fit_options, streams
+        As for :func:`permutation_sweep` (one GPU; the folds are the replicas).
+    prior_patient : float or None
+        Prior probability of the patient group; None: each fold's training proportion.
+
+    Returns
+    -------
+    dict with, per subject in column order, ``fold``, ``log_odds``, ``p_patient``,
+    ``control_loglik`` and ``patient_elbo`` ((S,) arrays), and ``folds``: per fold
+    the summary of its fit (fitted parameters, energy trace) with its final
+    ``free_energy``.
+    """
+    labels = np.asarray(labels, dtype=bool).reshape(-1)
+    fold = stratified_folds(labels, n_folds, seed)
+    dev = _dev.device()
+    corr_dev = corr if torch.is_tensor(corr) else torch.from_numpy(np.ascontiguousarray(corr, dtype=np.float64))
+    corr_dev = corr_dev.to(dev, torch.float64)
+    if corr_dev.dim() != 2 or int(corr_dev.shape[1]) != labels.size:
+        raise ValueError("corr must be (C, S) with S = %d labels (got shape %s)" % (labels.size, tuple(corr_dev.shape)))
+    model = UnsharedRegionModel() if model is None else model
+    shared = None
+    if not (fit_options or {}).get("update_mu_sigma"):
+        shared = SharedPlanes(corr_dev, model)
+
+    def run_one(i):
+        train = fold != i
+        con = torch.from_numpy(np.flatnonzero(train & ~labels)).to(dev)
+        pat = torch.from_numpy(np.flatnonzero(train & labels)).to(dev)
+        fit = UnsharedRegionFit()
+        fit.model = copy.deepcopy(model)
+        _configure(fit, fit_options)
+        if shared is not None:
+            fit.set_shared_inputs(shared, con, pat)
+        else:
+            fit.b = corr_dev.index_select(1, con)
+            fit.bt = corr_dev.index_select(1, pat)
+        fit.run()
+        held = np.flatnonzero(fold == i)
+        s = fit.classify_subjects(corr_dev.index_select(1, torch.from_numpy(held).to(dev)), prior_patient)
+        return dict(held=held, scores=s, summary=dict(_summary(fit), free_energy=float(fit.energy[-1])))
+
+    results = _run_replicas(list(range(n_folds)), run_one, default_streams() if streams is None else int(streams))
+    out = dict(fold=fold, folds=[results[i]["summary"] for i in range(n_folds)])
+    for name in ("log_odds", "p_patient", "control_loglik", "patient_elbo"):
+        v = np.empty(labels.size, dtype=np.float64)
+        for i in range(n_folds):
+            v[results[i]["held"]] = getattr(results[i]["scores"], name)
+        out[name] = v
+    return out
 
 
 def permutation_p_value(results, statistic=lambda r: -r["energy"][-1]):

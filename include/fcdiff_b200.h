@@ -475,6 +475,17 @@ FCD_API int fcd_connection_posteriors(const double* P, int64_t planeStride, int6
                               const fcd_theta* theta_host, double* qT, double* qFt, double* expected, double* rate,
                               double* ws, void* stream);
 
+/* Per-subject control log-likelihoods (csrc/fcd_patients.cu): one control's share of E_lp_B_g_F
+ * (fcdiff/fit.py:461-472) for each new column, with the Gaussian log density of fit.py:111-114:
+ *   out [S] = sum_c sum_k qF[c,k] (-((X[c][s] - mu_k) / sigma_k)^2 / 2 - log sigma_k - log sqrt(2 pi))
+ * X [C][pitchS] edge-major columns (C = N(N-1)/2, pitchS >= S >= 1); qF [C][3]; theta_host supplies mu, sigma.
+ * ws: fcd_control_terms_ws_bytes(C, S) bytes of device scratch (no zero fill needed).  A subject's value is
+ * bit-identical whichever other subjects, S or pitchS are in the call: the row partition depends on C only and
+ * the partials are added in a fixed order. */
+FCD_API int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S);
+FCD_API int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                              const fcd_theta* theta_host, double* out, double* ws, void* stream);
+
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
  * disabled pieces of a mu / sigma update, fcdiff/fit.py:232-237, 542-597,
