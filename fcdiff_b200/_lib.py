@@ -52,19 +52,25 @@ SIGNATURES = {
     "fcd_unpack_patients": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P]),
     "fcd_c_to_nm": (c_int, [c_int64, c_int64, _P, _P, _P]),
     "fcd_healthy_stats": (c_int, [_P, c_int64, c_int32, c_int64, _P, _P, _P]),
+    "fcd_healthy_stats_masked": (c_int, [_P, c_int64, c_int32, c_int64, _P, _P, _P, _P]),
     "fcd_row_logsums": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, _P]),
     "fcd_estep_qF_rowsums": (c_int, [_P, _P, c_int32, _P, c_int64, _D3, POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_estep_qF_rowsums_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, _D3, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_elm_rowsums": (c_int, [_P, _P, c_int64, _D3, _P, _P, _P]),
     "fcd_healthy_stats_cols": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P]),
+    "fcd_healthy_stats_cols_masked": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P, _P]),
     "fcd_gather_columns": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P, c_int64, c_int64, _P]),
     "fcd_gather_rows": (c_int, [_P, c_int64, c_int32, _P, c_int32, c_int64, _P, c_int64, _P]),
     "fcd_edge_table": (c_int, [c_int64, c_int64, _P, _P]),
     "fcd_resp_cache": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
+    "fcd_resp_cache_masked": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
     "fcd_map_labels": (c_int, [_P, c_int64, c_int32, _P, _P]),
     "fcd_peak_states_F": (c_int, [_P, c_int64, _P, _P]),
     "fcd_peak_states_R": (c_int, [_P, c_int32, c_int32, c_int64, _P, _P]),
     "fcd_estep_qF": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64, c_int32, _P,
                              POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_estep_qF_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64,
+                                    c_int32, _P, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_transpose_patients": (c_int, [_P, c_int64, c_int32, c_int64, c_int32, c_int32, _P, c_int64, _P]),
     "fcd_region_weights": (c_int, [_P, c_int64, c_int32, c_int64, c_int64, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P]),
     "fcd_estep_qR": (c_int, [_P, c_int64, c_int32, c_int32, c_int32, c_int32, _D3, c_int32, _P, _P, _P]),
@@ -87,9 +93,14 @@ SIGNATURES = {
                                  c_int32, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, _P, _P, _P]),
     "fcd_estep_qF_coded": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P,
                                    _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_estep_qF_coded_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32,
+                                          _P, _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_estep_qF_coded_solved": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P,
                                           _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, c_double, c_double,
                                           _P, _P, _P]),
+    "fcd_estep_qF_coded_solved_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P,
+                                                 c_int32, _P, _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P,
+                                                 c_double, c_double, _P, _P, _P]),
     "fcd_elm_coded": (c_int, [_P, _P, c_int64, _P, c_int64, _P, c_int64, POINTER(FcdTheta), c_int32, _P, _P, _P]),
     "fcd_solver_state_bytes": (c_int64, []),
     "fcd_solver_published_bytes": (c_int64, []),
@@ -106,6 +117,8 @@ SIGNATURES = {
     "fcd_solver_wait": (c_int, [_P, c_uint64, _P, c_int32]),
     "fcd_energy_terms": (c_int, [_P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
                                  POINTER(FcdTheta), c_double, _P, _P, _P, _P]),
+    "fcd_energy_terms_masked": (c_int, [_P, _P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
+                                        POINTER(FcdTheta), c_double, _P, _P, _P, _P]),
     "fcd_patient_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
     "fcd_patient_terms": (c_int, [_P, c_int64, _P, c_int64, c_int32, c_int64, _P, _P, _P, _P, c_int32, POINTER(FcdTheta),
                                   _P, _P, _P]),
@@ -115,9 +128,11 @@ SIGNATURES = {
                                           POINTER(FcdTheta), _P, _P, _P, _P, _P, _P]),
     "fcd_control_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
     "fcd_control_terms": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_control_terms_masked": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_state_moments": (c_int, [_P, _P, c_int32, _P, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int32, _P,
                                   POINTER(FcdTheta), _P, _P, _P]),
     "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),
+    "fcd_materialize_lps_masked": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),
     "fcd_eval_M": (c_int, [_P, c_int64, c_double, c_double, c_int32, c_int32, _P, _P]),
     "fcd_lqF_from_arrays": (c_int, [_P, _P, c_int64, c_int32, c_int32, _P, c_int32, _D3, _P, _P]),
     "fcd_region_weights_from_lM": (c_int, [_P, c_int64, c_int32, _P, _P, _P]),
@@ -134,6 +149,7 @@ SIGNATURES = {
     "fcd_sample_B_tilde": (c_int, [c_uint64, c_uint64, _P, c_int64, c_int64, c_int32, _D3, _D3, _P, _P]),
     "fcd_corr_workspace_bytes": (c_int64, [c_int32, c_int32, c_int32]),
     "fcd_corr_fisherz": (c_int, [_P, c_int32, c_int32, c_int32, _P, c_int64, c_int32, c_int32, _P, _P]),
+    "fcd_corr_mark_missing": (c_int, [_P, c_int32, c_int32, c_int32, _P, c_int64, c_int32, _P]),
 }
 
 class SolverState(ctypes.Structure):

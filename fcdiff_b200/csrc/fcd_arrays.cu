@@ -41,23 +41,37 @@ struct LpsParams {
     double mu[3], sigma[3], log_sigma[3], epsl[3];
 };
 
+// MASKED: a NaN entry is not observed; its caches hold the marginalised values
+//   lp_B_g_F = 0 (density factor 1), p_Bt_g_Ft = (1, 1, 1) and lM = 0 (M_kl = eps_l + (1 - eps_l) = 1).
+template <bool MASKED>
 __global__ void __launch_bounds__(kArrThreads)
 materialize_b_kernel(const double* __restrict__ b, int64_t n, const __grid_constant__ LpsParams p,
                      double* __restrict__ lpB) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
          i += (int64_t)gridDim.x * blockDim.x) {
         const double x = b[i];
+        if (MASKED && isnan(x)) {
+            lpB[i * 3] = lpB[i * 3 + 1] = lpB[i * 3 + 2] = 0.0;
+            continue;
+        }
 #pragma unroll
         for (int k = 0; k < 3; ++k) lpB[i * 3 + k] = sp_logpdf(sp_y(x, p.mu[k], p.sigma[k]), p.log_sigma[k]);
     }
 }
 
+template <bool MASKED>
 __global__ void __launch_bounds__(kArrThreads)
 materialize_bt_kernel(const double* __restrict__ bt, int64_t n, const __grid_constant__ LpsParams p,
                       double* __restrict__ pBt, double* __restrict__ lM) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n;
          i += (int64_t)gridDim.x * blockDim.x) {
         const double x = bt[i];
+        if (MASKED && isnan(x)) {
+            pBt[i * 3] = pBt[i * 3 + 1] = pBt[i * 3 + 2] = 1.0;
+#pragma unroll
+            for (int j = 0; j < 9; ++j) lM[i * 9 + j] = 0.0;
+            continue;
+        }
         double pk[3];
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
@@ -233,8 +247,8 @@ using namespace fcd;
 
 extern "C" {
 
-int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
-                        const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
+static int materialize_lps_launch(bool masked, const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
+                                  const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
     FCD_REQUIRE(theta_host != nullptr, "fcd_materialize_lps: theta is NULL");
     FCD_REQUIRE(C >= 0 && H >= 0 && U >= 0, "fcd_materialize_lps: bad shape");
     LpsParams p;
@@ -250,15 +264,29 @@ int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H,
     cudaStream_t st = (cudaStream_t)stream;
     int rc = 0;
     if (b != nullptr && lpB != nullptr && C * H > 0) {
-        materialize_b_kernel<<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
+        if (masked) materialize_b_kernel<true><<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
+        else materialize_b_kernel<false><<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
         rc = check_launch("fcd_materialize_lps(b)");
         if (rc) return rc;
     }
     if (bt != nullptr && pBt != nullptr && lM != nullptr && C * U > 0) {
-        materialize_bt_kernel<<<arr_grid(C * U, kArrThreads), kArrThreads, 0, st>>>(bt, C * U, p, pBt, lM);
+        if (masked)
+            materialize_bt_kernel<true><<<arr_grid(C * U, kArrThreads), kArrThreads, 0, st>>>(bt, C * U, p, pBt, lM);
+        else
+            materialize_bt_kernel<false><<<arr_grid(C * U, kArrThreads), kArrThreads, 0, st>>>(bt, C * U, p, pBt, lM);
         rc = check_launch("fcd_materialize_lps(bt)");
     }
     return rc;
+}
+
+int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
+                        const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
+    return materialize_lps_launch(false, b, bt, C, H, U, theta_host, lpB, pBt, lM, stream);
+}
+
+int fcd_materialize_lps_masked(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
+                               const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
+    return materialize_lps_launch(true, b, bt, C, H, U, theta_host, lpB, pBt, lM, stream);
 }
 
 int fcd_eval_M(const double* p, int64_t n, double eta, double epsilon, int32_t k, int32_t l,

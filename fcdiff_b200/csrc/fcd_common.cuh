@@ -63,6 +63,7 @@ struct ThetaDev {
     double eta;
     double epsilon;
     double log_pi2[2];
+    double hq_c1[3];     // hq_c of one control: the masked form takes H_c * hq_c1 with H_c = S0[c] observed controls
 };
 
 ThetaDev make_theta_dev(const fcd_theta& th, int H);
@@ -172,15 +173,24 @@ __device__ __forceinline__ void pair_weights(double2 qn, double2 qm, double (&w)
 __device__ __forceinline__ double sel3(int l, const double (&v)[3]) { return l == 0 ? v[0] : (l == 1 ? v[1] : v[2]); }
 
 // ---------------------------------------------------------------- K2 row end
+// Healthy term of edge c, sum_h log N_k(b[c,h]) = hq_a S2 + hq_b S1 + hq_c (fit.py:111-114, 171).  MASKED: the
+// sums run over the S0 = H_c observed controls of the edge and the constant is H_c hq_c1; hq_c1 = hq_c / (-H) up to
+// the sign only (make_theta_dev), so S0 = H gives the bits of the unmasked form.
+template <bool MASKED>
+__device__ __forceinline__ double healthy_term(const ThetaDev& th, int k, double s1, double s2, double s0) {
+    return fma(th.hq_a[k], s2, fma(th.hq_b[k], s1, MASKED ? __dmul_rn(s0, th.hq_c1[k]) : th.hq_c[k]));
+}
+
 // lane 0 of the warp that owns edge c: log gamma + healthy quadratic + A, then
 // scipy.special.logsumexp: a_max + log(sum exp(a - a_max))           (fit.py:165-174)
-__device__ __forceinline__ void k2_finish(int64_t c, const double (&A)[3], double s1, double s2,
+template <bool MASKED = false>
+__device__ __forceinline__ void k2_finish(int64_t c, const double (&A)[3], double s1, double s2, double s0,
                                           const ThetaDev& th, double* __restrict__ lqF,
                                           double* __restrict__ qF) {
     double l[3];
 #pragma unroll
     for (int k = 0; k < 3; ++k)
-        l[k] = th.log_gamma[k] + fma(th.hq_a[k], s2, fma(th.hq_b[k], s1, th.hq_c[k])) + A[k];
+        l[k] = th.log_gamma[k] + healthy_term<MASKED>(th, k, s1, s2, s0) + A[k];
     const double mx = fmax(l[0], fmax(l[1], l[2]));
     const double lse = mx + log(exp(l[0] - mx) + exp(l[1] - mx) + exp(l[2] - mx));
 #pragma unroll

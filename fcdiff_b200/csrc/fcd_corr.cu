@@ -101,6 +101,39 @@ gram_simt_kernel(const float* __restrict__ Z, int N, int Tp, int ntile,
         }
 }
 
+// Rows without a usable time series: one warp per (subject, region) row, the sums of standardise_kernel in
+// the same order.  A row with a non-finite sample, or of zero variance, gets NaN (not observed) on every
+// one of its N - 1 edges in column s0 + s.  (standardise_kernel cannot tell such a row from a real
+// zero correlation: it writes zeros, and a NaN sample ends up as the negative clip.)
+__global__ void __launch_bounds__(256)
+mark_missing_kernel(const float* __restrict__ ts, int S, int N, int T, double* __restrict__ out, int64_t pitch,
+                    int s0) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int64_t rows = (int64_t)S * N;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    for (int64_t r = warp0; r < rows; r += nwarps) {
+        const float* x = ts + r * T;
+        double s = 0.0;
+        for (int t = lane; t < T; t += 32) s += (double)x[t];
+        const double mean = warp_sum(s) / (double)T;
+        double ss = 0.0;
+        for (int t = lane; t < T; t += 32) {
+            const double d = (double)x[t] - mean;
+            ss = fma(d, d, ss);
+        }
+        ss = warp_sum(ss);
+        if (ss > 0.0) continue;                               // also false for NaN: an inf or NaN sample
+        const int subj = (int)(r / N), n = (int)(r - (int64_t)subj * N);
+        for (int m = lane; m < N; m += 32) {
+            if (m == n) continue;
+            const int64_t c = n > m ? (int64_t)n * (n - 1) / 2 + m : (int64_t)m * (m - 1) / 2 + n;
+            out[c * pitch + s0 + subj] = nan;
+        }
+    }
+}
+
 }  // namespace fcd
 
 using namespace fcd;
@@ -140,6 +173,20 @@ int fcd_corr_fisherz(const float* ts, int32_t S, int32_t N, int32_t T,
     dim3 grid((unsigned)(nt * (nt + 1) / 2), (unsigned)S);
     gram_simt_kernel<<<grid, 256, 0, st>>>(Z, N, Tp, nt, out, pitch, s0, fisher);
     return check_launch("fcd_corr_fisherz(gram_simt)");
+}
+
+int fcd_corr_mark_missing(const float* ts, int32_t S, int32_t N, int32_t T, double* out, int64_t pitch, int32_t s0,
+                          void* stream) {
+    FCD_REQUIRE(ts != nullptr && out != nullptr, "fcd_corr_mark_missing: NULL argument");
+    FCD_REQUIRE(S >= 0 && N >= 2 && T >= 2 && s0 >= 0 && pitch >= (int64_t)s0 + S,
+                "fcd_corr_mark_missing: bad shape S=%d N=%d T=%d s0=%d pitch=%lld", S, N, T, s0, (long long)pitch);
+    if (S == 0) return 0;
+    const int64_t rows = (int64_t)S * N;
+    int64_t g = (rows + 7) / 8;
+    const int64_t cap = (int64_t)sm_count() * 8;
+    if (g > cap) g = cap;
+    mark_missing_kernel<<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(ts, S, N, T, out, pitch, s0);
+    return check_launch("fcd_corr_mark_missing");
 }
 
 }  // extern "C"

@@ -36,26 +36,33 @@ __global__ void edge_table_kernel(int64_t c0, int64_t C, int32_t* __restrict__ n
 
 // ------------------------------------------------------------ healthy stats
 // S1[c] = sum_h b[c,h], S2[c] = sum_h b[c,h]^2.  One warp per edge row,
-// coalesced 64-bit loads along the subject axis.
+// coalesced 64-bit loads along the subject axis.  MASKED: NaN entries are not
+// observed and left out; S0[c] counts the observed ones (same sums, same order
+// as the unmasked form when nothing is missing).
+template <bool MASKED>
 __global__ void __launch_bounds__(kEdgeThreads)
 healthy_stats_kernel(const double* __restrict__ b, int64_t C, int H, int64_t pitchH,
-                     double* __restrict__ S1, double* __restrict__ S2) {
+                     double* __restrict__ S1, double* __restrict__ S2, double* __restrict__ S0) {
     const int lane = threadIdx.x & 31;
     const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t c = warp0; c < C; c += nwarps) {
         const double* row = b + c * pitchH;
-        double s1 = 0.0, s2 = 0.0;
+        double s1 = 0.0, s2 = 0.0, s0 = 0.0;
         for (int h = lane; h < H; h += 32) {
             double x = ldg_stream1(row + h);
+            if (MASKED && isnan(x)) continue;
             s1 += x;
             s2 = fma(x, x, s2);
+            if (MASKED) s0 += 1.0;
         }
         s1 = warp_sum(s1);
         s2 = warp_sum(s2);
+        if (MASKED) s0 = warp_sum(s0);
         if (lane == 0) {
             S1[c] = s1;
             S2[c] = s2;
+            if (MASKED) S0[c] = s0;
         }
     }
 }
@@ -64,6 +71,10 @@ healthy_stats_kernel(const double* __restrict__ b, int64_t C, int H, int64_t pit
 // P0 / P1 / P2 / L planes (see fcd_common.cuh) from the patient correlations; the
 // only place where exponentials of the data are taken.  Elementwise over the
 // padded [C][pitchU] rows (padding columns are written as zeros).
+// MASKED: a NaN entry is not observed and gets p_k = 1/3, L = log 3, so that
+// log M_kl = L + log(a_l + b_l / 3) = 0 for every (k, l) and theta: the element
+// drops out of every later pass, which read it through the planes only.
+template <bool MASKED>
 __global__ void __launch_bounds__(256)
 resp_cache_kernel(const double* __restrict__ bt, int64_t C, int U, int64_t pitchU,
                   const __grid_constant__ ThetaDev th,
@@ -74,7 +85,15 @@ resp_cache_kernel(const double* __restrict__ bt, int64_t C, int U, int64_t pitch
         const int u = (int)(i % pitchU);
         Resp r;
         r.p[0] = r.p[1] = r.p[2] = r.L = 0.0;
-        if (u < U) r = resp_eval(ldg_stream1(bt + i), th);
+        if (u < U) {
+            const double x = ldg_stream1(bt + i);
+            if (MASKED && isnan(x)) {
+                r.p[0] = r.p[1] = r.p[2] = 1.0 / 3.0;
+                r.L = 1.0986122886681098;                    // log 3
+            } else {
+                r = resp_eval(x, th);
+            }
+        }
         P[i] = r.p[0];
         P[planeStride + i] = r.p[1];
         P[2 * planeStride + i] = r.p[2];
@@ -146,9 +165,9 @@ map_labels_kernel(const double* __restrict__ lq, int64_t n, int width, uint8_t* 
 
 constexpr int kK2Seg = 128;
 
-template <bool FAST>
+template <bool FAST, bool MASKED>
 __global__ void __launch_bounds__(kStreamThreads, 1)
-estep_qF_kernel(const double* __restrict__ S1, const double* __restrict__ S2,
+estep_qF_kernel(const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S0,
                 const double* __restrict__ P, int64_t planeStride,
                 int64_t C, int U, int64_t pitchU,
                 const double* __restrict__ qR, const uint8_t* __restrict__ rstate, int64_t pitchS,
@@ -229,7 +248,9 @@ estep_qF_kernel(const double* __restrict__ S1, const double* __restrict__ S2,
     int64_t keep_c = -1;
     int rows_done = 0;
     auto finish_rows = [&]() {
-        if (keep_c >= 0) k2_finish(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), th, lqF, qF);
+        if (keep_c >= 0)
+            k2_finish<MASKED>(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), MASKED ? __ldg(S0 + keep_c) : 0.0,
+                              th, lqF, qF);
         keep_c = -1;
     };
     auto row_end = [&](int64_t c) {
@@ -264,9 +285,9 @@ constexpr int kK2cStage = 2 * kK2cSeg * 8 + kK2cSeg;          // bytes: p_0, p_1
 constexpr int kK2cMaxDepth = 5;
 constexpr size_t k2c_ring_bytes(int depth, int nw) { return (size_t)nw * depth * (kK2cStage + 8); }
 
-template <bool FAST, int NW>
+template <bool FAST, int NW, bool MASKED>
 __global__ void __launch_bounds__(NW * 32, 1)
-estep_qF_coded_kernel(const double* __restrict__ S1, const double* __restrict__ S2,
+estep_qF_coded_kernel(const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S0,
                       const double* __restrict__ P, int64_t planeStride, int64_t C, int U, int64_t pitchU,
                       const double* __restrict__ qR, const int32_t* __restrict__ nm,
                       const uint8_t* __restrict__ code, int64_t pitchQ, const int2* __restrict__ counts,
@@ -410,7 +431,9 @@ estep_qF_coded_kernel(const double* __restrict__ S1, const double* __restrict__ 
     int64_t keep_c = -1;
     int rows_done = 0;
     auto finish_rows = [&]() {
-        if (keep_c >= 0) k2_finish(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), th, lqF, qF);
+        if (keep_c >= 0)
+            k2_finish<MASKED>(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), MASKED ? __ldg(S0 + keep_c) : 0.0,
+                              th, lqF, qF);
         keep_c = -1;
     };
     // The half records of a row are taken off the critical path (they used to be a chain of dependent
@@ -1509,20 +1532,46 @@ int fcd_healthy_stats(const double* b, int64_t C, int32_t H, int64_t pitchH,
     FCD_REQUIRE(C >= 0 && H >= 1 && pitchH >= H, "fcd_healthy_stats: bad shape C=%lld H=%d pitch=%lld",
                 (long long)C, H, (long long)pitchH);
     if (C == 0) return 0;
-    healthy_stats_kernel<<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
-        b, C, H, pitchH, S1, S2);
+    healthy_stats_kernel<false><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
+        b, C, H, pitchH, S1, S2, nullptr);
     return check_launch("fcd_healthy_stats");
 }
 
-int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
+int fcd_healthy_stats_masked(const double* b, int64_t C, int32_t H, int64_t pitchH,
+                             double* S1, double* S2, double* S0, void* stream) {
+    FCD_REQUIRE(C >= 0 && H >= 1 && pitchH >= H, "fcd_healthy_stats_masked: bad shape C=%lld H=%d pitch=%lld",
+                (long long)C, H, (long long)pitchH);
+    FCD_REQUIRE(C == 0 || (b != nullptr && S1 != nullptr && S2 != nullptr && S0 != nullptr),
+                "fcd_healthy_stats_masked: NULL argument");
+    if (C == 0) return 0;
+    healthy_stats_kernel<true><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
+        b, C, H, pitchH, S1, S2, S0);
+    return check_launch("fcd_healthy_stats_masked");
+}
+
+static int resp_cache_launch(bool masked, const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                             const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && bt != nullptr && P != nullptr, "fcd_resp_cache: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && pitchU >= U && planeStride >= C * pitchU, "fcd_resp_cache: bad shape");
     if (C == 0) return 0;
     const ThetaDev th = make_theta_dev(*theta_host, 0);
-    resp_cache_kernel<<<grid_for_rows(C * pitchU, 256, 16), 256, 0, (cudaStream_t)stream>>>(
-        bt, C, U, pitchU, th, P, planeStride, L);
-    return check_launch("fcd_resp_cache");
+    if (masked)
+        resp_cache_kernel<true><<<grid_for_rows(C * pitchU, 256, 16), 256, 0, (cudaStream_t)stream>>>(
+            bt, C, U, pitchU, th, P, planeStride, L);
+    else
+        resp_cache_kernel<false><<<grid_for_rows(C * pitchU, 256, 16), 256, 0, (cudaStream_t)stream>>>(
+            bt, C, U, pitchU, th, P, planeStride, L);
+    return check_launch(masked ? "fcd_resp_cache_masked" : "fcd_resp_cache");
+}
+
+int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
+    return resp_cache_launch(false, bt, C, U, pitchU, theta_host, P, planeStride, L, stream);
+}
+
+int fcd_resp_cache_masked(const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                          const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
+    return resp_cache_launch(true, bt, C, U, pitchU, theta_host, P, planeStride, L, stream);
 }
 
 int fcd_map_labels(const double* lq, int64_t n, int32_t width, uint8_t* labels, void* stream) {
@@ -1547,10 +1596,11 @@ int fcd_peak_states_R(const double* qR, int32_t N, int32_t U, int64_t pitchS, ui
     return check_launch("fcd_peak_states_R");
 }
 
-int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
-                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
-                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+// S0 == NULL: every edge has all H controls (fcd_estep_qF); otherwise fcd_estep_qF_masked.
+static int estep_qF_launch(const double* S1, const double* S2, const double* S0, int32_t H,
+                           const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                           const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
+                           const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && P != nullptr && qR != nullptr && rstate != nullptr && nm != nullptr &&
                 lqF != nullptr, "fcd_estep_qF: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && U < 65536 && pitchU >= U && pitchS >= U && N >= 2 && N < 65536,
@@ -1569,22 +1619,43 @@ int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
     const size_t smem = tbytes + StreamGeom<2, kK2Seg>::bytes(kStreamWarps, depth);
     int64_t grid = (C + kStreamWarps - 1) / kStreamWarps;
     if (grid > sm_count()) grid = sm_count();                       // one persistent CTA per SM
-#define FCD_K2(F)                                                                                 \
-    do {                                                                                          \
-        cudaFuncSetAttribute(estep_qF_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize,     \
-                             (int)kSmemBudget);                                                   \
-        estep_qF_kernel<F><<<(unsigned)grid, kStreamThreads, smem, st>>>(                         \
-            S1, S2, P, planeStride, C, U, pitchU, qR, rstate, pitchS, nm, th, tab, depth, lqF, qF); \
+#define FCD_K2(F, M)                                                                                  \
+    do {                                                                                              \
+        cudaFuncSetAttribute(estep_qF_kernel<F, M>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
+                             (int)kSmemBudget);                                                       \
+        estep_qF_kernel<F, M><<<(unsigned)grid, kStreamThreads, smem, st>>>(                          \
+            S1, S2, S0, P, planeStride, C, U, pitchU, qR, rstate, pitchS, nm, th, tab, depth, lqF, qF); \
     } while (0)
-    if (fast) FCD_K2(true); else FCD_K2(false);
+    if (S0 != nullptr) {
+        if (fast) FCD_K2(true, true); else FCD_K2(false, true);
+    } else {
+        if (fast) FCD_K2(true, false); else FCD_K2(false, false);
+    }
 #undef FCD_K2
-    return check_launch("fcd_estep_qF");
+    return check_launch(S0 != nullptr ? "fcd_estep_qF_masked" : "fcd_estep_qF");
+}
+
+int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
+                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
+                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+    return estep_qF_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, rstate, pitchS, N, nm, theta_host,
+                           lqF, qF, stream);
+}
+
+int fcd_estep_qF_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                        const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                        const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
+                        const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_masked: S0 is NULL");
+    return estep_qF_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, rstate, pitchS, N, nm, theta_host,
+                           lqF, qF, stream);
 }
 
 // `solved` == NULL: (eta, epsilon) of theta_host; otherwise the solver state block a device-resident solve
 // enqueued BEFORE this launch leaves its solution in, with [eps_lo, eps_hi] the box of that solve (it
 // sizes the logarithm table like fcd_elm_coded_solve does).
-static int estep_qF_coded_launch(const double* S1, const double* S2, int32_t H,
+static int estep_qF_coded_launch(const double* S1, const double* S2, const double* S0, int32_t H,
                                  const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                                  const double* qR, int32_t N, const int32_t* nm,
                                  const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
@@ -1626,7 +1697,7 @@ static int estep_qF_coded_launch(const double* S1, const double* S2, int32_t H,
         return e != nullptr && strcmp(e, "rows") == 0;
     }();
     if (rows_form && solved == nullptr && estep_rows_supported(U, pitchU, pitchQ))
-        return estep_rows_launch(S1, S2, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, counts, keysF, keysH, rowoff,
+        return estep_rows_launch(S1, S2, S0, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, counts, keysF, keysH, rowoff,
                                  Hh, th, tab, fast, lqF, qF, st);
     // 16 warps per SM (127 registers each).  FCD_K2C_WARPS=24 selects the 24-warp build (80 registers, three
     // ring stages per warp): measured no faster (0.199 vs 0.193 ms at config 3) -- the kernel is bound by
@@ -1636,29 +1707,34 @@ static int estep_qF_coded_launch(const double* S1, const double* S2, int32_t H,
         return e != nullptr ? atoi(e) : 0;
     }();
     int nw = 16;
-    if ((forced_nw == 24 || forced_nw == 20) && tbytes + k2c_ring_bytes(2, forced_nw) <= kSmemBudget) nw = forced_nw;
+    if (S0 == nullptr && (forced_nw == 24 || forced_nw == 20) && tbytes + k2c_ring_bytes(2, forced_nw) <= kSmemBudget) nw = forced_nw;
     int depth = kK2cMaxDepth;
     while (depth > 2 && tbytes + k2c_ring_bytes(depth, nw) > kSmemBudget) --depth;
     FCD_REQUIRE(tbytes + k2c_ring_bytes(depth, nw) <= kSmemBudget, "fcd_estep_qF_coded: shared memory budget exceeded");
     const size_t smem = tbytes + k2c_ring_bytes(depth, nw);
     int64_t grid = (C + nw - 1) / nw;
     if (grid > sm_count()) grid = sm_count();                       // one persistent CTA per SM
-#define FCD_K2C_(F, NW_)                                                                              \
+#define FCD_K2C_(F, NW_, M)                                                                           \
     do {                                                                                              \
-        FCD_ALLOW_BIG_SMEM(estep_qF_coded_kernel<F, NW_>);                                            \
-        estep_qF_coded_kernel<F, NW_><<<(unsigned)grid, NW_ * 32, smem, st>>>(                        \
-            S1, S2, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, reinterpret_cast<const int2*>(counts), \
+        FCD_ALLOW_BIG_SMEM(estep_qF_coded_kernel<F, NW_, M>);                                         \
+        estep_qF_coded_kernel<F, NW_, M><<<(unsigned)grid, NW_ * 32, smem, st>>>(                     \
+            S1, S2, S0, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, reinterpret_cast<const int2*>(counts), \
             reinterpret_cast<const unsigned long long*>(keysF), reinterpret_cast<const unsigned long long*>(keysH), \
             reinterpret_cast<const longlong2*>(rowoff), reinterpret_cast<const double2*>(Hh), th, solved, tab, depth, lqF, qF); \
     } while (0)
 #define FCD_K2C(F)                                                                                    \
     do {                                                                                              \
-        if (nw == 24) FCD_K2C_(F, 24); else if (nw == 20) FCD_K2C_(F, 20); else FCD_K2C_(F, 16);      \
+        if (nw == 24) FCD_K2C_(F, 24, false); else if (nw == 20) FCD_K2C_(F, 20, false); else FCD_K2C_(F, 16, false); \
     } while (0)
-    if (fast) FCD_K2C(true); else FCD_K2C(false);
+    // the masked form is built for the default 16 warps only (the other widths are experiments)
+    if (S0 != nullptr) {
+        if (fast) FCD_K2C_(true, 16, true); else FCD_K2C_(false, 16, true);
+    } else {
+        if (fast) FCD_K2C(true); else FCD_K2C(false);
+    }
 #undef FCD_K2C
 #undef FCD_K2C_
-    return check_launch("fcd_estep_qF_coded");
+    return check_launch(S0 != nullptr ? "fcd_estep_qF_coded_masked" : "fcd_estep_qF_coded");
 }
 
 int fcd_estep_qF_coded(const double* S1, const double* S2, int32_t H,
@@ -1667,8 +1743,19 @@ int fcd_estep_qF_coded(const double* S1, const double* S2, int32_t H,
                        const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
                        const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
                        const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    return estep_qF_coded_launch(S1, S2, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts, keysF, keysH,
-                                 rowoff, Hh, theta_host, nullptr, 0.0, 0.0, lqF, qF, stream);
+    return estep_qF_coded_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
+                                 keysF, keysH, rowoff, Hh, theta_host, nullptr, 0.0, 0.0, lqF, qF, stream);
+}
+
+int fcd_estep_qF_coded_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                              const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                              const double* qR, int32_t N, const int32_t* nm,
+                              const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
+                              const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
+                              const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_coded_masked: S0 is NULL");
+    return estep_qF_coded_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
+                                 keysF, keysH, rowoff, Hh, theta_host, nullptr, 0.0, 0.0, lqF, qF, stream);
 }
 
 int fcd_estep_qF_coded_solved(const double* S1, const double* S2, int32_t H,
@@ -1680,9 +1767,24 @@ int fcd_estep_qF_coded_solved(const double* S1, const double* S2, int32_t H,
                               double* lqF, double* qF, void* stream) {
     FCD_REQUIRE(solver_state != nullptr && (reinterpret_cast<uintptr_t>(solver_state) & 7) == 0,
                 "fcd_estep_qF_coded_solved: solver state must be a device pointer (fcd_solver_init)");
-    return estep_qF_coded_launch(S1, S2, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts, keysF, keysH,
-                                 rowoff, Hh, theta_host, static_cast<const SolverState*>(solver_state), eps_lo, eps_hi,
-                                 lqF, qF, stream);
+    return estep_qF_coded_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
+                                 keysF, keysH, rowoff, Hh, theta_host, static_cast<const SolverState*>(solver_state),
+                                 eps_lo, eps_hi, lqF, qF, stream);
+}
+
+int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                                     const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                                     const double* qR, int32_t N, const int32_t* nm,
+                                     const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
+                                     const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
+                                     const fcd_theta* theta_host, const void* solver_state, double eps_lo,
+                                     double eps_hi, double* lqF, double* qF, void* stream) {
+    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_coded_solved_masked: S0 is NULL");
+    FCD_REQUIRE(solver_state != nullptr && (reinterpret_cast<uintptr_t>(solver_state) & 7) == 0,
+                "fcd_estep_qF_coded_solved_masked: solver state must be a device pointer (fcd_solver_init)");
+    return estep_qF_coded_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
+                                 keysF, keysH, rowoff, Hh, theta_host, static_cast<const SolverState*>(solver_state),
+                                 eps_lo, eps_hi, lqF, qF, stream);
 }
 
 int fcd_transpose_patients(const double* bt, int64_t C, int32_t U, int64_t pitchU,

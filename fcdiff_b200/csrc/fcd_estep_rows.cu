@@ -36,11 +36,11 @@ __device__ __forceinline__ void rw_tma_2d(uint32_t dst, const CUtensorMap* map, 
         ::"r"(dst), "l"(map), "r"(x), "r"(y), "r"(bar) : "memory");
 }
 
-template <bool FAST, int NW>
+template <bool FAST, int NW, bool MASKED>
 __global__ void __launch_bounds__(NW * 32, 1)
 estep_qF_rows_kernel(const __grid_constant__ CUtensorMap map_p0, const __grid_constant__ CUtensorMap map_p1,
                      const __grid_constant__ CUtensorMap map_code,
-                     const double* __restrict__ S1, const double* __restrict__ S2,
+                     const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S0,
                      const double* __restrict__ P, int64_t planeStride, int64_t C, int U, int64_t pitchU,
                      const double* __restrict__ qR, const int32_t* __restrict__ nm,
                      const int2* __restrict__ counts, const unsigned long long* __restrict__ keysF,
@@ -141,7 +141,9 @@ estep_qF_rows_kernel(const __grid_constant__ CUtensorMap map_p0, const __grid_co
     int64_t keep_c = -1;
     int groups_done = 0;
     auto finish_rows = [&]() {
-        if (keep_c >= 0) k2_finish(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), th, lqF, qF);
+        if (keep_c >= 0)
+            k2_finish<MASKED>(keep_c, keep, __ldg(S1 + keep_c), __ldg(S2 + keep_c), MASKED ? __ldg(S0 + keep_c) : 0.0,
+                              th, lqF, qF);
         keep_c = -1;
     };
 
@@ -300,9 +302,9 @@ bool estep_rows_supported(int U, int64_t pitchU, int64_t pitchQ) {
     return U >= 1 && pitchU % 2 == 0 && pitchQ % 16 == 0 && rw_encode_fn() != nullptr;
 }
 
-int estep_rows_launch(const double* S1, const double* S2, const double* P, int64_t planeStride, int64_t C, int U,
-                      int64_t pitchU, const double* qR, const int32_t* nm, const uint8_t* code, int64_t pitchQ,
-                      const int32_t* counts, const uint64_t* keysF, const uint64_t* keysH, const int64_t* rowoff,
+int estep_rows_launch(const double* S1, const double* S2, const double* S0, const double* P, int64_t planeStride,
+                      int64_t C, int U, int64_t pitchU, const double* qR, const int32_t* nm, const uint8_t* code,
+                      int64_t pitchQ, const int32_t* counts, const uint64_t* keysF, const uint64_t* keysH, const int64_t* rowoff,
                       const double* Hh, const ThetaDev& th, const LogTabWindow& tab, bool fast, double* lqF, double* qF,
                       cudaStream_t st) {
     alignas(64) CUtensorMap map_p0, map_p1, map_code;
@@ -318,7 +320,7 @@ int estep_rows_launch(const double* S1, const double* S2, const double* P, int64
         return e != nullptr ? atoi(e) : 0;
     }();
     int nw = 16;
-    if (forced_nw == 8 || forced_nw == 12 || forced_nw == 16) nw = forced_nw;
+    if (S0 == nullptr && (forced_nw == 8 || forced_nw == 12 || forced_nw == 16)) nw = forced_nw;
     int depth = kRwMaxDepth;
     while (depth > 2 && tbytes + rw_ring_bytes(depth, nw) > kSmemBudget) --depth;
     FCD_REQUIRE(tbytes + rw_ring_bytes(depth, nw) <= kSmemBudget, "fcd_estep_qF_coded: shared memory budget exceeded");
@@ -326,22 +328,27 @@ int estep_rows_launch(const double* S1, const double* S2, const double* P, int64
     const int64_t ngroups = (C + kRwRows - 1) / kRwRows;
     int64_t grid = (ngroups + nw - 1) / nw;
     if (grid > sm_count()) grid = sm_count();                       // one persistent CTA per SM
-#define FCD_K2R_(F, NW_)                                                                              \
+#define FCD_K2R_(F, NW_, M)                                                                           \
     do {                                                                                              \
-        FCD_ALLOW_BIG_SMEM(estep_qF_rows_kernel<F, NW_>);                                             \
-        estep_qF_rows_kernel<F, NW_><<<(unsigned)grid, NW_ * 32, smem, st>>>(                         \
-            map_p0, map_p1, map_code, S1, S2, P, planeStride, C, U, pitchU, qR, nm,                   \
+        FCD_ALLOW_BIG_SMEM(estep_qF_rows_kernel<F, NW_, M>);                                          \
+        estep_qF_rows_kernel<F, NW_, M><<<(unsigned)grid, NW_ * 32, smem, st>>>(                      \
+            map_p0, map_p1, map_code, S1, S2, S0, P, planeStride, C, U, pitchU, qR, nm,               \
             reinterpret_cast<const int2*>(counts), reinterpret_cast<const unsigned long long*>(keysF), \
             reinterpret_cast<const unsigned long long*>(keysH), reinterpret_cast<const longlong2*>(rowoff), \
             reinterpret_cast<const double2*>(Hh), th, tab, depth, lqF, qF);                           \
     } while (0)
 #define FCD_K2R(F)                                                                                    \
     do {                                                                                              \
-        if (nw == 16) FCD_K2R_(F, 16);                                                                \
-        else if (nw == 12) FCD_K2R_(F, 12);                                                           \
-        else FCD_K2R_(F, 8);                                                                          \
+        if (nw == 16) FCD_K2R_(F, 16, false);                                                         \
+        else if (nw == 12) FCD_K2R_(F, 12, false);                                                    \
+        else FCD_K2R_(F, 8, false);                                                                   \
     } while (0)
-    if (fast) FCD_K2R(true); else FCD_K2R(false);
+    // the masked form is built for the default 16 warps only (the other widths are experiments)
+    if (S0 != nullptr) {
+        if (fast) FCD_K2R_(true, 16, true); else FCD_K2R_(false, 16, true);
+    } else {
+        if (fast) FCD_K2R(true); else FCD_K2R(false);
+    }
 #undef FCD_K2R
 #undef FCD_K2R_
     return check_launch("fcd_estep_qF_coded(rows)");

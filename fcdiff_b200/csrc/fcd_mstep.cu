@@ -320,8 +320,10 @@ control_moments_kernel(const double* __restrict__ S1, const double* __restrict__
 //  v[0] E_lp_F = sum qF log gamma (fit.py:458)   v[1] E_lp_B_g_F (fit.py:472, via S1,S2)
 //  v[2] E_lp_R = sum qR log[1-pi, pi] (fit.py:486)
 //  v[4] E_lq_F = sum qF lqF (fit.py:525)         v[5] E_lq_R = sum qR lqR (fit.py:539)
+// MASKED: S0[c] observed controls of edge c (healthy_term).
+template <bool MASKED>
 __global__ void __launch_bounds__(kRedThreads)
-energy_small_kernel(const double* __restrict__ S1, const double* __restrict__ S2,
+energy_small_kernel(const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S0,
                     const double* __restrict__ lqF, const double* __restrict__ qF, int64_t C,
                     const double* __restrict__ lqR, const double* __restrict__ qR, int64_t NU,
                     const __grid_constant__ ThetaDev th, double elm_value, const SolverState* __restrict__ solved,
@@ -333,13 +335,13 @@ energy_small_kernel(const double* __restrict__ S1, const double* __restrict__ S2
     // finished just before this launch on the same stream (f = -E_lM at the solution; NaN if it has not)
     if (tid == 0) v[3] = solved != nullptr ? (solved->done ? -solved->f : __longlong_as_double(0x7ff8000000000000ll)) : elm_value;
     for (int64_t c = tid; c < C; c += nth) {
-        const double s1 = S1[c], s2 = S2[c];
+        const double s1 = S1[c], s2 = S2[c], s0 = MASKED ? S0[c] : 0.0;
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             const double l = lqF[c * 3 + k];
             const double q = qF[c * 3 + k];
             v[0] = fma(q, th.log_gamma[k], v[0]);
-            v[1] = fma(q, fma(th.hq_a[k], s2, fma(th.hq_b[k], s1, th.hq_c[k])), v[1]);
+            v[1] = fma(q, healthy_term<MASKED>(th, k, s1, s2, s0), v[1]);
             v[4] = fma(q, l, v[4]);
         }
     }
@@ -493,19 +495,43 @@ int fcd_elm_const(const double* L, int64_t C, int32_t U, int64_t pitchU,
     return check_launch("fcd_elm_const");
 }
 
-int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
-                     const double* lqF, const double* qF, int64_t C,
-                     const double* lqR, const double* qR, int32_t N, int32_t U,
-                     const fcd_theta* theta_host, double elm, const void* solver_state,
-                     double* out6, double* ws, void* stream) {
+static int energy_terms_launch(const double* S1, const double* S2, const double* S0, int32_t H,
+                               const double* lqF, const double* qF, int64_t C,
+                               const double* lqR, const double* qR, int32_t N, int32_t U,
+                               const fcd_theta* theta_host, double elm, const void* solver_state,
+                               double* out6, double* ws, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && ws != nullptr && out6 != nullptr, "fcd_energy_terms: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && N >= 2 && H >= 1, "fcd_energy_terms: bad shape");
     const ThetaDev th = make_theta_dev(*theta_host, H);
     const int64_t NU = (int64_t)N * U;
     const int64_t work = C > NU ? C : NU;
-    energy_small_kernel<<<red_grid(work, kRedThreads), kRedThreads, 0, (cudaStream_t)stream>>>(
-        S1, S2, lqF, qF, C, lqR, qR, NU, th, elm, static_cast<const SolverState*>(solver_state), out6, ws);
-    return check_launch("fcd_energy_terms");
+    const SolverState* solved = static_cast<const SolverState*>(solver_state);
+    if (S0 != nullptr)
+        energy_small_kernel<true><<<red_grid(work, kRedThreads), kRedThreads, 0, (cudaStream_t)stream>>>(
+            S1, S2, S0, lqF, qF, C, lqR, qR, NU, th, elm, solved, out6, ws);
+    else
+        energy_small_kernel<false><<<red_grid(work, kRedThreads), kRedThreads, 0, (cudaStream_t)stream>>>(
+            S1, S2, nullptr, lqF, qF, C, lqR, qR, NU, th, elm, solved, out6, ws);
+    return check_launch(S0 != nullptr ? "fcd_energy_terms_masked" : "fcd_energy_terms");
+}
+
+int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
+                     const double* lqF, const double* qF, int64_t C,
+                     const double* lqR, const double* qR, int32_t N, int32_t U,
+                     const fcd_theta* theta_host, double elm, const void* solver_state,
+                     double* out6, double* ws, void* stream) {
+    return energy_terms_launch(S1, S2, nullptr, H, lqF, qF, C, lqR, qR, N, U, theta_host, elm, solver_state, out6, ws,
+                               stream);
+}
+
+int fcd_energy_terms_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                            const double* lqF, const double* qF, int64_t C,
+                            const double* lqR, const double* qR, int32_t N, int32_t U,
+                            const fcd_theta* theta_host, double elm, const void* solver_state,
+                            double* out6, double* ws, void* stream) {
+    FCD_REQUIRE(S0 != nullptr, "fcd_energy_terms_masked: S0 is NULL");
+    return energy_terms_launch(S1, S2, S0, H, lqF, qF, C, lqR, qR, N, U, theta_host, elm, solver_state, out6, ws,
+                               stream);
 }
 
 int fcd_state_moments(const double* S1, const double* S2, int32_t H,

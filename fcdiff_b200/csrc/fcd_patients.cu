@@ -364,6 +364,8 @@ struct ControlConsts {
 
 constexpr int kCtRows = 8;                  // rows whose loads a thread has in flight at once
 
+// MASKED: a NaN entry is not observed and enters like a row past the block's end (weight 0, value 0).
+template <bool MASKED>
 __global__ void __launch_bounds__(kPtThreads)
 control_terms_rows_kernel(const double* __restrict__ X, int64_t C, int S, int64_t pitchS, const double* __restrict__ qF,
                           const __grid_constant__ ControlConsts cc, int64_t nb, int64_t rows, int lanesP,
@@ -385,12 +387,14 @@ control_terms_rows_kernel(const double* __restrict__ X, int64_t C, int S, int64_
         for (int j = 0; j < kCtRows; ++j) x[j] = ldg_stream1(X + (cb + j < c1 ? cb + j : c1 - 1) * pitchS + s);
 #pragma unroll
         for (int j = 0; j < kCtRows; ++j) {
-            const bool in = cb + j < c1;
-            const double* q = qF + (in ? cb + j : c1 - 1) * 3;
+            const bool obs = !MASKED || !isnan(x[j]);
+            const bool in = cb + j < c1 && obs;
+            const double xj = obs ? x[j] : 0.0;
+            const double* q = qF + (cb + j < c1 ? cb + j : c1 - 1) * 3;
             const double g0 = __ldg(q), g1 = __ldg(q + 1), g2 = __ldg(q + 2);   // straight-line code: no branch
             const double f0 = in ? g0 : 0.0, f1 = in ? g1 : 0.0, f2 = in ? g2 : 0.0;
-            const double z0 = (x[j] - cc.mu[0]) * cc.isig[0], z1 = (x[j] - cc.mu[1]) * cc.isig[1],
-                         z2 = (x[j] - cc.mu[2]) * cc.isig[2];
+            const double z0 = (xj - cc.mu[0]) * cc.isig[0], z1 = (xj - cc.mu[1]) * cc.isig[1],
+                         z2 = (xj - cc.mu[2]) * cc.isig[2];
             const double l0 = fma(-0.5 * z0, z0, -cc.nc[0]), l1 = fma(-0.5 * z1, z1, -cc.nc[1]),
                          l2 = fma(-0.5 * z2, z2, -cc.nc[2]);
             acc += fma(f0, l0, fma(f1, l1, f2 * l2));
@@ -493,8 +497,8 @@ int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S) {
     return pt_row_blocks(C) * (int64_t)S * (int64_t)sizeof(double);
 }
 
-int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                      const fcd_theta* theta_host, double* out, double* ws, void* stream) {
+static int control_terms_launch(bool masked, const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                                const fcd_theta* theta_host, double* out, double* ws, void* stream) {
     FCD_REQUIRE(X != nullptr && qF != nullptr && theta_host != nullptr && out != nullptr && ws != nullptr,
                 "fcd_control_terms: NULL argument");
     const int64_t N = (int64_t)((sqrt(8.0 * (double)C + 1.0) + 1.0) * 0.5);
@@ -518,12 +522,27 @@ int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, con
     const int64_t grid = (warps * 32 + kPtThreads - 1) / kPtThreads;
     FCD_REQUIRE(warps < ((int64_t)1 << 26), "fcd_control_terms: %lld subjects are too many for one launch",
                 (long long)S);
-    control_terms_rows_kernel<<<(unsigned)grid, kPtThreads, 0, st>>>(X, C, S, pitchS, qF, cc, nb, rows, lanesP, ws);
+    if (masked)
+        control_terms_rows_kernel<true><<<(unsigned)grid, kPtThreads, 0, st>>>(X, C, S, pitchS, qF, cc, nb, rows, lanesP,
+                                                                               ws);
+    else
+        control_terms_rows_kernel<false><<<(unsigned)grid, kPtThreads, 0, st>>>(X, C, S, pitchS, qF, cc, nb, rows, lanesP,
+                                                                                ws);
     int rc = check_launch("fcd_control_terms(rows)");
     if (rc != 0) return rc;
     connection_finish_kernel<<<(unsigned)((S + 31) / 32), kPtThreads, 0, st>>>(ws, nb, nullptr, C, S,
                                                                               (int)((S + 31) / 32), out, nullptr);
     return check_launch("fcd_control_terms(finish)");
+}
+
+int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                      const fcd_theta* theta_host, double* out, double* ws, void* stream) {
+    return control_terms_launch(false, X, C, S, pitchS, qF, theta_host, out, ws, stream);
+}
+
+int fcd_control_terms_masked(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                             const fcd_theta* theta_host, double* out, double* ws, void* stream) {
+    return control_terms_launch(true, X, C, S, pitchS, qF, theta_host, out, ws, stream);
 }
 
 int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,

@@ -16,26 +16,32 @@
 namespace fcd {
 
 // S1[c] = sum_h X[c][cols[h]], S2[c] = sum_h X[c][cols[h]]^2: one warp per edge row; the row (S doubles,
-// contiguous) is read through L1, the lanes walk the column list.
+// contiguous) is read through L1, the lanes walk the column list.  MASKED: NaN entries are left out and
+// S0[c] counts the observed ones (healthy_stats_kernel).
+template <bool MASKED>
 __global__ void __launch_bounds__(256)
 healthy_stats_cols_kernel(const double* __restrict__ X, int64_t C, int64_t pitchS, const int32_t* __restrict__ cols,
-                          int H, double* __restrict__ S1, double* __restrict__ S2) {
+                          int H, double* __restrict__ S1, double* __restrict__ S2, double* __restrict__ S0) {
     const int lane = threadIdx.x & 31;
     const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t c = warp0; c < C; c += nwarps) {
         const double* row = X + c * pitchS;
-        double s1 = 0.0, s2 = 0.0;
+        double s1 = 0.0, s2 = 0.0, s0 = 0.0;
         for (int h = lane; h < H; h += 32) {
             const double x = __ldg(row + __ldg(cols + h));
+            if (MASKED && isnan(x)) continue;
             s1 += x;
             s2 = fma(x, x, s2);
+            if (MASKED) s0 += 1.0;
         }
         s1 = warp_sum(s1);
         s2 = warp_sum(s2);
+        if (MASKED) s0 = warp_sum(s0);
         if (lane == 0) {
             S1[c] = s1;
             S2[c] = s2;
+            if (MASKED) S0[c] = s0;
         }
     }
 }
@@ -87,8 +93,21 @@ int fcd_healthy_stats_cols(const double* X, int64_t C, int64_t pitchS, const int
     if (C == 0) return 0;
     int64_t grid = (C + 7) / 8;
     if (grid > (int64_t)sm_count() * 16) grid = (int64_t)sm_count() * 16;
-    healthy_stats_cols_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2);
+    healthy_stats_cols_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2,
+                                                                                         nullptr);
     return check_launch("fcd_healthy_stats_cols");
+}
+
+int fcd_healthy_stats_cols_masked(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
+                                  double* S1, double* S2, double* S0, void* stream) {
+    FCD_REQUIRE(X != nullptr && cols != nullptr && S1 != nullptr && S2 != nullptr && S0 != nullptr,
+                "fcd_healthy_stats_cols_masked: NULL argument");
+    FCD_REQUIRE(C >= 0 && H >= 1 && pitchS >= 1, "fcd_healthy_stats_cols_masked: bad shape");
+    if (C == 0) return 0;
+    int64_t grid = (C + 7) / 8;
+    if (grid > (int64_t)sm_count() * 16) grid = (int64_t)sm_count() * 16;
+    healthy_stats_cols_kernel<true><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2, S0);
+    return check_launch("fcd_healthy_stats_cols_masked");
 }
 
 int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, int32_t nplanes, int64_t C,

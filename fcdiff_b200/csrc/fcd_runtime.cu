@@ -119,7 +119,9 @@ ThetaDev make_theta_dev(const fcd_theta& th, int H) {
         const double i2 = 0.5 * d.isig[k] * d.isig[k];
         d.hq_a[k] = -i2;
         d.hq_b[k] = 2.0 * th.mu[k] * i2;
-        d.hq_c[k] = -(double)H * (th.mu[k] * th.mu[k] * i2 + log(th.sigma[k]) + kHalfLog2Pi);
+        const double c1 = th.mu[k] * th.mu[k] * i2 + log(th.sigma[k]) + kHalfLog2Pi;
+        d.hq_c[k] = -(double)H * c1;
+        d.hq_c1[k] = -c1;                                   // H * hq_c1 == hq_c exactly: only the sign moves
     }
     // fcdiff/fit.py:433-444
     d.epsl[0] = 1.0 - th.epsilon;

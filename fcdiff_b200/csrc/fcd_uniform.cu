@@ -131,8 +131,10 @@ row_logsums_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C,
 
 // lqF[c,k] = log gamma_k + healthy_k(S1, S2) + sum_l w_l S[c][k][l] - logsumexp_k   (fit.py:165-174; the
 // theta-free term L sum_l w_l is common to the three states and cancels, as in estep_qF_kernel)
+template <bool MASKED>
 __global__ void __launch_bounds__(256)
-estep_qF_rowsums_kernel(const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S,
+estep_qF_rowsums_kernel(const double* __restrict__ S1, const double* __restrict__ S2, const double* __restrict__ S0,
+                        const double* __restrict__ S,
                         int64_t C, double w0, double w1, double w2, const __grid_constant__ ThetaDev th,
                         double* __restrict__ lqF, double* __restrict__ qF) {
     for (int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; c < C; c += (int64_t)gridDim.x * blockDim.x) {
@@ -140,7 +142,7 @@ estep_qF_rowsums_kernel(const double* __restrict__ S1, const double* __restrict_
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             const double a = fma(w0, S[c * 9 + k * 3], fma(w1, S[c * 9 + k * 3 + 1], w2 * S[c * 9 + k * 3 + 2]));
-            l[k] = th.log_gamma[k] + fma(th.hq_a[k], S2[c], fma(th.hq_b[k], S1[c], th.hq_c[k])) + a;
+            l[k] = th.log_gamma[k] + healthy_term<MASKED>(th, k, S1[c], S2[c], MASKED ? S0[c] : 0.0) + a;
         }
         const double mx = fmax(l[0], fmax(l[1], l[2]));
         const double lse = mx + log(exp(l[0] - mx) + exp(l[1] - mx) + exp(l[2] - mx));
@@ -201,17 +203,34 @@ int fcd_row_logsums(const double* P, int64_t planeStride, int64_t C, int32_t U, 
     return check_launch("fcd_row_logsums");
 }
 
-int fcd_estep_qF_rowsums(const double* S1, const double* S2, int32_t H, const double* S9, int64_t C,
-                         const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+static int estep_qF_rowsums_launch(const double* S1, const double* S2, const double* S0, int32_t H, const double* S9,
+                                   int64_t C, const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF,
+                                   void* stream) {
     FCD_REQUIRE(S1 != nullptr && S2 != nullptr && S9 != nullptr && w3_host != nullptr && theta_host != nullptr &&
                 lqF != nullptr && C >= 0 && H >= 1, "fcd_estep_qF_rowsums: bad argument");
     if (C == 0) return 0;
     const ThetaDev th = make_theta_dev(*theta_host, H);
     int64_t grid = (C + 255) / 256;
     if (grid > (int64_t)sm_count() * 8) grid = (int64_t)sm_count() * 8;
-    estep_qF_rowsums_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(S1, S2, S9, C, w3_host[0], w3_host[1],
-                                                                             w3_host[2], th, lqF, qF);
-    return check_launch("fcd_estep_qF_rowsums");
+    if (S0 != nullptr)
+        estep_qF_rowsums_kernel<true><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(
+            S1, S2, S0, S9, C, w3_host[0], w3_host[1], w3_host[2], th, lqF, qF);
+    else
+        estep_qF_rowsums_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(
+            S1, S2, nullptr, S9, C, w3_host[0], w3_host[1], w3_host[2], th, lqF, qF);
+    return check_launch(S0 != nullptr ? "fcd_estep_qF_rowsums_masked" : "fcd_estep_qF_rowsums");
+}
+
+int fcd_estep_qF_rowsums(const double* S1, const double* S2, int32_t H, const double* S9, int64_t C,
+                         const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+    return estep_qF_rowsums_launch(S1, S2, nullptr, H, S9, C, w3_host, theta_host, lqF, qF, stream);
+}
+
+int fcd_estep_qF_rowsums_masked(const double* S1, const double* S2, const double* S0, int32_t H, const double* S9,
+                                int64_t C, const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF,
+                                void* stream) {
+    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_rowsums_masked: S0 is NULL");
+    return estep_qF_rowsums_launch(S1, S2, S0, H, S9, C, w3_host, theta_host, lqF, qF, stream);
 }
 
 int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const double* w3_host, double* out1, double* ws,

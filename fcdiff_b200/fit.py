@@ -43,6 +43,7 @@ import torch
 from . import _dev, _lib, _opt, util
 
 _LOOKUP = {"reference": 0, "symmetric": 1}
+_MISSING = ("reject", "marginalize")
 
 # what UnsharedRegionFit.score_patients returns
 PatientScores = collections.namedtuple("PatientScores", "lq_R free_energy free_energy_typical sweeps max_change")
@@ -200,6 +201,13 @@ class UnsharedRegionFit(object):
         negative free energy (the usual case: densities > 1) any *decrease* makes the
         ratio negative, so the loop stops at the first decrease after the sign change.
         ``"magnitude"`` divides by ``|e|`` (new knob, not the default).
+    missing : "reject" | "marginalize"
+        What a NaN correlation in ``b``, ``bt`` or a read-out's columns means.  ``"reject"`` (default): an
+        error, as before.  ``"marginalize"``: the entry was not observed (a parcel outside a subject's field
+        of view, a scrubbed or masked entry) and is integrated out of the model: it contributes a density
+        factor of 1 to every term of the free energy, to the E-steps, the (eta, epsilon) objective and the
+        read-outs (DESIGN.md "Missing entries").  +-inf is rejected in both modes.  Not available with
+        ``update_mu_sigma``, edge ``shards`` or user-assigned ``_lp_B_g_F`` / ``_p_Bt_g_Ft`` / ``_lM``.
     """
 
     def __init__(self):
@@ -220,6 +228,7 @@ class UnsharedRegionFit(object):
         #                                    the E-step's edge-major planes (fcd_region_weights_em)
         self.elm_path = "auto"        # K3b form: "streams" (coded plane) | "tiered" | "auto" (coded unless most elements are undecided)
         self.convergence_rule = "reference"
+        self.missing = "reject"       # "marginalize": NaN correlations are unobserved entries, integrated out
         self.theta_solver = "newton"  # (eta, epsilon): device-resident Newton | host-driven SciPy L-BFGS-B
         self.solver_tol = 2e-4        # newton: a step with |dx_i| <= tol * min(x_i, 1 - x_i) is taken without another
         #                               evaluation (leaves a relative error ~ tol^2 = 4e-8 in eta, epsilon)
@@ -325,18 +334,42 @@ class UnsharedRegionFit(object):
     def _device_shard_inputs(self):
         return self.shards is not None and torch.is_tensor(self.b) and self.n_edges is not None
 
+    def _masked(self):
+        """True when NaN correlations are unobserved entries (``missing == "marginalize"``)."""
+        if self.missing not in _MISSING:
+            raise ValueError("missing must be 'reject' or 'marginalize' (got %r)" % (self.missing,))
+        return self.missing == "marginalize"
+
+    def _check_missing_mode(self):
+        """The combinations the masked form does not cover, rejected before any device work: the (mu, sigma)
+        update needs per-state counts of the observed entries, edge shards exchange unmasked planes, and
+        user-assigned caches are taken as they are."""
+        if not self._masked():
+            return
+        if self.update_mu_sigma:
+            raise ValueError("missing='marginalize' cannot be combined with update_mu_sigma")
+        if self.shards is not None:
+            raise ValueError("missing='marginalize' runs on one GPU: the fit has edge shards")
+        if any(n in self._explicit for n in ('_lp_B_g_F', '_p_Bt_g_Ft', '_lM')):
+            raise ValueError("missing='marginalize' cannot be combined with user-assigned _lp_B_g_F / _p_Bt_g_Ft / _lM")
+
     def _ensure_inputs(self):
         """Uploads b / bt (once per distinct array) and builds the healthy
         sufficient statistics.  The reference re-reads ``self.b`` / ``self.bt``
         at every ``_update_lps`` (fit.py:114-115); re-assign the attribute to
         have a changed array picked up."""
+        self._check_missing_mode()
         if self._shared is not None:
             return self._ensure_inputs_shared()
+        masked = self._masked()
         key = (self._input_stamp(self.b), self._input_stamp(self.bt),
-               None if self.shards is None else self.shards.key())
+               None if self.shards is None else self.shards.key(), masked)
         if (self._in is not None and self._in['key'] == key and self._in['src'][0] is self.b
                 and self._in['src'][1] is self.bt):
             return self._in
+        if masked:
+            self._check_finite(self.b, "b", allow_nan=True)
+            self._check_finite(self.bt, "bt", allow_nan=True)
         lib = _lib.load()
         (C, H, U) = self._global_shape()
         if self.shards is None:
@@ -367,6 +400,7 @@ class UnsharedRegionFit(object):
             bt_dev = _dev.empty((Cl, pitchU)) if pitchU == U else _dev.zeros((Cl, pitchU))
             S1 = _dev.empty((Cl,))
             S2 = _dev.empty((Cl,))
+            S0 = _dev.empty((Cl,)) if masked else None
             (cur, side) = (torch.cuda.current_stream(), _dev.side_stream())
             side.wait_stream(cur)
             with torch.cuda.stream(side):
@@ -375,8 +409,7 @@ class UnsharedRegionFit(object):
                 ev_bt.record(side)
                 b_dev.copy_(b_t, non_blocking=b_t.is_pinned())
                 if Cl > 0:
-                    _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2),
-                                                     _dev.stream()), "fcd_healthy_stats")
+                    self._healthy_stats(b_dev, Cl, H, S1, S2, S0)
                 ev_S = torch.cuda.Event()
                 ev_S.record(side)
             cur.wait_event(ev_bt)
@@ -384,19 +417,40 @@ class UnsharedRegionFit(object):
         if ev_S is None:
             S1 = _dev.empty((Cl,))
             S2 = _dev.empty((Cl,))
+            S0 = _dev.empty((Cl,)) if masked else None
             with _dev.timed(self.profile, "K0_healthy_stats"):
-                _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2),
-                                                 _dev.stream()), "fcd_healthy_stats")
+                self._healthy_stats(b_dev, Cl, H, S1, S2, S0)
             del b_dev
         nm = _dev.empty((max(Cl, 1),), torch.int32)
         _lib.check(lib.fcd_edge_table(c0, Cl, _dev.ptr(nm), _dev.stream()), "fcd_edge_table")
         # `src` keeps the source objects alive: identity (`is`) cannot be faked by a recycled id()
         self._in = dict(key=key, src=(self.b, self.bt), C=C, H=H, U=U, c0=c0, Cl=Cl, u0=u0, Ul=Ul, pitchU=pitchU,
-                        bt=bt_dev, S1=S1, S2=S2, nm=nm, cache_key=None, P=None, L=None, PT=None, WT=None,
+                        bt=bt_dev, S1=S1, S2=S2, S0=S0, nm=nm, cache_key=None, P=None, L=None, PT=None, WT=None,
                         ev_S=ev_S, b_dev=(b_dev if ev_S is not None else None))
         self._evals = []
         self._const = None
         return self._in
+
+    @staticmethod
+    def _healthy_entry(inp, name):
+        """(entry point, its name, leading S1 / S2 arguments) of a kernel that reads the healthy statistics: the
+        ``_masked`` form with S0 when missing entries are marginalised."""
+        lib = _lib.load()
+        head = (_dev.ptr(inp['S1']), _dev.ptr(inp['S2']))
+        if inp['S0'] is None:
+            return getattr(lib, name), name, head
+        return getattr(lib, name + "_masked"), name + "_masked", head + (_dev.ptr(inp['S0']),)
+
+    @staticmethod
+    def _healthy_stats(b_dev, Cl, H, S1, S2, S0):
+        """S1, S2 of the controls [Cl][H]; with S0 (missing entries marginalised) over the observed entries only."""
+        lib = _lib.load()
+        if S0 is None:
+            _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2), _dev.stream()),
+                       "fcd_healthy_stats")
+        else:
+            _lib.check(lib.fcd_healthy_stats_masked(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2),
+                                                    _dev.ptr(S0), _dev.stream()), "fcd_healthy_stats_masked")
 
     def set_shared_inputs(self, shared, controls, patients):
         """Replica mode (new; BASELINE.json configs[4]): the fit's inputs are COLUMNS of a correlation
@@ -413,20 +467,29 @@ class UnsharedRegionFit(object):
 
     def _ensure_inputs_shared(self):
         (sp, con, pat) = self._shared
-        key = ("shared", id(sp), id(con), id(pat))
+        key = ("shared", id(sp), id(con), id(pat), self.missing)
         if self._in is not None and self._in['key'] == key:
             return self._in
         if self.shards is not None:
             raise ValueError("shared-plane inputs cannot be combined with edge shards")
+        if sp.missing != self.missing:
+            raise ValueError("the shared planes were built with missing=%r, the fit has missing=%r"
+                             % (sp.missing, self.missing))
         lib = _lib.load()
         (C, H, U) = (int(sp.C), int(con.numel()), int(pat.numel()))
         S1 = _dev.empty((C,))
         S2 = _dev.empty((C,))
+        S0 = _dev.empty((C,)) if self._masked() else None
         with _dev.timed(self.profile, "K0_healthy_stats"):
-            _lib.check(lib.fcd_healthy_stats_cols(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H, _dev.ptr(S1),
-                                                  _dev.ptr(S2), _dev.stream()), "fcd_healthy_stats_cols")
+            if S0 is None:
+                _lib.check(lib.fcd_healthy_stats_cols(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H, _dev.ptr(S1),
+                                                      _dev.ptr(S2), _dev.stream()), "fcd_healthy_stats_cols")
+            else:
+                _lib.check(lib.fcd_healthy_stats_cols_masked(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H,
+                                                             _dev.ptr(S1), _dev.ptr(S2), _dev.ptr(S0), _dev.stream()),
+                           "fcd_healthy_stats_cols_masked")
         self._in = dict(key=key, src=(None, None), C=C, H=H, U=U, c0=0, Cl=C, u0=0, Ul=U, pitchU=_dev.even(U),
-                        bt=None, S1=S1, S2=S2, nm=sp.nm, cache_key=None, P=None, L=None, PT=None, WT=None,
+                        bt=None, S1=S1, S2=S2, S0=S0, nm=sp.nm, cache_key=None, P=None, L=None, PT=None, WT=None,
                         ev_S=None, b_dev=None)
         self._evals = []
         self._const = None
@@ -488,10 +551,11 @@ class UnsharedRegionFit(object):
                 inp['P'] = _dev.empty((3, max(Cl, 1), pitchU))
                 inp['L'] = _dev.empty((max(Cl, 1), pitchU))
             th = self._theta()
+            (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if inp['S0'] is not None
+                          else (lib.fcd_resp_cache, "fcd_resp_cache"))
             with _dev.timed(self.profile, "K0_resp_cache"):
-                _lib.check(lib.fcd_resp_cache(_dev.ptr(inp['bt']), Cl, U, pitchU, ctypes.byref(th),
-                                              _dev.ptr(inp['P']), max(Cl, 1) * pitchU, _dev.ptr(inp['L']),
-                                              _dev.stream()), "fcd_resp_cache")
+                _lib.check(fn(_dev.ptr(inp['bt']), Cl, U, pitchU, ctypes.byref(th), _dev.ptr(inp['P']),
+                              max(Cl, 1) * pitchU, _dev.ptr(inp['L']), _dev.stream()), name)
         inp['Lsum'] = None                          # total of the L plane, formed on first use (code pass)
         inp['PsE'] = None                           # dominant-state plane of the code pass: rebuilt with the planes
         inp['code_verR'] = None
@@ -712,9 +776,10 @@ class UnsharedRegionFit(object):
         U = bt_dev.shape[1]
         lpB, pBt, lM = _dev.empty((C, H, 3)), _dev.empty((C, U, 3)), _dev.empty((C, U, 3, 3))
         th = self._theta()
-        _lib.check(lib.fcd_materialize_lps(_dev.ptr(b_dev), _dev.ptr(bt_dev), C, H, U, ctypes.byref(th),
-                                           _dev.ptr(lpB), _dev.ptr(pBt), _dev.ptr(lM), _dev.stream()),
-                   "fcd_materialize_lps")
+        (fn, name) = ((lib.fcd_materialize_lps_masked, "fcd_materialize_lps_masked") if self._masked()
+                      else (lib.fcd_materialize_lps, "fcd_materialize_lps"))
+        _lib.check(fn(_dev.ptr(b_dev), _dev.ptr(bt_dev), C, H, U, ctypes.byref(th), _dev.ptr(lpB), _dev.ptr(pBt),
+                      _dev.ptr(lM), _dev.stream()), name)
         self._mat = {'_lp_B_g_F': _dev.download(lpB), '_p_Bt_g_Ft': _dev.download(pBt),
                      '_lM': _dev.download(lM)}
         return self._mat
@@ -733,6 +798,7 @@ class UnsharedRegionFit(object):
             msg = "Model has not been initialized."
             raise ValueError(msg)
         N = int(N)
+        self._check_missing_mode()
 
         self._init_lps(N, H, U)
         self._update_lps()
@@ -828,6 +894,7 @@ class UnsharedRegionFit(object):
         return ((e - e_star) / e) < self.rel_tol
 
     def _arrays_mode(self, *names):
+        self._check_missing_mode()
         return any(n in self._explicit for n in names) or self._lps_state != 'derived'
 
     def _eval_energy(self):
@@ -890,12 +957,13 @@ class UnsharedRegionFit(object):
         self._wait_healthy(inp)
         # the global E_lM is known: rank 0 contributes it, the others zero
         first = self.shards is None or self.shards.rank == 0
+        (fn, name, s12) = self._healthy_entry(inp, "fcd_energy_terms")
         with _dev.timed(self.profile, "K4_energy_small"):
-            _lib.check(lib.fcd_energy_terms(
-                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), Cl,
+            _lib.check(fn(
+                *s12, H, _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), Cl,
                 _dev.ptr(lqR), _dev.ptr(qR), N, U, ctypes.byref(th), float(elm) if first else 0.0,
                 solver_state if first else None,
-                _dev.ptr(res.dev), _dev.ptr(_dev.workspace()), _dev.stream()), "fcd_energy_terms")
+                _dev.ptr(res.dev), _dev.ptr(_dev.workspace()), _dev.stream()), name)
         if self.shards is not None:
             h = self.shards.reduce_begin(res)
             return ("shards", h, res)
@@ -1038,28 +1106,30 @@ class UnsharedRegionFit(object):
         if uni is not None:
             # q_R is the constant start: the row sums (shared with the initial free energy) give lq_F directly
             (S9, w3, _) = uni
+            (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_rowsums")
             with _dev.timed(self.profile, "K2_estep_qF_rowsums"):
-                _lib.check(lib.fcd_estep_qF_rowsums(_dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(S9), Cl, w3,
-                                                    ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]),
-                                                    _dev.stream()), "fcd_estep_qF_rowsums")
+                _lib.check(fn(*s12, H, _dev.ptr(S9), Cl, w3, ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]),
+                              _dev.ptr(qF[c0 * 3:]), _dev.stream()), name)
             self._set_lq_F_dev(lqF_buf, qF_buf, C)
             return
         if self.coded_estep and Cl > 0 and inp.get('code_verR') == self._mR.version and inp.get('PsE') is not None:
             # the code plane and key lists of the last M-step still describe q_R (fcd_estep_qF_coded)
+            (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_coded")
             with _dev.timed(self.profile, "K2_estep_qF_coded"):
-                _lib.check(lib.fcd_estep_qF_coded(
-                    _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
+                _lib.check(fn(
+                    *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
                     Cl, U, inp['pitchU'], _dev.ptr(qR), N, _dev.ptr(inp['nm']), _dev.ptr(inp['code']), inp['pitchQ'],
                     _dev.ptr(inp['bk_counts']), _dev.ptr(inp['bk_K']), _dev.ptr(inp['bk_KH']), _dev.ptr(inp['bk_rowoff']),
                     _dev.ptr(inp['bk_H']), ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()),
-                    "fcd_estep_qF_coded")
+                    name)
             self._set_lq_F_dev(lqF_buf, qF_buf, C)
             return
+        (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF")
         with _dev.timed(self.profile, "K2_estep_qF"):
-            _lib.check(lib.fcd_estep_qF(
-                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
+            _lib.check(fn(
+                *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
                 Cl, U, inp['pitchU'], _dev.ptr(qR), _dev.ptr(rstate), rstate.shape[1], N, _dev.ptr(inp['nm']),
-                ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()), "fcd_estep_qF")
+                ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()), name)
         self._set_lq_F_dev(lqF_buf, qF_buf, C)
 
     def _set_lq_F_dev(self, lqF_buf, qF_buf, C):
@@ -1098,13 +1168,14 @@ class UnsharedRegionFit(object):
         (lqF_buf, qF_buf) = (_dev.empty((nbuf,)), _dev.empty((nbuf,)))
         th = self._theta()
         self._wait_healthy(inp)
+        (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_coded_solved")
         with _dev.timed(self.profile, "K2_estep_qF_coded"):
-            _lib.check(lib.fcd_estep_qF_coded_solved(
-                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
+            _lib.check(fn(
+                *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
                 Cl, U, inp['pitchU'], _dev.ptr(qR), N, _dev.ptr(inp['nm']), _dev.ptr(inp['code']), inp['pitchQ'],
                 _dev.ptr(inp['bk_counts']), _dev.ptr(inp['bk_K']), _dev.ptr(inp['bk_KH']), _dev.ptr(inp['bk_rowoff']),
                 _dev.ptr(inp['bk_H']), ctypes.byref(th), solver_state, float(lo_e), float(hi_e),
-                _dev.ptr(lqF_buf[c0 * 3:]), _dev.ptr(qF_buf[c0 * 3:]), _dev.stream()), "fcd_estep_qF_coded_solved")
+                _dev.ptr(lqF_buf[c0 * 3:]), _dev.ptr(qF_buf[c0 * 3:]), _dev.stream()), name)
         self.spec_stats[0] += 1
         return dict(bufs=(lqF_buf, qF_buf), inp=inp, cache_key=inp['cache_key'], verR=self._mR.version, qR=qR,
                     dims=self._dims, rest=(tuple(th.gamma), tuple(th.mu), tuple(th.sigma)), x=None)
@@ -1261,6 +1332,8 @@ class UnsharedRegionFit(object):
         """`score_patients` up to the per-patient sums: (lq_R, (U', 4) {E_lM, E_lp_R, E_lq_R,
         sum_c sum_k q_F log M_k0}, sweeps, max_change)."""
         (C, N, U, lq_R0, max_sweeps) = self._check_score_args("score_patients", bt_new, lq_R0, max_sweeps)
+        if self._masked():
+            self._check_finite(bt_new, "bt_new", allow_nan=True)
         return self._score_columns(bt_new, C, N, U, lq_R0, max_sweeps, tol)
 
     def _check_score_args(self, what, bt_new, lq_R0, max_sweeps):
@@ -1333,6 +1406,7 @@ class UnsharedRegionFit(object):
             raise ValueError("The fit has no q_F (run() the fit or assign _lq_F first).")
         if self.shards is not None:
             raise ValueError("%s runs on one GPU: the fit has edge shards." % what)
+        self._masked()                                   # a valid `missing`
         if any(name in self._explicit for name in explicit):
             raise ValueError("%s needs the fused form: the fit holds user-assigned %s." % (what, " / ".join(explicit)))
         C = int(shF[0])
@@ -1352,12 +1426,16 @@ class UnsharedRegionFit(object):
         return U
 
     @staticmethod
-    def _check_finite(x, name):
+    def _check_finite(x, name, allow_nan=False):
         """Correlations enter the read-outs unvalidated otherwise: a NaN or inf would make every sum it enters
-        non-finite.  One device reduction for a CUDA tensor."""
-        ok = bool(torch.isfinite(x).all()) if torch.is_tensor(x) else bool(np.isfinite(np.asarray(x)).all())
+        non-finite.  ``allow_nan``: NaN marks an unobserved entry (``missing == "marginalize"``); +-inf is
+        still rejected.  One device reduction for a CUDA tensor."""
+        if allow_nan:
+            ok = not (bool(torch.isinf(x).any()) if torch.is_tensor(x) else bool(np.isinf(np.asarray(x)).any()))
+        else:
+            ok = bool(torch.isfinite(x).all()) if torch.is_tensor(x) else bool(np.isfinite(np.asarray(x)).all())
         if not ok:
-            raise ValueError("%s must hold finite correlations" % name)
+            raise ValueError("%s must hold finite correlations%s" % (name, " or NaN" if allow_nan else ""))
 
     @staticmethod
     def _columns_on_device(src, C, U, pitchU):
@@ -1378,9 +1456,11 @@ class UnsharedRegionFit(object):
         lib = _lib.load()
         bt = self._columns_on_device(bt_src, C, U, pitchU)
         PL = _dev.empty((4 if with_L else 3, C, pitchU))
+        (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if self._masked()
+                      else (lib.fcd_resp_cache, "fcd_resp_cache"))
         with _dev.timed(self.profile, "P0_resp_cache"):
-            _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
-                                          _dev.ptr(PL[3] if with_L else None), _dev.stream()), "fcd_resp_cache")
+            _lib.check(fn(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
+                          _dev.ptr(PL[3] if with_L else None), _dev.stream()), name)
         return PL
 
     def connection_posteriors(self, bt_new=None, lq_R=None, maps=True):
@@ -1439,6 +1519,8 @@ class UnsharedRegionFit(object):
                 bt_src = inp['bt'] if inp is not None else self.bt
         else:
             U = self._check_bt_new(bt_new, C)
+            if self._masked():
+                self._check_finite(bt_new, "bt_new", allow_nan=True)
             lq = np.ascontiguousarray(lq_R.cpu().numpy() if torch.is_tensor(lq_R) else lq_R, dtype=np.float64)
             if lq.shape != (N, U, 2):
                 raise ValueError("lq_R must be (N, U', 2) = %s (got %s)" % ((N, U, 2), lq.shape))
@@ -1492,7 +1574,7 @@ class UnsharedRegionFit(object):
             else:
                 raise ValueError("The fit has no controls (assign b or pass b_new).")
         S = self._check_bt_new(src, C, "b_new")
-        self._check_finite(src, "b_new")
+        self._check_finite(src, "b_new", allow_nan=self._masked())
         pitchS = _dev.even(S)
         return self._control_terms(self._columns_on_device(src, C, S, pitchS), C, S, pitchS)
 
@@ -1503,9 +1585,11 @@ class UnsharedRegionFit(object):
         (_, qF) = self._mF.get_dev()
         out = _dev.empty((S,))
         ws = _dev.empty((max(int(lib.fcd_control_terms_ws_bytes(C, S)) // 8, 1),))
+        (fn, name) = ((lib.fcd_control_terms_masked, "fcd_control_terms_masked") if self._masked()
+                      else (lib.fcd_control_terms, "fcd_control_terms"))
         with _dev.timed(self.profile, "P4_control_terms"):
-            _lib.check(lib.fcd_control_terms(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th),
-                                             _dev.ptr(out), _dev.ptr(ws), _dev.stream()), "fcd_control_terms")
+            _lib.check(fn(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th), _dev.ptr(out), _dev.ptr(ws),
+                          _dev.stream()), name)
         return _dev.download(out)
 
     def classify_subjects(self, x_new, prior_patient=None, lq_R0=None, max_sweeps=50, tol=1e-9):
@@ -1545,7 +1629,7 @@ class UnsharedRegionFit(object):
             rho = float(prior_patient)
         if not 0.0 < rho < 1.0:
             raise ValueError("prior_patient must lie in (0, 1) (got %r)" % rho)
-        self._check_finite(x_new, "x_new")
+        self._check_finite(x_new, "x_new", allow_nan=self._masked())
         pitchS = _dev.even(S)
         X = self._columns_on_device(x_new, C, S, pitchS)
         ps = self._patient_scores(*self._score_columns(X, C, N, S, lq_R0, max_sweeps, tol))
@@ -1659,6 +1743,8 @@ class UnsharedRegionFit(object):
         lib = _lib.load()
         if self._shared is not None:
             raise ValueError("update_mu_sigma is not available with shared-plane inputs (the planes are fixed)")
+        if self._masked():
+            raise ValueError("update_mu_sigma is not available with missing='marginalize'")
         if self._lps_state != 'derived':
             self._update_lps()
         inp = self._ensure_cache()

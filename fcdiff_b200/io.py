@@ -61,10 +61,12 @@ def load_timeseries(paths, time_major=False):
     return np.stack(subjects, axis=0)
 
 
-def correlations_from_files(control_paths, patient_paths, fisher=True, time_major=False):
+def correlations_from_files(control_paths, patient_paths, fisher=True, time_major=False, missing=False):
     """(b, bt): (C, H) and (C, U) float64 correlation matrices of the control and
-    the patient group, ready for ``UnsharedRegionFit.b`` / ``.bt``."""
+    the patient group, ready for ``UnsharedRegionFit.b`` / ``.bt``.  ``missing``:
+    regions without a usable time series in a subject give NaN connections
+    (``corr.correlations``), for a fit with ``missing="marginalize"``."""
     ts = load_timeseries(list(control_paths) + list(patient_paths), time_major)
-    c = corr.correlations(ts, fisher=fisher)
+    c = corr.correlations(ts, fisher=fisher, missing=missing)
     H = len(control_paths)
     return np.ascontiguousarray(c[:, :H]), np.ascontiguousarray(c[:, H:])

@@ -30,9 +30,12 @@ class SharedPlanes(object):
     PL [4][C][pitchS]    p_0, p_1, p_2, L of every (edge, subject)      (fcd_resp_cache)
     PT [3][S][pitchC]    p_k patient-major                              (fcd_transpose_patients)
     nm [C]               edge table
+
+    ``missing``: the ``UnsharedRegionFit.missing`` of the fits that use the planes; with ``"marginalize"`` a NaN
+    correlation is an unobserved entry (fcd_resp_cache_masked) and +-inf is rejected.
     """
 
-    def __init__(self, corr, model):
+    def __init__(self, corr, model, missing="reject"):
         import ctypes
         from . import _lib
         from .util import C_to_N
@@ -43,6 +46,11 @@ class SharedPlanes(object):
         (C, S) = (int(x.shape[0]), int(x.shape[1]))
         if (C_to_N(C) % 1) != 0:
             raise ValueError("Number of connections (%u) must be a triangular number." % C)
+        if missing not in ("reject", "marginalize"):
+            raise ValueError("missing must be 'reject' or 'marginalize' (got %r)" % (missing,))
+        if missing == "marginalize" and bool(torch.isinf(x).any()):
+            raise ValueError("corr must hold finite correlations or NaN")
+        self.missing = missing
         (self.C, self.S, self.pitchS, self.pitchC) = (C, S, _dev.even(S), _dev.even(C))
         if self.pitchS == S:
             self.X = x.contiguous()
@@ -53,8 +61,10 @@ class SharedPlanes(object):
                              np.asarray(model.gamma).reshape(-1), model.mu, model.sigma)
         self.cache_key = (tuple(float(v) for v in model.mu), tuple(float(v) for v in model.sigma))
         self.PL = _dev.empty((4, C, self.pitchS))
-        _lib.check(lib.fcd_resp_cache(_dev.ptr(self.X), C, S, self.pitchS, ctypes.byref(th), _dev.ptr(self.PL),
-                                      C * self.pitchS, _dev.ptr(self.PL[3]), _dev.stream()), "fcd_resp_cache")
+        (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if missing == "marginalize"
+                      else (lib.fcd_resp_cache, "fcd_resp_cache"))
+        _lib.check(fn(_dev.ptr(self.X), C, S, self.pitchS, ctypes.byref(th), _dev.ptr(self.PL), C * self.pitchS,
+                      _dev.ptr(self.PL[3]), _dev.stream()), name)
         self.PT = _dev.zeros((3, S, self.pitchC))
         for k in range(3):
             _lib.check(lib.fcd_transpose_patients(_dev.ptr(self.PL[k]), C, S, self.pitchS, 0, S, _dev.ptr(self.PT[k]),
@@ -177,7 +187,7 @@ def permutation_sweep(corr, labels, n_permutations, model=None, seed=0, fit_opti
         reference's defaults, fcdiff/model.py:31-38).
     fit_options : dict
         Attributes set on every ``UnsharedRegionFit`` (``max_iters``, ``rel_tol``,
-        ``edge_lookup``, ...).
+        ``edge_lookup``, ``missing``, ...).
     rank, world, group
         Replica sharding (see the module docstring); ``gather`` merges the
         results of all ranks.
@@ -203,7 +213,7 @@ def permutation_sweep(corr, labels, n_permutations, model=None, seed=0, fit_opti
     model = UnsharedRegionModel() if model is None else model
     shared = None
     if shared_planes and not (fit_options or {}).get("update_mu_sigma"):
-        shared = SharedPlanes(corr_dev, model)
+        shared = SharedPlanes(corr_dev, model, missing=(fit_options or {}).get("missing", "reject"))
     def run_one(i):
         pat = torch.from_numpy(np.flatnonzero(lab[i])).to(dev)
         con = torch.from_numpy(np.flatnonzero(~lab[i])).to(dev)
@@ -282,7 +292,7 @@ def cross_validate(corr, labels, n_folds=5, model=None, seed=0, fit_options=None
     model = UnsharedRegionModel() if model is None else model
     shared = None
     if not (fit_options or {}).get("update_mu_sigma"):
-        shared = SharedPlanes(corr_dev, model)
+        shared = SharedPlanes(corr_dev, model, missing=(fit_options or {}).get("missing", "reject"))
 
     def run_one(i):
         train = fold != i

@@ -127,6 +127,12 @@ FCD_API int fcd_c_to_nm(int64_t c0, int64_t C, int32_t* n_out, int32_t* m_out, v
  * healthy log-density sum of fit.py:171 is a quadratic in (S1, S2). */
 FCD_API int fcd_healthy_stats(const double* b, int64_t C, int32_t H, int64_t pitchH,
                       double* S1, double* S2, void* stream);
+/* Missing entries (fit.missing = "marginalize"): a NaN b[c,h] is not observed and is left out of S1, S2;
+ * S0[c] = H_c, the number of observed controls of edge c (a double).  The healthy sum of fit.py:171 over the
+ * observed entries is hq_a S2 + hq_b S1 + H_c hq_c1: the constant scales with H_c, so it cannot be folded into
+ * S1, S2.  With no NaN, S1 and S2 have the bits of fcd_healthy_stats and S0 = H. */
+FCD_API int fcd_healthy_stats_masked(const double* b, int64_t C, int32_t H, int64_t pitchH,
+                      double* S1, double* S2, double* S0, void* stream);
 
 /* Edge table of the local shard: nm[i] = n | m << 16 for the edge c0 + i
  * (fcdiff/util.py:62-84 c_to_nm; at most 65535 regions).  Built once per fit. */
@@ -141,6 +147,12 @@ FCD_API int fcd_edge_table(int64_t c0, int64_t C, int32_t* nm, void* stream);
  *   log M_kl = L + log(a_l + b_l p_k),  a_l = (1 - eps_l)/2,  b_l = eps_l - a_l,
  * exactly and without underflow; the kernels below read these planes, not bt. */
 FCD_API int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream);
+/* fcd_resp_cache for patient correlations with missing entries: a NaN bt[c,u] is not observed and is stored
+ * as p_0 = p_1 = p_2 = 1/3, L = log 3.  Then a_l + b_l / 3 = 1/3 for every l and theta, log M_kl = 0 for all
+ * (k, l) (fit.py:117-122): the element's density factor is 1 in every kernel that reads the planes.  Finite
+ * entries get the bits of fcd_resp_cache. */
+FCD_API int fcd_resp_cache_masked(const double* bt, int64_t C, int32_t U, int64_t pitchU,
                    const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream);
 
 /* Peak states of the posteriors (tier selection, DESIGN.md "Tiers"):
@@ -169,6 +181,11 @@ FCD_API int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
                  const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                  const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
                  const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
+/* fcd_estep_qF with S0 of fcd_healthy_stats_masked: the healthy sum of fit.py:171 over the observed controls. */
+FCD_API int fcd_estep_qF_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
+                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
 
 /* The same E-step driven by the code pass of the previous M-step (fcd_code_plane / fcd_code_records:
  * valid while q_R has not changed since): the coded elements need no peak-state decoding and no
@@ -178,6 +195,13 @@ FCD_API int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
  * the code pass for the same local rows; rows whose edge was unpeaked then (counts[c][0] == 3 U)
  * are evaluated in full. */
 FCD_API int fcd_estep_qF_coded(const double* S1, const double* S2, int32_t H,
+                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                       const double* qR, int32_t N, const int32_t* nm,
+                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
+                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
+                       const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
+/* fcd_estep_qF_coded with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
+FCD_API int fcd_estep_qF_coded_masked(const double* S1, const double* S2, const double* S0, int32_t H,
                        const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                        const double* qR, int32_t N, const int32_t* nm,
                        const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
@@ -198,6 +222,14 @@ FCD_API int fcd_estep_qF_coded_solved(const double* S1, const double* S2, int32_
                        const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
                        const fcd_theta* theta_host, const void* solver_state, double eps_lo, double eps_hi,
                        double* lqF, double* qF, void* stream);
+/* fcd_estep_qF_coded_solved with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
+FCD_API int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                       const double* qR, int32_t N, const int32_t* nm,
+                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
+                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
+                       const fcd_theta* theta_host, const void* solver_state, double eps_lo, double eps_hi,
+                       double* lqF, double* qF, void* stream);
 
 /* The uniform start (fcdiff/fit.py:84-102: lq_R = -ln 2, lq_F = -ln 3 everywhere).  With a CONSTANT q_R every
  * element has the same pair weights w (fit.py:382-406), and the sums of fit.py:165-173 / 489-511 factor through
@@ -211,6 +243,10 @@ FCD_API int fcd_row_logsums(const double* P, int64_t planeStride, int64_t C, int
                     const fcd_theta* theta_host, double* S9, void* stream);
 FCD_API int fcd_estep_qF_rowsums(const double* S1, const double* S2, int32_t H, const double* S9, int64_t C,
                          const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
+/* fcd_estep_qF_rowsums with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
+FCD_API int fcd_estep_qF_rowsums_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                         const double* S9, int64_t C, const double* w3_host, const fcd_theta* theta_host,
+                         double* lqF, double* qF, void* stream);
 FCD_API int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const double* w3_host, double* out1,
                     double* ws, void* stream);
 
@@ -224,6 +260,9 @@ FCD_API int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const
  * cols / rows: int32 device arrays. */
 FCD_API int fcd_healthy_stats_cols(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
                            double* S1, double* S2, void* stream);
+/* fcd_healthy_stats_cols over the observed (non-NaN) entries, with S0 as fcd_healthy_stats_masked. */
+FCD_API int fcd_healthy_stats_cols_masked(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
+                           double* S1, double* S2, double* S0, void* stream);
 FCD_API int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, int32_t nplanes, int64_t C,
                        const int32_t* cols, int32_t U, double* dst, int64_t planeStrideD, int64_t pitchD,
                        void* stream);
@@ -435,6 +474,13 @@ FCD_API int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
                      const double* lqR, const double* qR, int32_t N, int32_t U,
                      const fcd_theta* theta_host, double elm, const void* solver_state,
                      double* out6, double* ws, void* stream);
+/* fcd_energy_terms with S0 of fcd_healthy_stats_masked: E_lp_B_g_F (fit.py:461-472) over the observed
+ * controls. */
+FCD_API int fcd_energy_terms_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+                     const double* lqF, const double* qF, int64_t C,
+                     const double* lqR, const double* qR, int32_t N, int32_t U,
+                     const fcd_theta* theta_host, double elm, const void* solver_state,
+                     double* out6, double* ws, void* stream);
 
 /* Held-out scoring (csrc/fcd_patients.cu): with theta and q_F of a fitted model fixed, the free energy
  * (fcdiff/fit.py:142-155) is a sum over patient columns u; these entries keep the sums of `_eval_E_lp_R`,
@@ -485,6 +531,10 @@ FCD_API int fcd_connection_posteriors(const double* P, int64_t planeStride, int6
 FCD_API int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S);
 FCD_API int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
                               const fcd_theta* theta_host, double* out, double* ws, void* stream);
+/* fcd_control_terms over the observed entries: a NaN X[c][s] adds nothing (fit.py:461-472 with the
+ * entry marginalised), so that a subject's l_C and its patient free energy cover the same entries. */
+FCD_API int fcd_control_terms_masked(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                              const fcd_theta* theta_host, double* out, double* ws, void* stream);
 
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
@@ -508,6 +558,12 @@ FCD_API int fcd_state_moments(const double* S1, const double* S2, int32_t H,
 /* `_update_lps` (fcdiff/fit.py:104-122): lpB [C][H][3], pBt [C][U][3],
  * lM [C][U][3][3] (k major, l minor), scipy.stats.norm op order. */
 FCD_API int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
+                        const fcd_theta* theta_host,
+                        double* lpB, double* pBt, double* lM, void* stream);
+/* The same caches of a fit with missing entries (fcdiff/fit.py:104-122 with NaN marginalised): a NaN b[c,h]
+ * gives lpB[c][h][:] = 0, a NaN bt[c,u] gives pBt[c][u][:] = 1 and lM[c][u][:][:] = 0 (M_kl = eps_l +
+ * (1 - eps_l) = 1, fit.py:427-430). */
+FCD_API int fcd_materialize_lps_masked(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
                         const fcd_theta* theta_host,
                         double* lpB, double* pBt, double* lM, void* stream);
 
@@ -586,6 +642,12 @@ FCD_API int64_t fcd_corr_workspace_bytes(int32_t S, int32_t N, int32_t T);
 FCD_API int fcd_corr_fisherz(const float* ts, int32_t S, int32_t N, int32_t T,
                      double* out, int64_t pitch, int32_t s0, int32_t fisher,
                      void* zws, void* stream);
+/* After fcd_corr_fisherz on the same ts / out / pitch / s0: a (subject, region) row with a non-finite
+ * sample or of zero variance (the test the standardisation applies) has no usable time series; NaN (not
+ * observed, fit.missing = "marginalize") is written to all N - 1 edges of that region in column s0 + s.
+ * Every other entry is left as it is. */
+FCD_API int fcd_corr_mark_missing(const float* ts, int32_t S, int32_t N, int32_t T,
+                     double* out, int64_t pitch, int32_t s0, void* stream);
 
 #ifdef __cplusplus
 }
