@@ -142,7 +142,16 @@ def test_joint_sample_matches_oracle_sampler_in_distribution():
                                    # tensor-core path: odd subject counts (a lone subject in the last pair), tail
                                    # blocks of 2 / 16 / 72 rows (transposed tiles, UMMA N = 16 / 16 / 80), no tail,
                                    # more work items than SMs (persistent CTAs, both TMEM buffers reused)
-                                   (5, 130, 64), (3, 272, 96), (7, 200, 128), (1, 256, 64), (61, 300, 40)])
+                                   (5, 130, 64), (3, 272, 96), (7, 200, 128), (1, 256, 64), (61, 300, 40),
+                                   # the last SIMT size and the first tensor-core one (a single 64-row tile)
+                                   (3, 63, 64), (3, 64, 64),
+                                   # tail 112 (the widest transposed tile, UMMA N = 112), tail 113 (a full
+                                   # 128-wide tile with masked rows), tail 127, no tail with three tiles
+                                   (3, 240, 96), (3, 241, 96), (3, 255, 64), (3, 384, 64),
+                                   # Schaefer-1000: eight tiles, tail 104
+                                   (2, 1000, 96),
+                                   # T around kKChunk = 32: one K chunk with 1 / 0 padded columns, two chunks
+                                   (3, 130, 31), (3, 130, 32), (3, 130, 33), (3, 40, 33)])
 @pytest.mark.parametrize("fisher", [True, False])
 def test_corr_fisherz_vs_numpy(S, N, T, fisher):
     rng = np.random.RandomState(S * 1000 + N)
