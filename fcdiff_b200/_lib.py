@@ -150,6 +150,9 @@ SIGNATURES = {
     "fcd_corr_workspace_bytes": (c_int64, [c_int32, c_int32, c_int32]),
     "fcd_corr_fisherz": (c_int, [_P, c_int32, c_int32, c_int32, _P, c_int64, c_int32, c_int32, _P, _P]),
     "fcd_corr_mark_missing": (c_int, [_P, c_int32, c_int32, c_int32, _P, c_int64, c_int32, _P]),
+    "fcd_corr_clean_workspace_bytes": (c_int64, [c_int32, c_int32, c_int32, c_int32]),
+    "fcd_corr_fisherz_clean": (c_int, [_P, c_int32, c_int32, c_int32, _P, _P, c_int32, _P, c_int64, c_int32, c_int32,
+                                       c_int32, _P, _P, _P]),
 }
 
 class SolverState(ctypes.Structure):

@@ -19,27 +19,41 @@ namespace fcd {
 
 // One warp per (subject, region) row.  SPLIT: write the TF32 hi / lo parts
 // (both exactly representable in TF32) for the tensor-core path.
-template <bool SPLIT>
+// MASK (fcd_corr_fisherz_clean without confounds): only the frames t with keep[s][t] != 0 (every frame
+// when keep is NULL) are read; the others are written as zeros.  The sums are those of the unmasked form
+// in the same order, divided by the number of kept frames, so an all-kept mask gives the same bits.  A
+// row with a non-finite kept sample or of zero variance is written as zeros, and status[r] = 1 marks it.
+template <bool SPLIT, bool MASK = false>
 __global__ void __launch_bounds__(256)
 standardise_kernel(const float* __restrict__ ts, int64_t rows, int T, int Tp, float* __restrict__ Z,
-                   float* __restrict__ Zlo) {
+                   float* __restrict__ Zlo, const uint8_t* __restrict__ keep = nullptr, int N = 0,
+                   uint8_t* __restrict__ status = nullptr) {
     const int lane = threadIdx.x & 31;
     const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t r = warp0; r < rows; r += nwarps) {
         const float* x = ts + r * T;
+        const uint8_t* kp = MASK && keep != nullptr ? keep + (r / N) * T : nullptr;
         double s = 0.0;
-        for (int t = lane; t < T; t += 32) s += (double)x[t];
-        const double mean = warp_sum(s) / (double)T;
+        int cnt = 0;
+        for (int t = lane; t < T; t += 32) {
+            if (MASK && kp != nullptr && !kp[t]) continue;
+            s += (double)x[t];
+            if (MASK) ++cnt;
+        }
+        const double mean = warp_sum(s) / (double)(MASK ? __reduce_add_sync(0xffffffffu, cnt) : T);
         double ss = 0.0;
         for (int t = lane; t < T; t += 32) {
+            if (MASK && kp != nullptr && !kp[t]) continue;
             const double d = (double)x[t] - mean;
             ss = fma(d, d, ss);
         }
         ss = warp_sum(ss);
         const double inv = ss > 0.0 ? rsqrt(ss) : 0.0;
+        if (MASK && lane == 0) status[r] = ss > 0.0 ? 0 : 1;
         for (int t = lane; t < Tp; t += 32) {
-            const float z = t < T ? (float)(((double)x[t] - mean) * inv) : 0.0f;
+            const bool use = t < T && (!MASK || (ss > 0.0 && (kp == nullptr || kp[t])));
+            const float z = use ? (float)(((double)x[t] - mean) * inv) : 0.0f;
             if (SPLIT) {
                 uint32_t hb, lb;
                 asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(z));
@@ -134,6 +148,58 @@ mark_missing_kernel(const float* __restrict__ ts, int S, int N, int T, double* _
     }
 }
 
+// Rows flagged by the cleaning stage (status[s][n] != 0): NaN on their N - 1 edges of column s0 + s, one
+// warp per row; every other entry is left as it is.
+__global__ void __launch_bounds__(256)
+mark_status_kernel(const uint8_t* __restrict__ status, int S, int N, double* __restrict__ out, int64_t pitch,
+                   int s0) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp0 = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int64_t rows = (int64_t)S * N;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    for (int64_t r = warp0; r < rows; r += nwarps) {
+        if (!status[r]) continue;
+        const int subj = (int)(r / N), n = (int)(r - (int64_t)subj * N);
+        for (int m = lane; m < N; m += 32) {
+            if (m == n) continue;
+            const int64_t c = n > m ? (int64_t)n * (n - 1) / 2 + m : (int64_t)m * (m - 1) / 2 + n;
+            out[c * pitch + s0 + subj] = nan;
+        }
+    }
+}
+
+static int row_grid(int64_t rows) {
+    const int64_t g = (rows + 7) / 8;
+    const int64_t cap = (int64_t)sm_count() * 8;
+    return (int)(g < cap ? g : cap);
+}
+
+bool corr_use_tc(int N) { return corr_tc_supported(N) && getenv("FCD_CORR_SIMT") == nullptr; }
+
+int corr_gram(bool tc, const float* Z, const float* Zlo, int S, int N, int Tp, double* out, int64_t pitch, int s0,
+              int fisher, cudaStream_t st) {
+    if (tc) return corr_gram_tc(Z, Zlo, S, N, Tp, out, pitch, s0, fisher, st);
+    FCD_REQUIRE(S <= 65535, "fcd_corr_fisherz: S=%d too large for the SIMT Gram kernel", S);
+    const int nt = (N + 31) / 32;
+    dim3 grid((unsigned)(nt * (nt + 1) / 2), (unsigned)S);
+    gram_simt_kernel<<<grid, 256, 0, st>>>(Z, N, Tp, nt, out, pitch, s0, fisher);
+    return check_launch("fcd_corr_fisherz(gram_simt)");
+}
+
+int corr_standardise_masked(bool tc, const float* ts, const uint8_t* keep, int S, int N, int T, int Tp, float* Z,
+                            float* Zlo, uint8_t* status, cudaStream_t st) {
+    const int64_t rows = (int64_t)S * N;
+    if (tc) standardise_kernel<true, true><<<row_grid(rows), 256, 0, st>>>(ts, rows, T, Tp, Z, Zlo, keep, N, status);
+    else standardise_kernel<false, true><<<row_grid(rows), 256, 0, st>>>(ts, rows, T, Tp, Z, nullptr, keep, N, status);
+    return check_launch("fcd_corr_fisherz_clean(standardise)");
+}
+
+int corr_mark_status(const uint8_t* status, int S, int N, double* out, int64_t pitch, int s0, cudaStream_t st) {
+    mark_status_kernel<<<row_grid((int64_t)S * N), 256, 0, st>>>(status, S, N, out, pitch, s0);
+    return check_launch("fcd_corr_fisherz_clean(mark)");
+}
+
 }  // namespace fcd
 
 using namespace fcd;
@@ -167,12 +233,7 @@ int fcd_corr_fisherz(const float* ts, int32_t S, int32_t N, int32_t T,
     else standardise_kernel<false><<<grid1, 256, 0, st>>>(ts, rows, T, Tp, Z, nullptr);
     int rc = check_launch("fcd_corr_fisherz(standardise)");
     if (rc) return rc;
-    if (tc) return corr_gram_tc(Z, Zlo, S, N, Tp, out, pitch, s0, fisher, st);
-    FCD_REQUIRE(S <= 65535, "fcd_corr_fisherz: S=%d too large for the SIMT Gram kernel", S);
-    const int nt = (N + 31) / 32;
-    dim3 grid((unsigned)(nt * (nt + 1) / 2), (unsigned)S);
-    gram_simt_kernel<<<grid, 256, 0, st>>>(Z, N, Tp, nt, out, pitch, s0, fisher);
-    return check_launch("fcd_corr_fisherz(gram_simt)");
+    return corr_gram(tc, Z, Zlo, S, N, Tp, out, pitch, s0, fisher, st);
 }
 
 int fcd_corr_mark_missing(const float* ts, int32_t S, int32_t N, int32_t T, double* out, int64_t pitch, int32_t s0,

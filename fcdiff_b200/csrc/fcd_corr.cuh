@@ -38,4 +38,14 @@ bool corr_tc_supported(int N);
 int corr_gram_tc(const float* Zh, const float* Zl, int S, int N, int Tp, double* out, int64_t pitch, int s0,
                  int fisher, cudaStream_t st);
 
+// fcd_corr.cu: the Gram + epilogue of fcd_corr_fisherz on the tensor-core (tc) or SIMT path; corr_use_tc
+// is the path fcd_corr_fisherz takes for N (FCD_CORR_SIMT forces SIMT).  The masked standardisation
+// (standardise_kernel<SPLIT, true>) and the NaN marking of the rows it flags, for fcd_corr_fisherz_clean.
+bool corr_use_tc(int N);
+int corr_gram(bool tc, const float* Z, const float* Zlo, int S, int N, int Tp, double* out, int64_t pitch, int s0,
+              int fisher, cudaStream_t st);
+int corr_standardise_masked(bool tc, const float* ts, const uint8_t* keep, int S, int N, int T, int Tp, float* Z,
+                            float* Zlo, uint8_t* status, cudaStream_t st);
+int corr_mark_status(const uint8_t* status, int S, int N, double* out, int64_t pitch, int s0, cudaStream_t st);
+
 }  // namespace fcd

@@ -649,6 +649,26 @@ FCD_API int fcd_corr_fisherz(const float* ts, int32_t S, int32_t N, int32_t T,
 FCD_API int fcd_corr_mark_missing(const float* ts, int32_t S, int32_t N, int32_t T,
                      double* out, int64_t pitch, int32_t s0, void* stream);
 
+/* Correlations from cleaned time series: censored frames, per-subject scan lengths, confound regression.
+ * ts [S][N][T] float32 (T = the longest subject; shorter subjects padded), keep [S][T] uint8 (a frame t
+ * enters subject s's correlations iff keep[s][t] != 0; NULL: every frame), confounds [S][T][K] float64
+ * frame-major (NULL iff K == 0; 0 <= K <= 64).  Per subject, over its kept frames only, every region row
+ * is centred, cleared of the centred confounds by projection on their orthonormal basis (two passes of
+ * modified Gram-Schmidt in fp64; a confound whose residual norm is <= 1e-10 of its raw norm is dropped,
+ * rank[s] = the confounds kept, when rank != NULL), scaled to unit norm, and the Gram stage and output of
+ * fcd_corr_fisherz follow: columns [s0, s0 + S) of the (C, pitch) matrix out, every other column
+ * untouched.  r is then the partial correlation of the two regions given the confounds and a constant.
+ * Samples and confounds of frames that are not kept are never read into arithmetic.  A region row with a
+ * non-finite kept sample, or whose residual sum of squares is at most 2^-40 of its centred sum of squares
+ * (zero variance when K == 0), is unusable: r = 0 on its edges, or NaN on its N - 1 edges when
+ * mark_missing != 0.  With keep all ones and K == 0 the output has the bits of fcd_corr_fisherz (and,
+ * with mark_missing, of fcd_corr_mark_missing after it).  Every subject needs at least K + 2 kept frames
+ * (not checked here).  zws: device scratch of fcd_corr_clean_workspace_bytes(S, N, T, K) bytes. */
+FCD_API int64_t fcd_corr_clean_workspace_bytes(int32_t S, int32_t N, int32_t T, int32_t K);
+FCD_API int fcd_corr_fisherz_clean(const float* ts, int32_t S, int32_t N, int32_t T, const uint8_t* keep,
+                     const double* confounds, int32_t K, double* out, int64_t pitch, int32_t s0,
+                     int32_t fisher, int32_t mark_missing, int32_t* rank, void* zws, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
