@@ -60,7 +60,6 @@ SIGNATURES = {
     "fcd_healthy_stats_cols": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P]),
     "fcd_healthy_stats_cols_masked": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P, _P]),
     "fcd_gather_columns": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P, c_int64, c_int64, _P]),
-    "fcd_gather_rows": (c_int, [_P, c_int64, c_int32, _P, c_int32, c_int64, _P, c_int64, _P]),
     "fcd_edge_table": (c_int, [c_int64, c_int64, _P, _P]),
     "fcd_resp_cache": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
     "fcd_resp_cache_masked": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
@@ -71,12 +70,7 @@ SIGNATURES = {
                              POINTER(FcdTheta), _P, _P, _P]),
     "fcd_estep_qF_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64,
                                     c_int32, _P, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_transpose_patients": (c_int, [_P, c_int64, c_int32, c_int64, c_int32, c_int32, _P, c_int64, _P]),
-    "fcd_region_weights": (c_int, [_P, c_int64, c_int32, c_int64, c_int64, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P]),
     "fcd_estep_qR": (c_int, [_P, c_int64, c_int32, c_int32, c_int32, c_int32, _D3, c_int32, _P, _P, _P]),
-    "fcd_estep_qR_fused": (c_int, [_P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int32, c_int32, c_int32, c_int32,
-                                   _D3, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_pstar_refresh": (c_int, [_P, c_int64, c_int32, c_int64, c_int64, _P, _P, _P, _P]),
     "fcd_pstar_refresh_em": (c_int, [_P, c_int64, c_int64, c_int32, c_int32, c_int64, c_int64, _P, _P, _P, _P]),
     "fcd_region_weights_em": (c_int, [_P, c_int64, c_int64, c_int32, c_int32, c_int64, c_int64, _P, _P, _P, _P,
                                       POINTER(FcdTheta), _P, _P]),
@@ -184,7 +178,7 @@ def load():
         fn = getattr(lib, name)          # AttributeError if the symbol is missing
         fn.restype = restype
         fn.argtypes = argtypes
-    if lib.fcd_version() < 120:
+    if lib.fcd_version() < 121:
         raise FcdError("fcdiff_b200: stale libfcdiff_b200.so (version %d)" % lib.fcd_version())
     _lib = lib
     return lib

@@ -1,13 +1,11 @@
 // E-step kernels: healthy sufficient statistics, responsibility planes, peak
 // states, K2 (template posterior q_F), K2b (region-weight tensor W and the
 // Gauss-Seidel sweep for q_R).
-#include <cstdlib>
 #include <cstring>
 
 #include <type_traits>
 
 #include "fcd_common.cuh"
-#include "fcd_estep_rows.cuh"
 #include "fcd_solver.cuh"
 
 namespace fcd {
@@ -571,78 +569,15 @@ estep_qF_coded_kernel(const double* __restrict__ S1, const double* __restrict__ 
     finish_rows();
 }
 
-// ------------------------------------------------------ patient-major copy
-// btT[u - u0][c] = bt[c][u]; 32x32 tiles through padded shared memory so both
-// sides are coalesced.
-__global__ void __launch_bounds__(256)
-transpose_patients_kernel(const double* __restrict__ bt, int64_t C, int U, int64_t pitchU,
-                          int u0, int Ul, double* __restrict__ btT, int64_t pitchC) {
-    __shared__ double tile[32][33];
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;       // 32 x 8
-    const int64_t cb = (int64_t)blockIdx.x * 32;
-    const int ub = blockIdx.y * 32;
-#pragma unroll
-    for (int j = 0; j < 32; j += 8) {
-        const int64_t c = cb + ty + j;
-        const int u = ub + tx;
-        if (c < C && u < Ul) tile[ty + j][tx] = bt[c * pitchU + u0 + u];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < 32; j += 8) {
-        const int u = ub + ty + j;
-        const int64_t c = cb + tx;
-        if (c < C && u < Ul) btT[(int64_t)u * pitchC + c] = tile[tx][ty + j];
-    }
-}
-
 // ------------------------------------------------------------------- K2b/P*
-// PsT[u][c] = PT[k*(c)][u][c]: the patient-major plane of each edge's dominant
-// state.  q_F settles after the first iteration, so the plane is gathered once and
-// afterwards only the columns of edges whose state changed are refreshed
-// (kcache[c] = the state PsT[.][c] was gathered for; 255 = never).
-__global__ void __launch_bounds__(256)
-pstar_refresh_kernel(const double* __restrict__ PT, int64_t planeStride, int Ul, int64_t C, int64_t pitchC,
-                     const uint8_t* __restrict__ fstate, const uint8_t* __restrict__ kcache,
-                     double* __restrict__ PsT) {
-    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    const int k = fstate[c];
-    if ((k >= 3 ? 3 : k) == kcache[c]) return;
-    const int per = (Ul + gridDim.y - 1) / gridDim.y;
-    const int u1 = min(Ul, (int)(blockIdx.y + 1) * per);
-    if (k >= 3) {
-        // unpeaked edge: its column is marked with a negative "responsibility" -- the fused sweep, which reads
-        // nothing but this plane in its inner loop, takes the three-plane path for it (the other readers
-        // look at the edge's state first and never use the entry)
-        for (int u = blockIdx.y * per; u < u1; ++u) PsT[(int64_t)u * pitchC + c] = -1.0;
-        return;
-    }
-    const double* src = PT + (int64_t)k * planeStride + c;
-    // a thread that has to copy keeps eight loads in flight (the launch lasts as long as its slowest column)
-    int u = blockIdx.y * per;
-    for (; u + 8 <= u1; u += 8) {
-        double v[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) v[i] = ldg_stream1(src + (int64_t)(u + i) * pitchC);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) PsT[(int64_t)(u + i) * pitchC + c] = v[i];
-    }
-    for (; u < u1; ++u) PsT[(int64_t)u * pitchC + c] = ldg_stream1(src + (int64_t)u * pitchC);
-}
-
-__global__ void __launch_bounds__(256)
-pstar_commit_kernel(const uint8_t* __restrict__ fstate, int64_t C, uint8_t* __restrict__ kcache) {
-    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (c < C) kcache[c] = fstate[c] < 3 ? fstate[c] : 3;
-}
-
-// The same plane gathered straight from the E-step's EDGE-major planes Pe[k][c][u0 + u] (the patient-major copies
-// PT existed for this gather alone once every edge is peaked: three transposes and a gather, 1.9 GB + 0.6 GB of
-// traffic per fit, for what is ONE transposing pass over the dominant-state rows).  One CTA per 32 edges: it leaves
-// at once when none of its columns changed state (the usual launch), otherwise walks the patients in 32 x 32 tiles
-// through padded shared memory -- reads coalesced along u, writes along c; columns that did not change are
-// neither read nor written.
+// PsT[u][c] = Pe[k*(c)][c][u0 + u]: the patient-major plane of each edge's dominant state, gathered straight from
+// the E-step's EDGE-major planes by one transposing pass over the dominant-state rows.  q_F settles after the first
+// iteration, so the plane is gathered once and afterwards only the columns of edges whose state changed are
+// refreshed (kcache[c] = the state PsT[.][c] was gathered for; 255 = never).  The column of an unpeaked edge is
+// marked with a negative "responsibility": region_weights_kernel reads nothing but this plane per element and takes
+// the three-plane path for it.  One CTA per 32 edges: it leaves at once when none of its columns changed state (the
+// usual launch), otherwise walks the patients in 32 x 32 tiles through padded shared memory -- reads coalesced
+// along u, writes along c; columns that did not change are neither read nor written.
 __global__ void __launch_bounds__(256)
 pstar_refresh_em_kernel(const double* __restrict__ Pe, int64_t planeStride, int64_t pitchU, int u0, int Ul, int64_t C,
                         int64_t pitchC, const uint8_t* __restrict__ fstate, const uint8_t* __restrict__ kcache,
@@ -672,7 +607,7 @@ pstar_refresh_em_kernel(const double* __restrict__ Pe, int64_t planeStride, int6
         for (int j = 0; j < 32; j += 8) {                         // tile[c][u]: coalesced along u
             const int k = s_k[ty + j];
             const int u = ub + tx;
-            double v = -1.0;                                      // unpeaked edge: the negative mark (pstar_refresh_kernel)
+            double v = -1.0;                                      // unpeaked edge: the negative mark
             if (k >= 0 && k < 3 && u < Ul) v = ldg_stream1(Pe + (int64_t)k * planeStride + (cb + ty + j) * pitchU + u0 + u);
             tile[ty + j][tx] = v;
         }
@@ -686,9 +621,15 @@ pstar_refresh_em_kernel(const double* __restrict__ Pe, int64_t planeStride, int6
     }
 }
 
+__global__ void __launch_bounds__(256)
+pstar_commit_kernel(const uint8_t* __restrict__ fstate, int64_t C, uint8_t* __restrict__ kcache) {
+    const int64_t c = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (c < C) kcache[c] = fstate[c] < 3 ? fstate[c] : 3;
+}
+
 // ------------------------------------------------------------------- K2b/W
-// W_l[c,u] = sum_k qF[c,k] log(a_l + b_l p_k(c,u)) from the patient-major
-// responsibility planes PT[k][u][c].  The omitted per-(c,u) constant L sum_k qF[c,k]
+// W_l[c,u] = sum_k qF[c,k] log(a_l + b_l p_k(c,u)) from the responsibility
+// planes (see fcd_region_weights_em for the strides).  The omitted per-(c,u) constant L sum_k qF[c,k]
 // is the same for l = 0, 1, 2 and enters both states of fcdiff/fit.py:190,194
 // multiplied by (q_R[m,u,0] + q_R[m,u,1]), so it cancels at fit.py:196.
 // Only the DIFFERENCE of the two region states' sums survives the normalisation of
@@ -710,7 +651,7 @@ region_weights_kernel(const double* __restrict__ PT, int64_t planeStride, int64_
     // persistent CTAs over (patient, 1024-edge tile) work items: no wave tail, one table load per
     // CTA.  The kernel is bound by load latency, so (a) with the dominant-state plane ONE load per element
     // says everything: the responsibility of a peaked edge, or the negative mark of an unpeaked one
-    // (fcd_pstar_refresh) -- no state byte is fetched; and (b) the loads of the CTA's next tile are in
+    // (pstar_refresh_em_kernel) -- no state byte is fetched; and (b) the loads of the CTA's next tile are in
     // flight while the logs of the current one are taken.  Tile indices are 32-bit (the host checks the
     // count): no 64-bit division per tile.
     const unsigned tiles_per_row = (unsigned)((C + 1023) / 1024);
@@ -929,9 +870,9 @@ __device__ __forceinline__ int64_t sweep_edge(int n, int m, int64_t base_n) {
 }
 
 // q_R [Npad] | tiles [2 buffers][near, in-block][B x (B + 1)] | far sums [2][helper warps][B] | D [2][B]
-__host__ __device__ constexpr size_t sweep_blocked_smem(int N, int T, int B, int n7 = 0, int cs = 1) {
+__host__ __device__ constexpr size_t sweep_blocked_smem(int N, int T, int B, int cs = 1) {
     return (size_t)((N + 31) & ~31) * 16 + (size_t)4 * B * (B + 1) * 16 + (size_t)2 * cs * (T / 32 - 1) * B * 8 +
-           (size_t)2 * B * 8 + (size_t)n7 * 8;
+           (size_t)2 * B * 8;
 }
 
 // Thread-block cluster helpers (CS > 1 form of the blocked sweep: the CTAs of a cluster share one patient).
@@ -961,69 +902,18 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
                  ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 
-// FUSED: no weight tensor.  The kernel reads the patient-major dominant-state plane PsT (8 bytes per
-// edge-patient instead of WT's 16, and no region_weights pass that writes them) and forms
-//     {W_0 - W_2, W_2 - W_1},  W_l = log(a_l + b_l p*)                       (peaked edge: fcd_region_weights)
-// where it needs them: the far loop is bound by the latency of its loads and has the issue slots.  An
-// unpeaked edge is marked by a NEGATIVE entry of PsT (fcd_pstar_refresh) and takes all three planes and q_F
-// (rare after the first E-step).  The logarithm uses a 7-bit rounded reciprocal (every fourth slot of the
-// 9-bit table: a quarter of the shared memory, so that four CTAs still fit an SM) and two more terms of
-// log1p: |u| <= 2^-8, truncation u^6 / 6 < 6e-16.
-struct SweepFusedArgs {
-    const double* PT;          // [3][Ul][pitchC] responsibility planes, patient-major (unpeaked edges)
-    int64_t planeStride;
-    int64_t pitchC;
-    const double* qF;          // [C][3]
-    double al[3], bl[3];
-    const double* tab;         // 9-bit table (all slots)
-    int lo7, n7;               // window in 7-bit slots
-};
-
-constexpr int kLogTab7Base = (1023 + kLogTabMinExp) << 7;
-
-template <bool FAST>
-__device__ __forceinline__ double sweep_log7(double y, const double* s_tab7) {
-    if (!FAST) return log(y);
-    double r0;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(r0) : "d"(y));                // MUFU.RCP64H
-    const int hi = (__double2hiint(r0) + (1 << 12)) & ~((1 << 13) - 1);
-    const double r7 = __hiloint2double(hi, 0);
-    const double u = fma(y, r7, -1.0);
-    // log1p(u) = u - u^2/2 + u^3/3 - u^4/4 + u^5/5
-    double q = fma(u, 0.2, -0.25);
-    q = fma(u, q, 1.0 / 3.0);
-    q = fma(u, q, -0.5);
-    return s_tab7[(hi >> 13) - kLogTab7Base] + fma(u * u, q, u);
-}
-
-// The weights of an UNPEAKED edge e of patient row ul: sum_k q_F[e,k] log(a_l + b_l p_k) (rare: kept out of line)
-template <bool FAST>
-__device__ __noinline__ double2 sweep_weights_unpeaked(const SweepFusedArgs& fa, int ul, int64_t e, const double* tab7) {
-    const double* pk = fa.PT + (int64_t)ul * fa.pitchC + e;
-    double w0 = 0.0, w1 = 0.0, w2 = 0.0;
-    for (int k = 0; k < 3; ++k) {
-        const double q = __ldg(fa.qF + e * 3 + k), pp = __ldg(pk + k * fa.planeStride);
-        w0 = fma(q, sweep_log7<FAST>(fma(fa.bl[0], pp, fa.al[0]), tab7), w0);
-        w1 = fma(q, sweep_log7<FAST>(fma(fa.bl[1], pp, fa.al[1]), tab7), w1);
-        w2 = fma(q, sweep_log7<FAST>(fma(fa.bl[2], pp, fa.al[2]), tab7), w2);
-    }
-    return make_double2(w0 - w2, w2 - w1);
-}
-
 // CS > 1 (few patients on this GPU -- sharded fits: 63 patients on 148 SMs): the CS CTAs of a thread-block cluster
 // share ONE patient.  The launch lasts a patient's chain of blocks and a block lasts what its far sums take one SM to
 // pull from L2; the cluster splits the far columns over its CTAs, CTA r > 0 stores its warps' partial sums into CTA
 // 0's shared memory (DSMEM), CTA 0 alone holds the tiles, solves and writes the outputs, and sends every solved
 // block's q_R to the others' copies of s_q; the per-block barrier becomes a cluster barrier.
-template <int T, int B, int LOOKUP, bool FUSED, bool FAST, int CS = 1>
+template <int T, int B, int LOOKUP, int CS = 1>
 __global__ void __launch_bounds__(T, 512 / T)
 sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int u0, double lp0, double lp1,
-                     double* __restrict__ qR, double* __restrict__ lqR, const __grid_constant__ SweepFusedArgs fa) {
-    static_assert(CS == 1 || !FUSED, "the cluster form exists for the WT sweep");
+                     double* __restrict__ qR, double* __restrict__ lqR) {
     constexpr int NWH = T / 32 - 1, H = T - 32, Bp = B + 1, RH = kSwRH, TILE = B * Bp, NWP = CS * NWH;
     constexpr int LB = B == 32 ? 5 : 4;
     static_assert(B == 16 || B == 32, "block of 16 or 32 regions");
-    static_assert(!FUSED || LOOKUP == FCD_LOOKUP_REFERENCE, "the fused form reads contiguous windows (reference lookup)");
     extern __shared__ __align__(16) double s_sweep[];
     double2* s_q = reinterpret_cast<double2*>(s_sweep);                    // [Npad] q_R of the moment
     const int Npad = (N + 31) & ~31;
@@ -1033,24 +923,9 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
     const int crank = CS > 1 ? (int)cluster_ctarank() : 0;
     const int ul = CS > 1 ? blockIdx.x / CS : blockIdx.x, u = u0 + ul;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    using Elem = typename std::conditional<FUSED, double, double2>::type;  // what the far loop loads per edge
-    // WT form: {W_0 - W_2, W_2 - W_1} of this patient's edges; fused form: the patient's row of PsT
-    const Elem* Wu = reinterpret_cast<const Elem*>(WT) + (int64_t)ul * (FUSED ? fa.pitchC : C);
+    const double2* Wu = reinterpret_cast<const double2*>(WT) + (int64_t)ul * C;   // {W_0 - W_2, W_2 - W_1}
     const double2* qR2 = reinterpret_cast<const double2*>(qR);
     for (int m = tid; m < Npad; m += T) s_q[m] = m < N ? qR2[(int64_t)m * U + u] : make_double2(0.0, 0.0);
-    double* s_tab7 = s_D + 2 * B;                                          // [n7] -log r7 (fused form)
-    if (FUSED && FAST)
-        for (int i = tid; i < fa.n7; i += T) s_tab7[i] = fa.tab[(int64_t)(fa.lo7 + i) << 2];
-    const double* tab7 = s_tab7 - fa.lo7;
-    // weights of one edge from its dominant-state responsibility (fused form)
-    auto weights = [&](double pv, const double* addr) {
-        if (pv < 0.0)                                                      // unpeaked edge (marked by fcd_pstar_refresh)
-            return sweep_weights_unpeaked<FAST>(fa, ul, addr - reinterpret_cast<const double*>(Wu), tab7);
-        const double w0 = sweep_log7<FAST>(fma(fa.bl[0], pv, fa.al[0]), tab7);
-        const double w1 = sweep_log7<FAST>(fma(fa.bl[1], pv, fa.al[1]), tab7);
-        const double w2 = sweep_log7<FAST>(fma(fa.bl[2], pv, fa.al[2]), tab7);
-        return make_double2(w0 - w2, w2 - w1);
-    };
     if (CS > 1) cluster_sync_all(); else __syncthreads();
     const double dlp = lp0 - lp1;
     const int nblocks = (N + B - 1) / B;
@@ -1063,10 +938,7 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
         double2* tiles = s_tiles + (b & 1) * 2 * TILE;
         // (i) tiles: element e -> tile t (0 near, 1 in-block), row i, column j; lanes walk a row's columns
         // (contiguous edges: both tiles have m < n, where the two lookups agree)
-        // (fused form: the tiles are formed after the far loop, from responsibilities the previous phase's
-        // prefetch has already brought into L2)
-        if constexpr (!FUSED) {
-            if (crank == 0)
+        if (crank == 0)
             for (int e = ht; e < 2 * B * B; e += H) {
                 const int t = e >> (2 * LB), i = (e >> LB) & (B - 1), j = e & (B - 1);
                 double2* dst = tiles + t * TILE + j * Bp + i;
@@ -1075,7 +947,6 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
                 if (live) cp_async16(dst, Wu + (int64_t)n * (n - 1) / 2 + (n0 - (t == 0 ? B : 0)) + j);
                 else *dst = make_double2(0.0, 0.0);
             }
-        }
         // (ii) the rows of block b + 1 (what the NEXT prepare will read, one phase from now) into L2
         if (b + 1 < nblocks && lane == 0 && crank == 0) {                  // (the instruction takes warp-uniform operands)
             const int n1 = n0 + B, nl = n1 + B - 1 < N - 1 ? n1 + B - 1 : N - 1;
@@ -1083,7 +954,7 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
             int64_t e1 = (int64_t)nl * (nl - 1) / 2 + (LOOKUP == FCD_LOOKUP_REFERENCE ? N : nl);
             if (e1 > C) e1 = C;
             const char* g0 = reinterpret_cast<const char*>(Wu + e0);
-            const int64_t bytes = ((e1 - e0) * (int64_t)sizeof(Elem)) & ~(int64_t)15;
+            const int64_t bytes = ((e1 - e0) * (int64_t)sizeof(double2)) & ~(int64_t)15;
             for (int64_t off = (int64_t)hw * 8192; off < bytes; off += (int64_t)NWH * 8192) {
                 const uint32_t sz = (uint32_t)(bytes - off < 8192 ? bytes - off : 8192);
                 asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(g0 + off), "r"(sz) : "memory");
@@ -1103,31 +974,17 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
             for (int r = 0; r < RH; ++r) acc[r] = 0.0;
             // `masked` = false is the common case (a whole block of rows, a column outside the block): no
             // predicate per row -- a per-row predicate would cap the loads in flight at the 7 predicate registers
-            auto rows = [&](const Elem* p, int stride, auto tri, auto masked, int lim, double2 q) {
+            auto rows = [&](const double2* p, int stride, auto tri, auto masked, int lim, double2 q) {
                 p += h * stride + (decltype(tri)::value ? h * (h - 1) / 2 : 0);
                 // base(n0 + h + r) - base(n0 + h) = r (n0 + h) + r (r - 1) / 2
                 auto off = [&](int r) {
                     return r * (stride + (decltype(tri)::value ? h : 0)) + (decltype(tri)::value ? r * (r - 1) / 2 : 0);
                 };
-                if constexpr (FUSED) {
-                    double v[RH];                                          // all loads first, then the logarithms
 #pragma unroll
-                    for (int r = 0; r < RH; ++r)
-                        if (!decltype(masked)::value || h + r < lim) v[r] = __ldg(p + off(r));
-#pragma unroll
-                    for (int r = 0; r < RH; ++r) {
-                        if (!decltype(masked)::value || h + r < lim) {
-                            const double2 w = weights(v[r], p + off(r));
-                            acc[r] = fma(q.x, w.x, fma(q.y, w.y, acc[r]));
-                        }
-                    }
-                } else {
-#pragma unroll
-                    for (int r = 0; r < RH; ++r) {
-                        if (!decltype(masked)::value || h + r < lim) {
-                            const double2 w = __ldg(p + off(r));
-                            acc[r] = fma(q.x, w.x, fma(q.y, w.y, acc[r]));    // (fit.py:188-190) - (fit.py:192-194)
-                        }
+                for (int r = 0; r < RH; ++r) {
+                    if (!decltype(masked)::value || h + r < lim) {
+                        const double2 w = __ldg(p + off(r));
+                        acc[r] = fma(q.x, w.x, fma(q.y, w.y, acc[r]));    // (fit.py:188-190) - (fit.py:192-194)
                     }
                 }
             };
@@ -1136,7 +993,7 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
                 if (mb == b - 1) continue;                                 // near: the solver's (new q_R of block b - 1)
                 const double2 q = s_q[m];
                 const bool tri = LOOKUP == FCD_LOOKUP_REFERENCE || m < n0;
-                const Elem* p = tri ? Wu + base0 + m : Wu + (int64_t)m * (m - 1) / 2 + n0;
+                const double2* p = tri ? Wu + base0 + m : Wu + (int64_t)m * (m - 1) / 2 + n0;
                 if (mb != b && nb == B) {
                     if (tri) rows(p, n0, yes(), no(), B, q);
                     else rows(p, 1, no(), no(), B, q);
@@ -1166,17 +1023,7 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
                 else dsmem_store(dsmem_addr(dst, 0), acc[0]);              // into CTA 0's copy
             }
         }
-        if constexpr (FUSED) {
-            for (int e = ht; e < 2 * B * B; e += H) {
-                const int t = e >> (2 * LB), i = (e >> LB) & (B - 1), j = e & (B - 1);
-                const int n = n0 + i;
-                const bool live = i < nb && (t == 0 ? b > 0 : j < i);
-                const double* src = reinterpret_cast<const double*>(Wu + (int64_t)n * (n - 1) / 2 + (n0 - (t == 0 ? B : 0)) + j);
-                tiles[t * TILE + j * Bp + i] = live ? weights(__ldg(src), src) : make_double2(0.0, 0.0);
-            }
-        } else {
-            asm volatile("cp.async.wait_all;" ::: "memory");
-        }
+        asm volatile("cp.async.wait_all;" ::: "memory");
     };
 
     // ---- solve(b): warp 0 only (B = 16: lanes 16.. mirror lanes 0..15)
@@ -1274,229 +1121,6 @@ sweep_blocked_kernel(const double* __restrict__ WT, int64_t C, int N, int U, int
         if (CS > 1) cluster_sync_all(); else __syncthreads();     // (the last one also keeps every CTA alive while
     }                                                             //  CTA 0 may still store into its shared memory)
     if (warp == NWH && crank == 0) outputs(nblocks - 1);
-}
-
-// --------------------------------------------------------------- K2b fused
-// Gauss-Seidel sweep of fcdiff/fit.py:184-197 with the region weights computed
-// inside the kernel: no WT tensor (24 bytes per edge-patient written and read
-// back) and no region_weights pass.  With edge_lookup = "reference" the edges
-// read at step n are the contiguous window [n(n-1)/2, n(n-1)/2 + N)
-// (fit.py:185-186), and the windows of successive steps slide monotonically over
-// the patient's row of the dominant-state plane PsT (fcd_region_weights).
-// Warp-specialised, per patient a group of T sweep threads and TC converter
-// threads:
-//   * converter lane 0 streams the row by TMA bulk copies (64-edge chunks: p and
-//     the edges' peak states) into a staging ring;
-//   * the converter warps turn every edge ONCE into its three weights
-//     W_l = log(a_l + b_l p) and store them in a shared-memory ring of R edges,
-//     one window ahead of the sweep (iteration j prepares window j while the
-//     sweep works on step j - 1; handshake over two mbarriers: READY_j / START_j);
-//   * the sweep threads (thread t owns the regions m = t, t + T, ...; their q_R
-//     stay in registers) read their window from shared memory, reduce (warp
-//     shuffle + ONE named barrier) and only the owner of region n normalises
-//     (fit.py:196-197): no logarithm is left on the sweep's critical path.
-// PPC patient groups per CTA share the log table.  Ring capacity: window n (being
-// read) and window n + 1 (being prepared) must fit: 2N - 1 <= R.
-constexpr int kSwChunk = 64;
-
-template <int T, int R>
-struct SweepSmem {
-    static constexpr int NW = T / 32;
-    static constexpr int kSlots = R / kSwChunk;
-    static constexpr size_t bytes = (size_t)3 * R * 8 + (size_t)R * 8 + R + (kSlots + 2) * 8 + 2 * NW * 2 * 8;
-    static constexpr size_t padded = (bytes + 127) / 128 * 128;
-};
-
-template <int T, int TC, int MPT, int PPC, int R, bool FAST>
-__global__ void __launch_bounds__((T + TC) * PPC)
-sweep_fused_kernel(const double* __restrict__ PsT, const double* __restrict__ PT, int64_t planeStride,
-                   int64_t pitchC, const double* __restrict__ qF, const uint8_t* __restrict__ fstate,
-                   int64_t pitchF, int64_t C, int N, int U, int u0, int Ul, double lp0, double lp1,
-                   const __grid_constant__ ThetaDev th, const __grid_constant__ LogTabWindow tab,
-                   double* __restrict__ qR, double* __restrict__ lqR) {
-    constexpr int NW = T / 32, NCV = TC / 32, kSlots = R / kSwChunk, kAhead = 64;
-    extern __shared__ __align__(128) double s_dyn[];
-    const double* s_tab = load_log_table<FAST>(tab, s_dyn);
-    const int pp = threadIdx.x / (T + TC), gt = threadIdx.x % (T + TC);      // patient group, thread in group
-    const int ul = blockIdx.x * PPC + pp;
-    if (ul >= Ul) return;                                    // whole patient group leaves (its barriers are its own)
-    unsigned char* mine = reinterpret_cast<unsigned char*>(s_dyn + (FAST ? ((tab.n + 15) & ~15) : 0)) +
-                          (size_t)pp * SweepSmem<T, R>::padded;
-    double* wring = reinterpret_cast<double*>(mine);         // [3][R] weights
-    double* pring = wring + 3 * R;                           // [R] staged responsibilities
-    uint8_t* fring = reinterpret_cast<uint8_t*>(pring + R);  // [R] staged peak states
-    uint64_t* bars = reinterpret_cast<uint64_t*>(fring + R); // [kSlots] chunk arrival, then READY, START
-    uint64_t* ready = bars + kSlots;                         // completed by the NCV converter warps per window
-    uint64_t* start = ready + 1;                             // completed by the NW sweep warps per step
-    double* s_red = reinterpret_cast<double*>(start + 1);    // [2][NW][2]
-    // init by the group's first thread, published to the group by a named barrier over ALL its threads
-    if (gt == 0) {
-        for (int i = 0; i < kSlots; ++i) mbar_init(bars + i, 1);
-        mbar_init(ready, NCV);
-        mbar_init(start, NW);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (PPC == 1 || pp == 0) asm volatile("bar.sync 1, %0;" ::"n"(T + TC) : "memory");
-    else if (pp == 1) asm volatile("bar.sync 2, %0;" ::"n"(T + TC) : "memory");
-    else if (pp == 2) asm volatile("bar.sync 3, %0;" ::"n"(T + TC) : "memory");
-    else asm volatile("bar.sync 4, %0;" ::"n"(T + TC) : "memory");
-
-    const int u = u0 + ul;
-    auto clampC = [&](int64_t e) { return e < C ? e : C; };
-    // edges [0, target(j)) must be converted before the sweep reads window j
-    auto target = [&](int j) {
-        const int64_t base = (int64_t)j * (j - 1) / 2;
-        int64_t t = base + N + kAhead;                       // end of window j and a little ahead
-        if (j > 0) {                                         // window j - 1 is still being read: its slots stay
-            const int64_t cap = (int64_t)(j - 1) * (j - 2) / 2 + R;
-            if (t > cap) t = cap;
-        } else if (t > R) {
-            t = R;
-        }
-        return clampC(t);
-    };
-
-    if (gt >= T) {
-        // ------------------------------------------------------------ converter warps
-        const int ct = gt - T, lane = ct & 31;
-        const double* row = PsT + (int64_t)ul * pitchC;
-        const int nchunks = (int)((pitchC + kSwChunk - 1) / kSwChunk);
-        const double al[3] = {th.al[0], th.al[1], th.al[2]}, bl[3] = {th.bl[0], th.bl[1], th.bl[2]};
-        int next_issue = 0;                                  // meaningful in ct == 0 only
-        auto issue = [&](int g) {
-            uint64_t* bar = bars + (g % kSlots);
-            const int64_t e0 = (int64_t)g * kSwChunk;
-            const uint32_t ne = (uint32_t)(pitchC - e0 < kSwChunk ? pitchC - e0 : kSwChunk);
-            const uint32_t nf = (uint32_t)(pitchF - e0 < kSwChunk ? pitchF - e0 : kSwChunk);
-            const int so = (g % kSlots) * kSwChunk;
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            mbar_expect_tx(bar, ne * 8 + nf);
-            tma_load_1d(pring + so, row + e0, ne * 8, bar);
-            tma_load_1d(fring + so, fstate + e0, nf, bar);
-        };
-        if (ct == 0)
-            for (; next_issue < kSlots && next_issue < nchunks; ++next_issue) issue(next_issue);
-        int waited = -1;                                     // chunks 0..waited have arrived (per thread)
-        int64_t cv = 0;                                      // edges [0, cv) are converted (same in all converter threads)
-        for (int j = 0; j < N; ++j) {
-            if (j >= 1) mbar_wait(start, (uint32_t)((j - 1) & 1));       // sweep has begun step j-1: windows < j-1 are dead
-            const int64_t tg = target(j);
-            if (tg > cv) {
-                const int ghi = (int)((tg - 1) / kSwChunk);
-                for (; waited < ghi; ++waited) mbar_wait(bars + ((waited + 1) % kSlots), ((waited + 1) / kSlots) & 1);
-                for (int64_t e = cv + ct; e < tg; e += TC) {
-                    const int idx = (int)(e & (R - 1));
-                    const int k = fring[idx];
-                    double w[3];
-                    if (k < 3) {
-                        const double p = pring[idx];
-#pragma unroll
-                        for (int l = 0; l < 3; ++l) w[l] = fast_log<FAST>(fma(bl[l], p, al[l]), s_tab);
-                    } else {                                 // edge whose q_F is not peaked (rare): all three planes
-                        const double qf[3] = {__ldg(qF + e * 3), __ldg(qF + e * 3 + 1), __ldg(qF + e * 3 + 2)};
-                        w[0] = w[1] = w[2] = 0.0;
-#pragma unroll
-                        for (int kk = 0; kk < 3; ++kk) {
-                            const double p = ldg_stream1(PT + kk * planeStride + (int64_t)ul * pitchC + e);
-#pragma unroll
-                            for (int l = 0; l < 3; ++l)
-                                w[l] = fma(qf[kk], fast_log<FAST>(fma(bl[l], p, al[l]), s_tab), w[l]);
-                        }
-                    }
-                    wring[idx] = w[0];
-                    wring[R + idx] = w[1];
-                    wring[2 * R + idx] = w[2];
-                }
-                cv = tg;
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(ready);               // window j is in the ring (release)
-            if (ct == 0) {                                   // staged chunks every converter is done with: refill
-                mbar_wait(ready, (uint32_t)(j & 1));
-                const int done = (int)(cv / kSwChunk);
-                for (; next_issue < nchunks && next_issue - kSlots < done; ++next_issue) issue(next_issue);
-            }
-        }
-        return;
-    }
-
-    // ---------------------------------------------------------------- sweep warps
-    const int tid = gt, lane = tid & 31, warp = tid >> 5;
-    auto sweep_sync = [&]() {                                // immediate barrier ids: a register id reserves all 16
-        if (PPC == 1 || pp == 0) asm volatile("bar.sync 5, %0;" ::"n"(T) : "memory");
-        else if (pp == 1) asm volatile("bar.sync 6, %0;" ::"n"(T) : "memory");
-        else if (pp == 2) asm volatile("bar.sync 7, %0;" ::"n"(T) : "memory");
-        else asm volatile("bar.sync 8, %0;" ::"n"(T) : "memory");
-    };
-    double q0[MPT], q1[MPT];
-#pragma unroll
-    for (int j = 0; j < MPT; ++j) {
-        const int m = tid + j * T;
-        q0[j] = q1[j] = 0.0;
-        if (m < N) {
-            q0[j] = qR[((int64_t)m * U + u) * 2];
-            q1[j] = qR[((int64_t)m * U + u) * 2 + 1];
-        }
-    }
-    for (int n = 0; n < N; ++n) {
-        mbar_wait(ready, (uint32_t)(n & 1));                 // window n converted (acquire)
-        __syncwarp();
-        if (lane == 0) mbar_arrive(start);                   // step n has begun: the converters may prepare window n+1
-        const uint32_t base_lo = (uint32_t)((int64_t)n * (n - 1) / 2);
-        double s0 = 0.0, s1 = 0.0;
-#pragma unroll
-        for (int j = 0; j < MPT; ++j) {
-            const int m = tid + j * T;
-            const bool valid = m < N && m != n;
-            const uint32_t idx = (base_lo + (uint32_t)(valid ? m : 0)) & (R - 1);
-            const double w0 = valid ? wring[idx] : 0.0, w1 = valid ? wring[R + idx] : 0.0,
-                         w2 = valid ? wring[2 * R + idx] : 0.0;
-            s0 += fma(q0[j], w0, q1[j] * w2);                 // fit.py:188-190
-            s1 += fma(q1[j], w1, q0[j] * w2);                 // fit.py:192-194
-        }
-        s0 = warp_sum(s0);
-        s1 = warp_sum(s1);
-        if (lane == 0) {
-            s_red[((n & 1) * NW + warp) * 2] = s0;
-            s_red[((n & 1) * NW + warp) * 2 + 1] = s1;
-        }
-        sweep_sync();
-        if (tid == (n & (T - 1))) {                           // owner of region n
-            double a = 0.0, b = 0.0;
-#pragma unroll
-            for (int i = 0; i < NW; ++i) {
-                a += s_red[((n & 1) * NW + i) * 2];
-                b += s_red[((n & 1) * NW + i) * 2 + 1];
-            }
-            // lq = l - logsumexp(l), q = exp(lq) (fit.py:196-197) with one exponential
-            const double l0r = lp0 + a, l1r = lp1 + b;
-            const bool first = l0r >= l1r;
-            const double d = first ? l1r - l0r : l0r - l1r;
-            const double t = exp_nonpos(d);
-            // most regions are decided: below 2^-54, log1p(t) = t and 1/(1+t) = 1 to rounding
-            double lg = t, inv = 1.0;
-            if (t >= 5.551115123125783e-17) {
-                lg = log1p(t);
-                inv = 1.0 / (1.0 + t);
-            }
-            const double lmax = -lg, lmin = d - lg;
-            const double qmax = inv, qmin = t * inv;
-            const double l0 = first ? lmax : lmin, l1 = first ? lmin : lmax;
-            const double p0 = first ? qmax : qmin, p1 = first ? qmin : qmax;
-            const int slot = n / T;
-#pragma unroll
-            for (int j = 0; j < MPT; ++j)
-                if (j == slot) {
-                    q0[j] = p0;
-                    q1[j] = p1;
-                }
-            const int64_t o = ((int64_t)n * U + u) * 2;
-            lqR[o] = l0;
-            lqR[o + 1] = l1;
-            qR[o] = p0;
-            qR[o + 1] = p1;
-        }
-    }
 }
 
 static inline int grid_for_rows(int64_t rows, int rows_per_block, int waves) {
@@ -1619,7 +1243,7 @@ static int estep_qF_launch(const double* S1, const double* S2, const double* S0,
     const size_t smem = tbytes + StreamGeom<2, kK2Seg>::bytes(kStreamWarps, depth);
     int64_t grid = (C + kStreamWarps - 1) / kStreamWarps;
     if (grid > sm_count()) grid = sm_count();                       // one persistent CTA per SM
-#define FCD_K2(F, M)                                                                                  \
+#define K2_LAUNCH(F, M)                                                                               \
     do {                                                                                              \
         cudaFuncSetAttribute(estep_qF_kernel<F, M>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
                              (int)kSmemBudget);                                                       \
@@ -1627,11 +1251,11 @@ static int estep_qF_launch(const double* S1, const double* S2, const double* S0,
             S1, S2, S0, P, planeStride, C, U, pitchU, qR, rstate, pitchS, nm, th, tab, depth, lqF, qF); \
     } while (0)
     if (S0 != nullptr) {
-        if (fast) FCD_K2(true, true); else FCD_K2(false, true);
+        if (fast) K2_LAUNCH(true, true); else K2_LAUNCH(false, true);
     } else {
-        if (fast) FCD_K2(true, false); else FCD_K2(false, false);
+        if (fast) K2_LAUNCH(true, false); else K2_LAUNCH(false, false);
     }
-#undef FCD_K2
+#undef K2_LAUNCH
     return check_launch(S0 != nullptr ? "fcd_estep_qF_masked" : "fcd_estep_qF");
 }
 
@@ -1687,53 +1311,30 @@ static int estep_qF_coded_launch(const double* S1, const double* S2, const doubl
     FCD_REQUIRE(log_table_window(w_eps, w_al, st, tab, true), "fcd_estep_qF_coded: log table initialisation failed");
     const bool fast = log_table_covers(w_eps, w_al);
     const size_t tbytes = fast ? (size_t)((tab.n + 15) & ~15) * sizeof(double) : 0;
-    // Row-group form (fcd_estep_rows.cu; FCD_K2=rows): four lanes per row, eight rows per warp, 2-D TMA tiles, the
-    // half records taken from the tiles -- HALF the warp-instructions of the warp-per-row kernel below, and the
-    // same time (0.190 against 0.193 ms at config 3 with 16 warps; 0.208 / 0.242 with 12 / 8): with 122 registers
-    // and 4.3 KB stages an SM holds 16 warps with two stages each, and the kernel waits (shared-memory table
-    // reads of the half records' logarithms, tile arrival) instead of issuing.  Kept as a tested alternative.
-    static const bool rows_form = [] {
-        const char* e = getenv("FCD_K2");
-        return e != nullptr && strcmp(e, "rows") == 0;
-    }();
-    if (rows_form && solved == nullptr && estep_rows_supported(U, pitchU, pitchQ))
-        return estep_rows_launch(S1, S2, S0, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, counts, keysF, keysH, rowoff,
-                                 Hh, th, tab, fast, lqF, qF, st);
-    // 16 warps per SM (127 registers each).  FCD_K2C_WARPS=24 selects the 24-warp build (80 registers, three
-    // ring stages per warp): measured no faster (0.199 vs 0.193 ms at config 3) -- the kernel is bound by
-    // the instructions of its row-level work, not by the warps available to hide latency.
-    static const int forced_nw = [] {
-        const char* e = getenv("FCD_K2C_WARPS");
-        return e != nullptr ? atoi(e) : 0;
-    }();
-    int nw = 16;
-    if (S0 == nullptr && (forced_nw == 24 || forced_nw == 20) && tbytes + k2c_ring_bytes(2, forced_nw) <= kSmemBudget) nw = forced_nw;
+    // 16 warps per SM (127 registers each).  24 warps (80 registers, three ring stages per warp) were measured no
+    // faster (0.199 vs 0.193 ms at config 3): the kernel is bound by the instructions of its row-level work, not by
+    // the warps available to hide latency.
+    constexpr int NW = 16;
     int depth = kK2cMaxDepth;
-    while (depth > 2 && tbytes + k2c_ring_bytes(depth, nw) > kSmemBudget) --depth;
-    FCD_REQUIRE(tbytes + k2c_ring_bytes(depth, nw) <= kSmemBudget, "fcd_estep_qF_coded: shared memory budget exceeded");
-    const size_t smem = tbytes + k2c_ring_bytes(depth, nw);
-    int64_t grid = (C + nw - 1) / nw;
+    while (depth > 2 && tbytes + k2c_ring_bytes(depth, NW) > kSmemBudget) --depth;
+    FCD_REQUIRE(tbytes + k2c_ring_bytes(depth, NW) <= kSmemBudget, "fcd_estep_qF_coded: shared memory budget exceeded");
+    const size_t smem = tbytes + k2c_ring_bytes(depth, NW);
+    int64_t grid = (C + NW - 1) / NW;
     if (grid > sm_count()) grid = sm_count();                       // one persistent CTA per SM
-#define FCD_K2C_(F, NW_, M)                                                                           \
+#define K2C_LAUNCH(F, M)                                                                              \
     do {                                                                                              \
-        FCD_ALLOW_BIG_SMEM(estep_qF_coded_kernel<F, NW_, M>);                                         \
-        estep_qF_coded_kernel<F, NW_, M><<<(unsigned)grid, NW_ * 32, smem, st>>>(                     \
+        FCD_ALLOW_BIG_SMEM(estep_qF_coded_kernel<F, NW, M>);                                          \
+        estep_qF_coded_kernel<F, NW, M><<<(unsigned)grid, NW * 32, smem, st>>>(                       \
             S1, S2, S0, P, planeStride, C, U, pitchU, qR, nm, code, pitchQ, reinterpret_cast<const int2*>(counts), \
             reinterpret_cast<const unsigned long long*>(keysF), reinterpret_cast<const unsigned long long*>(keysH), \
             reinterpret_cast<const longlong2*>(rowoff), reinterpret_cast<const double2*>(Hh), th, solved, tab, depth, lqF, qF); \
     } while (0)
-#define FCD_K2C(F)                                                                                    \
-    do {                                                                                              \
-        if (nw == 24) FCD_K2C_(F, 24, false); else if (nw == 20) FCD_K2C_(F, 20, false); else FCD_K2C_(F, 16, false); \
-    } while (0)
-    // the masked form is built for the default 16 warps only (the other widths are experiments)
     if (S0 != nullptr) {
-        if (fast) FCD_K2C_(true, 16, true); else FCD_K2C_(false, 16, true);
+        if (fast) K2C_LAUNCH(true, true); else K2C_LAUNCH(false, true);
     } else {
-        if (fast) FCD_K2C(true); else FCD_K2C(false);
+        if (fast) K2C_LAUNCH(true, false); else K2C_LAUNCH(false, false);
     }
-#undef FCD_K2C
-#undef FCD_K2C_
+#undef K2C_LAUNCH
     return check_launch(S0 != nullptr ? "fcd_estep_qF_coded_masked" : "fcd_estep_qF_coded");
 }
 
@@ -1787,78 +1388,6 @@ int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2, const d
                                  eps_lo, eps_hi, lqF, qF, stream);
 }
 
-int fcd_transpose_patients(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                           int32_t u0, int32_t Ul, double* btT, int64_t pitchC, void* stream) {
-    FCD_REQUIRE(C >= 0 && U >= 1 && pitchU >= U && u0 >= 0 && Ul >= 0 && u0 + Ul <= U && pitchC >= C,
-                "fcd_transpose_patients: bad shape");
-    if (C == 0 || Ul == 0) return 0;
-    dim3 grid((unsigned)((C + 31) / 32), (unsigned)((Ul + 31) / 32));
-    transpose_patients_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(bt, C, U, pitchU, u0, Ul, btT, pitchC);
-    return check_launch("fcd_transpose_patients");
-}
-
-int fcd_pstar_refresh(const double* PT, int64_t planeStride, int32_t Ul, int64_t C, int64_t pitchC,
-                      const uint8_t* fstate, double* PsT, uint8_t* kcache, void* stream) {
-    FCD_REQUIRE(PT != nullptr && fstate != nullptr && PsT != nullptr && kcache != nullptr,
-                "fcd_pstar_refresh: NULL argument");
-    FCD_REQUIRE(C >= 0 && Ul >= 0 && pitchC >= C, "fcd_pstar_refresh: bad shape");
-    if (C == 0 || Ul == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    // (in most iterations no edge changes its state and every CTA leaves at once: 16 slices of the patients, not
-    // 64, keep that launch short -- 20,000 CTAs took 41 us to do nothing; a thread that does copy has Ul / 16 rows)
-    dim3 rgrid((unsigned)((C + 255) / 256), (unsigned)(Ul < 16 ? Ul : 16));
-    pstar_refresh_kernel<<<rgrid, 256, 0, st>>>(PT, planeStride, Ul, C, pitchC, fstate, kcache, PsT);
-    int rc = check_launch("fcd_pstar_refresh");
-    if (rc) return rc;
-    pstar_commit_kernel<<<(unsigned)((C + 255) / 256), 256, 0, st>>>(fstate, C, kcache);
-    return check_launch("fcd_pstar_refresh(commit)");
-}
-
-// The planes as (base, planeStride, strideU, strideC): patient-major PT [3][Ul][pitchC] is (PT, Ul pitchC, pitchC, 1),
-// the E-step's edge-major planes [3][C][pitchU] from patient u0 on are (Pe + u0, C pitchU, 1, pitchU).
-static int region_weights_launch(const double* PT, int64_t planeStride, int64_t strideU, int64_t strideC, int32_t Ul,
-                                 int64_t C, int64_t pitchC, const double* qF, const uint8_t* fstate, const double* PsT,
-                                 const fcd_theta* theta_host, double* WT, cudaStream_t st) {
-    const ThetaDev th = make_theta_dev(*theta_host, 0);
-    LogTabWindow tab;
-    FCD_REQUIRE(log_table_window(th.epsl, th.al, st, tab), "fcd_region_weights: log table initialisation failed");
-    int64_t ntiles = ((C + 1023) / 1024) * (int64_t)Ul;
-    FCD_REQUIRE(ntiles < ((int64_t)1 << 31) - 8 * sm_count(), "fcd_region_weights: %lld tiles exceed the 32-bit tile index",
-                (long long)ntiles);
-    if (log_table_covers(th.epsl, th.al)) {
-        int per_sm = (int)((200 * 1024) / (tab.bytes() + 1024));
-        if (per_sm > 8) per_sm = 8;
-        if (per_sm < 1) per_sm = 1;
-        int64_t grid = (int64_t)sm_count() * per_sm;
-        if (grid > ntiles) grid = ntiles;
-        cudaFuncSetAttribute(region_weights_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)kLogTabBytes);
-        region_weights_kernel<true><<<(unsigned)grid, 256, tab.bytes(), st>>>(
-            PT, planeStride, strideU, strideC, Ul, C, pitchC, qF, fstate, PsT, th, tab, WT);
-    } else {
-        int64_t grid = (int64_t)sm_count() * 4;
-        if (grid > ntiles) grid = ntiles;
-        region_weights_kernel<false><<<(unsigned)grid, 256, 0, st>>>(
-            PT, planeStride, strideU, strideC, Ul, C, pitchC, qF, fstate, PsT, th, tab, WT);
-    }
-    return check_launch("fcd_region_weights");
-}
-
-int fcd_region_weights(const double* PT, int64_t planeStride, int32_t Ul, int64_t C, int64_t pitchC,
-                       const double* qF, const uint8_t* fstate, double* PsT, uint8_t* kcache,
-                       const fcd_theta* theta_host, double* WT, void* stream) {
-    FCD_REQUIRE(theta_host != nullptr && fstate != nullptr, "fcd_region_weights: NULL argument");
-    FCD_REQUIRE(C >= 0 && Ul >= 0 && pitchC >= C, "fcd_region_weights: bad shape");
-    FCD_REQUIRE((PsT == nullptr) == (kcache == nullptr), "fcd_region_weights: PsT and kcache go together");
-    if (C == 0 || Ul == 0) return 0;
-    if (PsT != nullptr) {                                     // refresh the columns of edges whose state changed
-        int rc = fcd_pstar_refresh(PT, planeStride, Ul, C, pitchC, fstate, PsT, kcache, stream);
-        if (rc) return rc;
-    }
-    return region_weights_launch(PT, planeStride, pitchC, 1, Ul, C, pitchC, qF, fstate, PsT, theta_host, WT,
-                                 (cudaStream_t)stream);
-}
-
 int fcd_pstar_refresh_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,
                          int64_t pitchC, const uint8_t* fstate, double* PsT, uint8_t* kcache, void* stream) {
     FCD_REQUIRE(Pe != nullptr && fstate != nullptr && PsT != nullptr && kcache != nullptr,
@@ -1883,8 +1412,31 @@ int fcd_region_weights_em(const double* Pe, int64_t planeStride, int64_t pitchU,
     if (C == 0 || Ul == 0) return 0;
     int rc = fcd_pstar_refresh_em(Pe, planeStride, pitchU, u0, Ul, C, pitchC, fstate, PsT, kcache, stream);
     if (rc) return rc;
-    return region_weights_launch(Pe + u0, planeStride, 1, pitchU, Ul, C, pitchC, qF, fstate, PsT, theta_host, WT,
-                                 (cudaStream_t)stream);
+    cudaStream_t st = (cudaStream_t)stream;
+    const ThetaDev th = make_theta_dev(*theta_host, 0);
+    LogTabWindow tab;
+    FCD_REQUIRE(log_table_window(th.epsl, th.al, st, tab), "fcd_region_weights_em: log table initialisation failed");
+    int64_t ntiles = ((C + 1023) / 1024) * (int64_t)Ul;
+    FCD_REQUIRE(ntiles < ((int64_t)1 << 31) - 8 * sm_count(), "fcd_region_weights_em: %lld tiles exceed the 32-bit tile index",
+                (long long)ntiles);
+    // the edge-major planes [3][C][pitchU] from patient u0 on: element (k, u, c) at Pe + u0 + k planeStride + u + c pitchU
+    if (log_table_covers(th.epsl, th.al)) {
+        int per_sm = (int)((200 * 1024) / (tab.bytes() + 1024));
+        if (per_sm > 8) per_sm = 8;
+        if (per_sm < 1) per_sm = 1;
+        int64_t grid = (int64_t)sm_count() * per_sm;
+        if (grid > ntiles) grid = ntiles;
+        cudaFuncSetAttribute(region_weights_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)kLogTabBytes);
+        region_weights_kernel<true><<<(unsigned)grid, 256, tab.bytes(), st>>>(
+            Pe + u0, planeStride, 1, pitchU, Ul, C, pitchC, qF, fstate, PsT, th, tab, WT);
+    } else {
+        int64_t grid = (int64_t)sm_count() * 4;
+        if (grid > ntiles) grid = ntiles;
+        region_weights_kernel<false><<<(unsigned)grid, 256, 0, st>>>(
+            Pe + u0, planeStride, 1, pitchU, Ul, C, pitchC, qF, fstate, PsT, th, tab, WT);
+    }
+    return check_launch("fcd_region_weights_em");
 }
 
 int fcd_estep_qR(const double* WT, int64_t C, int32_t N, int32_t U, int32_t u0, int32_t Ul,
@@ -1902,13 +1454,8 @@ int fcd_estep_qR(const double* WT, int64_t C, int32_t N, int32_t U, int32_t u0, 
     FCD_REQUIRE(N <= 8192, "fcd_estep_qR: N=%d exceeds the 8192 regions the sweep kernel supports", N);
     cudaStream_t st = (cudaStream_t)stream;
     const double lp0 = log_pi2_host[0], lp1 = log_pi2_host[1];
-    // blocked forward substitution (sweep_blocked_kernel) from 64 regions on; FCD_SWEEP=stepwise selects the
-    // one-region-per-step kernel everywhere (experiments, cross-checks)
-    static const bool stepwise = [] {
-        const char* e = getenv("FCD_SWEEP");
-        return e != nullptr && strcmp(e, "stepwise") == 0;
-    }();
-    if (N >= 64 && !stepwise) {
+    // blocked forward substitution (sweep_blocked_kernel) from 64 regions on
+    if (N >= 64) {
         // launch shape (scripts/sweep_bench.py, profiles/r02_sweep_shapes.txt): blocks of B = 16 regions
         // everywhere (32 was measured, never faster).  Threads: 3 helper warps and FOUR CTAs per SM (25 KB of
         // shared memory at N = 400) when the GPU has patients to fill them with -- every patient of the bench
@@ -1917,27 +1464,15 @@ int fcd_estep_qR(const double* WT, int64_t C, int32_t N, int32_t U, int32_t u0, 
         constexpr int B = 16;
         int T = N >= 700 ? 512 : ((N <= 512 && Ul > 2 * sm_count()) ? 128 : 256);
         while (T < 512 && sweep_blocked_smem(N, T, B) > (size_t)(T == 128 ? 54 : 110) * 1024) T *= 2;
-        static const int forced_T = [] {                      // FCD_SWEEP_T=128|256|512: launch-shape experiments
-            const char* e = getenv("FCD_SWEEP_T");
-            return e != nullptr ? atoi(e) : 0;
-        }();
-        if (forced_T == 128 || forced_T == 256 || forced_T == 512) T = forced_T;
-        // Cluster form: two CTAs per patient when that still fits one wave (sharded fits: 63 patients on 148 SMs);
-        // FCD_SWEEP_CLUSTER=1|2 overrides.  Measured (scripts/sweep_bench.py, us, one CTA -> cluster of two):
-        // 1131 regions x 63 patients 310 -> 294 (undecided regime) / 290 -> 252 (decided); 400 x 63: 86 -> 91 /
-        // 74 -> 74; 800 x 125 (does not fit one wave): 204 -> 407.  At 63 patients the launch already moves
-        // the patients' 644 MB of weights at ~4 TB/s -- it is closer to the memory system's limit than to a single
-        // SM's, so the second SM buys little: used from ~700 regions on (512 threads), where it does gain.
-        static const int forced_cs = [] {
-            const char* e = getenv("FCD_SWEEP_CLUSTER");
-            return e != nullptr ? atoi(e) : 0;
-        }();
-        int cs = (T == 512 && 2 * (int64_t)Ul <= (int64_t)sm_count()) ? 2 : 1;
-        if (forced_cs == 1 || (forced_cs == 2 && T >= 256)) cs = forced_cs;
-        const size_t smem = sweep_blocked_smem(N, T, B, 0, cs);
+        // Cluster form: two CTAs per patient when that still fits one wave (sharded fits: 63 patients on 148 SMs).
+        // Measured (scripts/sweep_bench.py, us, one CTA -> cluster of two): 1131 regions x 63 patients 310 -> 294
+        // (undecided regime) / 290 -> 252 (decided); 400 x 63: 86 -> 91 / 74 -> 74; 800 x 125 (does not fit one
+        // wave): 204 -> 407.  At 63 patients the launch already moves the patients' 644 MB of weights at ~4 TB/s --
+        // it is closer to the memory system's limit than to a single SM's, so the second SM buys little: used from
+        // ~700 regions on (512 threads), where it does gain.
+        const int cs = (T == 512 && 2 * (int64_t)Ul <= (int64_t)sm_count()) ? 2 : 1;
+        const size_t smem = sweep_blocked_smem(N, T, B, cs);
         FCD_REQUIRE(smem <= kSmemBudget, "fcd_estep_qR: N=%d needs %zu bytes of shared memory", N, smem);
-        SweepFusedArgs nofuse;
-        memset(&nofuse, 0, sizeof(nofuse));
         if (cs == 2) {
             cudaLaunchConfig_t cfg;
             memset(&cfg, 0, sizeof(cfg));
@@ -1953,160 +1488,44 @@ int fcd_estep_qR(const double* WT, int64_t C, int32_t N, int32_t U, int32_t u0, 
             cfg.attrs = &attr;
             cfg.numAttrs = 1;
             cudaError_t e = cudaSuccess;
-#define FCD_SWC(T_, L_)                                                                                       \
+#define FCD_SWC(L_)                                                                                           \
             do {                                                                                              \
-                FCD_ALLOW_BIG_SMEM((sweep_blocked_kernel<T_, 16, L_, false, false, 2>));                      \
-                e = cudaLaunchKernelEx(&cfg, sweep_blocked_kernel<T_, 16, L_, false, false, 2>, WT, C, N, U, u0, lp0, lp1, \
-                                       qR, lqR, nofuse);                                                      \
+                FCD_ALLOW_BIG_SMEM((sweep_blocked_kernel<512, B, L_, 2>));                                    \
+                e = cudaLaunchKernelEx(&cfg, sweep_blocked_kernel<512, B, L_, 2>, WT, C, N, U, u0, lp0, lp1, qR, lqR); \
             } while (0)
-            if (T == 512) {
-                if (edge_lookup == FCD_LOOKUP_REFERENCE) FCD_SWC(512, FCD_LOOKUP_REFERENCE);
-                else FCD_SWC(512, FCD_LOOKUP_SYMMETRIC);
-            } else {
-                if (edge_lookup == FCD_LOOKUP_REFERENCE) FCD_SWC(256, FCD_LOOKUP_REFERENCE);
-                else FCD_SWC(256, FCD_LOOKUP_SYMMETRIC);
-            }
+            if (edge_lookup == FCD_LOOKUP_REFERENCE) FCD_SWC(FCD_LOOKUP_REFERENCE);
+            else FCD_SWC(FCD_LOOKUP_SYMMETRIC);
 #undef FCD_SWC
             FCD_REQUIRE(e == cudaSuccess, "fcd_estep_qR(cluster): %s", cudaGetErrorString(e));
             return check_launch("fcd_estep_qR(blocked, cluster)");
         }
-#define FCD_SWB(T_, B_)                                                                                      \
+#define FCD_SWB(T_)                                                                                          \
         do {                                                                                                 \
             if (edge_lookup == FCD_LOOKUP_REFERENCE) {                                                       \
-                FCD_ALLOW_BIG_SMEM(sweep_blocked_kernel<T_, B_, FCD_LOOKUP_REFERENCE, false, false>);                      \
-                sweep_blocked_kernel<T_, B_, FCD_LOOKUP_REFERENCE, false, false><<<Ul, T_, smem, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR, nofuse); \
+                FCD_ALLOW_BIG_SMEM(sweep_blocked_kernel<T_, B, FCD_LOOKUP_REFERENCE>);                       \
+                sweep_blocked_kernel<T_, B, FCD_LOOKUP_REFERENCE><<<Ul, T_, smem, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
             } else {                                                                                         \
-                FCD_ALLOW_BIG_SMEM(sweep_blocked_kernel<T_, B_, FCD_LOOKUP_SYMMETRIC, false, false>);                      \
-                sweep_blocked_kernel<T_, B_, FCD_LOOKUP_SYMMETRIC, false, false><<<Ul, T_, smem, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR, nofuse); \
+                FCD_ALLOW_BIG_SMEM(sweep_blocked_kernel<T_, B, FCD_LOOKUP_SYMMETRIC>);                       \
+                sweep_blocked_kernel<T_, B, FCD_LOOKUP_SYMMETRIC><<<Ul, T_, smem, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
             }                                                                                                \
         } while (0)
-        if (T == 512) FCD_SWB(512, 16);
-        else if (T == 256) FCD_SWB(256, 16);
-        else FCD_SWB(128, 16);
+        if (T == 512) FCD_SWB(512);
+        else if (T == 256) FCD_SWB(256);
+        else FCD_SWB(128);
 #undef FCD_SWB
         return check_launch("fcd_estep_qR(blocked)");
     }
-#define FCD_SWEEP(T, M)                                                                            \
+#define SWEEP_LAUNCH(M)                                                                            \
     do {                                                                                           \
         if (edge_lookup == FCD_LOOKUP_REFERENCE)                                                   \
-            sweep_kernel<T, M, FCD_LOOKUP_REFERENCE><<<Ul, T, 0, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
+            sweep_kernel<32, M, FCD_LOOKUP_REFERENCE><<<Ul, 32, 0, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
         else                                                                                       \
-            sweep_kernel<T, M, FCD_LOOKUP_SYMMETRIC><<<Ul, T, 0, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
+            sweep_kernel<32, M, FCD_LOOKUP_SYMMETRIC><<<Ul, 32, 0, st>>>(WT, C, N, U, u0, lp0, lp1, qR, lqR); \
     } while (0)
-    if (N <= 32) FCD_SWEEP(32, 1);
-    else if (N <= 64) FCD_SWEEP(32, 2);
-    else if (N <= 128) FCD_SWEEP(64, 2);
-    else if (N <= 256) FCD_SWEEP(128, 2);
-    else if (N <= 512) FCD_SWEEP(128, 4);
-    // larger atlases: with few patients on this GPU (sharded fits) the launch lasts N dependent steps
-    // and a step lasts what one warp has to issue -- more warps, fewer regions per thread; with many
-    // patients the SMs are full and total instructions count -- the compact shapes
-    else if (Ul < 2 * sm_count()) {
-        if (N <= 640) FCD_SWEEP(320, 2);
-        else if (N <= 768) FCD_SWEEP(384, 2);
-        else if (N <= 896) FCD_SWEEP(448, 2);
-        else if (N <= 1024) FCD_SWEEP(512, 2);
-        else if (N <= 1280) FCD_SWEEP(640, 2);
-        else if (N <= 1536) FCD_SWEEP(512, 3);
-        else if (N <= 2048) FCD_SWEEP(512, 4);
-        else if (N <= 4096) FCD_SWEEP(1024, 4);
-        else FCD_SWEEP(1024, 8);
-    }
-    else if (N <= 1024) FCD_SWEEP(256, 4);
-    else if (N <= 2048) FCD_SWEEP(256, 8);
-    else if (N <= 4096) FCD_SWEEP(512, 8);
-    else FCD_SWEEP(1024, 8);
-#undef FCD_SWEEP
+    if (N <= 32) SWEEP_LAUNCH(1);
+    else SWEEP_LAUNCH(2);
+#undef SWEEP_LAUNCH
     return check_launch("fcd_estep_qR");
-}
-
-int fcd_estep_qR_fused(const double* PsT, const double* PT, int64_t planeStride, int64_t pitchC,
-                       const double* qF, const uint8_t* fstate, int64_t pitchF,
-                       int64_t C, int32_t N, int32_t U, int32_t u0, int32_t Ul,
-                       const double* log_pi2_host, const fcd_theta* theta_host,
-                       double* qR, double* lqR, void* stream) {
-    FCD_REQUIRE(PsT != nullptr && PT != nullptr && qF != nullptr && fstate != nullptr && log_pi2_host != nullptr &&
-                theta_host != nullptr && qR != nullptr && lqR != nullptr, "fcd_estep_qR_fused: NULL argument");
-    FCD_REQUIRE(N >= 3 && N <= 8192 && C == (int64_t)N * (N - 1) / 2,
-                "fcd_estep_qR_fused: needs 3 <= N <= 8192 and C = N(N-1)/2 (got N=%d, C=%lld)", N, (long long)C);
-    FCD_REQUIRE(u0 >= 0 && Ul >= 0 && u0 + Ul <= U, "fcd_estep_qR_fused: bad patient range");
-    FCD_REQUIRE(pitchC >= C && pitchC % 2 == 0 && pitchF >= pitchC && pitchF % 16 == 0 &&
-                ((reinterpret_cast<uintptr_t>(PsT) | reinterpret_cast<uintptr_t>(fstate)) & 15) == 0,
-                "fcd_estep_qR_fused: plane / states must be 16-byte aligned, pitchC even, pitchF % 16 == 0");
-    if (Ul == 0) return 0;
-    const ThetaDev th = make_theta_dev(*theta_host, 0);
-    cudaStream_t st = (cudaStream_t)stream;
-    LogTabWindow tab;
-    FCD_REQUIRE(log_table_window(th.epsl, th.al, st, tab), "fcd_estep_qR_fused: log table initialisation failed");
-    const bool fast = log_table_covers(th.epsl, th.al);
-    const size_t tbytes = fast ? (size_t)((tab.n + 15) & ~15) * sizeof(double) : 0;
-    const double lp0 = log_pi2_host[0], lp1 = log_pi2_host[1];
-    static const bool ring_form = [] {                       // FCD_SWEEP=ring: the shared-memory-ring kernel everywhere
-        const char* e = getenv("FCD_SWEEP");
-        return e != nullptr && strcmp(e, "ring") == 0;
-    }();
-    if (N >= 64 && !ring_form) {
-        // blocked forward substitution with the weights formed in the far loop (sweep_blocked_kernel<FUSED>)
-        constexpr int B = 16;
-        SweepFusedArgs fa;
-        fa.PT = PT;
-        fa.planeStride = planeStride;
-        fa.pitchC = pitchC;
-        fa.qF = qF;
-        for (int l = 0; l < 3; ++l) {
-            fa.al[l] = th.al[l];
-            fa.bl[l] = th.bl[l];
-        }
-        fa.tab = tab.g;
-        fa.lo7 = fast ? tab.lo >> 2 : 0;
-        fa.n7 = fast ? ((tab.lo + tab.n + 3) >> 2) - fa.lo7 : 0;
-        int T = N >= 700 ? 512 : ((N <= 512 && Ul > 2 * sm_count()) ? 128 : 256);
-        while (T < 512 && sweep_blocked_smem(N, T, B, fa.n7) > (size_t)(T == 128 ? 54 : 110) * 1024) T *= 2;
-        static const int forced_T = [] {
-            const char* e = getenv("FCD_SWEEP_T");
-            return e != nullptr ? atoi(e) : 0;
-        }();
-        if (forced_T == 128 || forced_T == 256 || forced_T == 512) T = forced_T;
-        const size_t smem = sweep_blocked_smem(N, T, B, fa.n7);
-        FCD_REQUIRE(smem <= kSmemBudget, "fcd_estep_qR_fused: N=%d needs %zu bytes of shared memory", N, smem);
-#define FCD_SWBF(T_, F_)                                                                                     \
-        do {                                                                                                 \
-            FCD_ALLOW_BIG_SMEM(sweep_blocked_kernel<T_, B, FCD_LOOKUP_REFERENCE, true, F_>);                 \
-            sweep_blocked_kernel<T_, B, FCD_LOOKUP_REFERENCE, true, F_><<<Ul, T_, smem, st>>>(               \
-                PsT, C, N, U, u0, lp0, lp1, qR, lqR, fa);                                                    \
-        } while (0)
-#define FCD_SWBF_T(F_)                                                                                       \
-        do {                                                                                                 \
-            if (T == 512) FCD_SWBF(512, F_);                                                                 \
-            else if (T == 256) FCD_SWBF(256, F_);                                                            \
-            else FCD_SWBF(128, F_);                                                                          \
-        } while (0)
-        if (fast) FCD_SWBF_T(true); else FCD_SWBF_T(false);
-#undef FCD_SWBF_T
-#undef FCD_SWBF
-        return check_launch("fcd_estep_qR_fused(blocked)");
-    }
-    FCD_REQUIRE(N <= 1024, "fcd_estep_qR_fused: the ring form needs N <= 1024 (got %d)", N);
-#define FCD_SWF(T, TC, PPC, RR, F)                                                                      \
-    do {                                                                                                \
-        const size_t smem = tbytes + (size_t)(PPC) * SweepSmem<T, RR>::padded;                          \
-        cudaFuncSetAttribute(sweep_fused_kernel<T, TC, 4, PPC, RR, F>,                                  \
-                             cudaFuncAttributeMaxDynamicSharedMemorySize,                               \
-                             (int)(kLogTabBytes + 128 + (PPC) * SweepSmem<T, RR>::padded));              \
-        sweep_fused_kernel<T, TC, 4, PPC, RR, F><<<(Ul + (PPC) - 1) / (PPC), ((T) + (TC)) * (PPC), smem, st>>>( \
-            PsT, PT, planeStride, pitchC, qF, fstate, pitchF, C, N, U, u0, Ul, lp0, lp1, th, tab, qR, lqR); \
-    } while (0)
-#define FCD_SWF_N(F)                                                                                    \
-    do {                                                                                                \
-        if (N <= 128) FCD_SWF(32, 32, 4, 1024, F);                                                      \
-        else if (N <= 256) FCD_SWF(64, 64, 4, 1024, F);                                                 \
-        else if (N <= 512) FCD_SWF(128, 128, 4, 1024, F);                                               \
-        else FCD_SWF(256, 128, 2, 2048, F);                                                             \
-    } while (0)
-    if (fast) FCD_SWF_N(true); else FCD_SWF_N(false);
-#undef FCD_SWF_N
-#undef FCD_SWF
-    return check_launch("fcd_estep_qR_fused");
 }
 
 }  // extern "C"

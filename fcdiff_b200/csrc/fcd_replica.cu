@@ -3,12 +3,10 @@
 // A relabelling changes WHICH columns of the (C, S) correlation matrix are controls and which are
 // patients -- nothing else.  The responsibility planes p_k(x), L(x) (fcd_common.cuh) depend on the
 // correlation value and (mu, sigma) only, so they are built ONCE for all S subjects
-// (fcd_resp_cache over every column, fcd_transpose_patients for the patient-major copy), and a
-// replica's inputs are selections from them:
+// (fcd_resp_cache over every column), and a replica's inputs are selections from them:
 //   * healthy sufficient statistics of the replica's control columns (fcdiff/fit.py:111-114, 171
 //     reduce to S1, S2): fcd_healthy_stats_cols;
-//   * edge-major planes of its patient columns: fcd_gather_columns (all planes in one launch);
-//   * patient-major planes of its patients: fcd_gather_rows.
+//   * edge-major planes of its patient columns: fcd_gather_columns (all planes in one launch).
 // Pure data movement (+ one masked sum): no exponential is taken again.
 #include "fcdiff_b200.h"
 #include "fcd_common.cuh"
@@ -64,22 +62,6 @@ gather_columns_kernel(const double* __restrict__ src, int64_t planeStrideS, int6
     }
 }
 
-// dst[p][j][0..pitch) = src[p][rows[j]][0..pitch): whole rows of `pitch` doubles (pitch even, 16-byte
-// aligned rows): 128-bit copies, one CTA per (plane, row) slice.
-__global__ void __launch_bounds__(256)
-gather_rows_kernel(const double* __restrict__ src, int64_t planeStrideS, int nplanes, const int32_t* __restrict__ rows,
-                   int U, int64_t pitch, double* __restrict__ dst, int64_t planeStrideD) {
-    const int64_t nrow = (int64_t)nplanes * U;
-    for (int64_t r = blockIdx.y; r < nrow; r += gridDim.y) {
-        const int64_t p = r / U, j = r - p * U;
-        const double2* s = reinterpret_cast<const double2*>(src + p * planeStrideS + (int64_t)__ldg(rows + j) * pitch);
-        double2* d = reinterpret_cast<double2*>(dst + p * planeStrideD + j * pitch);
-        for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < pitch / 2;
-             i += (int64_t)gridDim.x * blockDim.x)
-            d[i] = ldg_stream2(reinterpret_cast<const double*>(s + i));
-    }
-}
-
 }  // namespace fcd
 
 using namespace fcd;
@@ -120,22 +102,6 @@ int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, 
     gather_columns_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(src, planeStrideS, pitchS, nplanes, C, cols, U,
                                                                             dst, planeStrideD, pitchD);
     return check_launch("fcd_gather_columns");
-}
-
-int fcd_gather_rows(const double* src, int64_t planeStrideS, int32_t nplanes, const int32_t* rows, int32_t U,
-                    int64_t pitch, double* dst, int64_t planeStrideD, void* stream) {
-    FCD_REQUIRE(src != nullptr && rows != nullptr && dst != nullptr, "fcd_gather_rows: NULL argument");
-    FCD_REQUIRE(U >= 1 && nplanes >= 1 && pitch >= 2 && pitch % 2 == 0 &&
-                ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0 &&
-                planeStrideS % 2 == 0 && planeStrideD % 2 == 0,
-                "fcd_gather_rows: rows must be 16-byte aligned with an even pitch");
-    int64_t gx = (pitch / 2 + 255) / 256;
-    if (gx > 8) gx = 8;
-    int64_t gy = (int64_t)nplanes * U;
-    if (gy > 65535) gy = 65535;
-    gather_rows_kernel<<<dim3((unsigned)gx, (unsigned)gy), 256, 0, (cudaStream_t)stream>>>(src, planeStrideS, nplanes, rows,
-                                                                                          U, pitch, dst, planeStrideD);
-    return check_launch("fcd_gather_rows");
 }
 
 }  // extern "C"

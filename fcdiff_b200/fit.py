@@ -223,9 +223,6 @@ class UnsharedRegionFit(object):
         self.optimise_theta_sub = True
         self.update_mu_sigma = False  # re-estimate mu, sigma (disabled in the reference, fit.py:232-237)
         self.coded_estep = True       # K2 from the previous M-step's code plane when it still describes q_R
-        self.fused_sweep = False      # K2b: weights computed inside the sweep (no WT tensor; reference lookup, N <= 1024)
-        self.patient_major_planes = False  # K2b weights from patient-major copies of the planes (the first form) instead of
-        #                                    the E-step's edge-major planes (fcd_region_weights_em)
         self.elm_path = "auto"        # K3b form: "streams" (coded plane) | "tiered" | "auto" (coded unless most elements are undecided)
         self.convergence_rule = "reference"
         self.missing = "reject"       # "marginalize": NaN correlations are unobserved entries, integrated out
@@ -425,7 +422,7 @@ class UnsharedRegionFit(object):
         _lib.check(lib.fcd_edge_table(c0, Cl, _dev.ptr(nm), _dev.stream()), "fcd_edge_table")
         # `src` keeps the source objects alive: identity (`is`) cannot be faked by a recycled id()
         self._in = dict(key=key, src=(self.b, self.bt), C=C, H=H, U=U, c0=c0, Cl=Cl, u0=u0, Ul=Ul, pitchU=pitchU,
-                        bt=bt_dev, S1=S1, S2=S2, S0=S0, nm=nm, cache_key=None, P=None, L=None, PT=None, WT=None,
+                        bt=bt_dev, S1=S1, S2=S2, S0=S0, nm=nm, cache_key=None, P=None, L=None, WT=None,
                         ev_S=ev_S, b_dev=(b_dev if ev_S is not None else None))
         self._evals = []
         self._const = None
@@ -489,7 +486,7 @@ class UnsharedRegionFit(object):
                                                              _dev.ptr(S1), _dev.ptr(S2), _dev.ptr(S0), _dev.stream()),
                            "fcd_healthy_stats_cols_masked")
         self._in = dict(key=key, src=(None, None), C=C, H=H, U=U, c0=0, Cl=C, u0=0, Ul=U, pitchU=_dev.even(U),
-                        bt=None, S1=S1, S2=S2, S0=S0, nm=sp.nm, cache_key=None, P=None, L=None, PT=None, WT=None,
+                        bt=None, S1=S1, S2=S2, S0=S0, nm=sp.nm, cache_key=None, P=None, L=None, WT=None,
                         ev_S=None, b_dev=None)
         self._evals = []
         self._const = None
@@ -560,44 +557,10 @@ class UnsharedRegionFit(object):
         inp['PsE'] = None                           # dominant-state plane of the code pass: rebuilt with the planes
         inp['code_verR'] = None
         inp['cache_key'] = ckey
-        inp['PT'] = None
         inp['Pblk'] = None
         inp['PsT'] = inp['kcache'] = None
         self._evals = []
         self._const = None
-        return inp
-
-    def _ensure_patient_major(self):
-        """Patient-major responsibility planes PT [3][U_local][C] of ALL edges: the fused sweep's input, and the
-        region weights' when ``patient_major_planes`` is set (the default path reads the edge-major planes,
-        `_ensure_patient_planes`)."""
-        inp = self._ensure_cache()
-        if inp['PT'] is not None:
-            return inp
-        lib = _lib.load()
-        (C, U, u0, Ul) = (inp['C'], inp['U'], inp['u0'], inp['Ul'])
-        if self._shared is not None:
-            (sp, con, pat) = self._shared
-            PT = _dev.empty((3, U, sp.pitchC))
-            with _dev.timed(self.profile, "K0_gather_patient_major"):
-                _lib.check(lib.fcd_gather_rows(_dev.ptr(sp.PT), sp.S * sp.pitchC, 3, _dev.ptr(pat), U, sp.pitchC,
-                                               _dev.ptr(PT), U * sp.pitchC, _dev.stream()), "fcd_gather_rows")
-            inp['PT'] = PT
-            inp['PsT'] = inp['kcache'] = None
-            return inp
-        (src, planeStride, pitchU, uu0) = self._ensure_patient_planes()
-        pitchC = _dev.even(C)                      # rows are moved by 16-byte-granular bulk copies
-        PT = _dev.empty((3, max(Ul, 1), pitchC))       # every edge column is written below; only the pad is zeroed
-        if pitchC != C or Ul == 0:
-            PT[:, :, C:].zero_() if Ul > 0 else PT.zero_()
-        if Ul > 0:
-            with _dev.timed(self.profile, "K0_transpose"):
-                for k in range(3):
-                    _lib.check(lib.fcd_transpose_patients(_dev.ptr(src[k]), C, uu0 + Ul, pitchU, uu0, Ul,
-                                                          _dev.ptr(PT[k]), pitchC, _dev.stream()),
-                               "fcd_transpose_patients")
-        inp['PT'] = PT
-        inp['PsT'] = inp['kcache'] = None
         return inp
 
     def _ensure_patient_planes(self):
@@ -804,11 +767,8 @@ class UnsharedRegionFit(object):
         self._update_lps()
         if self._in is not None and self._in.get('ev_S') is not None:
             # host inputs still uploading: everything that needs the patient correlations only
-            # (planes, patient-major planes of the region sweep) is enqueued under the upload
-            if self.fused_sweep or self.patient_major_planes:
-                self._ensure_patient_major()
-            else:
-                self._ensure_patient_planes()
+            # (the planes of the E-step and of the region sweep) is enqueued under the upload
+            self._ensure_patient_planes()
         elif self.shards is not None and torch.is_tensor(self.bt):
             self._prefetch_patient_block()
 
@@ -1214,15 +1174,9 @@ class UnsharedRegionFit(object):
                                             _dev.ptr(lqR_new), _dev.stream()), "fcd_estep_qR")
             self._mR.set_dev(lqR_new, qR_new, (N, U, 2))
             return
-        fused = lookup == 0 and self.fused_sweep
-        use_pt = fused or self.patient_major_planes
-        if use_pt:
-            inp = self._ensure_patient_major()
-            (PT, pitchC) = (inp['PT'], inp['PT'].shape[2])
-        else:
-            (Pe, peStride, pePitch, pe_u0) = self._ensure_patient_planes()
-            inp = self._in
-            pitchC = _dev.even(inp['C'])
+        planes = self._ensure_patient_planes()
+        inp = self._in
+        pitchC = _dev.even(inp['C'])
         (N, H, U) = self._dims
         (C, u0, Ul) = (inp['C'], inp['u0'], inp['Ul'])
         (lqF, qF) = self._mF.get_dev()
@@ -1233,23 +1187,10 @@ class UnsharedRegionFit(object):
         if inp.get('PsT') is None:                 # dominant-state plane, gathered on first use (q_F settles early)
             inp['PsT'] = _dev.empty((max(Ul, 1), pitchC))
             inp['kcache'] = torch.full((max(C, 1),), 255, dtype=torch.uint8, device=_dev.device())
-        if fused and 3 <= N <= 8192:
-            # every edge's weights are computed once inside the sweep and kept in a shared-memory ring: no WT tensor
-            lqR_new, qR_new = lqR.clone(), qR.clone()
-            with _dev.timed(self.profile, "K2b_sweep_fused"):
-                _lib.check(lib.fcd_pstar_refresh(_dev.ptr(PT), max(Ul, 1) * pitchC, Ul, C, pitchC, _dev.ptr(fstate),
-                                                 _dev.ptr(inp['PsT']), _dev.ptr(inp['kcache']), _dev.stream()),
-                           "fcd_pstar_refresh")
-                _lib.check(lib.fcd_estep_qR_fused(
-                    _dev.ptr(inp['PsT']), _dev.ptr(PT), max(Ul, 1) * pitchC, pitchC, _dev.ptr(qF), _dev.ptr(fstate),
-                    fstate.numel(), C, N, U, u0, Ul, log_pi2, ctypes.byref(th), _dev.ptr(qR_new), _dev.ptr(lqR_new),
-                    _dev.stream()), "fcd_estep_qR_fused")
-        else:
-            if inp['WT'] is None:
-                inp['WT'] = _dev.empty((Ul, C, 2))
-            planes = ("pt", PT, max(Ul, 1) * pitchC) if use_pt else ("em", Pe, peStride, pePitch, pe_u0)
-            (lqR_new, qR_new) = self._weights_and_sweep(planes, inp['WT'], inp['PsT'], inp['kcache'], qF, fstate, th,
-                                                        C, N, U, u0, Ul, pitchC, log_pi2, lookup, lqR, qR)
+        if inp['WT'] is None:
+            inp['WT'] = _dev.empty((Ul, C, 2))
+        (lqR_new, qR_new) = self._weights_and_sweep(planes, inp['WT'], inp['PsT'], inp['kcache'], qF, fstate, th,
+                                                    C, N, U, u0, Ul, pitchC, log_pi2, lookup, lqR, qR)
         if self.shards is not None:
             self.shards.allgather_patients(lqR_new, qR_new, N, U)
         self._mR.set_dev(lqR_new, qR_new, (N, U, 2))
@@ -1258,23 +1199,16 @@ class UnsharedRegionFit(object):
                            lqR, qR, weights=True):
         """Region weights WT of the patients [u0, u0 + Ul) (K2b part 1, q_R-independent half of fcdiff/fit.py:187-194)
         unless ``weights`` is False (WT already holds them), then one Gauss-Seidel sweep (fit.py:176-198) on copies
-        of (lqR, qR); returns the copies.  ``planes``: ("pt", PT, planeStride) patient-major or
-        ("em", Pe, planeStride, pitchU, u0) edge-major responsibility planes."""
+        of (lqR, qR); returns the copies.  ``planes``: (Pe, planeStride, pitchU, u0), the edge-major responsibility
+        planes of `_ensure_patient_planes`."""
         lib = _lib.load()
         if weights:
+            (Pe, peStride, pePitch, pe_u0) = planes
             with _dev.timed(self.profile, "K2b_region_weights"):
-                if planes[0] == "pt":
-                    (_, PT, ptStride) = planes
-                    _lib.check(lib.fcd_region_weights(_dev.ptr(PT), ptStride, Ul, C, pitchC, _dev.ptr(qF),
-                                                      _dev.ptr(fstate), _dev.ptr(PsT), _dev.ptr(kcache),
-                                                      ctypes.byref(th), _dev.ptr(WT), _dev.stream()),
-                               "fcd_region_weights")
-                else:
-                    (_, Pe, peStride, pePitch, pe_u0) = planes
-                    _lib.check(lib.fcd_region_weights_em(_dev.ptr(Pe), peStride, pePitch, pe_u0, Ul, C, pitchC,
-                                                         _dev.ptr(qF), _dev.ptr(fstate), _dev.ptr(PsT),
-                                                         _dev.ptr(kcache), ctypes.byref(th), _dev.ptr(WT),
-                                                         _dev.stream()), "fcd_region_weights_em")
+                _lib.check(lib.fcd_region_weights_em(_dev.ptr(Pe), peStride, pePitch, pe_u0, Ul, C, pitchC,
+                                                     _dev.ptr(qF), _dev.ptr(fstate), _dev.ptr(PsT),
+                                                     _dev.ptr(kcache), ctypes.byref(th), _dev.ptr(WT),
+                                                     _dev.stream()), "fcd_region_weights_em")
         # (the sweep's in-place arrays are copied in the shadow of the weights kernel: until that launch the
         # host is on the critical path -- the GPU has only the E-step launched ahead to work on)
         lqR_new, qR_new = lqR.clone(), qR.clone()
@@ -1373,7 +1307,7 @@ class UnsharedRegionFit(object):
             pitchC = _dev.even(C)
             (PsT, WT) = (_dev.empty((U, pitchC)), _dev.empty((U, C, 2)))
             kcache = torch.full((C,), 255, dtype=torch.uint8, device=_dev.device())
-            planes = ("em", PL, C * pitchU, pitchU, 0)
+            planes = (PL, C * pitchU, pitchU, 0)
             log_pi2 = _lib.d3(np.log(_pi2(self.model.pi)))
             lookup = _LOOKUP[self.edge_lookup]
             res = _dev.SmallResult(1)

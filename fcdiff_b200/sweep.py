@@ -28,7 +28,6 @@ class SharedPlanes(object):
 
     X  [C][pitchS]       the correlations (zero padded to an even pitch)
     PL [4][C][pitchS]    p_0, p_1, p_2, L of every (edge, subject)      (fcd_resp_cache)
-    PT [3][S][pitchC]    p_k patient-major                              (fcd_transpose_patients)
     nm [C]               edge table
 
     ``missing``: the ``UnsharedRegionFit.missing`` of the fits that use the planes; with ``"marginalize"`` a NaN
@@ -51,7 +50,7 @@ class SharedPlanes(object):
         if missing == "marginalize" and bool(torch.isinf(x).any()):
             raise ValueError("corr must hold finite correlations or NaN")
         self.missing = missing
-        (self.C, self.S, self.pitchS, self.pitchC) = (C, S, _dev.even(S), _dev.even(C))
+        (self.C, self.S, self.pitchS) = (C, S, _dev.even(S))
         if self.pitchS == S:
             self.X = x.contiguous()
         else:
@@ -65,10 +64,6 @@ class SharedPlanes(object):
                       else (lib.fcd_resp_cache, "fcd_resp_cache"))
         _lib.check(fn(_dev.ptr(self.X), C, S, self.pitchS, ctypes.byref(th), _dev.ptr(self.PL), C * self.pitchS,
                       _dev.ptr(self.PL[3]), _dev.stream()), name)
-        self.PT = _dev.zeros((3, S, self.pitchC))
-        for k in range(3):
-            _lib.check(lib.fcd_transpose_patients(_dev.ptr(self.PL[k]), C, S, self.pitchS, 0, S, _dev.ptr(self.PT[k]),
-                                                  self.pitchC, _dev.stream()), "fcd_transpose_patients")
         self.nm = _dev.empty((max(C, 1),), torch.int32)
         _lib.check(lib.fcd_edge_table(0, C, _dev.ptr(self.nm), _dev.stream()), "fcd_edge_table")
 

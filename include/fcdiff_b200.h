@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define FCD_VERSION 120
+#define FCD_VERSION 121
 
 #if defined(__GNUC__)
 #define FCD_API __attribute__((visibility("default")))
@@ -252,12 +252,11 @@ FCD_API int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const
 
 /* Replica sweeps (BASELINE.json configs[4]; no reference counterpart -- the reference stops at one
  * fit, fcdiff/fit.py:56-82): the responsibility planes of ALL S subjects are built once
- * (fcd_resp_cache on every column of the (C, S) correlation matrix, fcd_transpose_patients), and a
- * relabelling selects from them (csrc/fcd_replica.cu):
+ * (fcd_resp_cache on every column of the (C, S) correlation matrix), and a relabelling selects from
+ * them (csrc/fcd_replica.cu):
  *   fcd_healthy_stats_cols: S1 / S2 of fcd_healthy_stats over the columns cols[0..H) of X [C][pitchS];
- *   fcd_gather_columns: dst[p][c][j] = src[p][c][cols[j]], j < U (columns U..pitchD-1 zero), p < nplanes;
- *   fcd_gather_rows: dst[p][j][:] = src[p][rows[j]][:] (rows of `pitch` doubles, 16-byte aligned).
- * cols / rows: int32 device arrays. */
+ *   fcd_gather_columns: dst[p][c][j] = src[p][c][cols[j]], j < U (columns U..pitchD-1 zero), p < nplanes.
+ * cols: int32 device array. */
 FCD_API int fcd_healthy_stats_cols(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
                            double* S1, double* S2, void* stream);
 /* fcd_healthy_stats_cols over the observed (non-NaN) entries, with S0 as fcd_healthy_stats_masked. */
@@ -266,32 +265,31 @@ FCD_API int fcd_healthy_stats_cols_masked(const double* X, int64_t C, int64_t pi
 FCD_API int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, int32_t nplanes, int64_t C,
                        const int32_t* cols, int32_t U, double* dst, int64_t planeStrideD, int64_t pitchD,
                        void* stream);
-FCD_API int fcd_gather_rows(const double* src, int64_t planeStrideS, int32_t nplanes, const int32_t* rows, int32_t U,
-                    int64_t pitch, double* dst, int64_t planeStrideD, void* stream);
 
-/* Patient-major copy of an edge-major plane: dst[u - u0][c] = src[c][u]
- * for u in [u0, u0+Ul), c in [0, C).  Built once per fit. */
-FCD_API int fcd_transpose_patients(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                           int32_t u0, int32_t Ul, double* btT, int64_t pitchC, void* stream);
-
-/* K2b part 1 -- q_R-independent half of `_update_lq_R` (fcdiff/fit.py:187-194):
- *   W_l[c,u] = sum_k qF[c,k] * log M_kl(bt[c][u])   (PT[k][u][c] are the patient-major
- *   copies [Ul][pitchC] of the responsibility planes)
+/* K2b part 1 -- q_R-independent half of `_update_lq_R` (fcdiff/fit.py:187-194) for the patients [u0, u0 + Ul),
+ * from the E-step's edge-major responsibility planes Pe [3][C][pitchU] (fcd_resp_cache):
+ *   W_l[c,u] = sum_k qF[c,k] * log M_kl(bt[c][u])
  * up to an additive per-(c,u) constant common to all l, which cancels in the
  * normalisation of fit.py:196 (see DESIGN.md).  Only l_0 - l_1 survives that
  * normalisation, so the tensor holds two numbers per edge-patient (16 bytes):
  *   WT[u][c] = { W_0 - W_2, W_2 - W_1 }     ([Ul][C][2], patient-major)
  * qF / fstate cover ALL edges.
- * PsT / kcache (both or neither): caller-kept [Ul][pitchC] plane of each edge's
- * dominant-state responsibility and the [C] states it was gathered for (255 =
- * never; set by the caller once); the call refreshes the columns of edges whose
- * state changed and then reads one coalesced plane instead of three. */
-FCD_API int fcd_region_weights(const double* PT, int64_t planeStride, int32_t Ul, int64_t C, int64_t pitchC,
-                       const double* qF, const uint8_t* fstate, double* PsT, uint8_t* kcache,
-                       const fcd_theta* theta_host, double* WT, void* stream);
+ * PsT / kcache: caller-kept [Ul][pitchC] plane of each edge's dominant-state
+ * responsibility and the [C] states it was gathered for (255 = never; set by the
+ * caller once).  The call first refreshes the columns of edges whose state changed
+ * (fcd_pstar_refresh_em: one transposing pass over those edges' rows of Pe, all of
+ * them the first time) and then reads one coalesced plane instead of three; the
+ * three-plane path of an unpeaked edge reads Pe with a stride. */
+FCD_API int fcd_region_weights_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,
+                          int64_t pitchC, const double* qF, const uint8_t* fstate, double* PsT, uint8_t* kcache,
+                          const fcd_theta* theta_host, double* WT, void* stream);
+/* The refresh of PsT / kcache alone (see fcd_region_weights_em) for the current peak
+ * states, without computing region weights. */
+FCD_API int fcd_pstar_refresh_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,
+                         int64_t pitchC, const uint8_t* fstate, double* PsT, uint8_t* kcache, void* stream);
 
 /* K2b part 2 -- Gauss-Seidel sweep of `_update_lq_R` (fcdiff/fit.py:176-198)
- * for the patients [u0, u0+Ul) from WT [Ul][C][2] (fcd_region_weights).  qR/lqR are the full [N][U][2] arrays; only
+ * for the patients [u0, u0+Ul) from WT [Ul][C][2] (fcd_region_weights_em).  qR/lqR are the full [N][U][2] arrays; only
  * the [u0, u0+Ul) columns are read and written.  log_pi2_host = {log(1-pi),
  * log(pi)} (the 2-vector convention of test_fcdiff/test_fit.py:477-487).
  * edge_lookup: FCD_LOOKUP_REFERENCE reproduces nm_to_c(n, m) for all m != n
@@ -299,38 +297,6 @@ FCD_API int fcd_region_weights(const double* PT, int64_t planeStride, int32_t Ul
 FCD_API int fcd_estep_qR(const double* WT, int64_t C, int32_t N, int32_t U, int32_t u0, int32_t Ul,
                  const double* log_pi2_host, int32_t edge_lookup,
                  double* qR, double* lqR, void* stream);
-
-/* K2b fused -- the whole of `_update_lq_R` (fcdiff/fit.py:176-198) for the
- * patients [u0, u0+Ul) with edge_lookup = FCD_LOOKUP_REFERENCE, without the WT
- * tensor: every edge's weights W[c][l] = sum_k qF[c,k] log M_kl are computed once
- * inside the sweep from the dominant-state plane PsT (kept by
- * fcd_region_weights' refresh; row pitch pitchC even), streamed through shared
- * memory by TMA, and held in a shared-memory ring while the sweep's window
- * passes.  PT (3 planes) is read only for edges whose q_F is not peaked.
- * fstate: peak states of ALL edges, padded to pitchF >= pitchC bytes (pitchF %
- * 16 == 0).  3 <= N <= 1024.  Other arguments as fcd_estep_qR. */
-FCD_API int fcd_estep_qR_fused(const double* PsT, const double* PT, int64_t planeStride, int64_t pitchC,
-                       const double* qF, const uint8_t* fstate, int64_t pitchF,
-                       int64_t C, int32_t N, int32_t U, int32_t u0, int32_t Ul,
-                       const double* log_pi2_host, const fcd_theta* theta_host,
-                       double* qR, double* lqR, void* stream);
-
-/* Refreshes the dominant-state plane PsT / kcache (see fcd_region_weights) for the
- * current peak states without computing region weights. */
-FCD_API int fcd_pstar_refresh(const double* PT, int64_t planeStride, int32_t Ul, int64_t C, int64_t pitchC,
-                      const uint8_t* fstate, double* PsT, uint8_t* kcache, void* stream);
-
-/* The same two entries on the E-step's EDGE-major planes Pe [3][C][pitchU] (fcd_resp_cache), patients
- * [u0, u0 + Ul): no patient-major copy of the planes is needed -- the dominant-state plane PsT [Ul][pitchC] is
- * gathered by one transposing pass over the rows of the edges whose state changed (all of them the first time),
- * and the three-plane path of an unpeaked edge reads Pe with a stride.  Same results as fcd_region_weights /
- * fcd_pstar_refresh on the transposed planes (fcdiff/fit.py:176-198 needs the weights of every edge of a patient;
- * the layout they are read from is this implementation's business). */
-FCD_API int fcd_pstar_refresh_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,
-                         int64_t pitchC, const uint8_t* fstate, double* PsT, uint8_t* kcache, void* stream);
-FCD_API int fcd_region_weights_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,
-                          int64_t pitchC, const double* qF, const uint8_t* fstate, double* PsT, uint8_t* kcache,
-                          const fcd_theta* theta_host, double* WT, void* stream);
 
 /* K3a -- M-step sums; replaces `_update_pi` / `_update_gamma`
  * (fcdiff/fit.py:208-220).  out[0..2] = sum_c exp(lqF[c,k]),

@@ -21,7 +21,7 @@ for rep in range(3):
     fit._init_lps(N, H, U); t1 = sync()
     fit._ensure_inputs(); t2 = sync()
     fit._update_lps(); fit._ensure_cache(); t3 = sync()
-    fit._ensure_patient_major(); t4 = sync()
+    fit._ensure_patient_planes(); t4 = sync()
     e0 = fit._eval_energy(); t5 = sync()
     fit._update_lq_F(); t6 = sync()
     fit._update_lq_R(); t7 = sync()
@@ -29,7 +29,7 @@ for rep in range(3):
     fit._update_lps(); e1 = fit._eval_energy(); t9 = sync()
     a = fit._lq_F; c = fit._lq_R; t10 = sync()
     if rep == 2:
-        names = ["init_lps", "upload+healthy", "resp_cache", "patient_major", "energy0", "K2", "K2b", "theta(nfev=%d)" % fit.n_objective_evals[-1] if fit.n_objective_evals else "theta", "energy1", "download"]
+        names = ["init_lps", "upload+healthy", "resp_cache", "patient_planes", "energy0", "K2", "K2b", "theta(nfev=%d)" % fit.n_objective_evals[-1] if fit.n_objective_evals else "theta", "energy1", "download"]
         ts = [t0, t1, t2, t3, t4, t5, t6, t7, t8, t9, t10]
         for i, nm in enumerate(names):
             print("%-18s %7.2f ms" % (nm, (ts[i + 1] - ts[i]) * 1e3))

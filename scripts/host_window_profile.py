@@ -27,7 +27,7 @@ for rep in range(3):
     (fit.b, fit.bt) = (b, bt); fit.max_iters = 10; fit.rel_tol = -1.0
     if rep == 2:
         for n in ("_update_lq_F", "_update_lq_R", "_update_theta", "_update_lps", "_eval_energy", "_is_converged",
-                  "_ensure_inputs", "_ensure_cache", "_ensure_patient_major", "_theta", "_energy_key", "_speculative_estep",
+                  "_ensure_inputs", "_ensure_cache", "_ensure_patient_planes", "_theta", "_energy_key", "_speculative_estep",
                   "_update_pi_gamma", "_update_theta_sub", "_solver_context", "_build_streams"):
             wrap(fit, n)
     torch.cuda.synchronize(); t0 = time.perf_counter(); fit.run(); torch.cuda.synchronize()

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """K2 in isolation on FIXED inputs: config 3 fitted for a few iterations, then the coded E-step launched
-repeatedly on the state the last M-step left (same code plane, same records) -- per-variant timings that do not
-depend on the fit's trajectory.  usage: python scripts/k2_probe.py [iters ...]   (FCD_K2DBG values via K2_DBG="0 1 ...")"""
+repeatedly on the state the last M-step left (same code plane, same records) -- timings that do not depend on
+the fit's trajectory.  usage: python scripts/k2_probe.py [iters ...]"""
 import os
 import sys
 
@@ -14,7 +14,6 @@ import fcdiff_b200 as fcdiff  # noqa: E402
 
 def main():
     iters = [int(a) for a in sys.argv[1:]] or [2, 8]
-    variants = os.environ.get("K2_DBG", "").split() or [""]
     (N, H, U) = (400, 500, 500)
     model = fcdiff.UnsharedRegionModel()
     (_, _, _, _, b, bt) = model.sample_device(N, H, U)
@@ -32,19 +31,16 @@ def main():
             print("after %d iterations: full records %d (rows with any %d, unpeaked rows %d), half records %d (rows > 64: %d)" % (
                 it, int(cnt[:, 0][cnt[:, 0] != 3 * U].sum()), int(((cnt[:, 0] > 0) & (cnt[:, 0] != 3 * U)).sum()),
                 int((cnt[:, 0] == 3 * U).sum()), int(cnt[:, 1].sum()), int((cnt[:, 1] > 64).sum())))
-        for v in variants:
-            if v:
-                os.environ["FCD_K2DBG"] = v
-            ms = []
-            for r in range(40):
-                (e0, e1) = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-                e0.record()
-                f._update_lq_F()
-                e1.record()
-                torch.cuda.synchronize()
-                ms.append(e0.elapsed_time(e1))
-            ms = sorted(ms[4:])
-            print("  iters %d  variant %-4s  K2 min %.4f  median %.4f ms" % (it, v or "-", ms[0], ms[len(ms) // 2]))
+        ms = []
+        for r in range(40):
+            (e0, e1) = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+            e0.record()
+            f._update_lq_F()
+            e1.record()
+            torch.cuda.synchronize()
+            ms.append(e0.elapsed_time(e1))
+        ms = sorted(ms[4:])
+        print("  iters %d  K2 min %.4f  median %.4f ms" % (it, ms[0], ms[len(ms) // 2]))
 
 
 if __name__ == "__main__":

@@ -42,7 +42,7 @@ def main():
         from fcdiff_b200 import dist as fdist
         shards = fdist.init_from_env("nccl")
     # config 1; a cut of config 2 (AAL-90); 70 regions: the blocked region sweep (N >= 64: cp.async tiles, L2 bulk
-    # prefetch, double-buffered shared-memory tiles between the solver warp and the helper warps) and its fused form
+    # prefetch, double-buffered shared-memory tiles between the solver warp and the helper warps)
     for (N, H, U) in ((10, 20, 20), (40, 50, 50), (70, 12, 16)):
         (b, bt) = problem(N, H, U, N)
         one_fit(b, bt, shards)
@@ -51,7 +51,6 @@ def main():
         one_fit(b, bt, edge_lookup="symmetric")
         one_fit(b, bt, elm_path="tiered", coded_estep=False)
         one_fit(b, bt, elm_path="streams")
-        one_fit(b, bt, fused_sweep=True)
         one_fit(b, bt, update_mu_sigma=True, edge_lookup="symmetric")
         for solver in ("newton",):
             if hasattr(fcdiff.fit.UnsharedRegionFit(), "theta_solver"):

@@ -1,29 +1,26 @@
-"""Launch-shape study of the region sweep (fcd_estep_qR) on one GPU: the one-region-per-step kernel against the
-blocked forward substitution, per thread count, at the shapes the bench meets.  The launch shape is chosen
-once per process (FCD_SWEEP / FCD_SWEEP_T), so every variant runs in a child process.
-    python scripts/sweep_bench.py            # table to stdout
+"""Timing of the region sweep (fcd_estep_qR) on one GPU at the shapes the bench meets, in the launch shape the
+code chooses from the region and patient counts.
+    python scripts/sweep_bench.py                # table to stdout
+    python scripts/sweep_bench.py 400x63 1131x63 # only these (regions x patients) shapes
 """
 import os
-import subprocess
 import sys
 
+import numpy as np
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+from fcdiff_b200 import _dev, _lib      # noqa: E402
+
 SHAPES = [(400, 500), (400, 63), (566, 250), (800, 125), (1131, 63), (1000, 1000), (1000, 125)]
-if os.environ.get("FCD_SWEEP_SHAPES"):                       # e.g. "400x63,1131x63" (profiling one shape under ncu)
-    SHAPES = [tuple(int(v) for v in t.split("x")) for t in os.environ["FCD_SWEEP_SHAPES"].split(",")]
-VARIANTS = [("stepwise", {"FCD_SWEEP": "stepwise"}), ("blocked/auto", {}), ("auto, 1 CTA", {"FCD_SWEEP_CLUSTER": "1"})] + \
-           [("blocked/%d" % t, {"FCD_SWEEP_T": str(t), "FCD_SWEEP_CLUSTER": "1"}) for t in (128, 256, 512)] + \
-           [("cluster/%d" % t, {"FCD_SWEEP_T": str(t), "FCD_SWEEP_CLUSTER": "2"}) for t in (256, 512)]
 
 
-def child():
-    import numpy as np
-    import torch
-    sys.path.insert(0, ROOT)
-    from fcdiff_b200 import _dev, _lib
+def main(shapes):
     lib = _lib.load()
-    out = []
-    for (N, Ul) in SHAPES:
+    print("%-22s %12s   %s" % ("N, patients, regime", "time", "checksum"))
+    for (N, Ul) in shapes:
         C = N * (N - 1) // 2
         for (regime, scale) in (("undecided", 0.02), ("decided", 3.0)):
             g = torch.Generator(device="cuda").manual_seed(N + Ul)
@@ -47,32 +44,10 @@ def child():
                 run()
             e1.record()
             torch.cuda.synchronize()
-            out.append("%d,%d,%s,%.1f,%.6f" % (N, Ul, regime, e0.elapsed_time(e1) / R * 1e3, float(q.reshape(-1, 2)[:, 0].sum().item())))
+            print("%-22s %9.1f us   %.6f" % ("%d, %d, %s" % (N, Ul, regime), e0.elapsed_time(e1) / R * 1e3,
+                                             float(q.reshape(-1, 2)[:, 0].sum().item())))
             del WT, q, lq
-    print("\n".join(out))
-
-
-def main():
-    table = {}
-    for (name, env) in VARIANTS:
-        e = dict(os.environ, **env)
-        r = subprocess.run([sys.executable, os.path.abspath(__file__), "child"], env=e, capture_output=True, text=True)
-        if r.returncode != 0:
-            print(name, "failed:", r.stderr[-400:])
-            continue
-        for line in r.stdout.strip().splitlines():
-            (N, Ul, regime, us, chk) = line.split(",")
-            table.setdefault((int(N), int(Ul), regime), {})[name] = (float(us), float(chk))
-    names = [v[0] for v in VARIANTS]
-    print("%-22s" % "N, patients, regime" + "".join("%12s" % n for n in names) + "   checksum spread")
-    for (key, row) in table.items():
-        chks = [row[n][1] for n in names if n in row]
-        print("%-22s" % ("%d, %d, %s" % key) + "".join("%9.1f us" % row[n][0] if n in row else "%12s" % "-" for n in names)
-              + "   %.2e" % (max(chks) - min(chks)))
 
 
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "child":
-        child()
-    else:
-        main()
+    main([tuple(int(v) for v in a.split("x")) for a in sys.argv[1:]] or SHAPES)

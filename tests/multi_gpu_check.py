@@ -16,9 +16,8 @@ from fcdiff_b200 import dist as fdist       # noqa: E402
 from oracle import iar_oracle as O          # noqa: E402
 
 
-def run(b, bt, shards, device_shards=False, n_edges=None, fused=False):
+def run(b, bt, shards, device_shards=False, n_edges=None):
     fit = fcdiff.fit.UnsharedRegionFit()
-    fit.fused_sweep = fused
     fit.model = fcdiff.UnsharedRegionModel()
     fit.model.eta += 0.1
     fit.b, fit.bt = b, bt
@@ -41,8 +40,7 @@ def main():
         (c0, Cl) = shards.span(C)
         dev = run(torch.from_numpy(b[c0:c0 + Cl]).cuda(), torch.from_numpy(bt[c0:c0 + Cl]).cuda(), shards,
                   device_shards=True, n_edges=C)             # device edge shards + all-to-all re-layout
-        fus = run(b, bt, shards, fused=True)                 # fused sweep on the patient shards
-        for name, f in (("host-sharded", sharded), ("device-sharded", dev), ("host-sharded, fused sweep", fus)):
+        for name, f in (("host-sharded", sharded), ("device-sharded", dev)):
             e = np.max(np.abs(np.array(f.energy) / np.array(single.energy) - 1))
             dF = np.max(np.abs(f._lq_F - single._lq_F))
             dR = np.max(np.abs(f._lq_R - single._lq_R))

@@ -220,11 +220,13 @@ def test_patient_gather_staging_roundtrip(N, U, world):
 
 
 @pytest.mark.parametrize("N,U,lookup,scale",
-                         [(37, 5, 0, 0.05), (600, 3, 0, 0.05), (600, 2, 1, 0.05), (1100, 2, 0, 0.05), (1400, 2, 1, 0.05),
+                         [(37, 5, 0, 0.05),                 # N < 64: one region per step
+                          # blocked forward substitution (N >= 64): 256 threads below 700 regions, 512 from 700 on
+                          (600, 3, 0, 0.05), (600, 2, 1, 0.05), (1100, 2, 0, 0.05), (1400, 2, 1, 0.05),
                           (2100, 1, 0, 0.05),
-                          (530, 300, 0, 0.05),              # U >= 2 x SMs: the compact launch shapes
-                          # blocked forward substitution (N >= 64): whole / ragged last blocks, both
-                          # lookups, the three thread counts, shared memory beyond 48 KB
+                          # more than 2 x SMs patients: 128 threads up to 512 regions, 256 above
+                          (100, 300, 1, 0.05), (530, 300, 0, 0.05),
+                          # whole / ragged last blocks, both lookups, shared memory beyond 48 KB
                           (64, 9, 0, 0.05), (65, 4, 1, 0.05), (96, 3, 0, 0.05), (100, 3, 1, 0.05), (400, 6, 0, 0.05),
                           (400, 5, 1, 0.05), (3300, 1, 1, 0.05),
                           # large weights: most regions come out decided (|l_0 - l_1| > 37.5, the short form of
@@ -236,7 +238,8 @@ def test_patient_gather_staging_roundtrip(N, U, world):
                           (800, 3, 1, 0.5), (715, 2, 0, 0.02)])
 def test_sweep_launch_shapes_match_numpy(N, U, lookup, scale):
     """Gauss-Seidel sweep of fit.py:184-197 over the two weight differences, for every launch shape of
-    fcd_estep_qR (regions per thread / warps per patient depend on N), both edge lookups."""
+    fcd_estep_qR (the kernel and its threads per patient depend on N and on the number of patients), both edge
+    lookups."""
     lib = _lib.load()
     rng = np.random.RandomState(N + U)
     C = N * (N - 1) // 2
@@ -265,24 +268,3 @@ def test_sweep_launch_shapes_match_numpy(N, U, lookup, scale):
             want_q[n, u] = np.exp(l)
     nptest.assert_allclose(lqd.cpu().numpy().reshape(N, U, 2), want_lq, rtol=1e-9, atol=1e-11)
     nptest.assert_allclose(qd.cpu().numpy().reshape(N, U, 2), want_q, rtol=1e-9, atol=1e-13)
-
-
-def test_alternative_kernel_forms_in_a_child_process():
-    """Kernel forms selected by an environment variable read once per process: the row-group form of the coded
-    E-step (FCD_K2=rows, csrc/fcd_estep_rows.cu) and the one-region-per-step sweep (FCD_SWEEP=stepwise) run
-    the same parity tests as the defaults, in a child interpreter."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get("FCD_CHILD_FORMS"):
-        pytest.skip("already inside the child run")
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, FCD_K2="rows", FCD_SWEEP="stepwise", FCD_CHILD_FORMS="1")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu", "-p", "no:cacheprovider",
-                        os.path.join(root, "tests", "test_gpu_code_pass.py"),
-                        os.path.join(root, "tests", "test_gpu_parity.py"),
-                        "-k", "code_plane_and_evaluator or sweep_launch_shapes or fused_steps or config3_properties "
-                              "or config3_two_iterations or cfg2_full_run or config4_edge_shard"],
-                       cwd=root, env=env, capture_output=True, text=True, timeout=1500)
-    tail = "\n".join(r.stdout.splitlines()[-25:]) + "\n" + "\n".join(r.stderr.splitlines()[-5:])
-    assert r.returncode == 0, tail

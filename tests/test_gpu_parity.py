@@ -310,34 +310,23 @@ def test_speculative_estep_is_bit_identical(N, H, U, iters):
 
 @pytest.mark.parametrize("N,H,U,iters,lookup", [(12, 9, 11, 3, "reference"), (33, 20, 70, 4, "symmetric"),
                                                  (90, 50, 50, 4, "reference"), (120, 30, 333, 5, "reference")])
-def test_region_weights_from_edge_major_planes_is_bit_identical(N, H, U, iters, lookup):
+def test_region_weights_from_edge_major_planes_vs_oracle(N, H, U, iters, lookup):
     """The region weights read the E-step's edge-major planes (fcd_region_weights_em: the dominant-state plane
-    gathered by a transposing pass, unpeaked edges through strided reads); the first form made patient-major
-    copies of the three planes for it (`patient_major_planes = True`).  Same numbers bit for bit -- the small
-    problems keep unpeaked edges and undecided regions for several iterations, the odd sizes exercise the
-    partial 32 x 32 tiles of the gather."""
+    gathered by a transposing pass, unpeaked edges through strided reads).  The small problems keep unpeaked
+    edges and undecided regions for several iterations, the odd sizes exercise the partial 32 x 32 tiles of the
+    gather."""
     (_, _, _, _, b, bt) = O.sample(O.Theta(), N, H, U, np.random.RandomState(7 * N + U))
-
-    def run(pm):
-        fit = _fit_for(b, bt, eta_shift=0.1, solver="newton")
-        fit.patient_major_planes = pm
-        fit.edge_lookup = lookup
-        fit.max_iters = iters
-        fit.rel_tol = -1.0
-        fit.run()
-        return fit
-
-    (f0, f1) = (run(False), run(True))
-    assert f0.energy == f1.energy
-    nptest.assert_array_equal(f0._lq_R, f1._lq_R)
-    nptest.assert_array_equal(f0._lq_F, f1._lq_F)
-    assert f0._in.get('PT') is None and f1._in.get('PT') is not None
-    # and against the oracle (polished optimiser = the device Newton solver's fixed point)
+    fit = _fit_for(b, bt, eta_shift=0.1, solver="newton")
+    fit.edge_lookup = lookup
+    fit.max_iters = iters
+    fit.rel_tol = -1.0
+    fit.run()
+    # against the oracle (polished optimiser = the device Newton solver's fixed point)
     tho = O.Theta()
     tho.eta += 0.1
     out = O.run(b, bt, tho, max_iters=iters, rel_tol=-1.0, edge_lookup=lookup, polish=True)
-    nptest.assert_allclose(f0.energy, out["energy"], rtol=1e-6)
-    nptest.assert_allclose(np.exp(f0._lq_R), np.exp(out["lq_R"]), rtol=1e-6, atol=1e-300)
+    nptest.assert_allclose(fit.energy, out["energy"], rtol=1e-6)
+    nptest.assert_allclose(np.exp(fit._lq_R), np.exp(out["lq_R"]), rtol=1e-6, atol=1e-300)
 
 
 def test_newton_solver_reaches_active_bounds_and_leaves_the_table_window():
@@ -427,14 +416,8 @@ def test_fused_steps_vs_oracle(N, H, U, lookup, peaked):
     exp_F = O.update_lq_F(th.gamma, lpB, lM, lq_R)
     nptest.assert_allclose(fit._lq_F, exp_F, rtol=1e-9, atol=1e-10)
     nptest.assert_allclose(np.exp(fit._lq_F).sum(axis=2), 1.0, rtol=1e-12)
-    # K2b (both forms: region weights + sweep over WT, and the fused sweep)
+    # K2b: region weights + sweep over WT
     exp_R = O.update_lq_R(np.array([1 - th.pi, th.pi]), exp_F, lM, lq_R, lookup)
-    if lookup == "reference" and N >= 3:
-        fit.fused_sweep = True
-        fit._update_lq_R()
-        nptest.assert_allclose(fit._lq_R, exp_R, rtol=1e-9, atol=1e-10)
-        fit._lq_R = lq_R
-        fit.fused_sweep = False
     fit._update_lq_R()
     nptest.assert_allclose(fit._lq_R, exp_R, rtol=1e-9, atol=1e-10)
     # K3a
@@ -690,15 +673,6 @@ def test_config3_properties(N, H, U):
     whole = estep(0, C, rstate)
     nptest.assert_array_equal(estep(a, e, rstate), whole[a * 3:])
     nptest.assert_allclose(estep(0, C, r_mixed), whole, rtol=1e-12, atol=1e-9)
-    # -- K2b: the fused sweep (weights from TMA-streamed planes) equals region weights + sweep over WT
-    lqR0 = fit._lq_R.copy()
-    fit.fused_sweep = True
-    fit._update_lq_R()
-    fused = fit._lq_R.copy()
-    fit._lq_R = lqR0
-    fit.fused_sweep = False
-    fit._update_lq_R()
-    nptest.assert_allclose(fused, fit._lq_R, rtol=1e-9, atol=1e-9)
 
 
 @pytest.mark.parametrize("N,H,U", [(4, 2, 3), (10, 20, 20), (24, 8, 129), (33, 17, 300)])
