@@ -147,6 +147,9 @@ SIGNATURES = {
     "fcd_corr_clean_workspace_bytes": (c_int64, [c_int32, c_int32, c_int32, c_int32]),
     "fcd_corr_fisherz_clean": (c_int, [_P, c_int32, c_int32, c_int32, _P, _P, c_int32, _P, c_int64, c_int32, c_int32,
                                        c_int32, _P, _P, _P]),
+    "fcd_corr_partial_workspace_bytes": (c_int64, [c_int32, c_int32, c_int32, c_int32]),
+    "fcd_corr_partial": (c_int, [_P, c_int32, c_int32, c_int32, _P, _P, c_int32, c_double, _P, c_int64, c_int32,
+                                 c_int32, c_int32, _P, _P, _P, _P, _P]),
 }
 
 class SolverState(ctypes.Structure):

@@ -11,6 +11,10 @@ transformed (``arctanh``) by default.  Oracle: ``numpy.corrcoef`` +
 Cleaned time series (``sample_mask`` / ``confounds``, ``fcd_corr_fisherz_clean``): frames can be censored
 per subject, subjects can differ in length, and nuisance regressors are projected out of every region on
 the GPU before the correlations.  Oracle: ``oracle/clean.py``.
+
+Partial correlations (``kind="partial"``, ``fcd_corr_partial``): per subject the cleaned rows in fp64, a
+Ledoit-Wolf shrunk correlation matrix and its inverse P on the GPU, r_nm = -P_nm / sqrt(P_nn P_mm).
+Oracle: ``oracle/partial.py``.
 """
 import numpy as np
 import torch
@@ -20,6 +24,31 @@ from .util import N_to_C
 
 
 MAX_CONFOUNDS = 64
+KINDS = ("pearson", "partial")
+
+
+def check_kind(kind, shrinkage):
+    """Validates ``kind`` and ``shrinkage`` on the host; returns the shrinkage the library takes (-1.0 for
+    Ledoit-Wolf).  Raises ``ValueError`` for an unknown kind or a shrinkage that is neither
+    ``"ledoit-wolf"`` nor a number in [0, 1]."""
+    if kind not in KINDS:
+        raise ValueError("kind: expected one of %s, got %r" % (KINDS, kind))
+    if isinstance(shrinkage, str):
+        if shrinkage != "ledoit-wolf":
+            raise ValueError("shrinkage: expected \"ledoit-wolf\" or a number in [0, 1], got %r" % shrinkage)
+        return -1.0
+    d = float(shrinkage)
+    if not 0.0 <= d <= 1.0:
+        raise ValueError("shrinkage: %r outside [0, 1]" % (shrinkage,))
+    return d
+
+
+def _check_not_singular(n, N, K, d):
+    """shrinkage = 0 leaves the sample correlation matrix, singular when a subject keeps n_s <= N + K frames."""
+    if d == 0.0 and (n <= N + K).any():
+        s = int(np.argmax(n <= N + K))
+        raise ValueError("shrinkage=0: subject %d keeps %d frames, its correlation matrix of %d regions after %d "
+                         "confounds is singular (needs more than %d)" % (s, int(n[s]), N, K, N + K))
 
 
 def pack_clean(ts, sample_mask=None, confounds=None):
@@ -110,20 +139,26 @@ def pack_clean(ts, sample_mask=None, confounds=None):
 
 
 def correlations_device(ts_dev, fisher=True, out=None, s0=0, missing=False, sample_mask=None, confounds=None,
-                        rank=None):
+                        rank=None, kind="pearson", shrinkage="ledoit-wolf", shrinkage_out=None):
     """ts_dev: float32 CUDA tensor (S, N, T).  Returns / fills a float64 CUDA
     tensor (C, pitch) with columns [s0, s0 + S) written.  ``missing``: see
     :func:`correlations`.  ``sample_mask`` ((S, T) bool) and ``confounds``
     ((S, T, K) float64), as arrays or CUDA tensors, select the cleaned path
     (:func:`correlations`; checked as :func:`pack_clean` does); ``rank``: an
-    optional (S,) int32 CUDA tensor that receives the confounds kept per subject."""
+    optional (S,) int32 CUDA tensor that receives the confounds kept per subject.
+    ``kind`` / ``shrinkage``: see :func:`correlations`; ``shrinkage_out``: an
+    optional (S,) float64 CUDA tensor that receives the shrinkage of each subject
+    (partial correlations only)."""
+    d = check_kind(kind, shrinkage)
     lib = _lib.load()
     (S, N, T) = ts_dev.shape
     C = N_to_C(N)
     if out is None:
         out = _dev.empty((C, s0 + S))
     pitch = out.shape[1]
-    if sample_mask is None and confounds is None:
+    if kind == "pearson" and shrinkage_out is not None:
+        raise ValueError("shrinkage_out: only kind=\"partial\" has a shrinkage")
+    if kind == "pearson" and sample_mask is None and confounds is None:
         zws = torch.empty(lib.fcd_corr_workspace_bytes(S, N, T), dtype=torch.uint8, device=ts_dev.device)
         _lib.check(lib.fcd_corr_fisherz(_dev.ptr(ts_dev), S, N, T, _dev.ptr(out), pitch, s0, 1 if fisher else 0,
                                         _dev.ptr(zws), _dev.stream()), "fcd_corr_fisherz")
@@ -155,6 +190,22 @@ def correlations_device(ts_dev, fisher=True, out=None, s0=0, missing=False, samp
     n = keep.sum(dim=1) if keep is not None else torch.full((S,), T, device=ts_dev.device)
     if bool((n < K + 2).any()):
         raise ValueError("a subject keeps fewer than K + 2 = %d frames" % (K + 2))
+    if kind == "partial":
+        _check_not_singular(n.cpu().numpy(), N, K, d)
+        if shrinkage_out is not None and (shrinkage_out.dtype != torch.float64 or tuple(shrinkage_out.shape) != (S,)
+                                          or not shrinkage_out.is_contiguous()):
+            raise ValueError("shrinkage_out: expected a contiguous (%d,) float64 tensor" % S)
+        status = torch.empty((S,), dtype=torch.int32, device=ts_dev.device)
+        zws = torch.empty(lib.fcd_corr_partial_workspace_bytes(S, N, T, K), dtype=torch.uint8, device=ts_dev.device)
+        _lib.check(lib.fcd_corr_partial(_dev.ptr(ts_dev), S, N, T, _dev.ptr(keep), _dev.ptr(conf), K, d, _dev.ptr(out),
+                                        pitch, s0, 1 if fisher else 0, 1 if missing else 0, _dev.ptr(rank),
+                                        _dev.ptr(shrinkage_out), _dev.ptr(status), _dev.ptr(zws), _dev.stream()),
+                   "fcd_corr_partial")
+        bad = torch.nonzero(status).flatten().tolist()
+        if bad:
+            raise ValueError("partial correlations: the shrunk correlation matrix of subject(s) %s is singular to "
+                             "working precision (their columns are NaN); use a shrinkage > 0" % bad)
+        return out
     zws = torch.empty(lib.fcd_corr_clean_workspace_bytes(S, N, T, K), dtype=torch.uint8, device=ts_dev.device)
     _lib.check(lib.fcd_corr_fisherz_clean(_dev.ptr(ts_dev), S, N, T, _dev.ptr(keep), _dev.ptr(conf), K, _dev.ptr(out),
                                           pitch, s0, 1 if fisher else 0, 1 if missing else 0, _dev.ptr(rank),
@@ -162,7 +213,8 @@ def correlations_device(ts_dev, fisher=True, out=None, s0=0, missing=False, samp
     return out
 
 
-def correlations(ts, fisher=True, missing=False, sample_mask=None, confounds=None):
+def correlations(ts, fisher=True, missing=False, sample_mask=None, confounds=None, kind="pearson",
+                 shrinkage="ledoit-wolf", return_shrinkage=False):
     """
     Computes subject correlations from region time series.
 
@@ -193,6 +245,26 @@ def correlations(ts, fisher=True, missing=False, sample_mask=None, confounds=Non
         signals, trends).  Each region is cleared of them and of a constant
         over the kept frames on the GPU: r is the partial correlation given
         the confounds.  Collinear columns are dropped.
+    kind : ``"pearson"`` (default) or ``"partial"``
+        ``"partial"``: the partial correlation of every two regions given all
+        other regions (and the confounds and a constant), as nilearn's
+        ``ConnectivityMeasure(kind="partial correlation")``: per subject the
+        cleaned rows are scaled to unit variance (1/n_s normalisation over its
+        n_s kept frames), their correlation matrix R is shrunk to
+        Sigma = (1 - delta) R + delta mu I (mu = tr R / N) and inverted in
+        fp64 on the GPU, r_nm = -P_nm / sqrt(P_nn P_mm) with P = Sigma^-1.
+        Unusable regions (as above) are left out of their subject's problem.
+        Partial correlations are smaller in magnitude than full ones: set the
+        fit's ``model.mu`` / ``model.sigma`` or use ``update_mu_sigma=True``.
+    shrinkage : ``"ledoit-wolf"`` (default) or a float in [0, 1]
+        delta of ``kind="partial"``: the Ledoit-Wolf estimate of
+        ``sklearn.covariance.ledoit_wolf`` on the unit-variance rows (which
+        counts n_s samples; the K + 1 fitted confound columns are not
+        subtracted), or a fixed value.  0 needs more than N + K kept frames per
+        subject; a subject whose shrunk matrix is still singular to working
+        precision raises ``ValueError``.
+    return_shrinkage : bool
+        Also return the (S,) delta of every subject (``kind="partial"``).
 
     With ``sample_mask`` and ``confounds`` both None and an array ``ts`` this
     is the plain path (``fcd_corr_fisherz``); otherwise the inputs are packed
@@ -200,8 +272,22 @@ def correlations(ts, fisher=True, missing=False, sample_mask=None, confounds=Non
 
     Returns
     -------
-    :class:`numpy.ndarray`, (C, S), float64 -- connection-major, subject-minor.
+    :class:`numpy.ndarray`, (C, S), float64 -- connection-major, subject-minor;
+    with ``return_shrinkage`` the pair (correlations, (S,) float64 delta).
     """
+    d = check_kind(kind, shrinkage)
+    if return_shrinkage and kind != "partial":
+        raise ValueError("return_shrinkage: only kind=\"partial\" has a shrinkage")
+    if kind == "partial":
+        (packed, keep, conf) = pack_clean(ts, sample_mask, confounds)
+        _check_not_singular(keep.sum(axis=1), packed.shape[1], 0 if conf is None else conf.shape[2], d)
+        delta = _dev.empty((packed.shape[0],))
+        out = _dev.download(correlations_device(
+            _dev.upload(packed, np.float32), fisher=fisher, missing=missing,
+            sample_mask=_dev.upload(keep.astype(np.bool_), np.bool_),
+            confounds=_dev.upload(conf, np.float64) if conf is not None else None, kind=kind, shrinkage=shrinkage,
+            shrinkage_out=delta))
+        return (out, _dev.download(delta)) if return_shrinkage else out
     if sample_mask is None and confounds is None and not isinstance(ts, (list, tuple)):
         ts_dev = _dev.upload(np.asarray(ts), np.float32)
         return _dev.download(correlations_device(ts_dev, fisher=fisher, missing=missing))

@@ -23,9 +23,10 @@ namespace fcd {
 // when keep is NULL) are read; the others are written as zeros.  The sums are those of the unmasked form
 // in the same order, divided by the number of kept frames, so an all-kept mask gives the same bits.  A
 // row with a non-finite kept sample or of zero variance is written as zeros, and status[r] = 1 marks it.
-template <bool SPLIT, bool MASK = false>
+// OutT = double (fcd_corr_partial, MASK only): the fp64 rows are stored as they are computed.
+template <bool SPLIT, bool MASK = false, typename OutT = float>
 __global__ void __launch_bounds__(256)
-standardise_kernel(const float* __restrict__ ts, int64_t rows, int T, int Tp, float* __restrict__ Z,
+standardise_kernel(const float* __restrict__ ts, int64_t rows, int T, int Tp, OutT* __restrict__ Z,
                    float* __restrict__ Zlo, const uint8_t* __restrict__ keep = nullptr, int N = 0,
                    uint8_t* __restrict__ status = nullptr) {
     const int lane = threadIdx.x & 31;
@@ -53,8 +54,8 @@ standardise_kernel(const float* __restrict__ ts, int64_t rows, int T, int Tp, fl
         if (MASK && lane == 0) status[r] = ss > 0.0 ? 0 : 1;
         for (int t = lane; t < Tp; t += 32) {
             const bool use = t < T && (!MASK || (ss > 0.0 && (kp == nullptr || kp[t])));
-            const float z = use ? (float)(((double)x[t] - mean) * inv) : 0.0f;
-            if (SPLIT) {
+            const OutT z = use ? (OutT)(((double)x[t] - mean) * inv) : (OutT)0;
+            if constexpr (SPLIT) {
                 uint32_t hb, lb;
                 asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(z));
                 const float zh = __uint_as_float(hb);
@@ -193,6 +194,14 @@ int corr_standardise_masked(bool tc, const float* ts, const uint8_t* keep, int S
     if (tc) standardise_kernel<true, true><<<row_grid(rows), 256, 0, st>>>(ts, rows, T, Tp, Z, Zlo, keep, N, status);
     else standardise_kernel<false, true><<<row_grid(rows), 256, 0, st>>>(ts, rows, T, Tp, Z, nullptr, keep, N, status);
     return check_launch("fcd_corr_fisherz_clean(standardise)");
+}
+
+int corr_standardise_masked_f64(const float* ts, const uint8_t* keep, int S, int N, int T, int Tp, double* Z,
+                                uint8_t* status, cudaStream_t st) {
+    const int64_t rows = (int64_t)S * N;
+    standardise_kernel<false, true, double><<<row_grid(rows), 256, 0, st>>>(ts, rows, T, Tp, Z, nullptr, keep, N,
+                                                                            status);
+    return check_launch("fcd_corr_partial(standardise)");
 }
 
 int corr_mark_status(const uint8_t* status, int S, int N, double* out, int64_t pitch, int s0, cudaStream_t st) {

@@ -48,4 +48,12 @@ int corr_standardise_masked(bool tc, const float* ts, const uint8_t* keep, int S
                             float* Zlo, uint8_t* status, cudaStream_t st);
 int corr_mark_status(const uint8_t* status, int S, int N, double* out, int64_t pitch, int s0, cudaStream_t st);
 
+// fp64 forms of the two standardisations for fcd_corr_partial: the same rows as fcd_corr_fisherz_clean forms
+// (K == 0: standardise_kernel<false, true>; K >= 1: confound_basis_kernel into Q [S][K][Tp], then
+// clean_kernel), stored as fp64 Z [S][N][Tp] without the rounding to fp32.
+int corr_standardise_masked_f64(const float* ts, const uint8_t* keep, int S, int N, int T, int Tp, double* Z,
+                                uint8_t* status, cudaStream_t st);
+int corr_clean_f64(const float* ts, const uint8_t* keep, const double* confounds, int S, int N, int T, int Tp, int K,
+                   double* Q, double* Z, uint8_t* status, int32_t* rank, cudaStream_t st);
+
 }  // namespace fcd

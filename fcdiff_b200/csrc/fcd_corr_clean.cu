@@ -112,11 +112,11 @@ confound_basis_kernel(const double* __restrict__ confounds, const uint8_t* __res
 // products accumulate in registers (KMAX >= K, unrolled) and are reduced once per row.
 // A row is unusable when a kept sample is non-finite or its residual sum of squares is at most 2^-40 of
 // its centred sum of squares (the region is explained by the confounds to the rounding of its fp32
-// input): it is written as zeros and status = 1.
-template <bool SPLIT, int KMAX>
+// input): it is written as zeros and status = 1.  OutT = double (fcd_corr_partial): the fp64 rows are stored.
+template <bool SPLIT, int KMAX, typename OutT = float>
 __global__ void __launch_bounds__(256)
 clean_kernel(const float* __restrict__ ts, const uint8_t* __restrict__ keep, const double* __restrict__ Q, int N,
-             int T, int Tp, int K, float* __restrict__ Z, float* __restrict__ Zlo, uint8_t* __restrict__ status) {
+             int T, int Tp, int K, OutT* __restrict__ Z, float* __restrict__ Zlo, uint8_t* __restrict__ status) {
     extern __shared__ double smem_d[];
     const int W = blockDim.x >> 5;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -207,8 +207,8 @@ clean_kernel(const float* __restrict__ ts, const uint8_t* __restrict__ keep, con
     if (lane == 0) status[r] = usable ? 0 : 1;
     for (int t = lane; t < Tp; t += 32) {
         const bool kept = t < T && (kp == nullptr || kp[t]);
-        const float z = usable && kept ? (float)(buf[t] * inv) : 0.0f;
-        if (SPLIT) {
+        const OutT z = usable && kept ? (OutT)(buf[t] * inv) : (OutT)0;
+        if constexpr (SPLIT) {
             uint32_t hb, lb;
             asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(z));
             const float zh = __uint_as_float(hb);
@@ -228,24 +228,33 @@ static int clean_warps(int Tp, int K) {
     return (int)(w < 8 ? w : 8);
 }
 
-template <bool SPLIT, int KMAX>
+template <bool SPLIT, int KMAX, typename OutT>
 static int launch_clean(const float* ts, const uint8_t* keep, const double* Q, int S, int N, int T, int Tp, int K,
-                        float* Z, float* Zlo, uint8_t* status, cudaStream_t st) {
+                        OutT* Z, float* Zlo, uint8_t* status, cudaStream_t st) {
     const int W = clean_warps(Tp, K);
     const size_t smem = ((size_t)K * kCleanChunk + (size_t)W * Tp) * sizeof(double);
-    FCD_ALLOW_BIG_SMEM(clean_kernel<SPLIT, KMAX>);
+    FCD_ALLOW_BIG_SMEM(clean_kernel<SPLIT, KMAX, OutT>);
     dim3 grid((unsigned)((N + W - 1) / W), (unsigned)S);
-    clean_kernel<SPLIT, KMAX><<<grid, 32 * W, smem, st>>>(ts, keep, Q, N, T, Tp, K, Z, Zlo, status);
+    clean_kernel<SPLIT, KMAX, OutT><<<grid, 32 * W, smem, st>>>(ts, keep, Q, N, T, Tp, K, Z, Zlo, status);
     return check_launch("fcd_corr_fisherz_clean(clean)");
 }
 
-template <bool SPLIT>
+template <bool SPLIT, typename OutT = float>
 static int launch_clean_k(const float* ts, const uint8_t* keep, const double* Q, int S, int N, int T, int Tp, int K,
-                          float* Z, float* Zlo, uint8_t* status, cudaStream_t st) {
+                          OutT* Z, float* Zlo, uint8_t* status, cudaStream_t st) {
     if (K <= 8) return launch_clean<SPLIT, 8>(ts, keep, Q, S, N, T, Tp, K, Z, Zlo, status, st);
     if (K <= 16) return launch_clean<SPLIT, 16>(ts, keep, Q, S, N, T, Tp, K, Z, Zlo, status, st);
     if (K <= 32) return launch_clean<SPLIT, 32>(ts, keep, Q, S, N, T, Tp, K, Z, Zlo, status, st);
     return launch_clean<SPLIT, 64>(ts, keep, Q, S, N, T, Tp, K, Z, Zlo, status, st);
+}
+
+int corr_clean_f64(const float* ts, const uint8_t* keep, const double* confounds, int S, int N, int T, int Tp, int K,
+                   double* Q, double* Z, uint8_t* status, int32_t* rank, cudaStream_t st) {
+    FCD_REQUIRE(clean_warps(Tp, K) >= 1, "fcd_corr_partial: T=%d too long for K=%d confounds", T, K);
+    confound_basis_kernel<<<S, kBasisThreads, 0, st>>>(confounds, keep, T, Tp, K, Q, rank);
+    const int rc = check_launch("fcd_corr_partial(basis)");
+    if (rc) return rc;
+    return launch_clean_k<false>(ts, keep, Q, S, N, T, Tp, K, Z, nullptr, status, st);
 }
 
 // Workspace layout: Z and Zlo planes (as fcd_corr_fisherz), the status bytes [S][N], Q [S][K][Tp].

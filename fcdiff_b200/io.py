@@ -67,13 +67,16 @@ def load_timeseries(paths, time_major=False):
     return np.stack(subjects, axis=0)
 
 
-def correlations_from_files(control_paths, patient_paths, fisher=True, time_major=False, missing=False):
+def correlations_from_files(control_paths, patient_paths, fisher=True, time_major=False, missing=False,
+                            kind="pearson", shrinkage="ledoit-wolf"):
     """(b, bt): (C, H) and (C, U) float64 correlation matrices of the control and
     the patient group, ready for ``UnsharedRegionFit.b`` / ``.bt``.  ``missing``:
     regions without a usable time series in a subject give NaN connections
-    (``corr.correlations``), for a fit with ``missing="marginalize"``."""
+    (``corr.correlations``), for a fit with ``missing="marginalize"``.
+    ``kind`` / ``shrinkage``: ``"partial"`` for partial correlations
+    (``corr.correlations``)."""
     ts = load_timeseries(list(control_paths) + list(patient_paths), time_major)
-    c = corr.correlations(ts, fisher=fisher, missing=missing)
+    c = corr.correlations(ts, fisher=fisher, missing=missing, kind=kind, shrinkage=shrinkage)
     H = len(control_paths)
     return np.ascontiguousarray(c[:, :H]), np.ascontiguousarray(c[:, H:])
 
@@ -132,11 +135,12 @@ def load_confounds(path, columns=None):
 
 
 def cleaned_correlations_from_files(control_paths, patient_paths, confound_paths=None, confound_columns=None,
-                                    sample_masks=None, fisher=True, missing=False, time_major=False):
+                                    sample_masks=None, fisher=True, missing=False, time_major=False,
+                                    kind="pearson", shrinkage="ledoit-wolf"):
     """(b, bt) as ``correlations_from_files`` returns them, from cleaned time series: subjects may differ in
     length; ``sample_masks`` (one (T_s,) bool array per subject, controls then patients) censors frames;
     ``confound_paths`` (one file per subject, same order) with ``confound_columns`` gives the regressors
-    projected out of every region (``corr.correlations``)."""
+    projected out of every region (``corr.correlations``); ``kind`` / ``shrinkage`` as there."""
     paths = list(control_paths) + list(patient_paths)
     ts = load_timeseries_list(paths, time_major)
     conf = None
@@ -146,6 +150,7 @@ def cleaned_correlations_from_files(control_paths, patient_paths, confound_paths
             raise ValueError("%d confound files for %d subjects" % (len(confound_paths), len(paths)))
         conf = [load_confounds(p, confound_columns) for p in confound_paths]
     masks = None if sample_masks is None else [np.asarray(m, dtype=bool) for m in sample_masks]
-    c = corr.correlations(ts, fisher=fisher, missing=missing, sample_mask=masks, confounds=conf)
+    c = corr.correlations(ts, fisher=fisher, missing=missing, sample_mask=masks, confounds=conf, kind=kind,
+                          shrinkage=shrinkage)
     H = len(control_paths)
     return np.ascontiguousarray(c[:, :H]), np.ascontiguousarray(c[:, H:])

@@ -635,6 +635,31 @@ FCD_API int fcd_corr_fisherz_clean(const float* ts, int32_t S, int32_t N, int32_
                      const double* confounds, int32_t K, double* out, int64_t pitch, int32_t s0,
                      int32_t fisher, int32_t mark_missing, int32_t* rank, void* zws, void* stream);
 
+/* Partial correlations from cleaned time series: r_nm = -P_nm / sqrt(P_nn P_mm), P = Sigma^-1, Sigma the
+ * Ledoit-Wolf shrunk correlation matrix of a subject's usable regions.  Inputs as fcd_corr_fisherz_clean
+ * (ts, keep, confounds, K <= 64), and the same rows: over the kept frames each region row is centred, cleared
+ * of the confounds, and scaled to unit variance with the 1/n_s normalisation (n_s the subject's kept frames),
+ * all in fp64 (X, n_s x N_s).  R = X^T X / n_s, mu = tr(R) / N_s, and, when shrinkage < 0, Ledoit-Wolf as
+ * sklearn.covariance.ledoit_wolf(X, assume_centered=True) computes it: d2 = |R - mu I|_F^2 / N_s,
+ * b2 = min(d2, (sum_t |x_t|^4 / n_s - |R|_F^2) / (n_s N_s)), delta = b2 / d2 (0 unless b2 > 0); a
+ * shrinkage in [0, 1] is delta itself.  Sigma = (1 - delta) R + delta mu I, inverted in fp64 (blocked
+ * symmetric sweep, one CTA per subject); r goes through the clip / atanh of fcd_corr_fisherz into columns
+ * [s0, s0 + S) of the (C, pitch) matrix out, every other column untouched.  With confounds r is the partial
+ * correlation given all other regions, the confounds and a constant (at delta = 0); n_s is not reduced by
+ * the K + 1 fitted columns.  An unusable region (the rule of fcd_corr_fisherz_clean) is left out of its
+ * subject's problem: the subject's other edges and delta are those of its usable regions alone, and the
+ * region's edges are 0, or NaN when mark_missing != 0.  delta = 1 gives r = 0 on every edge.  A pivot of
+ * the inverse <= 2^-40 (Sigma singular to working precision: shrinkage 0 with n_s <= N + K, or collinear
+ * regions) sets status[s] = 1 and writes NaN to all of column s0 + s; otherwise status[s] = 0.  rank[s]:
+ * the confounds kept (when rank != NULL); shrinkage_out[s]: delta (when != NULL).  Subjects are processed
+ * in batches inside the call; no result depends on the batch.  Every subject needs at least K + 2 kept
+ * frames (not checked here).  zws: device scratch of fcd_corr_partial_workspace_bytes(S, N, T, K) bytes. */
+FCD_API int64_t fcd_corr_partial_workspace_bytes(int32_t S, int32_t N, int32_t T, int32_t K);
+FCD_API int fcd_corr_partial(const float* ts, int32_t S, int32_t N, int32_t T, const uint8_t* keep,
+                     const double* confounds, int32_t K, double shrinkage, double* out, int64_t pitch,
+                     int32_t s0, int32_t fisher, int32_t mark_missing, int32_t* rank, double* shrinkage_out,
+                     int32_t* status, void* zws, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
