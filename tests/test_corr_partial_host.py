@@ -114,3 +114,77 @@ def test_unshrunk_singular_subject_raises(K):
     with pytest.raises(ValueError, match="subject 0"):
         corr.correlations(lists, kind="partial", shrinkage=0.0,
                           confounds=None if g is None else [g[s][:N + K] for s in range(S)])
+
+
+# ------------------------------------------------------------------ the longdouble reference
+def factor_series(N, T, K, seed):
+    """Planted 8-factor series with confound components: well conditioned (kappa ~ 10 under Ledoit-Wolf)."""
+    rng = np.random.RandomState(seed)
+    a = np.where(rng.rand(N) < 0.5, 0.55, -0.27)
+    f = rng.standard_normal((8, T))
+    g = rng.standard_normal((T, K))
+    x = np.sqrt(1 - a * a)[:, None] * rng.standard_normal((N, T)) + a[:, None] * f[np.arange(N) % 8]
+    x += 0.5 * rng.standard_normal((N, K)) @ g.T + rng.uniform(-5, 5, (N, 1))
+    return x.astype(np.float32), g
+
+
+@pytest.mark.parametrize("N,T,K,shrinkage", [(40, 300, 0, None), (70, 200, 3, None), (65, 500, 2, 0.0),
+                                             (30, 20, 1, None)])
+def test_longdouble_reference_is_the_fp64_oracle_when_well_conditioned(N, T, K, shrinkage):
+    (x, g) = factor_series(N, T, K, N + K)
+    keep = np.random.RandomState(T).rand(T) > 0.15
+    (r, bad, delta, piv, kappa) = OP.subject_partial_ld(x, keep, g if K else None, shrinkage)
+    (r64, bad64, delta64) = OP.subject_partial(x, keep, g if K else None, shrinkage)
+    assert kappa < 100 and (bad == bad64).all() and not bad.any()
+    assert np.abs(r.astype(np.float64) - r64).max() <= 1e-14
+    assert abs(float(delta) - delta64) <= 1e-14
+    assert piv.dtype == np.longdouble and (piv > 0).all()
+
+
+def test_longdouble_reference_closed_forms():
+    # N = 2: Sigma = [[1, (1 - delta) rho], [(1 - delta) rho, 1]], so r = (1 - delta) rho, rho the Pearson
+    # correlation of the cleaned rows
+    LD = np.longdouble
+    (x, g) = factor_series(2, 90, 2, 3)
+    x[1] += 2 * x[0]                                    # strongly correlated: delta < 1
+    keep = np.ones(90, bool)
+    keep[::7] = False
+    (r, _, delta, _, _) = OP.subject_partial_ld(x, keep, g)
+    assert 0 < delta < 1
+    (z, _) = OP.unit_rows_ld(x, keep, g)
+    rho = np.sum(z[0] * z[1]) / np.sqrt(np.sum(z[0] * z[0]) * np.sum(z[1] * z[1]))
+    assert abs(r[0, 1] - (1 - delta) * rho) <= 1e-17
+    # N = 3: the three-variable formula r_ab.c = (s_ab - s_ac s_bc) / sqrt((1 - s_ac^2)(1 - s_bc^2)) on the
+    # shrunk Sigma with its diagonal scaled to 1
+    (x, _) = factor_series(3, 60, 0, 4)
+    x[2] += x[0] - x[1]
+    keep = np.ones(60, bool)
+    (r, _, delta, _, _) = OP.subject_partial_ld(x, keep)
+    xc = x.astype(LD) - np.sum(x.astype(LD), axis=1, keepdims=True) / LD(60)
+    R = (xc @ xc.T) / np.sqrt(np.outer(np.sum(xc * xc, axis=1), np.sum(xc * xc, axis=1)))
+    sig = (1 - delta) * R + delta * np.trace(R) / 3 * np.eye(3, dtype=LD)
+    s = sig / np.sqrt(np.outer(np.diag(sig), np.diag(sig)))
+    for (a, b, c) in ((0, 1, 2), (0, 2, 1), (1, 2, 0)):
+        want = (s[a, b] - s[a, c] * s[b, c]) / np.sqrt((1 - s[a, c] ** 2) * (1 - s[b, c] ** 2))
+        assert abs(r[a, b] - want) <= 1e-17 and r[a, b] == r[b, a]
+
+
+def test_longdouble_pivots_are_the_squared_cholesky_diagonal():
+    LD = np.longdouble
+    (x, _) = factor_series(150, 170, 0, 9)             # three sweep blocks, the last partial
+    (z, _) = OP.unit_rows_ld(x, np.ones(170, bool))
+    (sigma, _) = OP.ledoit_wolf_ld(z, 0.0)
+    (mP, piv) = OP.sweep_ld(sigma)
+    L = np.zeros_like(sigma)
+    for j in range(150):                                # left-looking Cholesky, column by column
+        d = sigma[j, j] - np.sum(L[j, :j] * L[j, :j])
+        L[j, j] = np.sqrt(d)
+        L[j + 1:, j] = (sigma[j + 1:, j] - L[j + 1:, :j] @ L[j, :j]) / L[j, j]
+    assert np.abs(piv / np.diag(L) ** 2 - 1).max() <= 1e-15
+    assert piv.min() < 0.1                               # n_s = N + 20: small pivots late in the chain
+    assert np.abs((-mP).astype(np.float64) @ sigma.astype(np.float64) - np.eye(150)).max() <= 1e-9
+    # a singular matrix stops at its first pivot <= 0
+    z[5] = z[2]
+    (sigma, _) = OP.ledoit_wolf_ld(z, 0.0)
+    (mP, piv) = OP.sweep_ld(sigma)
+    assert mP is None and abs(piv[5]) <= 1e-17 and np.isnan(piv[6:].astype(np.float64)).all()
