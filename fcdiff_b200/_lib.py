@@ -108,6 +108,9 @@ SIGNATURES = {
                                      c_int32, _P, _P]),
     "fcd_solver_init_host": (c_int, [_P, c_double, c_double, _D3, _D3, c_double, c_int32]),
     "fcd_solver_step_host": (c_int, [_P, _D3]),
+    "fcd_solver_moments": (c_int64, []),
+    "fcd_solver_step_host_moments": (c_int, [_P, _D3, c_int32]),
+    "fcd_solver_model_host": (c_int, [_D3, c_int32, c_double, c_double, _D3, _D3]),
     "fcd_solver_wait": (c_int, [_P, c_uint64, _P, c_int32]),
     "fcd_energy_terms": (c_int, [_P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
                                  POINTER(FcdTheta), c_double, _P, _P, _P, _P]),

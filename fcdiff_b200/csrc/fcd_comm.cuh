@@ -8,7 +8,7 @@
 namespace fcd {
 
 constexpr int kCommMaxWorld = 16;
-constexpr int kCommMaxVals = 8;
+constexpr int kCommMaxVals = 16;
 
 struct CommWindow {
     double slot[2][kCommMaxWorld][kCommMaxVals];

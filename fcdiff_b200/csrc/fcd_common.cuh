@@ -43,7 +43,7 @@ constexpr double kHalfLog2Pi = 0.91893853320467274178032973640562;   // log(sqrt
 // Workspace layout (doubles): [0, kWsPartials) per-CTA partial sums,
 // then one 64-bit slot holding the arrival ticket, then 16 scratch doubles.
 constexpr int     kMaxReduceBlocks = 2048;
-constexpr int     kMaxReduceVals   = 9;
+constexpr int     kMaxReduceVals   = 16;
 constexpr int64_t kWsPartials      = (int64_t)kMaxReduceBlocks * kMaxReduceVals;
 constexpr int64_t kWsScratch       = kWsPartials + 2;      // 16 doubles of scratch for chained reductions
 constexpr int64_t kWsDoubles       = kWsScratch + 16;
@@ -521,26 +521,39 @@ __device__ __forceinline__ void grid_reduce_store(double (&v)[NV], double* ws, d
 // Same reduction, but the sums stay in the CTA that arrived last: returns true there (for all of
 // its threads, with s_out[0..NV) valid in shared memory after the internal barrier) and false in
 // every other CTA.  For kernels whose last CTA continues with an epilogue (fcd_solver.cuh).
+// The warp partials go through shared memory in rounds of at most 8 values: the static shared memory
+// stays inside the 2 KB that kSmemBudget leaves for it whatever NV is.
+template <int NV, int THREADS>
+__device__ __forceinline__ void cta_sum_rounds(const double (&v)[NV], double (*s_part)[THREADS / 32], double* dst) {
+    constexpr int R = NV < 8 ? NV : 8;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int r0 = 0; r0 < NV; r0 += R) {
+#pragma unroll
+        for (int i = r0; i < r0 + R && i < NV; ++i) {
+            double x = warp_sum(v[i]);
+            if (lane == 0) s_part[i - r0][warp] = x;
+        }
+        __syncthreads();
+        if (warp == 0) {
+#pragma unroll
+            for (int i = r0; i < r0 + R && i < NV; ++i) {
+                double x = (lane < THREADS / 32) ? s_part[i - r0][lane] : 0.0;
+                x = warp_sum(x);
+                if (lane == 0) dst[i] = x;
+            }
+        }
+        if (r0 + R < NV) __syncthreads();          // s_part reuse
+    }
+}
+
 template <int NV, int THREADS>
 __device__ __forceinline__ bool grid_reduce_last(double (&v)[NV], double* ws, double* s_out) {
     static_assert(NV <= kMaxReduceVals, "too many values");
-    __shared__ double s_part[NV][THREADS / 32];
+    __shared__ double s_part[NV < 8 ? NV : 8][THREADS / 32];
     __shared__ bool s_last;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        double x = warp_sum(v[i]);
-        if (lane == 0) s_part[i][warp] = x;
-    }
-    __syncthreads();
-    if (warp == 0) {
-#pragma unroll
-        for (int i = 0; i < NV; ++i) {
-            double x = (lane < THREADS / 32) ? s_part[i][lane] : 0.0;
-            x = warp_sum(x);
-            if (lane == 0) ws[(int64_t)blockIdx.x * NV + i] = x;
-        }
-    }
+    cta_sum_rounds<NV, THREADS>(v, s_part, ws + (int64_t)blockIdx.x * NV);
     unsigned long long* ticket = reinterpret_cast<unsigned long long*>(ws + kWsPartials);
     if (threadIdx.x == 0) {
         __threadfence();
@@ -558,21 +571,8 @@ __device__ __forceinline__ bool grid_reduce_last(double (&v)[NV], double* ws, do
         for (int i = 0; i < NV; ++i) acc[i] += __ldcg(ws + (int64_t)b * NV + i);
     }
     __syncthreads();      // s_part reuse
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        double x = warp_sum(acc[i]);
-        if (lane == 0) s_part[i][warp] = x;
-    }
-    __syncthreads();
-    if (warp == 0) {
-#pragma unroll
-        for (int i = 0; i < NV; ++i) {
-            double x = (lane < THREADS / 32) ? s_part[i][lane] : 0.0;
-            x = warp_sum(x);
-            if (lane == 0) s_out[i] = x;
-        }
-        if (lane == 0) *ticket = 0ull;
-    }
+    cta_sum_rounds<NV, THREADS>(acc, s_part, s_out);
+    if (warp == 0 && lane == 0) *ticket = 0ull;
     __syncthreads();
     return true;
 }

@@ -42,12 +42,12 @@ mstep_stats_kernel(const double* __restrict__ lqF, int64_t C,
 // with num_k = (3 p_k - 1)/2.  Tiers T1 / T2 / T3 as described in fcd_common.cuh.
 struct ElmAcc {
     double obj, ge, gh;       // objective, sum s_l w_l d_l, sum w_2 d_2
-    double qa, qb;            // SOLVE: sum_{l < 2} w_l g_l^2, sum w_2 g_2^2 (fcd_solver.cuh)
 };
 
 constexpr int kElmSeg = 256;
 
-// SOLVE: evaluation point from the solver state, Hessian sums, optimiser step in the last CTA
+// SOLVE: evaluation point from the solver state, the series model's moments (fcd_solver.cuh), optimiser
+// step in the last CTA
 // (see elm_coded_kernel, fcd_streams.cu).
 template <bool GRAD, bool FAST, bool SOLVE>
 __global__ void __launch_bounds__(kStreamThreads, 1)
@@ -81,15 +81,18 @@ elm_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C, int U, 
     const double al[3] = {T.al[0], T.al[1], T.al[2]}, bl[3] = {T.bl[0], T.bl[1], T.bl[2]};
     const double sl[3] = {-1.0, 1.0, 2.0 * T.eta - 1.0};
     const double2* qR2 = reinterpret_cast<const double2*>(qR);
-    ElmAcc acc = {0.0, 0.0, 0.0, 0.0, 0.0}, acc1 = {0.0, 0.0, 0.0, 0.0, 0.0};
-    // per-l constants of the T1 body {a_l, b_l, s_l, [l == 2]} (+ [l < 2] for the Hessian sums); row 3 is
+    ElmAcc acc = {0.0, 0.0, 0.0}, acc1 = {0.0, 0.0, 0.0};
+    SolverMoments mo;
+#pragma unroll
+    for (int k = 0; k < kSolverK - 1; ++k) mo.a[k] = mo.b[k] = 0.0;
+    // per-l constants of the T1 body {a_l, b_l, s_l, [l == 2]} (+ [l < 2] s_l for the moments); row 3 is
     // the neutral element for deferred / padding slots: log(1 + 0 p) = 0 exactly, zero gradient weight
     __shared__ double4 s_lc[4];
     __shared__ double s_lq[4];
     if (threadIdx.x < 4) {
         const int l = threadIdx.x;
         s_lc[l] = l < 3 ? make_double4(sel3(l, al), sel3(l, bl), sel3(l, sl), l == 2 ? 1.0 : 0.0) : make_double4(1.0, 0.0, 0.0, 0.0);
-        s_lq[l] = l < 2 ? 1.0 : 0.0;
+        s_lq[l] = l < 2 ? sel3(l, sl) : 0.0;
     }
     __syncthreads();
 
@@ -120,9 +123,8 @@ elm_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C, int U, 
             a.ge = fma(k.z, d, a.ge);
             a.gh = fma(k.w, d, a.gh);
             if (SOLVE) {
-                const double dd = d * d;
-                a.qa = fma(s_lq[lp], dd, a.qa);
-                a.qb = fma(k.w, dd, a.qb);
+                add_powers1(mo.a, s_lq[lp] * d);
+                add_powers1(mo.b, k.w * d);
             }
         }
         if (e == 1 && ++nf == kProdMax) flush();              // warp-uniform
@@ -156,8 +158,8 @@ elm_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C, int U, 
                 acc.ge = fma(sl[l], d, acc.ge);
                 if (l == 2) acc.gh += d;
                 if (SOLVE) {
-                    if (l == 2) acc.qb = fma(d, g, acc.qb);
-                    else acc.qa = fma(d, g, acc.qa);
+                    if (l == 2) add_powers(mo.b, qw[l], g);
+                    else add_powers(mo.a, qw[l], sl[l] * g);
                 }
             } else {
                 acc.obj = fma(qw[l], fast_log<FAST>(M, s_tab), acc.obj);
@@ -187,8 +189,9 @@ elm_kernel(const double* __restrict__ P, int64_t planeStride, int64_t C, int U, 
                                                          [](int64_t) {});
     flush();
     if (SOLVE) {
-        double v[5] = {acc.obj + acc1.obj, acc.ge + acc1.ge, acc.gh + acc1.gh, acc.qa + acc1.qa, acc.qb + acc1.qb};
-        if (grid_reduce_last<5, kStreamThreads>(v, ws, s_sums))
+        double v[kSolverVals];
+        solver_sums(acc.obj + acc1.obj, acc.ge + acc1.ge, acc.gh + acc1.gh, mo, v);
+        if (grid_reduce_last<kSolverVals, kStreamThreads>(v, ws, s_sums))
             solver_epilogue(s_sums, state, konst_dev, peers, rank, world, pub, seq);
     } else {
         double v[3] = {acc.obj + acc1.obj, -(2.0 * T.epsilon - 1.0) * (acc.gh + acc1.gh), -(acc.ge + acc1.ge)};

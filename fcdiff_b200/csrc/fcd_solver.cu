@@ -26,11 +26,27 @@ __global__ void solver_init_kernel(SolverState* st, double eta, double eps, doub
     *st = s;
 }
 
+template <int K>
+static void step_host(SolverState& s, const double* sums) {
+    solver_step<K>(s, sums);
+}
+
+template <int K>
+static void model_host(const double* sums, double eta0, double eps0, const double* z, double* out4) {
+    const SeriesModel<K> m = series_model<K>(sums, eta0, eps0, -(sums[0] + sums[5]));
+    double g[2], H[3];
+    out4[0] = model_eval<K>(m, z, g, H);
+    model_bounds<K>(m, z, out4[1], out4[2]);
+    out4[3] = model_radius<K>(m, z);
+}
+
 }  // namespace fcd
 
 using namespace fcd;
 
 extern "C" {
+
+int64_t fcd_solver_moments(void) { return kSolverK; }
 
 int64_t fcd_solver_state_bytes(void) { return (int64_t)sizeof(SolverState); }
 int64_t fcd_solver_published_bytes(void) { return (int64_t)sizeof(SolverPublished); }
@@ -64,9 +80,12 @@ int fcd_solver_init(void* state, double eta0, double eps0, const double* lo2_hos
     return check_launch("fcd_solver_init");
 }
 
-/* One optimiser transition on the HOST from six global sums {obj, ge, G_2, Q_0 + Q_1, Q_2, theta-free
- * part} (the same code the evaluation kernels' last CTA runs): lets the CPU tests drive the state
- * machine with NumPy-made sums.  state_host: an fcd_solver_state initialised by fcd_solver_init_host. */
+/* One optimiser transition on the HOST (the same code the evaluation kernels' last CTA runs): lets the
+ * CPU tests drive the state machine with NumPy-made sums.  state_host: an fcd_solver_state initialised by
+ * fcd_solver_init_host.  fcd_solver_step_host takes the six sums {obj, ge, G_2, Q_0 + Q_1, Q_2, theta-free
+ * part} (the quadratic model), fcd_solver_step_host_moments the layout of kSolverVals with K moments per
+ * series; fcd_solver_model_host evaluates the series model of such sums made at (eta0, eps0) at z2:
+ * {value, position bound, value bound, radius}. */
 int fcd_solver_init_host(void* state_host, double eta0, double eps0, const double* lo2_host, const double* hi2_host,
                          double tol, int32_t max_evals) {
     FCD_REQUIRE(state_host != nullptr && lo2_host != nullptr && hi2_host != nullptr, "fcd_solver_init_host: NULL argument");
@@ -86,13 +105,27 @@ int fcd_solver_init_host(void* state_host, double eta0, double eps0, const doubl
     return 0;
 }
 
-int fcd_solver_step_host(void* state_host, const double* sums6_host) {
-    FCD_REQUIRE(state_host != nullptr && sums6_host != nullptr, "fcd_solver_step_host: NULL argument");
+int fcd_solver_step_host_moments(void* state_host, const double* sums_host, int32_t K) {
+    FCD_REQUIRE(state_host != nullptr && sums_host != nullptr, "fcd_solver_step_host_moments: NULL argument");
+    FCD_REQUIRE(K == 2 || K == 4 || K == 6 || K == 8, "fcd_solver_step_host_moments: K must be 2, 4, 6 or 8");
     SolverState s;
     memcpy(&s, state_host, sizeof(s));
-    if (!s.done) solver_step(s, sums6_host);
+    if (!s.done) (K == 2 ? step_host<2> : K == 4 ? step_host<4> : K == 6 ? step_host<6> : step_host<8>)(s, sums_host);
     memcpy(state_host, &s, sizeof(s));
     return 0;
+}
+
+int fcd_solver_model_host(const double* sums_host, int32_t K, double eta0, double eps0, const double* z2_host,
+                          double* out4_host) {
+    FCD_REQUIRE(sums_host != nullptr && z2_host != nullptr && out4_host != nullptr, "fcd_solver_model_host: NULL argument");
+    FCD_REQUIRE(K == 2 || K == 4 || K == 6 || K == 8, "fcd_solver_model_host: K must be 2, 4, 6 or 8");
+    (K == 2 ? model_host<2> : K == 4 ? model_host<4> : K == 6 ? model_host<6> : model_host<8>)(sums_host, eta0, eps0,
+                                                                                            z2_host, out4_host);
+    return 0;
+}
+
+int fcd_solver_step_host(void* state_host, const double* sums6_host) {
+    return fcd_solver_step_host_moments(state_host, sums6_host, 2);
 }
 
 /* Spins until the launch `seq` of a solver batch has published; copies the state to state_out_host. */

@@ -20,10 +20,12 @@
 //     d2f/d eta2 = (2 eps - 1)^2 Q_2                  d2f/d eps2 = Q_0 + Q_1 + (2 eta - 1)^2 Q_2
 //     d2f/d eta d eps = (2 eps - 1)(2 eta - 1) Q_2 - 2 G_2
 // An evaluation delivers {obj, ge, gh, qa, qb} = {sum w_l log y_l, sum s_l w_l g_l with
-// s = (-1, 1, 2 eta - 1), G_2, Q_0 + Q_1, Q_2}: two accumulators more than the gradient alone.
-// f is convex along each parameter (a sum of -log of affine functions), not jointly (eps_2 is
-// bilinear): the step falls back to the diagonal when the 2 x 2 Hessian is not safely positive
-// definite, never moves a parameter more than 3/4 of the way to 0 or 1 (the scale on which
+// s = (-1, 1, 2 eta - 1), G_2, Q_0 + Q_1, Q_2} and the higher moments sum w (s_l g_l)^k of the
+// series model below (k = 3..kSolverK), from which one evaluation models the objective exactly up
+// to the truncation of two one-dimensional series: the solve usually ends on the model of the first
+// evaluation.  f is convex along each parameter (a sum of -log of affine functions), not jointly
+// (eps_2 is bilinear): a step falls back to the diagonal when the 2 x 2 Hessian is not safely
+// positive definite, never moves a parameter more than 3/4 of the way to 0 or 1 (the scale on which
 // -log(A + eps D) changes), projects onto the box, and is halved back towards the last accepted
 // iterate whenever the objective went up.
 #pragma once
@@ -36,12 +38,12 @@ struct SolverState {
     double x[2];          // (eta, epsilon) the NEXT evaluation is made at; the solution when done
     double xprev[2];      // last accepted iterate
     double fprev;         // objective there
-    double f;             // objective at the last accepted iterate (when done: f(x), by the quadratic model
-                          //   for a final step below `tol`)
+    double f;             // objective at the last accepted iterate (when done on the series model: the model's
+                          //   value at x)
     double g[2];          // gradient at the last evaluated point
     double lo[2], hi[2];  // box
-    double tol;           // a Newton step with |dx_i| <= tol * min(x_i, 1 - x_i) for both parameters is taken WITHOUT
-                          //   another evaluation
+    double tol;           // the solve ends on the series model when its remainder bound puts the model's minimiser
+                          //   within tol^2 of the objective's, relative to min(x_i, 1 - x_i)
     double step;          // max |dx| of the last step
     int32_t have_prev;    // an accepted iterate exists
     int32_t nfev;         // evaluations consumed
@@ -58,7 +60,13 @@ struct SolverPublished {
     unsigned long long seq;
 };
 
-constexpr int kSolverVals = 6;        // obj, ge, gh, qa, qb, theta-free part of E_lM
+// Moments per series the evaluation kernels accumulate (A_k, B_k for k <= kSolverK) and the sums an
+// evaluation delivers: obj, ge, gh, qa, qb, the theta-free part of E_lM, then A_3..A_K and B_3..B_K.
+constexpr int kSolverK = 4;
+constexpr int solver_vals(int K) { return 6 + 2 * (K - 2); }
+constexpr int kSolverVals = solver_vals(kSolverK);
+// Trust region of the series model: |d eps| G_01 <= rho and |d eps_2| G_2 <= rho (G_l bounds |g_l|)
+constexpr double kSolverRho = 0.25;
 
 #ifdef __CUDACC__
 #define FCD_HD __host__ __device__
@@ -66,13 +74,150 @@ constexpr int kSolverVals = 6;        // obj, ge, gh, qa, qb, theta-free part of
 #define FCD_HD
 #endif
 
-// One optimiser transition from the GLOBAL sums of the evaluation made at st.x.  One thread.
-// (Plain C++: also compiled for the host, where the CPU tests drive it with NumPy-made sums.)
+FCD_HD inline double solver_eps2(double eta, double eps) {
+    double e2 = eta * eps;
+    e2 += (1.0 - eta) * (1.0 - eps);                          // as sub_theta forms it
+    return e2;
+}
+
+// The objective as a function of the three mixture scalars.  Every term is w log(A + eps_l D), and
+// moving eps_l by d multiplies y_l by 1 + d g_l (g_l = D / y_l at the evaluated point), so with
+// d eps_0 = -d eps_1 = -delta, d eps_2 = delta_2 (bilinear in eta, eps: no cross terms in the series)
+//     f(eta', eps') = f - sum_k (-1)^(k+1) / k (delta^k A_k + delta_2^k B_k),
+//     A_k = sum_{l < 2} w (s_l g_l)^k (s = -1, +1),   B_k = sum_{l = 2} w g_2^k,
+// exactly but for the truncation of two one-dimensional series after K terms.  |g_l| <= G_l =
+// max(1 / eps_l, 1 / (1 - eps_l)) (g is a Moebius function of p in [0, 1]) and for even K the net
+// weights are non-negative (half records: the plane's l = 2 entry and the record's -q_s add up to
+// 1 - q_s), so |A_k| <= G^(k-K) A_K and, with r = |delta| G < 1, the remainder of the value is at
+// most |delta|^(K+1) G A_K / ((K+1)(1 - r)) and that of the slope |delta|^K G A_K / (1 - r).
+template <int K>
+struct SeriesModel {
+    double a[K + 1], b[K + 1];                                // A_k, B_k (index 0 unused)
+    double f, eps, e2, G01, G2;                               // at the evaluated point
+};
+
+template <int K>
+FCD_HD inline SeriesModel<K> series_model(const double* sums, double eta, double eps, double f) {
+    SeriesModel<K> m;
+    const double th = 2.0 * eta - 1.0;
+    m.a[0] = m.b[0] = 0.0;
+    m.a[1] = sums[1] - th * sums[2];                          // ge carries the l = 2 part as (2 eta - 1) gh
+    m.b[1] = sums[2];
+    m.a[2] = sums[3];
+    m.b[2] = sums[4];
+    for (int k = 3; k <= K; ++k) {
+        m.a[k] = sums[6 + (k - 3)];
+        m.b[k] = sums[6 + (K - 2) + (k - 3)];
+    }
+    m.f = f;
+    m.eps = eps;
+    m.e2 = solver_eps2(eta, eps);
+    m.G01 = fmax(1.0 / eps, 1.0 / (1.0 - eps));
+    m.G2 = fmax(1.0 / m.e2, 1.0 / (1.0 - m.e2));
+    return m;
+}
+
+// sum_{k <= K} (-1)^(k+1) d^k m_k / k and its first two derivatives in d
+template <int K>
+FCD_HD inline void series_sum(const double* mk, double d, double& v, double& d1, double& d2) {
+    v = d1 = d2 = 0.0;
+    double pk = 1.0;                                          // d^(k-1)
+    double pk2 = 0.0;                                         // d^(k-2)
+    for (int k = 1; k <= K; ++k) {
+        const double c = (k & 1) ? mk[k] : -mk[k];
+        d1 = fma(c, pk, d1);
+        d2 = fma((double)(k - 1) * c, pk2, d2);
+        v = fma(c * pk, d / (double)k, v);
+        pk2 = pk;
+        pk *= d;
+    }
+}
+
+// the model's value, gradient and Hessian {H00, H01, H11} at z = (eta', eps')
+template <int K>
+FCD_HD inline double model_eval(const SeriesModel<K>& m, const double z[2], double g[2], double H[3]) {
+    const double dA = z[1] - m.eps, dB = solver_eps2(z[0], z[1]) - m.e2;
+    double va, a1, a2, vb, b1, b2;
+    series_sum<K>(m.a, dA, va, a1, a2);
+    series_sum<K>(m.b, dB, vb, b1, b2);
+    const double te = 2.0 * z[1] - 1.0, th = 2.0 * z[0] - 1.0;   // d delta_2 / d eta', d delta_2 / d eps'
+    g[0] = -b1 * te;
+    g[1] = -(a1 + b1 * th);
+    H[0] = -b2 * te * te;
+    H[1] = -(b2 * te * th + 2.0 * b1);
+    H[2] = -(a2 + b2 * th * th);
+    return m.f - va - vb;
+}
+
+template <int K>
+FCD_HD inline double model_radius(const SeriesModel<K>& m, const double z[2]) {
+    return fmax(fabs(z[1] - m.eps) * m.G01, fabs(solver_eps2(z[0], z[1]) - m.e2) * m.G2);
+}
+
+// Remainder bounds at z: the largest relative error of the position the model's slope implies (the
+// slope's remainder over the curvature, |delta|^K G^2 M_K (1 + r)^2 / ((1 - r) M_2), relative to
+// 1 / G = min(eps_l, 1 - eps_l)), and the absolute error of the model's value.
+template <int K>
+FCD_HD inline void model_bounds(const SeriesModel<K>& m, const double z[2], double& pos, double& val) {
+    const double d[2] = {fabs(z[1] - m.eps), fabs(solver_eps2(z[0], z[1]) - m.e2)};
+    const double G[2] = {m.G01, m.G2}, M2[2] = {m.a[2], m.b[2]}, MK[2] = {fabs(m.a[K]), fabs(m.b[K])};
+    pos = val = 0.0;
+    for (int i = 0; i < 2; ++i) {
+        const double r = d[i] * G[i];
+        if (!(r < 1.0)) {
+            pos = val = 1.7976931348623157e308;
+            return;
+        }
+        double dk = 1.0;
+        for (int k = 0; k < K; ++k) dk *= d[i];
+        if (M2[i] > 0.0) pos = fmax(pos, dk * G[i] * G[i] * MK[i] * (1.0 + r) * (1.0 + r) / ((1.0 - r) * M2[i]));
+        val += dk * d[i] * G[i] * MK[i] / ((K + 1) * (1.0 - r));
+    }
+}
+
+// Safeguarded projected Newton point from x (gradient g, Hessian {H00, H01, H11}): active set at the
+// box, the diagonal when the 2 x 2 Hessian is not safely positive definite, never more than 3/4 of
+// the way to 0 or 1 (one common factor: the direction is kept), projection onto the box.
+FCD_HD inline void newton_point(const SolverState& st, const double x[2], const double g[2], const double H[3],
+                                double xn[2]) {
+    const double H00 = H[0], H01 = H[1], H11 = H[2], Hd[2] = {H00, H11};
+    bool fr[2];
+    const double flat = 1e-14 * (H00 + H11);                  // a parameter the objective does not depend on stays put
+    for (int i = 0; i < 2; ++i)                               // active set: at a bound with the gradient pointing out
+        fr[i] = !((x[i] <= st.lo[i] && g[i] > 0.0) || (x[i] >= st.hi[i] && g[i] < 0.0)) && Hd[i] > flat;
+    double d[2] = {0.0, 0.0};
+    const double det = H00 * H11 - H01 * H01;
+    if (fr[0] && fr[1] && det > 1e-8 * H00 * H11) {
+        d[0] = -(H11 * g[0] - H01 * g[1]) / det;
+        d[1] = -(H00 * g[1] - H01 * g[0]) / det;
+    } else {
+        for (int i = 0; i < 2; ++i)
+            if (fr[i]) d[i] = -g[i] / Hd[i];
+    }
+    double a = 1.0;
+    for (int i = 0; i < 2; ++i) {
+        const double room = d[i] < 0.0 ? 0.75 * x[i] : 0.75 * (1.0 - x[i]);
+        if (fabs(d[i]) > room) a = fmin(a, room / fabs(d[i]));
+    }
+    for (int i = 0; i < 2; ++i) xn[i] = fmin(st.hi[i], fmax(st.lo[i], x[i] + a * d[i]));
+}
+
+// One optimiser transition from the GLOBAL sums (layout of kSolverVals with K moments per series) of
+// the evaluation made at st.x.  One thread.  (Plain C++: also compiled for the host, where the CPU
+// tests drive it with NumPy-made sums; K = 2 is the quadratic model of the gradient and Hessian sums.)
+//
+// The first Newton step from the evaluated point is the step of the quadratic model.  If it leaves the
+// trust region the model is not used: the step is taken as it is and evaluated.  Otherwise projected
+// Newton runs on the series model to its minimiser; if the iteration leaves the region it stops on the
+// boundary, and that point is evaluated next.  A minimiser strictly inside the region is the solution,
+// without another evaluation, when the remainder bounds put it within tol^2 (relative) of the
+// objective's and its value within 1e-12 of |f|.
+template <int K>
 FCD_HD inline void solver_step(SolverState& st, const double* sums) {
     const double eta = st.x[0], eps = st.x[1];
     const double obj = sums[0], ge = sums[1], G2 = sums[2], QA = sums[3], Q2 = sums[4], konst = sums[5];
     const double f = -(obj + konst);
-    const double te = 2.0 * eps - 1.0, th = 2.0 * eta - 1.0;
+    const double te = 2.0 * eps - 1.0;
     const double g0 = -te * G2, g1 = -ge;
     st.nfev += 1;
     st.g[0] = g0;
@@ -96,51 +241,71 @@ FCD_HD inline void solver_step(SolverState& st, const double* sums) {
         return;
     }
     st.nback = 0;
-    const double H00 = te * te * Q2, H11 = QA + th * th * Q2, H01 = te * th * Q2 - 2.0 * G2;
-    const double x[2] = {eta, eps}, g[2] = {g0, g1}, Hd[2] = {H00, H11};
-    bool fr[2];
-    const double flat = 1e-14 * (H00 + H11);                  // a parameter the objective does not depend on stays put
-    for (int i = 0; i < 2; ++i)                               // active set: at a bound with the gradient pointing out
-        fr[i] = !((x[i] <= st.lo[i] && g[i] > 0.0) || (x[i] >= st.hi[i] && g[i] < 0.0)) && Hd[i] > flat;
-    double d[2] = {0.0, 0.0};
-    const double det = H00 * H11 - H01 * H01;
-    if (fr[0] && fr[1] && det > 1e-8 * H00 * H11) {
-        d[0] = -(H11 * g0 - H01 * g1) / det;
-        d[1] = -(H00 * g1 - H01 * g0) / det;
-    } else {
-        for (int i = 0; i < 2; ++i)
-            if (fr[i]) d[i] = -g[i] / Hd[i];
+    const SeriesModel<K> m = series_model<K>(sums, eta, eps, f);
+    const double x[2] = {eta, eps};
+    double z[2] = {eta, eps}, gz[2] = {g0, g1}, Hz[3], fz = f;
+    {
+        double gx[2];
+        model_eval<K>(m, z, gx, Hz);                          // the Hessian at x; the gradient as delivered
     }
-    // never more than 3/4 of the way to 0 or to 1 (one common factor: the direction is kept)
-    double a = 1.0;
-    for (int i = 0; i < 2; ++i) {
-        const double room = d[i] < 0.0 ? 0.75 * x[i] : 0.75 * (1.0 - x[i]);
-        if (fabs(d[i]) > room) a = fmin(a, room / fabs(d[i]));
+    bool conv = false;
+    for (int it = 0; it < 24; ++it) {
+        double zn[2];
+        newton_point(st, z, gz, Hz, zn);
+        if (model_radius<K>(m, zn) > kSolverRho) {
+            if (it == 0) {                                    // beyond the model's region: the quadratic model's step
+                z[0] = zn[0];
+                z[1] = zn[1];
+                break;
+            }
+            double in = 0.0, out = 1.0;                       // stop on the boundary
+            for (int j = 0; j < 24; ++j) {
+                const double a = 0.5 * (in + out);
+                const double za[2] = {z[0] + a * (zn[0] - z[0]), z[1] + a * (zn[1] - z[1])};
+                if (model_radius<K>(m, za) > kSolverRho) out = a;
+                else in = a;
+            }
+            z[0] += in * (zn[0] - z[0]);
+            z[1] += in * (zn[1] - z[1]);
+            break;
+        }
+        double gn[2], Hn[3];
+        double fn = model_eval<K>(m, zn, gn, Hn);
+        for (int j = 0; j < 30 && fn > fz + 1e-14 * fabs(fz); ++j) {   // the model went up: halve the step
+            zn[0] = 0.5 * (z[0] + zn[0]);
+            zn[1] = 0.5 * (z[1] + zn[1]);
+            fn = model_eval<K>(m, zn, gn, Hn);
+        }
+        double srel = 0.0;
+        for (int i = 0; i < 2; ++i) srel = fmax(srel, fabs(zn[i] - z[i]) / fmin(z[i], 1.0 - z[i]));
+        z[0] = zn[0];
+        z[1] = zn[1];
+        fz = fn;
+        gz[0] = gn[0];
+        gz[1] = gn[1];
+        Hz[0] = Hn[0];
+        Hz[1] = Hn[1];
+        Hz[2] = Hn[2];
+        if (srel <= 1e-12) {                                  // Newton converges quadratically: z is the minimiser
+            conv = true;
+            break;
+        }
     }
-    double xn[2], step = 0.0;
-    bool small = true;
-    for (int i = 0; i < 2; ++i) {
-        xn[i] = fmin(st.hi[i], fmax(st.lo[i], x[i] + a * d[i]));
-        step = fmax(step, fabs(xn[i] - x[i]));
-        // RELATIVE to the distance from 0 / 1: the mixture weights are linear in eps_l and the terms with
-        // y ~ eps_l dominate the curvature, so f''' / f'' ~ 1 / min(x, 1 - x) and the error a Newton step of
-        // relative size t leaves behind is ~ t^2 of the parameter (t = 2e-4: 4e-8, against the 1e-6 of north_star)
-        small = small && fabs(xn[i] - x[i]) <= st.tol * fmin(x[i], 1.0 - x[i]);
-    }
-    st.step = step;
+    st.step = fmax(fabs(z[0] - x[0]), fabs(z[1] - x[1]));
     st.xprev[0] = x[0];
     st.xprev[1] = x[1];
     st.fprev = f;
     st.have_prev = 1;
-    st.x[0] = xn[0];
-    st.x[1] = xn[1];
-    if (small) {
-        // final step: second-order model of f at the new point (the cubic term, ~ n t^3 / 3 for n elements with
-        // y ~ eps_l, is below 1e-11 of |f| ~ n for t = 2e-4)
-        const double e0 = xn[0] - x[0], e1 = xn[1] - x[1];
-        st.f = f + (g0 * e0 + g1 * e1) + 0.5 * (H00 * e0 * e0 + 2.0 * H01 * e0 * e1 + H11 * e1 * e1);
-        st.done = 1;
-        return;
+    st.x[0] = z[0];
+    st.x[1] = z[1];
+    if (conv) {
+        double pos, val;
+        model_bounds<K>(m, z, pos, val);
+        if (pos <= st.tol * st.tol && val <= 1e-12 * fabs(fz)) {
+            st.f = fz;
+            st.done = 1;
+            return;
+        }
     }
     st.f = f;
     if (st.nfev >= st.max_evals) {                            // budget: stay at the evaluated point
@@ -171,6 +336,53 @@ __device__ __forceinline__ SubTheta sub_theta(double eta, double epsilon) {
     return t;
 }
 
+// Moments of the series model an evaluation accumulates: a[k - 2] = A_k, b[k - 2] = B_k, k = 2..K
+struct SolverMoments {
+    double a[kSolverK - 1], b[kSolverK - 1];
+};
+static_assert(kSolverK >= 2 && kSolverK <= 8 && kSolverK % 2 == 0, "the remainder bound needs an even K");
+
+// m[k - 2] += x^k, k = 2..K (elements of weight 1: a power tree, one instruction per moment)
+__device__ __forceinline__ void add_powers1(double* m, double x) {
+    const double x2 = x * x, x3 = x2 * x;
+    m[0] += x2;
+    if (kSolverK >= 3) m[1] += x3;
+    if (kSolverK >= 4) m[2] = fma(x2, x2, m[2]);
+    if (kSolverK >= 5) m[3] = fma(x3, x2, m[3]);
+    if (kSolverK >= 6) m[4] = fma(x3, x3, m[4]);
+    if (kSolverK >= 7) {
+        const double x4 = x2 * x2;
+        m[5] = fma(x4, x3, m[5]);
+        m[6] = fma(x4, x4, m[6]);
+    }
+}
+
+// m[k - 2] += w x^k, k = 2..K
+__device__ __forceinline__ void add_powers(double* m, double w, double x) {
+    double pw = w * x;
+#pragma unroll
+    for (int k = 2; k <= kSolverK; ++k) {
+        pw *= x;
+        m[k - 2] += pw;
+    }
+}
+
+// The values the last CTA reduces: {obj, ge, gh, A_2, B_2, (slot of the theta-free part), A_3.., B_3..}
+__device__ __forceinline__ void solver_sums(double obj, double ge, double gh, const SolverMoments& mo,
+                                            double (&v)[kSolverVals]) {
+    v[0] = obj;
+    v[1] = ge;
+    v[2] = gh;
+    v[3] = mo.a[0];
+    v[4] = mo.b[0];
+    v[5] = 0.0;
+#pragma unroll
+    for (int k = 3; k <= kSolverK; ++k) {
+        v[6 + (k - 3)] = mo.a[k - 2];
+        v[6 + (kSolverK - 2) + (k - 3)] = mo.b[k - 2];
+    }
+}
+
 __device__ __forceinline__ void solver_publish(const SolverState& st, SolverPublished* pub, unsigned long long seq) {
     if (pub == nullptr) return;
     const double* src = reinterpret_cast<const double*>(&st);
@@ -183,8 +395,8 @@ __device__ __forceinline__ void solver_publish(const SolverState& st, SolverPubl
 }
 
 // Epilogue of an evaluation kernel, run by ALL threads of the CTA that arrived last: s_sums holds
-// this rank's {obj, ge, gh, qa, qb} (shared memory, kSolverVals slots); the theta-free part of
-// E_lM is read from konst_dev (this rank's share); exchange, step, publication.
+// this rank's sums (shared memory, kSolverVals slots, slot 5 free); the theta-free part of E_lM is
+// read from konst_dev (this rank's share) into slot 5; exchange, step, publication.
 __device__ __forceinline__ void solver_epilogue(double* s_sums, SolverState* state, const double* konst_dev,
                                                 const CommPeers& peers, int rank, int world,
                                                 SolverPublished* pub, unsigned long long seq) {
@@ -193,7 +405,7 @@ __device__ __forceinline__ void solver_epilogue(double* s_sums, SolverState* sta
     const bool ok = comm_exchange_cta(s_sums, kSolverVals, peers, rank, world, kCommSpinCycles);
     if (threadIdx.x == 0) {
         SolverState st = *state;
-        if (ok) solver_step(st, s_sums);
+        if (ok) solver_step<kSolverK>(st, s_sums);
         else st.done = 3;
         *state = st;
         __threadfence();

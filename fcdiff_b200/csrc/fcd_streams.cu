@@ -447,16 +447,18 @@ constexpr int kEvStage = kEvChunk * 8 + kEvChunk;            // bytes: p, then c
 constexpr size_t ev_ring_bytes(int depth) { return (size_t)kEvWarps * depth * (kEvStage + 8); }
 
 struct CodedAcc {
-    double obj, ge, gh, prod, qa, qb;
+    double obj, ge, gh, prod;
 };
 
-// HESS: also the two sums of squares the Newton step needs (fcd_solver.cuh): qa over l < 2, qb over l = 2.
+// HESS: also the moments of the solver's series model (fcd_solver.cuh), one set for both accumulators:
+// sum t^k (A_k, l < 2) and sum v^k (B_k, l = 2), k = 2..K.
 // The gradient weights are formed from the code in the ALU (it has the headroom; the shared-memory pipe,
 // with one 16-byte table read per element for {a_l, b_l} already, does not): sgn = -1, +1 for l = 0, 1 and
 // y = [l = 2] (codes 2, 4, 5).  acc.ge collects sum sgn d only: the l = 2
 // part of sum s_l d is (2 eta - 1) acc.gh and is added once, after the plane.
 template <bool GRAD, bool FAST, bool HESS>
-__device__ __forceinline__ void coded_elem(double p, int code, const double2* s_ab, const double* s_tab, CodedAcc& acc) {
+__device__ __forceinline__ void coded_elem(double p, int code, const double2* s_ab, const double* s_tab, CodedAcc& acc,
+                                           SolverMoments& mo) {
     const double2 ab = s_ab[code];
     const double M = fma(ab.y, p, ab.x);
     double rcp = 0.0;
@@ -480,8 +482,8 @@ __device__ __forceinline__ void coded_elem(double p, int code, const double2* s_
         acc.ge += t;
         acc.gh += v;
         if (HESS) {
-            acc.qa = fma(t, t, acc.qa);
-            acc.qb = fma(v, v, acc.qb);
+            add_powers1(mo.a, t);
+            add_powers1(mo.b, v);
         }
     }
 }
@@ -579,7 +581,10 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
     // the table and the constants are staged while the first chunks are in flight
     const double* s_tab = load_log_table<FAST>(tab, s_dyn);
 
-    CodedAcc a0 = {0.0, 0.0, 0.0, 1.0, 0.0, 0.0}, a1 = {0.0, 0.0, 0.0, 1.0, 0.0, 0.0};
+    CodedAcc a0 = {0.0, 0.0, 0.0, 1.0}, a1 = {0.0, 0.0, 0.0, 1.0};
+    SolverMoments mo;
+#pragma unroll
+    for (int k = 0; k < kSolverK - 1; ++k) mo.a[k] = mo.b[k] = 0.0;
     int nf = 0;                                              // factors in each running product
     int d = 0;
     uint32_t phase = 0;
@@ -607,8 +612,8 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
         for (int j = 0; j < kEvChunk / 64; ++j) {
             const double2 v = *reinterpret_cast<const double2*>(st + (64 * j + 2 * lane) * 8);
             const uint32_t c2 = *reinterpret_cast<const unsigned short*>(st + kEvChunk * 8 + 64 * j + 2 * lane);
-            coded_elem<GRAD, FAST, SOLVE>(v.x, c2 & 0xff, s_ab, s_tab, a0);
-            coded_elem<GRAD, FAST, SOLVE>(v.y, c2 >> 8, s_ab, s_tab, a1);
+            coded_elem<GRAD, FAST, SOLVE>(v.x, c2 & 0xff, s_ab, s_tab, a0, mo);
+            coded_elem<GRAD, FAST, SOLVE>(v.y, c2 >> 8, s_ab, s_tab, a1, mo);
         }
         nf += kEvChunk / 64;
         if (nf + kEvChunk / 64 > kProdMax) flush();
@@ -619,12 +624,13 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
         const unsigned char* st = ring + d * kEvStage;
         flush();
         for (int e = lane; e < left; e += 32)
-            coded_elem<GRAD, FAST, SOLVE>(reinterpret_cast<const double*>(st)[e], st[kEvChunk * 8 + e], s_ab, s_tab, a0);
+            coded_elem<GRAD, FAST, SOLVE>(reinterpret_cast<const double*>(st)[e], st[kEvChunk * 8 + e], s_ab, s_tab, a0,
+                                          mo);
     }
     flush();
     const double al[3] = {T.al[0], T.al[1], T.al[2]}, bl[3] = {T.bl[0], T.bl[1], T.bl[2]};
     const double sl[3] = {-1.0, 1.0, 2.0 * T.eta - 1.0};
-    double obj = a0.obj + a1.obj, gh = a0.gh + a1.gh, qa = a0.qa + a1.qa, qb = a0.qb + a1.qb;
+    double obj = a0.obj + a1.obj, gh = a0.gh + a1.gh;
     double ge = fma(sl[2], gh, a0.ge + a1.ge);               // sum s_l d over the plane: l < 2 signed, l = 2 through gh
     for (; cp < nq01; advance()) {                           // records {p, w_0, w_1, w_2}: real weights, three logs each
         const long long left = (n3 - (cp - nq0) * kEvChunk) >> 2;
@@ -649,8 +655,8 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
                         ge = fma(sl[l], dd, ge);
                         if (l == 2) gh += dd;
                         if (SOLVE) {
-                            if (l == 2) qb = fma(dd, g, qb);
-                            else qa = fma(dd, g, qa);
+                            if (l == 2) add_powers(mo.b, w[l], g);
+                            else add_powers(mo.a, w[l], sl[l] * g);
                         }
                     } else {
                         obj = fma(w[l], fast_log<FAST>(M, s_tab), obj);
@@ -682,8 +688,8 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
                     ge += fma(sx ? 1.0 : -1.0, dx, -sl[2] * d2);
                     gh -= d2;
                     if (SOLVE) {
-                        qa = fma(dx, gx, qa);
-                        qb = fma(-d2, g2, qb);
+                        add_powers(mo.a, q, sx ? gx : -gx);
+                        add_powers(mo.b, -q, g2);
                     }
                 } else {
                     obj = fma(q, fast_log<FAST>(Mx, s_tab) - fast_log<FAST>(M2, s_tab), obj);
@@ -692,8 +698,9 @@ elm_coded_kernel(const double* __restrict__ PsE, const uint8_t* __restrict__ cod
         }
     }
     if (SOLVE) {
-        double v[5] = {obj, ge, gh, qa, qb};
-        if (grid_reduce_last<5, kEvThreads>(v, ws, s_sums))
+        double v[kSolverVals];
+        solver_sums(obj, ge, gh, mo, v);
+        if (grid_reduce_last<kSolverVals, kEvThreads>(v, ws, s_sums))
             solver_epilogue(s_sums, state, konst_dev, peers, rank, world, pub, seq);
     } else {
         // dE/d eta = -(2 eps - 1) sum_{l = 2} d;  dE/d eps = -sum s_l d                 (fit.py:600-697)

@@ -227,8 +227,8 @@ class UnsharedRegionFit(object):
         self.convergence_rule = "reference"
         self.missing = "reject"       # "marginalize": NaN correlations are unobserved entries, integrated out
         self.theta_solver = "newton"  # (eta, epsilon): device-resident Newton | host-driven SciPy L-BFGS-B
-        self.solver_tol = 2e-4        # newton: a step with |dx_i| <= tol * min(x_i, 1 - x_i) is taken without another
-        #                               evaluation (leaves a relative error ~ tol^2 = 4e-8 in eta, epsilon)
+        self.solver_tol = 2e-4        # newton: the solve ends on the series model of the last evaluation when its
+        #                               remainder bound puts eta, epsilon within tol^2 = 4e-8 (relative) of the optimum
         self.energy_behind_solver = True   # newton: enqueue K4 behind the first batch of evaluations (one wait for both)
         self.uniform_fast_path = True      # constant q_R (the start): row log-sums as running products (fcd_uniform.cu)
         self.speculative_estep = True      # newton, inside run(): the next iteration's K2 enqueued behind the solve
@@ -1935,7 +1935,7 @@ class UnsharedRegionFit(object):
         terms = None
         spec = None
         self._spec = None
-        first = max(2, min(6, self._last_nfev))
+        first = max(1, min(6, self._last_nfev))    # one launch when the last solve ended on its first evaluation
         while True:
             # the epsilon box of this pass: the reference's bounds, at most a factor 8 towards 0 or 1
             # from the start point -- it sizes the shared-memory logarithm table of the kernels

@@ -424,6 +424,14 @@ FCD_API int fcd_elm_tiered_solve(const double* P, int64_t planeStride, int64_t C
 FCD_API int fcd_solver_init_host(void* state_host, double eta0, double eps0, const double* lo2_host,
                          const double* hi2_host, double tol, int32_t max_evals);
 FCD_API int fcd_solver_step_host(void* state_host, const double* sums6_host);
+/* The same with K moments per series (K = 2, 4, 6, 8): sums = the six above, then A_3..A_K, B_3..B_K
+ * (csrc/fcd_solver.cuh, series model); the evaluation kernels deliver fcd_solver_moments() of them.
+ * fcd_solver_model_host: the series model of such sums made at (eta0, eps0), at z2 = (eta, eps):
+ * out4 = {model value, position bound, value bound, trust-region radius}. */
+FCD_API int64_t fcd_solver_moments(void);
+FCD_API int fcd_solver_step_host_moments(void* state_host, const double* sums_host, int32_t K);
+FCD_API int fcd_solver_model_host(const double* sums_host, int32_t K, double eta0, double eps0, const double* z2_host,
+                                  double* out4_host);
 FCD_API int fcd_solver_wait(const void* published_host, uint64_t seq, void* state_out_host, int32_t timeout_ms);
 
 /* K4 -- free-energy terms; replaces `_eval_energy` and `_eval_E_*`
