@@ -51,25 +51,19 @@ SIGNATURES = {
     "fcd_pack_patients": (c_int, [_P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P]),
     "fcd_unpack_patients": (c_int, [_P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P]),
     "fcd_c_to_nm": (c_int, [c_int64, c_int64, _P, _P, _P]),
-    "fcd_healthy_stats": (c_int, [_P, c_int64, c_int32, c_int64, _P, _P, _P]),
-    "fcd_healthy_stats_masked": (c_int, [_P, c_int64, c_int32, c_int64, _P, _P, _P, _P]),
+    "fcd_healthy_stats": (c_int, [_P, c_int64, c_int32, c_int64, _P, _P, _P, _P]),
     "fcd_row_logsums": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, _P]),
-    "fcd_estep_qF_rowsums": (c_int, [_P, _P, c_int32, _P, c_int64, _D3, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_estep_qF_rowsums_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, _D3, POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_estep_qF_rowsums": (c_int, [_P, _P, _P, c_int32, _P, c_int64, _D3, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_elm_rowsums": (c_int, [_P, _P, c_int64, _D3, _P, _P, _P]),
-    "fcd_healthy_stats_cols": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P]),
-    "fcd_healthy_stats_cols_masked": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P, _P]),
+    "fcd_healthy_stats_cols": (c_int, [_P, c_int64, c_int64, _P, c_int32, _P, _P, _P, _P]),
     "fcd_gather_columns": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P, c_int64, c_int64, _P]),
     "fcd_edge_table": (c_int, [c_int64, c_int64, _P, _P]),
-    "fcd_resp_cache": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
-    "fcd_resp_cache_masked": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, _P]),
+    "fcd_resp_cache": (c_int, [_P, c_int64, c_int32, c_int64, POINTER(FcdTheta), _P, c_int64, _P, c_int32, _P]),
     "fcd_map_labels": (c_int, [_P, c_int64, c_int32, _P, _P]),
     "fcd_peak_states_F": (c_int, [_P, c_int64, _P, _P]),
     "fcd_peak_states_R": (c_int, [_P, c_int32, c_int32, c_int64, _P, _P]),
-    "fcd_estep_qF": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64, c_int32, _P,
+    "fcd_estep_qF": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64, c_int32, _P,
                              POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_estep_qF_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int64,
-                                    c_int32, _P, POINTER(FcdTheta), _P, _P, _P]),
     "fcd_estep_qR": (c_int, [_P, c_int64, c_int32, c_int32, c_int32, c_int32, _D3, c_int32, _P, _P, _P]),
     "fcd_pstar_refresh_em": (c_int, [_P, c_int64, c_int64, c_int32, c_int32, c_int64, c_int64, _P, _P, _P, _P]),
     "fcd_region_weights_em": (c_int, [_P, c_int64, c_int64, c_int32, c_int32, c_int64, c_int64, _P, _P, _P, _P,
@@ -85,16 +79,9 @@ SIGNATURES = {
                                _P, _P]),
     "fcd_code_records": (c_int, [_P, c_int64, _P, _P, c_int64, _P, _P, c_int64, c_int32, c_int64, _P, _P, _P, _P, c_int64,
                                  c_int32, _P, _P, _P, _P, _P, _P, _P, c_int64, _P, c_int64, _P, _P, _P]),
-    "fcd_estep_qF_coded": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P,
-                                   _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_estep_qF_coded_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32,
-                                          _P, _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_estep_qF_coded_solved": (c_int, [_P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P,
-                                          _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, c_double, c_double,
-                                          _P, _P, _P]),
-    "fcd_estep_qF_coded_solved_masked": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P,
-                                                 c_int32, _P, _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P,
-                                                 c_double, c_double, _P, _P, _P]),
+    "fcd_estep_qF_coded": (c_int, [_P, _P, _P, c_int32, _P, c_int64, c_int64, c_int32, c_int64, _P, c_int32, _P,
+                                   _P, c_int64, _P, _P, _P, _P, _P, POINTER(FcdTheta), _P, c_double, c_double,
+                                   _P, _P, _P]),
     "fcd_elm_coded": (c_int, [_P, _P, c_int64, _P, c_int64, _P, c_int64, POINTER(FcdTheta), c_int32, _P, _P, _P]),
     "fcd_solver_state_bytes": (c_int64, []),
     "fcd_solver_published_bytes": (c_int64, []),
@@ -112,10 +99,8 @@ SIGNATURES = {
     "fcd_solver_step_host_moments": (c_int, [_P, _D3, c_int32]),
     "fcd_solver_model_host": (c_int, [_D3, c_int32, c_double, c_double, _D3, _D3]),
     "fcd_solver_wait": (c_int, [_P, c_uint64, _P, c_int32]),
-    "fcd_energy_terms": (c_int, [_P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
+    "fcd_energy_terms": (c_int, [_P, _P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
                                  POINTER(FcdTheta), c_double, _P, _P, _P, _P]),
-    "fcd_energy_terms_masked": (c_int, [_P, _P, _P, c_int32, _P, _P, c_int64, _P, _P, c_int32, c_int32,
-                                        POINTER(FcdTheta), c_double, _P, _P, _P, _P]),
     "fcd_patient_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
     "fcd_patient_terms": (c_int, [_P, c_int64, _P, c_int64, c_int32, c_int64, _P, _P, _P, _P, c_int32, POINTER(FcdTheta),
                                   _P, _P, _P]),
@@ -124,12 +109,10 @@ SIGNATURES = {
     "fcd_connection_posteriors": (c_int, [_P, c_int64, c_int64, c_int32, c_int64, _P, _P, _P, c_int32,
                                           POINTER(FcdTheta), _P, _P, _P, _P, _P, _P]),
     "fcd_control_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
-    "fcd_control_terms": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_control_terms_masked": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, _P]),
+    "fcd_control_terms": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, c_int32, _P]),
     "fcd_state_moments": (c_int, [_P, _P, c_int32, _P, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int32, _P,
                                   POINTER(FcdTheta), _P, _P, _P]),
-    "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),
-    "fcd_materialize_lps_masked": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, _P]),
+    "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, c_int32, _P]),
     "fcd_eval_M": (c_int, [_P, c_int64, c_double, c_double, c_int32, c_int32, _P, _P]),
     "fcd_lqF_from_arrays": (c_int, [_P, _P, c_int64, c_int32, c_int32, _P, c_int32, _D3, _P, _P]),
     "fcd_region_weights_from_lM": (c_int, [_P, c_int64, c_int32, _P, _P, _P]),
@@ -184,7 +167,7 @@ def load():
         fn = getattr(lib, name)          # AttributeError if the symbol is missing
         fn.restype = restype
         fn.argtypes = argtypes
-    if lib.fcd_version() < 121:
+    if lib.fcd_version() < 122:
         raise FcdError("fcdiff_b200: stale libfcdiff_b200.so (version %d)" % lib.fcd_version())
     _lib = lib
     return lib

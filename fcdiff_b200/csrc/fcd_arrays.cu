@@ -247,10 +247,12 @@ using namespace fcd;
 
 extern "C" {
 
-static int materialize_lps_launch(bool masked, const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
-                                  const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
+int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
+                        const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, int32_t missing,
+                        void* stream) {
     FCD_REQUIRE(theta_host != nullptr, "fcd_materialize_lps: theta is NULL");
     FCD_REQUIRE(C >= 0 && H >= 0 && U >= 0, "fcd_materialize_lps: bad shape");
+    FCD_REQUIRE(missing == 0 || missing == 1, "fcd_materialize_lps: missing must be 0 or 1, got %d", missing);
     LpsParams p;
     for (int k = 0; k < 3; ++k) {
         p.mu[k] = theta_host->mu[k];
@@ -264,29 +266,19 @@ static int materialize_lps_launch(bool masked, const double* b, const double* bt
     cudaStream_t st = (cudaStream_t)stream;
     int rc = 0;
     if (b != nullptr && lpB != nullptr && C * H > 0) {
-        if (masked) materialize_b_kernel<true><<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
+        if (missing) materialize_b_kernel<true><<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
         else materialize_b_kernel<false><<<arr_grid(C * H, kArrThreads), kArrThreads, 0, st>>>(b, C * H, p, lpB);
         rc = check_launch("fcd_materialize_lps(b)");
         if (rc) return rc;
     }
     if (bt != nullptr && pBt != nullptr && lM != nullptr && C * U > 0) {
-        if (masked)
+        if (missing)
             materialize_bt_kernel<true><<<arr_grid(C * U, kArrThreads), kArrThreads, 0, st>>>(bt, C * U, p, pBt, lM);
         else
             materialize_bt_kernel<false><<<arr_grid(C * U, kArrThreads), kArrThreads, 0, st>>>(bt, C * U, p, pBt, lM);
         rc = check_launch("fcd_materialize_lps(bt)");
     }
     return rc;
-}
-
-int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
-                        const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
-    return materialize_lps_launch(false, b, bt, C, H, U, theta_host, lpB, pBt, lM, stream);
-}
-
-int fcd_materialize_lps_masked(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
-                               const fcd_theta* theta_host, double* lpB, double* pBt, double* lM, void* stream) {
-    return materialize_lps_launch(true, b, bt, C, H, U, theta_host, lpB, pBt, lM, stream);
 }
 
 int fcd_eval_M(const double* p, int64_t n, double eta, double epsilon, int32_t k, int32_t l,

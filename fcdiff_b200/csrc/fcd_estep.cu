@@ -1151,51 +1151,39 @@ int fcd_edge_table(int64_t c0, int64_t C, int32_t* nm, void* stream) {
     return check_launch("fcd_edge_table");
 }
 
+// S0 == NULL: every control is observed (the unmasked kernel); otherwise NaN entries are left out and S0 counts
+// the observed controls of each edge.
 int fcd_healthy_stats(const double* b, int64_t C, int32_t H, int64_t pitchH,
-                      double* S1, double* S2, void* stream) {
+                      double* S1, double* S2, double* S0, void* stream) {
     FCD_REQUIRE(C >= 0 && H >= 1 && pitchH >= H, "fcd_healthy_stats: bad shape C=%lld H=%d pitch=%lld",
                 (long long)C, H, (long long)pitchH);
+    FCD_REQUIRE(S0 == nullptr || C == 0 || (b != nullptr && S1 != nullptr && S2 != nullptr),
+                "fcd_healthy_stats: NULL argument");
     if (C == 0) return 0;
-    healthy_stats_kernel<false><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
-        b, C, H, pitchH, S1, S2, nullptr);
+    if (S0 == nullptr)
+        healthy_stats_kernel<false><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
+            b, C, H, pitchH, S1, S2, nullptr);
+    else
+        healthy_stats_kernel<true><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
+            b, C, H, pitchH, S1, S2, S0);
     return check_launch("fcd_healthy_stats");
 }
 
-int fcd_healthy_stats_masked(const double* b, int64_t C, int32_t H, int64_t pitchH,
-                             double* S1, double* S2, double* S0, void* stream) {
-    FCD_REQUIRE(C >= 0 && H >= 1 && pitchH >= H, "fcd_healthy_stats_masked: bad shape C=%lld H=%d pitch=%lld",
-                (long long)C, H, (long long)pitchH);
-    FCD_REQUIRE(C == 0 || (b != nullptr && S1 != nullptr && S2 != nullptr && S0 != nullptr),
-                "fcd_healthy_stats_masked: NULL argument");
-    if (C == 0) return 0;
-    healthy_stats_kernel<true><<<grid_for_rows(C, kEdgeThreads / 32, 8), kEdgeThreads, 0, (cudaStream_t)stream>>>(
-        b, C, H, pitchH, S1, S2, S0);
-    return check_launch("fcd_healthy_stats_masked");
-}
-
-static int resp_cache_launch(bool masked, const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                             const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
+int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, int32_t missing,
+                   void* stream) {
     FCD_REQUIRE(theta_host != nullptr && bt != nullptr && P != nullptr, "fcd_resp_cache: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && pitchU >= U && planeStride >= C * pitchU, "fcd_resp_cache: bad shape");
+    FCD_REQUIRE(missing == 0 || missing == 1, "fcd_resp_cache: missing must be 0 or 1, got %d", missing);
     if (C == 0) return 0;
     const ThetaDev th = make_theta_dev(*theta_host, 0);
-    if (masked)
+    if (missing)
         resp_cache_kernel<true><<<grid_for_rows(C * pitchU, 256, 16), 256, 0, (cudaStream_t)stream>>>(
             bt, C, U, pitchU, th, P, planeStride, L);
     else
         resp_cache_kernel<false><<<grid_for_rows(C * pitchU, 256, 16), 256, 0, (cudaStream_t)stream>>>(
             bt, C, U, pitchU, th, P, planeStride, L);
-    return check_launch(masked ? "fcd_resp_cache_masked" : "fcd_resp_cache");
-}
-
-int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
-    return resp_cache_launch(false, bt, C, U, pitchU, theta_host, P, planeStride, L, stream);
-}
-
-int fcd_resp_cache_masked(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                          const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream) {
-    return resp_cache_launch(true, bt, C, U, pitchU, theta_host, P, planeStride, L, stream);
+    return check_launch("fcd_resp_cache");
 }
 
 int fcd_map_labels(const double* lq, int64_t n, int32_t width, uint8_t* labels, void* stream) {
@@ -1220,11 +1208,11 @@ int fcd_peak_states_R(const double* qR, int32_t N, int32_t U, int64_t pitchS, ui
     return check_launch("fcd_peak_states_R");
 }
 
-// S0 == NULL: every edge has all H controls (fcd_estep_qF); otherwise fcd_estep_qF_masked.
-static int estep_qF_launch(const double* S1, const double* S2, const double* S0, int32_t H,
-                           const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                           const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
-                           const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
+// S0 == NULL: every edge has all H controls (the unmasked kernel).
+int fcd_estep_qF(const double* S1, const double* S2, const double* S0, int32_t H,
+                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
+                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && P != nullptr && qR != nullptr && rstate != nullptr && nm != nullptr &&
                 lqF != nullptr, "fcd_estep_qF: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && U < 65536 && pitchU >= U && pitchS >= U && N >= 2 && N < 65536,
@@ -1256,52 +1244,39 @@ static int estep_qF_launch(const double* S1, const double* S2, const double* S0,
         if (fast) K2_LAUNCH(true, false); else K2_LAUNCH(false, false);
     }
 #undef K2_LAUNCH
-    return check_launch(S0 != nullptr ? "fcd_estep_qF_masked" : "fcd_estep_qF");
+    return check_launch("fcd_estep_qF");
 }
 
-int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
-                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
-                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    return estep_qF_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, rstate, pitchS, N, nm, theta_host,
-                           lqF, qF, stream);
-}
-
-int fcd_estep_qF_masked(const double* S1, const double* S2, const double* S0, int32_t H,
-                        const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                        const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
-                        const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_masked: S0 is NULL");
-    return estep_qF_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, rstate, pitchS, N, nm, theta_host,
-                           lqF, qF, stream);
-}
-
-// `solved` == NULL: (eta, epsilon) of theta_host; otherwise the solver state block a device-resident solve
-// enqueued BEFORE this launch leaves its solution in, with [eps_lo, eps_hi] the box of that solve (it
-// sizes the logarithm table like fcd_elm_coded_solve does).
-static int estep_qF_coded_launch(const double* S1, const double* S2, const double* S0, int32_t H,
-                                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                                 const double* qR, int32_t N, const int32_t* nm,
-                                 const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                                 const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                                 const fcd_theta* theta_host, const SolverState* solved, double eps_lo, double eps_hi,
-                                 double* lqF, double* qF, void* stream) {
+// S0 == NULL: every edge has all H controls (the unmasked kernel).  solver_state == NULL: (eta, epsilon) of
+// theta_host; otherwise the solver state block a device-resident solve enqueued BEFORE this launch leaves its
+// solution in, with [eps_lo, eps_hi] the box of that solve (it sizes the logarithm table like
+// fcd_elm_coded_solve does).
+int fcd_estep_qF_coded(const double* S1, const double* S2, const double* S0, int32_t H,
+                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
+                       const double* qR, int32_t N, const int32_t* nm,
+                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
+                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
+                       const fcd_theta* theta_host, const void* solver_state, double eps_lo, double eps_hi,
+                       double* lqF, double* qF, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && S1 != nullptr && S2 != nullptr && P != nullptr && qR != nullptr &&
                 nm != nullptr && code != nullptr && counts != nullptr && keysF != nullptr && keysH != nullptr &&
                 rowoff != nullptr && Hh != nullptr && lqF != nullptr, "fcd_estep_qF_coded: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && U < 65536 && pitchU >= U && N >= 2 && N < 65536, "fcd_estep_qF_coded: bad shape");
+    FCD_REQUIRE((reinterpret_cast<uintptr_t>(solver_state) & 7) == 0,
+                "fcd_estep_qF_coded: solver state must be a device pointer (fcd_solver_init)");
     FCD_REQUIRE(((reinterpret_cast<uintptr_t>(P) | reinterpret_cast<uintptr_t>(code) | reinterpret_cast<uintptr_t>(rowoff) |
                   reinterpret_cast<uintptr_t>(Hh)) & 15) == 0 && (reinterpret_cast<uintptr_t>(counts) & 7) == 0 &&
                 pitchU % 2 == 0 && planeStride % 2 == 0 && pitchQ >= pitchU && pitchQ % 16 == 0,
                 "fcd_estep_qF_coded: planes / code / rowoff / half records must be 16-byte aligned (even pitchU, pitchQ % 16 == 0)");
     if (C == 0) return 0;
+    const SolverState* solved = static_cast<const SolverState*>(solver_state);
     const ThetaDev th = make_theta_dev(*theta_host, H);
     cudaStream_t st = (cudaStream_t)stream;
     LogTabWindow tab;
     double w_eps[3] = {th.epsl[0], th.epsl[1], th.epsl[2]}, w_al[3] = {th.al[0], th.al[1], th.al[2]};
     if (solved != nullptr) {
         // every mixture weight the solve can have ended at lies in [m / 2, 1], m = min(eps_lo, 1 - eps_hi)
-        FCD_REQUIRE(eps_lo > 0.0 && eps_lo <= eps_hi && eps_hi < 1.0, "fcd_estep_qF_coded_solved: bad box");
+        FCD_REQUIRE(eps_lo > 0.0 && eps_lo <= eps_hi && eps_hi < 1.0, "fcd_estep_qF_coded: bad box");
         const double m = eps_lo < 1.0 - eps_hi ? eps_lo : 1.0 - eps_hi;
         for (int l = 0; l < 3; ++l) {
             w_eps[l] = m;
@@ -1335,57 +1310,7 @@ static int estep_qF_coded_launch(const double* S1, const double* S2, const doubl
         if (fast) K2C_LAUNCH(true, false); else K2C_LAUNCH(false, false);
     }
 #undef K2C_LAUNCH
-    return check_launch(S0 != nullptr ? "fcd_estep_qF_coded_masked" : "fcd_estep_qF_coded");
-}
-
-int fcd_estep_qF_coded(const double* S1, const double* S2, int32_t H,
-                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                       const double* qR, int32_t N, const int32_t* nm,
-                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                       const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    return estep_qF_coded_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
-                                 keysF, keysH, rowoff, Hh, theta_host, nullptr, 0.0, 0.0, lqF, qF, stream);
-}
-
-int fcd_estep_qF_coded_masked(const double* S1, const double* S2, const double* S0, int32_t H,
-                              const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                              const double* qR, int32_t N, const int32_t* nm,
-                              const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                              const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                              const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_coded_masked: S0 is NULL");
-    return estep_qF_coded_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
-                                 keysF, keysH, rowoff, Hh, theta_host, nullptr, 0.0, 0.0, lqF, qF, stream);
-}
-
-int fcd_estep_qF_coded_solved(const double* S1, const double* S2, int32_t H,
-                              const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                              const double* qR, int32_t N, const int32_t* nm,
-                              const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                              const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                              const fcd_theta* theta_host, const void* solver_state, double eps_lo, double eps_hi,
-                              double* lqF, double* qF, void* stream) {
-    FCD_REQUIRE(solver_state != nullptr && (reinterpret_cast<uintptr_t>(solver_state) & 7) == 0,
-                "fcd_estep_qF_coded_solved: solver state must be a device pointer (fcd_solver_init)");
-    return estep_qF_coded_launch(S1, S2, nullptr, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
-                                 keysF, keysH, rowoff, Hh, theta_host, static_cast<const SolverState*>(solver_state),
-                                 eps_lo, eps_hi, lqF, qF, stream);
-}
-
-int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2, const double* S0, int32_t H,
-                                     const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                                     const double* qR, int32_t N, const int32_t* nm,
-                                     const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                                     const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                                     const fcd_theta* theta_host, const void* solver_state, double eps_lo,
-                                     double eps_hi, double* lqF, double* qF, void* stream) {
-    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_coded_solved_masked: S0 is NULL");
-    FCD_REQUIRE(solver_state != nullptr && (reinterpret_cast<uintptr_t>(solver_state) & 7) == 0,
-                "fcd_estep_qF_coded_solved_masked: solver state must be a device pointer (fcd_solver_init)");
-    return estep_qF_coded_launch(S1, S2, S0, H, P, planeStride, C, U, pitchU, qR, N, nm, code, pitchQ, counts,
-                                 keysF, keysH, rowoff, Hh, theta_host, static_cast<const SolverState*>(solver_state),
-                                 eps_lo, eps_hi, lqF, qF, stream);
+    return check_launch("fcd_estep_qF_coded");
 }
 
 int fcd_pstar_refresh_em(const double* Pe, int64_t planeStride, int64_t pitchU, int32_t u0, int32_t Ul, int64_t C,

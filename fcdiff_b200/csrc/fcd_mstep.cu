@@ -498,11 +498,12 @@ int fcd_elm_const(const double* L, int64_t C, int32_t U, int64_t pitchU,
     return check_launch("fcd_elm_const");
 }
 
-static int energy_terms_launch(const double* S1, const double* S2, const double* S0, int32_t H,
-                               const double* lqF, const double* qF, int64_t C,
-                               const double* lqR, const double* qR, int32_t N, int32_t U,
-                               const fcd_theta* theta_host, double elm, const void* solver_state,
-                               double* out6, double* ws, void* stream) {
+// S0 == NULL: every edge has all H controls (the unmasked kernel).
+int fcd_energy_terms(const double* S1, const double* S2, const double* S0, int32_t H,
+                     const double* lqF, const double* qF, int64_t C,
+                     const double* lqR, const double* qR, int32_t N, int32_t U,
+                     const fcd_theta* theta_host, double elm, const void* solver_state,
+                     double* out6, double* ws, void* stream) {
     FCD_REQUIRE(theta_host != nullptr && ws != nullptr && out6 != nullptr, "fcd_energy_terms: NULL argument");
     FCD_REQUIRE(C >= 0 && U >= 1 && N >= 2 && H >= 1, "fcd_energy_terms: bad shape");
     const ThetaDev th = make_theta_dev(*theta_host, H);
@@ -515,26 +516,7 @@ static int energy_terms_launch(const double* S1, const double* S2, const double*
     else
         energy_small_kernel<false><<<red_grid(work, kRedThreads), kRedThreads, 0, (cudaStream_t)stream>>>(
             S1, S2, nullptr, lqF, qF, C, lqR, qR, NU, th, elm, solved, out6, ws);
-    return check_launch(S0 != nullptr ? "fcd_energy_terms_masked" : "fcd_energy_terms");
-}
-
-int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
-                     const double* lqF, const double* qF, int64_t C,
-                     const double* lqR, const double* qR, int32_t N, int32_t U,
-                     const fcd_theta* theta_host, double elm, const void* solver_state,
-                     double* out6, double* ws, void* stream) {
-    return energy_terms_launch(S1, S2, nullptr, H, lqF, qF, C, lqR, qR, N, U, theta_host, elm, solver_state, out6, ws,
-                               stream);
-}
-
-int fcd_energy_terms_masked(const double* S1, const double* S2, const double* S0, int32_t H,
-                            const double* lqF, const double* qF, int64_t C,
-                            const double* lqR, const double* qR, int32_t N, int32_t U,
-                            const fcd_theta* theta_host, double elm, const void* solver_state,
-                            double* out6, double* ws, void* stream) {
-    FCD_REQUIRE(S0 != nullptr, "fcd_energy_terms_masked: S0 is NULL");
-    return energy_terms_launch(S1, S2, S0, H, lqF, qF, C, lqR, qR, N, U, theta_host, elm, solver_state, out6, ws,
-                               stream);
+    return check_launch("fcd_energy_terms");
 }
 
 int fcd_state_moments(const double* S1, const double* S2, int32_t H,

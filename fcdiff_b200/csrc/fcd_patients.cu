@@ -497,10 +497,11 @@ int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S) {
     return pt_row_blocks(C) * (int64_t)S * (int64_t)sizeof(double);
 }
 
-static int control_terms_launch(bool masked, const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                                const fcd_theta* theta_host, double* out, double* ws, void* stream) {
+int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
+                      const fcd_theta* theta_host, double* out, double* ws, int32_t missing, void* stream) {
     FCD_REQUIRE(X != nullptr && qF != nullptr && theta_host != nullptr && out != nullptr && ws != nullptr,
                 "fcd_control_terms: NULL argument");
+    FCD_REQUIRE(missing == 0 || missing == 1, "fcd_control_terms: missing must be 0 or 1, got %d", missing);
     const int64_t N = (int64_t)((sqrt(8.0 * (double)C + 1.0) + 1.0) * 0.5);
     FCD_REQUIRE(C >= 1 && N * (N - 1) / 2 == C, "fcd_control_terms: C=%lld is not N(N-1)/2", (long long)C);
     FCD_REQUIRE(S >= 1 && pitchS >= S, "fcd_control_terms: bad shape");
@@ -522,7 +523,7 @@ static int control_terms_launch(bool masked, const double* X, int64_t C, int32_t
     const int64_t grid = (warps * 32 + kPtThreads - 1) / kPtThreads;
     FCD_REQUIRE(warps < ((int64_t)1 << 26), "fcd_control_terms: %lld subjects are too many for one launch",
                 (long long)S);
-    if (masked)
+    if (missing)
         control_terms_rows_kernel<true><<<(unsigned)grid, kPtThreads, 0, st>>>(X, C, S, pitchS, qF, cc, nb, rows, lanesP,
                                                                                ws);
     else
@@ -533,16 +534,6 @@ static int control_terms_launch(bool masked, const double* X, int64_t C, int32_t
     connection_finish_kernel<<<(unsigned)((S + 31) / 32), kPtThreads, 0, st>>>(ws, nb, nullptr, C, S,
                                                                               (int)((S + 31) / 32), out, nullptr);
     return check_launch("fcd_control_terms(finish)");
-}
-
-int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                      const fcd_theta* theta_host, double* out, double* ws, void* stream) {
-    return control_terms_launch(false, X, C, S, pitchS, qF, theta_host, out, ws, stream);
-}
-
-int fcd_control_terms_masked(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                             const fcd_theta* theta_host, double* out, double* ws, void* stream) {
-    return control_terms_launch(true, X, C, S, pitchS, qF, theta_host, out, ws, stream);
 }
 
 int fcd_qR_change(const double* qR_old, const double* qR_new, int32_t N, int32_t U, double* maxU, double* out1,

@@ -68,28 +68,21 @@ using namespace fcd;
 
 extern "C" {
 
+// S0 == NULL: every control is observed (the unmasked kernel); otherwise NaN entries are left out and S0 counts
+// the observed controls of each edge.
 int fcd_healthy_stats_cols(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H, double* S1,
-                           double* S2, void* stream) {
+                           double* S2, double* S0, void* stream) {
     FCD_REQUIRE(X != nullptr && cols != nullptr && S1 != nullptr && S2 != nullptr, "fcd_healthy_stats_cols: NULL argument");
     FCD_REQUIRE(C >= 0 && H >= 1 && pitchS >= 1, "fcd_healthy_stats_cols: bad shape");
     if (C == 0) return 0;
     int64_t grid = (C + 7) / 8;
     if (grid > (int64_t)sm_count() * 16) grid = (int64_t)sm_count() * 16;
-    healthy_stats_cols_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2,
-                                                                                         nullptr);
+    if (S0 == nullptr)
+        healthy_stats_cols_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2,
+                                                                                             nullptr);
+    else
+        healthy_stats_cols_kernel<true><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2, S0);
     return check_launch("fcd_healthy_stats_cols");
-}
-
-int fcd_healthy_stats_cols_masked(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
-                                  double* S1, double* S2, double* S0, void* stream) {
-    FCD_REQUIRE(X != nullptr && cols != nullptr && S1 != nullptr && S2 != nullptr && S0 != nullptr,
-                "fcd_healthy_stats_cols_masked: NULL argument");
-    FCD_REQUIRE(C >= 0 && H >= 1 && pitchS >= 1, "fcd_healthy_stats_cols_masked: bad shape");
-    if (C == 0) return 0;
-    int64_t grid = (C + 7) / 8;
-    if (grid > (int64_t)sm_count() * 16) grid = (int64_t)sm_count() * 16;
-    healthy_stats_cols_kernel<true><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(X, C, pitchS, cols, H, S1, S2, S0);
-    return check_launch("fcd_healthy_stats_cols_masked");
 }
 
 int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, int32_t nplanes, int64_t C,

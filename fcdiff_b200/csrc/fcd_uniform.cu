@@ -203,9 +203,10 @@ int fcd_row_logsums(const double* P, int64_t planeStride, int64_t C, int32_t U, 
     return check_launch("fcd_row_logsums");
 }
 
-static int estep_qF_rowsums_launch(const double* S1, const double* S2, const double* S0, int32_t H, const double* S9,
-                                   int64_t C, const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF,
-                                   void* stream) {
+// S0 == NULL: every edge has all H controls (the unmasked kernel).
+int fcd_estep_qF_rowsums(const double* S1, const double* S2, const double* S0, int32_t H, const double* S9,
+                         int64_t C, const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF,
+                         void* stream) {
     FCD_REQUIRE(S1 != nullptr && S2 != nullptr && S9 != nullptr && w3_host != nullptr && theta_host != nullptr &&
                 lqF != nullptr && C >= 0 && H >= 1, "fcd_estep_qF_rowsums: bad argument");
     if (C == 0) return 0;
@@ -218,19 +219,7 @@ static int estep_qF_rowsums_launch(const double* S1, const double* S2, const dou
     else
         estep_qF_rowsums_kernel<false><<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(
             S1, S2, nullptr, S9, C, w3_host[0], w3_host[1], w3_host[2], th, lqF, qF);
-    return check_launch(S0 != nullptr ? "fcd_estep_qF_rowsums_masked" : "fcd_estep_qF_rowsums");
-}
-
-int fcd_estep_qF_rowsums(const double* S1, const double* S2, int32_t H, const double* S9, int64_t C,
-                         const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF, void* stream) {
-    return estep_qF_rowsums_launch(S1, S2, nullptr, H, S9, C, w3_host, theta_host, lqF, qF, stream);
-}
-
-int fcd_estep_qF_rowsums_masked(const double* S1, const double* S2, const double* S0, int32_t H, const double* S9,
-                                int64_t C, const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF,
-                                void* stream) {
-    FCD_REQUIRE(S0 != nullptr, "fcd_estep_qF_rowsums_masked: S0 is NULL");
-    return estep_qF_rowsums_launch(S1, S2, S0, H, S9, C, w3_host, theta_host, lqF, qF, stream);
+    return check_launch("fcd_estep_qF_rowsums");
 }
 
 int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const double* w3_host, double* out1, double* ws,

@@ -406,7 +406,8 @@ class UnsharedRegionFit(object):
                 ev_bt.record(side)
                 b_dev.copy_(b_t, non_blocking=b_t.is_pinned())
                 if Cl > 0:
-                    self._healthy_stats(b_dev, Cl, H, S1, S2, S0)
+                    _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2),
+                                                     _dev.ptr(S0), _dev.stream()), "fcd_healthy_stats")
                 ev_S = torch.cuda.Event()
                 ev_S.record(side)
             cur.wait_event(ev_bt)
@@ -416,7 +417,8 @@ class UnsharedRegionFit(object):
             S2 = _dev.empty((Cl,))
             S0 = _dev.empty((Cl,)) if masked else None
             with _dev.timed(self.profile, "K0_healthy_stats"):
-                self._healthy_stats(b_dev, Cl, H, S1, S2, S0)
+                _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2), _dev.ptr(S0),
+                                                 _dev.stream()), "fcd_healthy_stats")
             del b_dev
         nm = _dev.empty((max(Cl, 1),), torch.int32)
         _lib.check(lib.fcd_edge_table(c0, Cl, _dev.ptr(nm), _dev.stream()), "fcd_edge_table")
@@ -427,27 +429,6 @@ class UnsharedRegionFit(object):
         self._evals = []
         self._const = None
         return self._in
-
-    @staticmethod
-    def _healthy_entry(inp, name):
-        """(entry point, its name, leading S1 / S2 arguments) of a kernel that reads the healthy statistics: the
-        ``_masked`` form with S0 when missing entries are marginalised."""
-        lib = _lib.load()
-        head = (_dev.ptr(inp['S1']), _dev.ptr(inp['S2']))
-        if inp['S0'] is None:
-            return getattr(lib, name), name, head
-        return getattr(lib, name + "_masked"), name + "_masked", head + (_dev.ptr(inp['S0']),)
-
-    @staticmethod
-    def _healthy_stats(b_dev, Cl, H, S1, S2, S0):
-        """S1, S2 of the controls [Cl][H]; with S0 (missing entries marginalised) over the observed entries only."""
-        lib = _lib.load()
-        if S0 is None:
-            _lib.check(lib.fcd_healthy_stats(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2), _dev.stream()),
-                       "fcd_healthy_stats")
-        else:
-            _lib.check(lib.fcd_healthy_stats_masked(_dev.ptr(b_dev), Cl, H, H, _dev.ptr(S1), _dev.ptr(S2),
-                                                    _dev.ptr(S0), _dev.stream()), "fcd_healthy_stats_masked")
 
     def set_shared_inputs(self, shared, controls, patients):
         """Replica mode (new; BASELINE.json configs[4]): the fit's inputs are COLUMNS of a correlation
@@ -478,13 +459,8 @@ class UnsharedRegionFit(object):
         S2 = _dev.empty((C,))
         S0 = _dev.empty((C,)) if self._masked() else None
         with _dev.timed(self.profile, "K0_healthy_stats"):
-            if S0 is None:
-                _lib.check(lib.fcd_healthy_stats_cols(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H, _dev.ptr(S1),
-                                                      _dev.ptr(S2), _dev.stream()), "fcd_healthy_stats_cols")
-            else:
-                _lib.check(lib.fcd_healthy_stats_cols_masked(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H,
-                                                             _dev.ptr(S1), _dev.ptr(S2), _dev.ptr(S0), _dev.stream()),
-                           "fcd_healthy_stats_cols_masked")
+            _lib.check(lib.fcd_healthy_stats_cols(_dev.ptr(sp.X), C, sp.pitchS, _dev.ptr(con), H, _dev.ptr(S1),
+                                                  _dev.ptr(S2), _dev.ptr(S0), _dev.stream()), "fcd_healthy_stats_cols")
         self._in = dict(key=key, src=(None, None), C=C, H=H, U=U, c0=0, Cl=C, u0=0, Ul=U, pitchU=_dev.even(U),
                         bt=None, S1=S1, S2=S2, S0=S0, nm=sp.nm, cache_key=None, P=None, L=None, WT=None,
                         ev_S=None, b_dev=None)
@@ -548,11 +524,10 @@ class UnsharedRegionFit(object):
                 inp['P'] = _dev.empty((3, max(Cl, 1), pitchU))
                 inp['L'] = _dev.empty((max(Cl, 1), pitchU))
             th = self._theta()
-            (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if inp['S0'] is not None
-                          else (lib.fcd_resp_cache, "fcd_resp_cache"))
             with _dev.timed(self.profile, "K0_resp_cache"):
-                _lib.check(fn(_dev.ptr(inp['bt']), Cl, U, pitchU, ctypes.byref(th), _dev.ptr(inp['P']),
-                              max(Cl, 1) * pitchU, _dev.ptr(inp['L']), _dev.stream()), name)
+                _lib.check(lib.fcd_resp_cache(_dev.ptr(inp['bt']), Cl, U, pitchU, ctypes.byref(th), _dev.ptr(inp['P']),
+                                              max(Cl, 1) * pitchU, _dev.ptr(inp['L']), int(self._masked()),
+                                              _dev.stream()), "fcd_resp_cache")
         inp['Lsum'] = None                          # total of the L plane, formed on first use (code pass)
         inp['PsE'] = None                           # dominant-state plane of the code pass: rebuilt with the planes
         inp['code_verR'] = None
@@ -616,7 +591,7 @@ class UnsharedRegionFit(object):
         if Ul > 0:
             th = self._theta()
             _lib.check(lib.fcd_resp_cache(_dev.ptr(blk), C, Ul, Ul, ctypes.byref(th), _dev.ptr(src),
-                                          C * max(Ul, 1), None, _dev.stream()), "fcd_resp_cache")
+                                          C * max(Ul, 1), None, 0, _dev.stream()), "fcd_resp_cache")
         else:
             src.zero_()
         return src
@@ -739,10 +714,9 @@ class UnsharedRegionFit(object):
         U = bt_dev.shape[1]
         lpB, pBt, lM = _dev.empty((C, H, 3)), _dev.empty((C, U, 3)), _dev.empty((C, U, 3, 3))
         th = self._theta()
-        (fn, name) = ((lib.fcd_materialize_lps_masked, "fcd_materialize_lps_masked") if self._masked()
-                      else (lib.fcd_materialize_lps, "fcd_materialize_lps"))
-        _lib.check(fn(_dev.ptr(b_dev), _dev.ptr(bt_dev), C, H, U, ctypes.byref(th), _dev.ptr(lpB), _dev.ptr(pBt),
-                      _dev.ptr(lM), _dev.stream()), name)
+        _lib.check(lib.fcd_materialize_lps(_dev.ptr(b_dev), _dev.ptr(bt_dev), C, H, U, ctypes.byref(th), _dev.ptr(lpB),
+                                           _dev.ptr(pBt), _dev.ptr(lM), int(self._masked()), _dev.stream()),
+                   "fcd_materialize_lps")
         self._mat = {'_lp_B_g_F': _dev.download(lpB), '_p_Bt_g_Ft': _dev.download(pBt),
                      '_lM': _dev.download(lM)}
         return self._mat
@@ -917,13 +891,12 @@ class UnsharedRegionFit(object):
         self._wait_healthy(inp)
         # the global E_lM is known: rank 0 contributes it, the others zero
         first = self.shards is None or self.shards.rank == 0
-        (fn, name, s12) = self._healthy_entry(inp, "fcd_energy_terms")
         with _dev.timed(self.profile, "K4_energy_small"):
-            _lib.check(fn(
-                *s12, H, _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), Cl,
-                _dev.ptr(lqR), _dev.ptr(qR), N, U, ctypes.byref(th), float(elm) if first else 0.0,
-                solver_state if first else None,
-                _dev.ptr(res.dev), _dev.ptr(_dev.workspace()), _dev.stream()), name)
+            _lib.check(lib.fcd_energy_terms(
+                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), _dev.ptr(inp['S0']), H, _dev.ptr(lqF[c0 * 3:]),
+                _dev.ptr(qF[c0 * 3:]), Cl, _dev.ptr(lqR), _dev.ptr(qR), N, U, ctypes.byref(th),
+                float(elm) if first else 0.0, solver_state if first else None,
+                _dev.ptr(res.dev), _dev.ptr(_dev.workspace()), _dev.stream()), "fcd_energy_terms")
         if self.shards is not None:
             h = self.shards.reduce_begin(res)
             return ("shards", h, res)
@@ -1066,31 +1039,39 @@ class UnsharedRegionFit(object):
         if uni is not None:
             # q_R is the constant start: the row sums (shared with the initial free energy) give lq_F directly
             (S9, w3, _) = uni
-            (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_rowsums")
             with _dev.timed(self.profile, "K2_estep_qF_rowsums"):
-                _lib.check(fn(*s12, H, _dev.ptr(S9), Cl, w3, ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]),
-                              _dev.ptr(qF[c0 * 3:]), _dev.stream()), name)
+                _lib.check(lib.fcd_estep_qF_rowsums(_dev.ptr(inp['S1']), _dev.ptr(inp['S2']), _dev.ptr(inp['S0']), H,
+                                                    _dev.ptr(S9), Cl, w3, ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]),
+                                                    _dev.ptr(qF[c0 * 3:]), _dev.stream()), "fcd_estep_qF_rowsums")
             self._set_lq_F_dev(lqF_buf, qF_buf, C)
             return
         if self.coded_estep and Cl > 0 and inp.get('code_verR') == self._mR.version and inp.get('PsE') is not None:
-            # the code plane and key lists of the last M-step still describe q_R (fcd_estep_qF_coded)
-            (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_coded")
-            with _dev.timed(self.profile, "K2_estep_qF_coded"):
-                _lib.check(fn(
-                    *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
-                    Cl, U, inp['pitchU'], _dev.ptr(qR), N, _dev.ptr(inp['nm']), _dev.ptr(inp['code']), inp['pitchQ'],
-                    _dev.ptr(inp['bk_counts']), _dev.ptr(inp['bk_K']), _dev.ptr(inp['bk_KH']), _dev.ptr(inp['bk_rowoff']),
-                    _dev.ptr(inp['bk_H']), ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()),
-                    name)
+            # the code plane and key lists of the last M-step still describe q_R
+            self._estep_qF_coded(inp, th, qR, lqF_buf, qF_buf)
             self._set_lq_F_dev(lqF_buf, qF_buf, C)
             return
-        (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF")
         with _dev.timed(self.profile, "K2_estep_qF"):
-            _lib.check(fn(
-                *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
-                Cl, U, inp['pitchU'], _dev.ptr(qR), _dev.ptr(rstate), rstate.shape[1], N, _dev.ptr(inp['nm']),
-                ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()), name)
+            _lib.check(lib.fcd_estep_qF(
+                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), _dev.ptr(inp['S0']), H, _dev.ptr(inp['P']),
+                max(Cl, 1) * inp['pitchU'], Cl, U, inp['pitchU'], _dev.ptr(qR), _dev.ptr(rstate), rstate.shape[1], N,
+                _dev.ptr(inp['nm']), ctypes.byref(th), _dev.ptr(lqF[c0 * 3:]), _dev.ptr(qF[c0 * 3:]), _dev.stream()),
+                "fcd_estep_qF")
         self._set_lq_F_dev(lqF_buf, qF_buf, C)
+
+    def _estep_qF_coded(self, inp, th, qR, lqF_buf, qF_buf, solver_state=None, lo_e=0.0, hi_e=0.0):
+        """Enqueues the E-step from the code plane and key lists of the last M-step into the local rows of
+        lqF_buf / qF_buf.  ``solver_state``: take eta and epsilon from the device-resident solve enqueued before,
+        whose epsilon box is [lo_e, hi_e]; otherwise they are th's."""
+        (N, H, U) = self._dims
+        (c0, Cl, pitchU) = (inp['c0'], inp['Cl'], inp['pitchU'])
+        with _dev.timed(self.profile, "K2_estep_qF_coded"):
+            _lib.check(_lib.load().fcd_estep_qF_coded(
+                _dev.ptr(inp['S1']), _dev.ptr(inp['S2']), _dev.ptr(inp['S0']), H, _dev.ptr(inp['P']),
+                max(Cl, 1) * pitchU, Cl, U, pitchU, _dev.ptr(qR), N, _dev.ptr(inp['nm']), _dev.ptr(inp['code']),
+                inp['pitchQ'], _dev.ptr(inp['bk_counts']), _dev.ptr(inp['bk_K']), _dev.ptr(inp['bk_KH']),
+                _dev.ptr(inp['bk_rowoff']), _dev.ptr(inp['bk_H']), ctypes.byref(th), solver_state, float(lo_e),
+                float(hi_e), _dev.ptr(lqF_buf[c0 * 3:]), _dev.ptr(qF_buf[c0 * 3:]), _dev.stream()),
+                "fcd_estep_qF_coded")
 
     def _set_lq_F_dev(self, lqF_buf, qF_buf, C):
         """Publishes an E-step's result.  Edge shards: q_F is gathered now (the region sweep reads every
@@ -1120,22 +1101,13 @@ class UnsharedRegionFit(object):
         inp = self._in
         if inp is None or inp.get('PsE') is None or inp.get('code_verR') != self._mR.version or inp['Cl'] <= 0:
             return None
-        lib = _lib.load()
-        (N, H, U) = self._dims
-        (C, c0, Cl) = (inp['C'], inp['c0'], inp['Cl'])
+        C = inp['C']
         (_, qR) = self._mR.get_dev()
         nbuf = C * 3 if self.shards is None else self.shards.edge_buffer_len(C)
         (lqF_buf, qF_buf) = (_dev.empty((nbuf,)), _dev.empty((nbuf,)))
         th = self._theta()
         self._wait_healthy(inp)
-        (fn, name, s12) = self._healthy_entry(inp, "fcd_estep_qF_coded_solved")
-        with _dev.timed(self.profile, "K2_estep_qF_coded"):
-            _lib.check(fn(
-                *s12, H, _dev.ptr(inp['P']), max(Cl, 1) * inp['pitchU'],
-                Cl, U, inp['pitchU'], _dev.ptr(qR), N, _dev.ptr(inp['nm']), _dev.ptr(inp['code']), inp['pitchQ'],
-                _dev.ptr(inp['bk_counts']), _dev.ptr(inp['bk_K']), _dev.ptr(inp['bk_KH']), _dev.ptr(inp['bk_rowoff']),
-                _dev.ptr(inp['bk_H']), ctypes.byref(th), solver_state, float(lo_e), float(hi_e),
-                _dev.ptr(lqF_buf[c0 * 3:]), _dev.ptr(qF_buf[c0 * 3:]), _dev.stream()), name)
+        self._estep_qF_coded(inp, th, qR, lqF_buf, qF_buf, solver_state, lo_e, hi_e)
         self.spec_stats[0] += 1
         return dict(bufs=(lqF_buf, qF_buf), inp=inp, cache_key=inp['cache_key'], verR=self._mR.version, qR=qR,
                     dims=self._dims, rest=(tuple(th.gamma), tuple(th.mu), tuple(th.sigma)), x=None)
@@ -1390,11 +1362,10 @@ class UnsharedRegionFit(object):
         lib = _lib.load()
         bt = self._columns_on_device(bt_src, C, U, pitchU)
         PL = _dev.empty((4 if with_L else 3, C, pitchU))
-        (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if self._masked()
-                      else (lib.fcd_resp_cache, "fcd_resp_cache"))
         with _dev.timed(self.profile, "P0_resp_cache"):
-            _lib.check(fn(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
-                          _dev.ptr(PL[3] if with_L else None), _dev.stream()), name)
+            _lib.check(lib.fcd_resp_cache(_dev.ptr(bt), C, U, pitchU, ctypes.byref(th), _dev.ptr(PL), C * pitchU,
+                                          _dev.ptr(PL[3] if with_L else None), int(self._masked()), _dev.stream()),
+                       "fcd_resp_cache")
         return PL
 
     def connection_posteriors(self, bt_new=None, lq_R=None, maps=True):
@@ -1519,11 +1490,9 @@ class UnsharedRegionFit(object):
         (_, qF) = self._mF.get_dev()
         out = _dev.empty((S,))
         ws = _dev.empty((max(int(lib.fcd_control_terms_ws_bytes(C, S)) // 8, 1),))
-        (fn, name) = ((lib.fcd_control_terms_masked, "fcd_control_terms_masked") if self._masked()
-                      else (lib.fcd_control_terms, "fcd_control_terms"))
         with _dev.timed(self.profile, "P4_control_terms"):
-            _lib.check(fn(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th), _dev.ptr(out), _dev.ptr(ws),
-                          _dev.stream()), name)
+            _lib.check(lib.fcd_control_terms(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th), _dev.ptr(out),
+                                             _dev.ptr(ws), int(self._masked()), _dev.stream()), "fcd_control_terms")
         return _dev.download(out)
 
     def classify_subjects(self, x_new, prior_patient=None, lq_R0=None, max_sweeps=50, tol=1e-9):

@@ -31,7 +31,7 @@ class SharedPlanes(object):
     nm [C]               edge table
 
     ``missing``: the ``UnsharedRegionFit.missing`` of the fits that use the planes; with ``"marginalize"`` a NaN
-    correlation is an unobserved entry (fcd_resp_cache_masked) and +-inf is rejected.
+    correlation is an unobserved entry (fcd_resp_cache with missing = 1) and +-inf is rejected.
     """
 
     def __init__(self, corr, model, missing="reject"):
@@ -60,10 +60,9 @@ class SharedPlanes(object):
                              np.asarray(model.gamma).reshape(-1), model.mu, model.sigma)
         self.cache_key = (tuple(float(v) for v in model.mu), tuple(float(v) for v in model.sigma))
         self.PL = _dev.empty((4, C, self.pitchS))
-        (fn, name) = ((lib.fcd_resp_cache_masked, "fcd_resp_cache_masked") if missing == "marginalize"
-                      else (lib.fcd_resp_cache, "fcd_resp_cache"))
-        _lib.check(fn(_dev.ptr(self.X), C, S, self.pitchS, ctypes.byref(th), _dev.ptr(self.PL), C * self.pitchS,
-                      _dev.ptr(self.PL[3]), _dev.stream()), name)
+        _lib.check(lib.fcd_resp_cache(_dev.ptr(self.X), C, S, self.pitchS, ctypes.byref(th), _dev.ptr(self.PL),
+                                      C * self.pitchS, _dev.ptr(self.PL[3]), int(missing == "marginalize"),
+                                      _dev.stream()), "fcd_resp_cache")
         self.nm = _dev.empty((max(C, 1),), torch.int32)
         _lib.check(lib.fcd_edge_table(0, C, _dev.ptr(self.nm), _dev.stream()), "fcd_edge_table")
 

@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define FCD_VERSION 121
+#define FCD_VERSION 122
 
 #if defined(__GNUC__)
 #define FCD_API __attribute__((visibility("default")))
@@ -124,14 +124,14 @@ FCD_API int fcd_c_to_nm(int64_t c0, int64_t C, int32_t* n_out, int32_t* m_out, v
 /* Healthy-subject sufficient statistics, computed once per fit:
  *   S1[c] = sum_h b[c,h],  S2[c] = sum_h b[c,h]^2.
  * They replace the (C,H,3) cache `_lp_B_g_F` of fcdiff/fit.py:111-114: the
- * healthy log-density sum of fit.py:171 is a quadratic in (S1, S2). */
+ * healthy log-density sum of fit.py:171 is a quadratic in (S1, S2).
+ * S0 == NULL: every b[c,h] is taken as observed.  S0 != NULL, for missing entries (fit.missing =
+ * "marginalize"): a NaN b[c,h] is not observed and is left out of S1, S2; S0[c] = H_c, the number of observed
+ * controls of edge c (a double).  The healthy sum of fit.py:171 over the observed entries is
+ * hq_a S2 + hq_b S1 + H_c hq_c1: the constant scales with H_c, so it cannot be folded into S1, S2.  With no NaN,
+ * S1 and S2 have the bits of the S0 == NULL form and S0 = H.  The kernels below that take S0 read it the same
+ * way: NULL means every edge has all H controls, and S0 = H gives the bits of the NULL form. */
 FCD_API int fcd_healthy_stats(const double* b, int64_t C, int32_t H, int64_t pitchH,
-                      double* S1, double* S2, void* stream);
-/* Missing entries (fit.missing = "marginalize"): a NaN b[c,h] is not observed and is left out of S1, S2;
- * S0[c] = H_c, the number of observed controls of edge c (a double).  The healthy sum of fit.py:171 over the
- * observed entries is hq_a S2 + hq_b S1 + H_c hq_c1: the constant scales with H_c, so it cannot be folded into
- * S1, S2.  With no NaN, S1 and S2 have the bits of fcd_healthy_stats and S0 = H. */
-FCD_API int fcd_healthy_stats_masked(const double* b, int64_t C, int32_t H, int64_t pitchH,
                       double* S1, double* S2, double* S0, void* stream);
 
 /* Edge table of the local shard: nm[i] = n | m << 16 for the edge c0 + i
@@ -145,15 +145,14 @@ FCD_API int fcd_edge_table(int64_t c0, int64_t C, int32_t* nm, void* stream);
  *   L[c][u]    = log(N_0 + N_1 + N_2)      (may be NULL)
  * each with the shape and pitch of bt.  Then (fit.py:117-122, 409-444)
  *   log M_kl = L + log(a_l + b_l p_k),  a_l = (1 - eps_l)/2,  b_l = eps_l - a_l,
- * exactly and without underflow; the kernels below read these planes, not bt. */
-FCD_API int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream);
-/* fcd_resp_cache for patient correlations with missing entries: a NaN bt[c,u] is not observed and is stored
- * as p_0 = p_1 = p_2 = 1/3, L = log 3.  Then a_l + b_l / 3 = 1/3 for every l and theta, log M_kl = 0 for all
+ * exactly and without underflow; the kernels below read these planes, not bt.
+ * missing = 1 for patient correlations with missing entries: a NaN bt[c,u] is not observed and is stored as
+ * p_0 = p_1 = p_2 = 1/3, L = log 3.  Then a_l + b_l / 3 = 1/3 for every l and theta, log M_kl = 0 for all
  * (k, l) (fit.py:117-122): the element's density factor is 1 in every kernel that reads the planes.  Finite
- * entries get the bits of fcd_resp_cache. */
-FCD_API int fcd_resp_cache_masked(const double* bt, int64_t C, int32_t U, int64_t pitchU,
-                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, void* stream);
+ * entries get the bits of missing = 0.  Any other value of `missing` is rejected. */
+FCD_API int fcd_resp_cache(const double* bt, int64_t C, int32_t U, int64_t pitchU,
+                   const fcd_theta* theta_host, double* P, int64_t planeStride, double* L, int32_t missing,
+                   void* stream);
 
 /* Peak states of the posteriors (tier selection, DESIGN.md "Tiers"):
  *   fstate[c]   = k if qF[c,k] == 1.0 and the other two <= 2^-60, else 3;
@@ -176,13 +175,9 @@ FCD_API int fcd_map_labels(const double* lq, int64_t n, int32_t width, uint8_t* 
  *   lqF[c,k] = log gamma_k + sum_h logN_k(b[c,h])
  *            + sum_u sum_l w_l(n,m,u) log M_kl(bt[c,u]),  minus logsumexp_k.
  * P: planes of the local edge rows; qR [N][U][2] probabilities, rstate their peak
- * states; nm the shard's edge table.  Outputs lqF [C][3] and qF=exp(lqF) [C][3]. */
-FCD_API int fcd_estep_qF(const double* S1, const double* S2, int32_t H,
-                 const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                 const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
-                 const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
-/* fcd_estep_qF with S0 of fcd_healthy_stats_masked: the healthy sum of fit.py:171 over the observed controls. */
-FCD_API int fcd_estep_qF_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+ * states; nm the shard's edge table.  Outputs lqF [C][3] and qF=exp(lqF) [C][3].
+ * S0 (may be NULL) of fcd_healthy_stats: the healthy sum of fit.py:171 over the observed controls. */
+FCD_API int fcd_estep_qF(const double* S1, const double* S2, const double* S0, int32_t H,
                  const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                  const double* qR, const uint8_t* rstate, int64_t pitchS, int32_t N, const int32_t* nm,
                  const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
@@ -193,37 +188,17 @@ FCD_API int fcd_estep_qF_masked(const double* S1, const double* S2, const double
  * mixed region are taken from the row's key lists (half records: three differences of logs with
  * one weight; full records: nine logs).  code / counts / keysF / keysH / rowoff / Hh as written by
  * the code pass for the same local rows; rows whose edge was unpeaked then (counts[c][0] == 3 U)
- * are evaluated in full. */
-FCD_API int fcd_estep_qF_coded(const double* S1, const double* S2, int32_t H,
-                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                       const double* qR, int32_t N, const int32_t* nm,
-                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                       const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
-/* fcd_estep_qF_coded with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
-FCD_API int fcd_estep_qF_coded_masked(const double* S1, const double* S2, const double* S0, int32_t H,
-                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                       const double* qR, int32_t N, const int32_t* nm,
-                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                       const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
-
-/* The same launch for the E-step of the NEXT iteration, enqueued behind a device-resident (eta, epsilon) solve
- * (fcd_elm_coded_solve / fcd_elm_tiered_solve, fcdiff/fit.py:228-241) whose result the host has not read yet:
- * eta and epsilon are taken from `solver_state` on the device when the kernel starts (theta_host supplies gamma,
- * mu, sigma; its eta / epsilon are ignored); [eps_lo, eps_hi] is the epsilon box of that solve and sizes the
- * logarithm table.  The reference runs these steps one after the other (fit.py:73-79); here the E-step fills the
- * GPU while the host waits for the solve and the free energy.  The caller discards lqF / qF when the solve had not
- * finished in the launches enqueued before (state.done == 0), ended pinned at the box, or the fit stops. */
-FCD_API int fcd_estep_qF_coded_solved(const double* S1, const double* S2, int32_t H,
-                       const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
-                       const double* qR, int32_t N, const int32_t* nm,
-                       const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
-                       const uint64_t* keysH, const int64_t* rowoff, const double* Hh,
-                       const fcd_theta* theta_host, const void* solver_state, double eps_lo, double eps_hi,
-                       double* lqF, double* qF, void* stream);
-/* fcd_estep_qF_coded_solved with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
-FCD_API int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+ * are evaluated in full.  S0 (may be NULL) of fcd_healthy_stats (fit.py:157-174 over the observed controls).
+ * solver_state == NULL: eta and epsilon come from theta_host, and eps_lo / eps_hi are ignored.
+ * solver_state != NULL (device, fcd_solver_init, 8-byte aligned): the E-step of the NEXT iteration, enqueued
+ * behind a device-resident (eta, epsilon) solve (fcd_elm_coded_solve / fcd_elm_tiered_solve,
+ * fcdiff/fit.py:228-241) whose result the host has not read yet: eta and epsilon are taken from `solver_state` on
+ * the device when the kernel starts (theta_host supplies gamma, mu, sigma; its eta / epsilon are ignored);
+ * [eps_lo, eps_hi] (0 < eps_lo <= eps_hi < 1) is the epsilon box of that solve and sizes the logarithm table.
+ * The reference runs these steps one after the other (fit.py:73-79); here the E-step fills the GPU while the
+ * host waits for the solve and the free energy.  The caller discards lqF / qF when the solve had not finished in
+ * the launches enqueued before (state.done == 0), ended pinned at the box, or the fit stops. */
+FCD_API int fcd_estep_qF_coded(const double* S1, const double* S2, const double* S0, int32_t H,
                        const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                        const double* qR, int32_t N, const int32_t* nm,
                        const uint8_t* code, int64_t pitchQ, const int32_t* counts, const uint64_t* keysF,
@@ -236,15 +211,13 @@ FCD_API int fcd_estep_qF_coded_solved_masked(const double* S1, const double* S2,
  *   S9[c][k*3 + l] = sum_u log(a_l + b_l p_k(c,u))       (a_l, b_l: fit.py:427-444 relative to the total density)
  * -- nine running products per row instead of nine logarithms per element (csrc/fcd_uniform.cu):
  *   fcd_row_logsums: S9 [C][9] from the planes P_0, P_1 ([C][pitchU], 16-byte aligned rows);
- *   fcd_estep_qF_rowsums: `_update_lq_F` (fit.py:157-174) from S9 and w3_host = {q0^2, q1^2, 2 q0 q1};
+ *   fcd_estep_qF_rowsums: `_update_lq_F` (fit.py:157-174) from S9 and w3_host = {q0^2, q1^2, 2 q0 q1}, with S0
+ *     (may be NULL) of fcd_healthy_stats (the healthy sum over the observed controls);
  *   fcd_elm_rowsums: out1[0] = sum_c sum_k qF[c,k] sum_l w_l S9[c][k][l], the theta-dependent part of E_lM
  *     (fit.py:489-511); the theta-free part is (sum_l w_l) sum_c (sum_k qF[c,k]) sum_u L[c,u]. */
 FCD_API int fcd_row_logsums(const double* P, int64_t planeStride, int64_t C, int32_t U, int64_t pitchU,
                     const fcd_theta* theta_host, double* S9, void* stream);
-FCD_API int fcd_estep_qF_rowsums(const double* S1, const double* S2, int32_t H, const double* S9, int64_t C,
-                         const double* w3_host, const fcd_theta* theta_host, double* lqF, double* qF, void* stream);
-/* fcd_estep_qF_rowsums with S0 of fcd_healthy_stats_masked (fit.py:157-174 over the observed controls). */
-FCD_API int fcd_estep_qF_rowsums_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+FCD_API int fcd_estep_qF_rowsums(const double* S1, const double* S2, const double* S0, int32_t H,
                          const double* S9, int64_t C, const double* w3_host, const fcd_theta* theta_host,
                          double* lqF, double* qF, void* stream);
 FCD_API int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const double* w3_host, double* out1,
@@ -254,13 +227,11 @@ FCD_API int fcd_elm_rowsums(const double* S9, const double* qF, int64_t C, const
  * fit, fcdiff/fit.py:56-82): the responsibility planes of ALL S subjects are built once
  * (fcd_resp_cache on every column of the (C, S) correlation matrix), and a relabelling selects from
  * them (csrc/fcd_replica.cu):
- *   fcd_healthy_stats_cols: S1 / S2 of fcd_healthy_stats over the columns cols[0..H) of X [C][pitchS];
+ *   fcd_healthy_stats_cols: S1 / S2 (and S0, may be NULL) of fcd_healthy_stats over the columns cols[0..H) of
+ *     X [C][pitchS]; with S0 != NULL only the observed (non-NaN) entries are summed;
  *   fcd_gather_columns: dst[p][c][j] = src[p][c][cols[j]], j < U (columns U..pitchD-1 zero), p < nplanes.
  * cols: int32 device array. */
 FCD_API int fcd_healthy_stats_cols(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
-                           double* S1, double* S2, void* stream);
-/* fcd_healthy_stats_cols over the observed (non-NaN) entries, with S0 as fcd_healthy_stats_masked. */
-FCD_API int fcd_healthy_stats_cols_masked(const double* X, int64_t C, int64_t pitchS, const int32_t* cols, int32_t H,
                            double* S1, double* S2, double* S0, void* stream);
 FCD_API int fcd_gather_columns(const double* src, int64_t planeStrideS, int64_t pitchS, int32_t nplanes, int64_t C,
                        const int32_t* cols, int32_t U, double* dst, int64_t planeStrideD, int64_t pitchD,
@@ -442,15 +413,9 @@ FCD_API int fcd_solver_wait(const void* published_host, uint64_t seq, void* stat
  * shard's C rows.  `elm` = E_lM of the shard (fcd_elm_obj_grad + fcd_elm_const
  * at the same q_F, q_R, theta); or, with `solver_state` != NULL (device, fcd_solver_init): the E_lM
  * of the device-resident (eta, epsilon) solve enqueued before this call on the same stream (the
- * GLOBAL value: pass it on one rank only) -- NaN if that solve has not finished. */
-FCD_API int fcd_energy_terms(const double* S1, const double* S2, int32_t H,
-                     const double* lqF, const double* qF, int64_t C,
-                     const double* lqR, const double* qR, int32_t N, int32_t U,
-                     const fcd_theta* theta_host, double elm, const void* solver_state,
-                     double* out6, double* ws, void* stream);
-/* fcd_energy_terms with S0 of fcd_healthy_stats_masked: E_lp_B_g_F (fit.py:461-472) over the observed
- * controls. */
-FCD_API int fcd_energy_terms_masked(const double* S1, const double* S2, const double* S0, int32_t H,
+ * GLOBAL value: pass it on one rank only) -- NaN if that solve has not finished.  S0 (may be NULL) of
+ * fcd_healthy_stats: E_lp_B_g_F (fit.py:461-472) over the observed controls. */
+FCD_API int fcd_energy_terms(const double* S1, const double* S2, const double* S0, int32_t H,
                      const double* lqF, const double* qF, int64_t C,
                      const double* lqR, const double* qR, int32_t N, int32_t U,
                      const fcd_theta* theta_host, double elm, const void* solver_state,
@@ -501,14 +466,12 @@ FCD_API int fcd_connection_posteriors(const double* P, int64_t planeStride, int6
  * X [C][pitchS] edge-major columns (C = N(N-1)/2, pitchS >= S >= 1); qF [C][3]; theta_host supplies mu, sigma.
  * ws: fcd_control_terms_ws_bytes(C, S) bytes of device scratch (no zero fill needed).  A subject's value is
  * bit-identical whichever other subjects, S or pitchS are in the call: the row partition depends on C only and
- * the partials are added in a fixed order. */
+ * the partials are added in a fixed order.  missing = 1 sums over the observed entries: a NaN X[c][s] adds
+ * nothing (fit.py:461-472 with the entry marginalised), so that a subject's l_C and its patient free energy
+ * cover the same entries.  missing = 0 takes every entry as observed; any other value is rejected. */
 FCD_API int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S);
 FCD_API int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                              const fcd_theta* theta_host, double* out, double* ws, void* stream);
-/* fcd_control_terms over the observed entries: a NaN X[c][s] adds nothing (fit.py:461-472 with the
- * entry marginalised), so that a subject's l_C and its patient free energy cover the same entries. */
-FCD_API int fcd_control_terms_masked(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
-                              const fcd_theta* theta_host, double* out, double* ws, void* stream);
+                              const fcd_theta* theta_host, double* out, double* ws, int32_t missing, void* stream);
 
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
@@ -530,16 +493,13 @@ FCD_API int fcd_state_moments(const double* S1, const double* S2, int32_t H,
  * path above never materialises them). */
 
 /* `_update_lps` (fcdiff/fit.py:104-122): lpB [C][H][3], pBt [C][U][3],
- * lM [C][U][3][3] (k major, l minor), scipy.stats.norm op order. */
+ * lM [C][U][3][3] (k major, l minor), scipy.stats.norm op order.
+ * missing = 1: the same caches of a fit with missing entries (fit.py:104-122 with NaN marginalised): a NaN
+ * b[c,h] gives lpB[c][h][:] = 0, a NaN bt[c,u] gives pBt[c][u][:] = 1 and lM[c][u][:][:] = 0 (M_kl = eps_l +
+ * (1 - eps_l) = 1, fit.py:427-430).  missing = 0 takes every entry as observed; any other value is rejected. */
 FCD_API int fcd_materialize_lps(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
                         const fcd_theta* theta_host,
-                        double* lpB, double* pBt, double* lM, void* stream);
-/* The same caches of a fit with missing entries (fcdiff/fit.py:104-122 with NaN marginalised): a NaN b[c,h]
- * gives lpB[c][h][:] = 0, a NaN bt[c,u] gives pBt[c][u][:] = 1 and lM[c][u][:][:] = 0 (M_kl = eps_l +
- * (1 - eps_l) = 1, fit.py:427-430). */
-FCD_API int fcd_materialize_lps_masked(const double* b, const double* bt, int64_t C, int32_t H, int32_t U,
-                        const fcd_theta* theta_host,
-                        double* lpB, double* pBt, double* lM, void* stream);
+                        double* lpB, double* pBt, double* lM, int32_t missing, void* stream);
 
 /* `_eval_M` (fcdiff/fit.py:409-430): M[i] from p[i][3], i < n. */
 FCD_API int fcd_eval_M(const double* p, int64_t n, double eta, double epsilon, int32_t k, int32_t l,

@@ -9,9 +9,10 @@ device, 10 iterations from theta_true with eta + 0.1.  Prints one JSON line:
   the time of fit.run() (host clock around a call that ends in a synchronise; median of --repeat, alternated) for
     the default path, the masked path on the same complete data, and the masked path with 10 % of the
     (region, subject) pairs dropped out (every edge of a dropped region NaN in that subject);
-  fcd_resp_cache_masked and fcd_healthy_stats_masked alone (CUDA events around 20 launches on the dropout data):
-    their algorithmic bytes over their time, as a fraction of the device-to-device copy rate measured in the same
-    run, beside fcd_resp_cache / fcd_healthy_stats on the complete data;
+  fcd_resp_cache and fcd_healthy_stats alone in their missing-entry forms (missing=1: the flag, or an S0 output;
+    CUDA events around 20 launches on the dropout data): their algorithmic bytes over their time, as a fraction of
+    the device-to-device copy rate measured in the same run, beside their complete-data forms (missing=0) on the
+    complete data;
   classify_subjects end to end on 500 + 500 held-out columns of the same draw with the same dropout;
   the GPU's name and power limit, read in the same run.
 """
@@ -91,16 +92,17 @@ def main():
     (S1, S2, S0) = (_dev.empty((C,)), _dev.empty((C,)), _dev.empty((C,)))
     (bd, btd) = data["dropout"]
     (bc, btc) = data["complete"]
-    calls = dict(
-        resp_cache_masked=lambda: lib.fcd_resp_cache_masked(_dev.ptr(btd), C, U, U, ctypes.byref(th), _dev.ptr(P),
-                                                             C * U, _dev.ptr(P[3]), _dev.stream()),
-        resp_cache=lambda: lib.fcd_resp_cache(_dev.ptr(btc), C, U, U, ctypes.byref(th), _dev.ptr(P), C * U,
-                                              _dev.ptr(P[3]), _dev.stream()),
-        healthy_stats_masked=lambda: lib.fcd_healthy_stats_masked(_dev.ptr(bd), C, H, H, _dev.ptr(S1), _dev.ptr(S2),
-                                                                  _dev.ptr(S0), _dev.stream()),
-        healthy_stats=lambda: lib.fcd_healthy_stats(_dev.ptr(bc), C, H, H, _dev.ptr(S1), _dev.ptr(S2), _dev.stream()))
-    algo_bytes = dict(resp_cache_masked=8 * C * U * 5, resp_cache=8 * C * U * 5,
-                      healthy_stats_masked=8 * C * H + 24 * C, healthy_stats=8 * C * H + 16 * C)
+    calls = {
+        "resp_cache missing=1": lambda: lib.fcd_resp_cache(_dev.ptr(btd), C, U, U, ctypes.byref(th), _dev.ptr(P),
+                                                           C * U, _dev.ptr(P[3]), 1, _dev.stream()),
+        "resp_cache missing=0": lambda: lib.fcd_resp_cache(_dev.ptr(btc), C, U, U, ctypes.byref(th), _dev.ptr(P),
+                                                           C * U, _dev.ptr(P[3]), 0, _dev.stream()),
+        "healthy_stats missing=1": lambda: lib.fcd_healthy_stats(_dev.ptr(bd), C, H, H, _dev.ptr(S1), _dev.ptr(S2),
+                                                                 _dev.ptr(S0), _dev.stream()),
+        "healthy_stats missing=0": lambda: lib.fcd_healthy_stats(_dev.ptr(bc), C, H, H, _dev.ptr(S1), _dev.ptr(S2),
+                                                                 None, _dev.stream())}
+    algo_bytes = {"resp_cache missing=1": 8 * C * U * 5, "resp_cache missing=0": 8 * C * U * 5,
+                  "healthy_stats missing=1": 8 * C * H + 24 * C, "healthy_stats missing=0": 8 * C * H + 16 * C}
     kernels = {}
     for (name, call) in calls.items():
         _lib.check(call(), name)

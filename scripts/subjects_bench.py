@@ -112,7 +112,7 @@ def main():
     out = _dev.empty((S,))
     ws = _dev.empty((int(lib.fcd_control_terms_ws_bytes(C, S)) // 8,))
     call = lambda: _lib.check(lib.fcd_control_terms(_dev.ptr(held), C, S, S, _dev.ptr(qF), ctypes.byref(th),
-                                                    _dev.ptr(out), _dev.ptr(ws), _dev.stream()), "fcd_control_terms")
+                                                    _dev.ptr(out), _dev.ptr(ws), 0, _dev.stream()), "fcd_control_terms")
     call()
     reps = 20
     (e0, e1) = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))

@@ -70,7 +70,7 @@ for (name, fst, rst) in variants():
                                      _dev.stream()))
 
     def k2():
-        _lib.check(lib.fcd_estep_qF(_dev.ptr(inp['S1']), _dev.ptr(inp['S2']), H, _dev.ptr(P), C * pitch, C, U, pitch,
+        _lib.check(lib.fcd_estep_qF(_dev.ptr(inp['S1']), _dev.ptr(inp['S2']), None, H, _dev.ptr(P), C * pitch, C, U, pitch,
                                     _dev.ptr(qR), _dev.ptr(rst), pitchS, N, _dev.ptr(inp['nm']), ctypes.byref(th),
                                     _dev.ptr(lq), None, _dev.stream()))
     if PROFILE:

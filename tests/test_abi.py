@@ -29,6 +29,9 @@ def test_header_declares_entry_points():
     for must in ("fcd_estep_qF", "fcd_estep_qR", "fcd_elm_obj_grad", "fcd_energy_terms",
                  "fcd_mstep_stats", "fcd_sample_B_tilde", "fcd_corr_fisherz"):
         assert must in syms
+    # one entry point per step: missing entries (S0 / `missing`) and the coded E-step's solver state are
+    # arguments, not separate `_masked` / `_solved` symbols
+    assert not [s for s in syms if s.endswith(("_masked", "_solved"))]
 
 
 def test_library_exports_every_declared_symbol(lib):

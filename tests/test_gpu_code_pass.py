@@ -31,7 +31,7 @@ def _pair_code(sn, sm):
 
 
 @pytest.mark.parametrize("N,U", [(9, 7), (23, 130), (40, 300)])
-def test_code_plane_and_evaluator_match_numpy(N, U):
+def test_code_plane_evaluator_and_estep_match_numpy(N, U):
     lib = _lib.load()
     rng = np.random.RandomState(N * 1000 + U)
     C = N * (N - 1) // 2
@@ -159,13 +159,13 @@ def test_code_plane_and_evaluator_match_numpy(N, U):
     (S1, S2) = (rng.randn(C), np.abs(rng.randn(C)) + 1.0)
     (lqF_c, qF_c) = (_dev.zeros((C * 3,)), _dev.zeros((C * 3,)))
     (S1d, S2d) = (_dev.upload(S1), _dev.upload(S2))
-    _lib.check(lib.fcd_estep_qF_coded(_dev.ptr(S1d), _dev.ptr(S2d), H, _dev.ptr(d['P']), C * pitchU, C, U, pitchU,
-                                      _dev.ptr(d['qR']), N, _dev.ptr(nmd), _dev.ptr(code), pitchQ, _dev.ptr(counts),
-                                      _dev.ptr(K), _dev.ptr(KH), _dev.ptr(RO), _dev.ptr(Hh), ctypes.byref(th), _dev.ptr(lqF_c),
-                                      _dev.ptr(qF_c), st),
+    _lib.check(lib.fcd_estep_qF_coded(_dev.ptr(S1d), _dev.ptr(S2d), None, H, _dev.ptr(d['P']), C * pitchU, C, U,
+                                      pitchU, _dev.ptr(d['qR']), N, _dev.ptr(nmd), _dev.ptr(code), pitchQ,
+                                      _dev.ptr(counts), _dev.ptr(K), _dev.ptr(KH), _dev.ptr(RO), _dev.ptr(Hh),
+                                      ctypes.byref(th), None, 0.0, 0.0, _dev.ptr(lqF_c), _dev.ptr(qF_c), st),
                "fcd_estep_qF_coded")
     (lqF_p, qF_p) = (_dev.zeros((C * 3,)), _dev.zeros((C * 3,)))
-    _lib.check(lib.fcd_estep_qF(_dev.ptr(S1d), _dev.ptr(S2d), H, _dev.ptr(d['P']), C * pitchU, C, U, pitchU,
+    _lib.check(lib.fcd_estep_qF(_dev.ptr(S1d), _dev.ptr(S2d), None, H, _dev.ptr(d['P']), C * pitchU, C, U, pitchU,
                                 _dev.ptr(d['qR']), _dev.ptr(rs), pitchS, N, _dev.ptr(nmd), ctypes.byref(th),
                                 _dev.ptr(lqF_p), _dev.ptr(qF_p), st), "fcd_estep_qF")
     # NumPy: lqF[c,k] = log gamma_k + healthy_k + sum_u sum_l w_l log(a_l + b_l p_k) - logsumexp_k  (L cancels)

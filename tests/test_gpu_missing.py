@@ -1,6 +1,6 @@
-"""GPU: missing entries marginalised (``UnsharedRegionFit.missing = "marginalize"``; csrc: fcd_resp_cache_masked,
-fcd_healthy_stats_masked, the S0 forms of K2 / K4, fcd_control_terms_masked, fcd_materialize_lps_masked,
-fcd_corr_mark_missing) against the default path on complete data (bit for bit) and the masked NumPy oracle
+"""GPU: missing entries marginalised (``UnsharedRegionFit.missing = "marginalize"``; csrc: fcd_resp_cache,
+fcd_control_terms and fcd_materialize_lps with missing = 1, fcd_healthy_stats and the K2 / K4 launches with an S0
+array, fcd_corr_mark_missing) against the default path on complete data (bit for bit) and the masked NumPy oracle
 (oracle/missing.py) on data with NaN entries."""
 import copy
 

@@ -277,7 +277,7 @@ def test_newton_solver_full_run_vs_polished_oracle(N, H, U, iters, lookup):
 @pytest.mark.parametrize("N,H,U,iters", [(24, 9, 33, 5), (90, 50, 50, 4), (160, 40, 400, 10)])
 def test_speculative_estep_is_bit_identical(N, H, U, iters):
     """`run()` enqueues the next iteration's E-step behind the device-resident (eta, epsilon) solve
-    (fcd_estep_qF_coded_solved: theta read from the solver's state block on the device) and adopts it
+    (fcd_estep_qF_coded with a solver state: theta read from the solver's state block on the device) and adopts it
     when nothing changed: the same fit with the feature off must give the same numbers bit for bit, the
     launches must actually be adopted, and a fit that stops leaves no stray result behind."""
     (_, _, _, _, b, bt) = O.sample(O.Theta(), N, H, U, np.random.RandomState(3 * N + 1))
@@ -570,7 +570,7 @@ def test_config3_two_iterations_vs_oracle_golden(solver, variant):
 
 
 @pytest.mark.parametrize("N,H,U", [(400, 500, 500)])
-def test_config3_properties(N, H, U):
+def test_config3_invariants(N, H, U):
     """Schaefer-400 x 1000 subjects: shard additivity, determinism,
     normalisation, energy consistency -- no CPU oracle at this size."""
     import ctypes
@@ -665,8 +665,8 @@ def test_config3_properties(N, H, U):
 
     def estep(a, e, rst):
         lq = _dev.empty(((e - a) * 3,))
-        _lib.check(lib.fcd_estep_qF(_dev.ptr(inp['S1'][a:]), _dev.ptr(inp['S2'][a:]), H, _dev.ptr(P[0, a:]), C * pitch,
-                                    e - a, U, pitch, _dev.ptr(qR), _dev.ptr(rst), pitchS, N, _dev.ptr(inp['nm'][a:]),
+        _lib.check(lib.fcd_estep_qF(_dev.ptr(inp['S1'][a:]), _dev.ptr(inp['S2'][a:]), None, H, _dev.ptr(P[0, a:]),
+                                    C * pitch, e - a, U, pitch, _dev.ptr(qR), _dev.ptr(rst), pitchS, N, _dev.ptr(inp['nm'][a:]),
                                     ctypes.byref(th), _dev.ptr(lq), None, _dev.stream()))
         return _dev.download(lq)
 

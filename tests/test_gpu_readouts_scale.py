@@ -460,7 +460,7 @@ def test_cohort_sums_equal_the_fit_energy_terms(native):
 
 # ------------------------------------------------------------------ empty row blocks through the C-ABI
 @gpu
-def test_empty_blocks_write_zero_partials(native):
+def test_empty_row_blocks_write_zero_partials(native):
     """N = 257: 2048 blocks of 17 rows, the last 112 hold no edge.  Their workspace partials must be exactly
     +0.0 in all three row kernels (for fcd_patient_terms, log_pos(1.0) of the two empty running products is
     exactly 0), and every other partial finite; the workspaces start as NaN, so a partial not written shows.
@@ -515,11 +515,11 @@ def test_empty_blocks_write_zero_partials(native):
     x = O.sample(O.Theta(), N, S, 1, np.random.RandomState(2573))[4]
     pitchS = _dev.even(S)
     X = fit._columns_on_device(x, C, S, pitchS)
-    for (fn, name) in ((lib.fcd_control_terms, "fcd_control_terms"),
-                       (lib.fcd_control_terms_masked, "fcd_control_terms_masked")):
+    for missing in (0, 1):
+        name = "fcd_control_terms missing=%d" % missing
         ws = nan_ws(lib.fcd_control_terms_ws_bytes(C, S))
         out = _dev.empty((S,))
-        _lib.check(fn(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th_c), _dev.ptr(out), _dev.ptr(ws),
-                      _dev.stream()), name)
+        _lib.check(lib.fcd_control_terms(_dev.ptr(X), C, S, pitchS, _dev.ptr(qF), ctypes.byref(th_c), _dev.ptr(out),
+                                         _dev.ptr(ws), missing, _dev.stream()), name)
         check_parts(ws.cpu().numpy().reshape(nb, S), name)
         nptest.assert_array_equal(out.cpu().numpy(), fit.score_controls(x))

@@ -130,7 +130,7 @@ def test_sums_equal_the_fit_energy_term_in_replica_mode():
     nptest.assert_array_equal(got, fit.score_controls(b))
 
 
-def test_batch_invariance_and_determinism():
+def test_batch_pitch_invariance_and_determinism():
     (th, lq_F) = _fitted_state(90)
     (_, _, _, _, b, _) = O.sample(O.Theta(), 90, 45, 1, np.random.RandomState(61))
     fit = _fit_at(th, lq_F, "reference")
@@ -149,7 +149,7 @@ def test_batch_invariance_and_determinism():
     ws = _dev.empty((int(lib.fcd_control_terms_ws_bytes(C, S)) // 8,))
     th_c = fit._theta(use_snapshot=False)
     _lib.check(lib.fcd_control_terms(_dev.ptr(X), C, S, pitchS, _dev.ptr(fit._mF.get_dev()[1]), ctypes.byref(th_c),
-                                     _dev.ptr(out), _dev.ptr(ws), _dev.stream()), "fcd_control_terms")
+                                     _dev.ptr(out), _dev.ptr(ws), 0, _dev.stream()), "fcd_control_terms")
     nptest.assert_array_equal(out.cpu().numpy(), whole)
 
 
