@@ -110,6 +110,8 @@ SIGNATURES = {
                                           POINTER(FcdTheta), _P, _P, _P, _P, _P, _P]),
     "fcd_control_terms_ws_bytes": (c_int64, [c_int64, c_int32]),
     "fcd_control_terms": (c_int, [_P, c_int64, c_int32, c_int64, _P, POINTER(FcdTheta), _P, _P, c_int32, _P]),
+    "fcd_maxt_ws_bytes": (c_int64, [c_int64, c_int64]),
+    "fcd_maxt_counts": (c_int, [_P, c_int64, c_int64, c_int64, _P, c_int64, c_int64, _P, _P, _P, _P]),
     "fcd_state_moments": (c_int, [_P, _P, c_int32, _P, _P, c_int64, c_int64, c_int32, c_int64, _P, _P, c_int32, _P,
                                   POINTER(FcdTheta), _P, _P, _P]),
     "fcd_materialize_lps": (c_int, [_P, _P, c_int64, c_int32, c_int32, POINTER(FcdTheta), _P, _P, _P, c_int32, _P]),
@@ -167,7 +169,7 @@ def load():
         fn = getattr(lib, name)          # AttributeError if the symbol is missing
         fn.restype = restype
         fn.argtypes = argtypes
-    if lib.fcd_version() < 122:
+    if lib.fcd_version() < 123:
         raise FcdError("fcdiff_b200: stale libfcdiff_b200.so (version %d)" % lib.fcd_version())
     _lib = lib
     return lib

@@ -1398,31 +1398,10 @@ class UnsharedRegionFit(object):
         if (bt_new is None) != (lq_R is None):
             raise ValueError("connection_posteriors takes bt_new and lq_R together (held-out patients) or "
                              "neither (the fit's own patients)")
-        (P, planeStride, pitchU, bt_src) = (None, 0, 0, None)
         if bt_new is None:
-            shR = self._mirror_shape(self._mR)
-            if shR is None:
-                raise ValueError("The fit has no q_R (run() the fit or assign _lq_R first).")
-            inp = self._in
-            if self._shared is not None:
-                U = int(self._shared[2].numel())
-            elif inp is not None:
-                U = int(inp['U'])
-            elif self.bt is not None:
-                U = self._check_bt_new(self.bt, C)
-            else:
-                raise ValueError("The fit has no patients (assign bt or run() the fit first).")
-            if tuple(shR) != (N, U, 2):
-                raise ValueError("the fit's q_R is %s, not (N, U, 2) = %s" % (tuple(shR), (N, U, 2)))
-            key = (tuple(float(v) for v in self.model.mu), tuple(float(v) for v in self.model.sigma))
-            if inp is not None and inp['P'] is not None and inp['cache_key'] == key:
-                (P, planeStride, pitchU) = (inp['P'], max(inp['Cl'], 1) * inp['pitchU'], inp['pitchU'])
-            elif self._shared is not None:
-                raise ValueError("connection_posteriors: the replica-mode fit has no planes for the model's "
-                                 "(mu, sigma) (run() the fit first).")
-            else:
-                bt_src = inp['bt'] if inp is not None else self.bt
+            (U, P, planeStride, pitchU, bt_src) = self._own_connection_inputs(C, N)
         else:
+            (P, planeStride, pitchU) = (None, 0, 0)
             U = self._check_bt_new(bt_new, C)
             if self._masked():
                 self._check_finite(bt_new, "bt_new", allow_nan=True)
@@ -1430,7 +1409,42 @@ class UnsharedRegionFit(object):
             if lq.shape != (N, U, 2):
                 raise ValueError("lq_R must be (N, U', 2) = %s (got %s)" % ((N, U, 2), lq.shape))
             bt_src = bt_new
+        rate = _dev.empty((C,))
+        (qT, qFt, expected) = self._launch_connection_posteriors(
+            C, N, U, P, planeStride, pitchU, bt_src, None if bt_new is None else np.exp(lq).reshape(-1), maps, rate)
+        return ConnectionPosteriors(_dev.download(qT) if maps else None, _dev.download(qFt) if maps else None,
+                                    _dev.download(expected), _dev.download(rate))
 
+    def _own_connection_inputs(self, C, N):
+        """(U, P, planeStride, pitchU, bt_src) of the fit's own patients for the connection read-outs: the planes
+        the fit holds when they were built for the model's (mu, sigma) (always, for a replica-mode fit), else
+        P = None and the patient columns ``bt_src`` whose planes are to be built."""
+        shR = self._mirror_shape(self._mR)
+        if shR is None:
+            raise ValueError("The fit has no q_R (run() the fit or assign _lq_R first).")
+        inp = self._in
+        if self._shared is not None:
+            U = int(self._shared[2].numel())
+        elif inp is not None:
+            U = int(inp['U'])
+        elif self.bt is not None:
+            U = self._check_bt_new(self.bt, C)
+        else:
+            raise ValueError("The fit has no patients (assign bt or run() the fit first).")
+        if tuple(shR) != (N, U, 2):
+            raise ValueError("the fit's q_R is %s, not (N, U, 2) = %s" % (tuple(shR), (N, U, 2)))
+        key = (tuple(float(v) for v in self.model.mu), tuple(float(v) for v in self.model.sigma))
+        if inp is not None and inp['P'] is not None and inp['cache_key'] == key:
+            return (U, inp['P'], max(inp['Cl'], 1) * inp['pitchU'], inp['pitchU'], None)
+        if self._shared is not None:
+            raise ValueError("connection_posteriors: the replica-mode fit has no planes for the model's "
+                             "(mu, sigma) (run() the fit first).")
+        return (U, None, 0, 0, inp['bt'] if inp is not None else self.bt)
+
+    def _launch_connection_posteriors(self, C, N, U, P, planeStride, pitchU, bt_src, qR_host, maps, rate):
+        """One fcd_connection_posteriors call: builds the planes of ``bt_src`` when P is None, takes q_R from the
+        fit (``qR_host`` None) or from the host array, and writes the (C,) anomalous rates into the float64
+        device tensor ``rate``.  Returns the device tensors (qT, qFt or None, expected)."""
         lib = _lib.load()
         th = self._theta(use_snapshot=False)
         if P is None:
@@ -1439,18 +1453,27 @@ class UnsharedRegionFit(object):
             planeStride = C * pitchU
         (_, qF) = self._mF.get_dev()
         fstate = self._mF.get_state()
-        qR = self._mR.get_dev()[1] if bt_new is None else _dev.upload(np.exp(lq).reshape(-1))
+        qR = self._mR.get_dev()[1] if qR_host is None else _dev.upload(qR_host)
         qT = _dev.empty((C, U))                     # scratch of the rates without maps
         qFt = _dev.empty((C, U, 3)) if maps else None
-        (expected, rate) = (_dev.empty((U,)), _dev.empty((C,)))
+        expected = _dev.empty((U,))
         ws = _dev.empty((max(int(lib.fcd_connection_ws_bytes(C, U)) // 8, 1),))
         with _dev.timed(self.profile, "P3_connection_posteriors"):
             _lib.check(lib.fcd_connection_posteriors(_dev.ptr(P), planeStride, C, U, pitchU, _dev.ptr(qF),
                                                      _dev.ptr(fstate), _dev.ptr(qR), N, ctypes.byref(th),
                                                      _dev.ptr(qT), _dev.ptr(qFt), _dev.ptr(expected), _dev.ptr(rate),
                                                      _dev.ptr(ws), _dev.stream()), "fcd_connection_posteriors")
-        return ConnectionPosteriors(_dev.download(qT) if maps else None, _dev.download(qFt) if maps else None,
-                                    _dev.download(expected), _dev.download(rate))
+        return (qT, qFt, expected)
+
+    def _connection_rate_into(self, rate):
+        """Writes the ``anomalous_rate`` of ``connection_posteriors(maps=False)`` (the fit's own patients) into
+        ``rate``, a (C,) float64 device view (a row of the statistics of ``sweep.permutation_inference``), with
+        the same launch: the same bits, nothing downloaded."""
+        (C, N) = self._check_readout("connection_posteriors", ('_lM', '_lp_B_g_F', '_p_Bt_g_Ft'))
+        if tuple(rate.shape) != (C,) or rate.dtype != torch.float64 or not rate.is_cuda or rate.stride(0) != 1:
+            raise ValueError("rate must be a contiguous (C,) = (%d,) float64 CUDA tensor" % C)
+        (U, P, planeStride, pitchU, bt_src) = self._own_connection_inputs(C, N)
+        self._launch_connection_posteriors(C, N, U, P, planeStride, pitchU, bt_src, None, False, rate)
 
     # ------------------------------------------------------------------ held-out controls, subjects of unknown group (new)
     def score_controls(self, b_new=None):

@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define FCD_VERSION 122
+#define FCD_VERSION 123
 
 #if defined(__GNUC__)
 #define FCD_API __attribute__((visibility("default")))
@@ -472,6 +472,22 @@ FCD_API int fcd_connection_posteriors(const double* P, int64_t planeStride, int6
 FCD_API int64_t fcd_control_terms_ws_bytes(int64_t C, int32_t S);
 FCD_API int fcd_control_terms(const double* X, int64_t C, int32_t S, int64_t pitchS, const double* qF,
                               const fcd_theta* theta_host, double* out, double* ws, int32_t missing, void* stream);
+
+/* Westfall-Young step-down max-T counts of a permutation test (csrc/fcd_permutation.cu; no reference
+ * counterpart: the reference has no permutation driver, fcdiff/fit.py:56-82).  T [R1][pitch] (pitch >= K):
+ * row 0 the observed statistics, rows 1..R1-1 those of relabelled data.  One family is the column range
+ * [k0, k1), 0 <= k0 < k1 <= K; order [k1 - k0] (int64) lists its columns k, k0 <= k < k1, ascending by
+ * (T[0][k], k): the permutation sigma, formed on the host and not checked here.  Then
+ *   count_unc [k1 - k0] (by column, k - k0) = #{r : T[r][k] >= T[0][k]}
+ *   count_sd  [k1 - k0] (by position j)     = #{r : max_{i <= j} T[r][sigma(i)] >= T[0][sigma(j)]}
+ * so p[k] = count_unc / R1 and p_fwer[sigma(j)] = max_{i >= j} count_sd[i] / R1 (the suffix maximum is left
+ * to the caller).  Both outputs are int64 and written whole; T must be finite (not checked here).  The counts
+ * are exact integers: they do not depend on the launch shape or the order of the atomics.  1 <= R1 <= 2^20,
+ * 1 <= K <= 2^24; larger sizes are rejected before any launch.  ws: fcd_maxt_ws_bytes(R1, K) bytes of device
+ * scratch (no zero fill needed; 0 for sizes out of range). */
+FCD_API int64_t fcd_maxt_ws_bytes(int64_t R1, int64_t K);
+FCD_API int fcd_maxt_counts(const double* T, int64_t R1, int64_t K, int64_t pitch, const int64_t* order, int64_t k0,
+                            int64_t k1, int64_t* count_unc, int64_t* count_sd, double* ws, void* stream);
 
 /* K3c -- per-state sufficient statistics of the correlations for the control
  * and the patient group (north_star subsystem 3; the reference ships only
